@@ -13,6 +13,10 @@ subset-dominance prune, results left on the device.  `value` = sets scored by al
 time.  `e2e` repeats the same through the public API with HOST buffers: the H2D copy of the data from pinned
 memory and the D2H fetch of every variable's surviving (mask, score) list are inside the timed region.
 
+--dump-outputs DIR: the timed steps drop their results on the device, so after them one more pass of the same step, outside
+the timed region, reads every score cache back and writes it (dump_outputs).  The step is deterministic, so these are the
+caches each timed step computed; two builds can be compared output for output on the same seeded inputs.
+
 --impl reference times the CPU oracle's restatement of the reference path (oracle/, or oracle/_ref when the
 reference's own sources were compiled) on the host cores, on a bounded sample of the same workload.
 """
@@ -479,6 +483,10 @@ def run_gpu(args):
         t = torch.tensor([t16_fallbacks, t16_warm], device="cuda", dtype=torch.int64)
         dist.all_reduce(t)
         t16_fallbacks, t16_warm = int(t[0].item()), int(t[1].item())
+    if args.dump_outputs:
+        # the step is deterministic (integer counts, fixed-order reductions, bit-identical caches on every context), so one
+        # more pass over the same inputs that reads the caches back returns what the last timed step left on the device
+        dump_outputs(args.dump_outputs, pool.run(items, wl["K"], stype, lam=lam, flags=flags, fetch=True, costs=costs))
     if rank == 0:
         peak, peak_src = load_peaks()
         fam = {"count": st["ms_count"], "cube": st["ms_cube"], "tree": st["ms_tree"], "cbic": st["ms_cbic"], "accept": st["ms_accept"],
@@ -572,6 +580,32 @@ def run_gpu(args):
     if pool is not None:
         pool.close()
 
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, caches, limit=DUMP_LIMIT, seed=0):
+    """Write the per-variable score caches {variable: (masks uint64 [n, words], scores float32 [n])} as .npy files, one row
+    per stored parent set, variables ascending and each cache in its canonical (|S|, mask) order:
+      variable.npy  float64 [N]            the child variable
+      parents.npy   float64 [N, 2*words]   every 64-bit parent-mask word as two exact 32-bit halves, low half first
+      scores.npy    float32 [N]            the stored score
+      index.npy     float64 [N]            the row's position in the full output
+    When the full output exceeds `limit` bytes, a fixed seeded sample of rows (kept in order) is written instead."""
+    vs = sorted(caches)
+    masks = np.concatenate([np.asarray(caches[v][0], dtype=np.uint64) for v in vs])
+    scores = np.concatenate([np.asarray(caches[v][1], dtype=np.float32) for v in vs])
+    variable = np.concatenate([np.full(len(caches[v][1]), v, dtype=np.float64) for v in vs])
+    index = np.arange(len(scores), dtype=np.int64)
+    rows = (limit - 4 * 128) // (8 + 8 * 2 * masks.shape[1] + 4 + 8)   # 128: one .npy header
+    if len(scores) > rows:
+        index = np.sort(np.random.default_rng(seed).choice(len(scores), size=rows, replace=False))
+    halves = np.stack([masks[index] & np.uint64(0xFFFFFFFF), masks[index] >> np.uint64(32)], axis=2).reshape(len(index), -1)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("variable", variable[index]), ("parents", halves.astype(np.float64)), ("scores", scores[index]),
+                    ("index", index.astype(np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------- sub-records of the default line
@@ -1000,7 +1034,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-subrecords", action="store_true", help="skip the cBIC configs[2] and score-file wall-time sub-records of the default line")
     ap.add_argument("--one-pass", action="store_true", help="profiling aid: one warm pass, then one pass on one context inside cudaProfilerStart/Stop; no bench line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, run the step once more, untimed, and write the score caches it reads back (every "
+                         "variable's stored parent sets and scores) to DIR/*.npy, at most 64 MB (a seeded sample of rows beyond that); "
+                         "bic and cbic, one GPU")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "urlgpu" or args.workload == "cbic5" or args.gpus != 1 or args.one_pass):
+        ap.error("--dump-outputs needs --impl urlgpu, --workload bic or cbic, --gpus 1 and no --one-pass")
     args.cpu_seconds_given = any(a == "--cpu-seconds" or a.startswith("--cpu-seconds=") for a in sys.argv[1:])
     if args.impl == "reference":
         run_reference(args)

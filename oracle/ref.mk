@@ -1,7 +1,10 @@
-# oracle/_ref: the reference's OWN discrete-BIC sources, compiled where they lie under /root/reference against the
-# shim headers in oracle/shim/ (Boost is absent).  Only ref_driver.cpp is ours.  Output: oracle/_ref/libref_bic.so
+# oracle/_ref: the reference's OWN discrete-BIC sources, compiled where they lie in an urlearning-cpp checkout (REF, by
+# default $URLEARNING_CPP_SRC: the directory that holds urlearning/) against the shim headers in oracle/shim/ (Boost is absent).  Only ref_driver.cpp is ours.  Output: oracle/_ref/libref_bic.so
 # (git-ignored, travels to the GPU box).  Reference sources are never copied into the repo.
-REF ?= /root/reference
+REF ?= $(URLEARNING_CPP_SRC)
+ifeq ($(strip $(REF)),)
+$(error set REF or URLEARNING_CPP_SRC to an urlearning-cpp source checkout)
+endif
 CXX = $(shell test -x /usr/bin/g++ && echo /usr/bin/g++ || echo g++)
 # the reference's own flags (urlearning/Jamroot:14-45): -std=c++11 -fno-strict-aliasing; -w: its warnings are not ours
 CXXFLAGS = -std=c++11 -fno-strict-aliasing -O2 -fPIC -w -pthread -I shim -I $(REF)

@@ -1,6 +1,6 @@
 """fNML (SURVEY.md §8f rank 4): the regret tables and the oracle's fNML restatement, pinned against the reference's own
-code (oracle/_ref: fnml_scoring_function.cpp + getRegretCache compiled from /root/reference) and, for the K = 2 table,
-against the literals in the reference's header when it is present."""
+code (oracle/_ref: fnml_scoring_function.cpp + getRegretCache compiled from the checkout URLEARNING_CPP_SRC names) and,
+for the K = 2 table, against the literals in the reference's header when that checkout is present."""
 import os
 import re
 import struct
@@ -13,7 +13,8 @@ import ref_lib
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEP = os.path.join(ROOT, "tests", "data", "hepatitis.clean.csv")
-REF_HEADER = "/root/reference/urlearning/scoring_function/fnml_scoring_function.h"
+REF_SRC = os.environ.get("URLEARNING_CPP_SRC")
+REF_HEADER = os.path.join(REF_SRC, "urlearning", "scoring_function", "fnml_scoring_function.h") if REF_SRC else None
 R2_CRC = 0x85246587   # crc32 of the 1001 float32 bit patterns (tools/gen_regret_table.py)
 
 
@@ -33,7 +34,7 @@ def test_generated_r2_tables_are_identical_and_match_their_crc():
     assert np.all(np.diff(f) > 0)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_HEADER), reason="reference sources not present")
+@pytest.mark.skipif(not (REF_HEADER and os.path.exists(REF_HEADER)), reason="reference sources not present")
 def test_r2_table_equals_the_reference_literals_as_float32():
     src = open(REF_HEADER).read()
     body = src[src.index("r2_1000[] = {") + len("r2_1000[] = {"):]

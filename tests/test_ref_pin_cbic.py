@@ -1,5 +1,5 @@
 """Pins the oracle's continuous-BIC restatement against the REFERENCE'S OWN CODE: scoring_function/BIC_OLS.cpp and
-score_calculator.cpp compiled from /root/reference (oracle/_ref/libref_cbic.so, oracle/ref.mk) over shim Boost headers and a
+score_calculator.cpp compiled from an urlearning-cpp checkout (oracle/_ref/libref_cbic.so, oracle/ref.mk) over shim Boost headers and a
 minimal Armadillo / mlpack (oracle/shim_arma: matrices, mean, var, a no-intercept linear regression written from their
 published algorithms in the oracle's arithmetic order).  Pinned here: the standardisation, the score formula, the acceptance
 test with its recursion exactly AS WRITTEN (SURVEY.md Q5: arma::uvec zero-filled) and the enumeration / store loop — the

@@ -1,4 +1,4 @@
-"""The reference's OWN `score` program (score/score_main.cpp with its own main(), compiled from /root/reference by oracle/ref.mk
+"""The reference's OWN `score` program (score/score_main.cpp with its own main(), compiled from an urlearning-cpp checkout by oracle/ref.mk
 over shim Boost headers — program_options that parses, threads that run — and, for cBIC, the minimal Armadillo / mlpack of
 oracle/shim_arma) against the oracle's restatement of the whole run (orc_score_file): the header block byte for byte, the
 same variables, arities and parent sets, and the scores — bit-identical text for cBIC (same arithmetic on both sides),

@@ -24,9 +24,10 @@ def S():
 @pytest.fixture(scope="module")
 def ref():
     if not os.path.exists(REF_SO):
-        if not os.path.isdir("/root/reference/urlearning"):
-            pytest.skip("oracle/_ref/libref_search.so was not built and /root/reference is absent")
-        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "-f", "ref.mk"])
+        src = os.environ.get("URLEARNING_CPP_SRC")
+        if not src or not os.path.isdir(os.path.join(src, "urlearning")):
+            pytest.skip("oracle/_ref/libref_search.so was not built and URLEARNING_CPP_SRC names no reference checkout")
+        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "-f", "ref.mk", "REF=" + os.path.abspath(src)])
     L = C.CDLL(REF_SO)
     vp, i32, i64 = C.c_void_p, C.c_int, C.c_int64
     L.refs_open.restype = vp
