@@ -197,8 +197,8 @@ typedef struct urlgpu_stats {
     double algorithmic_bytes;  /* BIC: sum over scored sets of n*(|S|+1) */
     double algorithmic_flops;  /* cBIC: sum over scored sets of k^3/3+2k^2+2k */
     double gram_flops;         /* K2: 2*n*p^2 per Gram formed */
-    uint64_t launches_tree;    /* K1 on-chip count + marginalise + score kernel */
-    double ms_tree;
+    uint64_t launches_tree;    /* always 0: kept so the struct layout stays compatible */
+    double ms_tree;            /* always 0 */
     double k1_bytes_read;      /* cube path: bytes the K1 kernels load from global memory (rows + parent tables; L2 may absorb re-reads) */
     double k1_bytes_written;   /* cube path: bytes of contingency tables the K1 kernels store */
     double ms_standardise;     /* K2: column moments + standardisation passes (HBM bound); ms_gram is the DMMA Gram kernel + combine */

@@ -83,38 +83,13 @@ def test_all_tiers_arity4(pkg, orc, bic_engine):
         _check_variable(pkg, orc, engine, codes, card, None, v, 9)
 
 
-@pytest.mark.parametrize("budget,run,unit", [(1024, 2, 64), (3072, 6, 256), (12288, 6, 1024), (24576, 8, 2048), (4096, 3, 256)])
-def test_tree_path_slicing_variants(pkg, orc, budget, run, unit):
-    """the on-chip tree path under different slice budgets / run limits: deep slicing with many row segments, single-unit
-    slices, long runs; every variant must reproduce the oracle bit for bit"""
-    keys = {"URLGPU_BIC_MODE": "tree", "URLGPU_TREE_BUDGET": str(budget), "URLGPU_TREE_RUN": str(run), "URLGPU_TREE_UNIT": str(unit)}
-    old = {k: os.environ.get(k) for k in keys}
-    os.environ.update(keys)
-    try:
-        eng = pkg.Engine(0)
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-    codes, card, edges, _ = pkg.datagen.discrete_bn(p=14, n=40009, seed=21, arities=(2, 3, 4), window=6, max_indegree=3)
-    eng.set_discrete(codes, card)
-    eng.reset_stats()
-    for v, K in ((0, 13), (6, 8), (13, 5), (9, 1), (3, 0)):
-        _check_variable(pkg, orc, eng, codes, card, None, v, K)
-    _check_variable(pkg, orc, eng, codes, card, edges, 7, 6, flags=pkg.PRUNE_DOMINATED)
-    assert eng.stats()["launches_tree"] >= 3  # the tree kernel really ran (no silent fall-back to the cube path)
-    eng.close()
-
-
-@pytest.mark.parametrize("fuse,budget,leaves", [("1", 22528, "1"), ("1", 2048, "1"), ("0", 22528, "1"), ("1", 40000, "0"), ("0", 22528, "0")])
-def test_cube_roots_counted_in_slices_and_fused(pkg, orc, fuse, budget, leaves):
+@pytest.mark.parametrize("fuse,budget", [("1", 22528), ("1", 2048), ("0", 22528), ("1", 40000), ("0", 2048)])
+def test_cube_roots_counted_in_slices_and_fused(pkg, orc, fuse, budget):
     """the cube path's big roots: counted in shared-memory slices of the packed rows; ancestor-only roots (layer K+1) hand
     their children straight to the next layer (fused) or, with URLGPU_FUSE_ROOTS=0 / a run that does not fit the slice
-    budget, are written out and marginalised through HBM; sets without the lowest candidate are scored by the pass that
-    produces their parent table (URLGPU_FUSE_LEAVES).  All variants bit-exact against the oracle."""
-    keys = {"URLGPU_BIC_MODE": "cube", "URLGPU_FUSE_ROOTS": fuse, "URLGPU_ROOT_BUDGET": str(budget), "URLGPU_FUSE_LEAVES": leaves}
+    budget, are written out and marginalised through HBM.  Edge shapes: every set a root's descendant (K = c - 1), a
+    single parent, the empty set alone.  All variants bit-exact against the oracle."""
+    keys = {"URLGPU_BIC_MODE": "cube", "URLGPU_FUSE_ROOTS": fuse, "URLGPU_ROOT_BUDGET": str(budget)}
     old = {k: os.environ.get(k) for k in keys}
     os.environ.update(keys)
     try:
@@ -127,7 +102,7 @@ def test_cube_roots_counted_in_slices_and_fused(pkg, orc, fuse, budget, leaves):
                 os.environ[k] = v
     codes, card, edges, _ = pkg.datagen.discrete_bn(p=14, n=70003, seed=31, arities=(2, 3, 4), window=6, max_indegree=3)
     eng.set_discrete(codes, card)
-    for v, K in ((2, 9), (11, 8), (5, 10)):
+    for v, K in ((2, 9), (11, 8), (5, 10), (0, 13), (9, 1), (3, 0)):
         _check_variable(pkg, orc, eng, codes, card, None, v, K)
     _check_variable(pkg, orc, eng, codes, card, None, 7, 9, flags=pkg.PRUNE_DOMINATED)
     eng.close()

@@ -15,7 +15,7 @@ import re
 import sys
 
 K1 = re.compile(r"bic_root_kernel|cube_derive_kernel|cube_map_kernel|root_map_kernel|tree_key_kernel|tree_scatter_kernel|bic_count_smem_kernel|"
-                r"bic_count_global_kernel|bic_score_tables_kernel|bic_tree_kernel|tree_map_kernel|DeviceScan|bucket_scan_kernel|sparse_bic")
+                r"bic_count_global_kernel|bic_score_tables_kernel|DeviceScan|bucket_scan_kernel|sparse_bic")
 scale = {"byte": 1.0, "Kbyte": 1e3, "Mbyte": 1e6, "Gbyte": 1e9, "ns": 1e-3, "us": 1.0, "ms": 1e3, "s": 1e6,
          "nsecond": 1e-3, "usecond": 1.0, "msecond": 1e3, "second": 1e6}
 

@@ -23,6 +23,6 @@ for rep in range(2):
         eng.synchronize()
         dt = time.time() - t0
         st = eng.stats()
-        print(f"v={v} c={c} K={K} sets={res.scored()} wall={dt*1e3:.1f} ms  count_ms={st['ms_count']:.2f} cube_ms={st['ms_cube']:.2f} tree_ms={st['ms_tree']:.2f} "
+        print(f"v={v} c={c} K={K} sets={res.scored()} wall={dt*1e3:.1f} ms  count_ms={st['ms_count']:.2f} cube_ms={st['ms_cube']:.2f} "
               f"launches={st['launches_total']} sets/s={res.scored()/dt:.3e} alg_GB/s={st['algorithmic_bytes']/dt/1e9:.1f}")
         res.free()

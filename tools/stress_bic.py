@@ -12,10 +12,9 @@ rng = np.random.default_rng(seed)
 t_end = time.time() + budget_s
 cases = 0
 while time.time() < t_end:
-    mode = str(rng.choice(["cube", "cube", "tree", "direct"]))
-    env = {"URLGPU_BIC_MODE": mode, "URLGPU_FUSE_ROOTS": str(rng.integers(0, 2)), "URLGPU_FUSE_LEAVES": str(rng.integers(0, 2)),
-           "URLGPU_ROOT_BUDGET": str(int(rng.choice([1024, 4096, 24576, 40000]))), "URLGPU_TREE_BUDGET": str(int(rng.choice([2048, 8192, 16384]))),
-           "URLGPU_TREE_RUN": str(int(rng.integers(1, 9)))}
+    mode = str(rng.choice(["cube", "cube", "direct"]))
+    env = {"URLGPU_BIC_MODE": mode, "URLGPU_FUSE_ROOTS": str(rng.integers(0, 2)),
+           "URLGPU_ROOT_BUDGET": str(int(rng.choice([1024, 4096, 24576, 40000])))}
     os.environ.update(env)
     eng = pkg.Engine(0)
     p = int(rng.integers(3, 15))

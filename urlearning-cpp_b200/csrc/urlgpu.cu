@@ -33,7 +33,7 @@ namespace {
 thread_local std::string g_create_error;
 std::atomic<int> g_ctx_on_device[64];   // live contexts per device: each budgets its share of the free memory
 
-enum Family { F_COUNT = 0, F_CUBE, F_CBIC, F_ACCEPT, F_PRUNE, F_GRAM, F_TREE, F_OTHER, F_STD, F_N };
+enum Family { F_COUNT = 0, F_CUBE, F_CBIC, F_ACCEPT, F_PRUNE, F_GRAM, F_OTHER, F_STD, F_N };
 
 struct EvPair { cudaEvent_t a, b; int fam; };
 
@@ -87,10 +87,6 @@ struct urlgpu_ctx {
     uint16_t *d_low_sorted = nullptr; int low_bits = -1; std::vector<int> low_off;
     bool use_slice_count = true; // cube path: count big roots in shared-memory slices (URLGPU_SLICE_COUNT=0 disables)
     bool fuse_roots = true;      // cube path: ancestor-only roots hand their children straight to HBM (URLGPU_FUSE_ROOTS=0 disables)
-    // cube path: sets without cube bit 0 scored by the pass that produces their parent (URLGPU_FUSE_LEAVES=1 enables).  Bit-exact and
-    // 16 % fewer issued bytes, but measured neutral to slightly slower at config 4 (the saved reads were L2 hits; the grouped
-    // access pattern halves the sector efficiency of each load), so off by default
-    bool fuse_leaves = false;
     // cube path: tables of layers >= table16_min_layer are written with uint16 cells, speculatively (URLGPU_TABLE16=0 disables,
     // URLGPU_TABLE16_MINLAYER sets the layer); a count that does not fit flags the call and the variable is recomputed in 32 bits
     bool table16 = true;
@@ -98,13 +94,9 @@ struct urlgpu_ctx {
     uint32_t root_budget = 24 * 1024; // cells of a root slice (URLGPU_ROOT_BUDGET): 96 KB + segment tables, two 512-thread CTAs per SM
     uint32_t root_seg_cap = 1024;     // row segments of a slice kept in shared memory (URLGPU_ROOT_SEGS)
     int root_warps = 16;              // warps per CTA of bic_root_kernel (URLGPU_ROOT_WARPS = 8, 12 or 16)
-    // K1 strategy (URLGPU_BIC_MODE=cube|tree|direct): 2 = cube (default: roots counted in shared-memory slices, the rest
-    // marginalised through HBM), 0 = tree (every table counted or marginalised in shared memory; measured 0.6-0.9x the cube
-    // path on config 4, instruction bound — kept as an opt-in strategy), 1 = direct counting of every set
-    int bic_mode = 2;
-    uint32_t tree_budget = 8 * 1024;    // cells of a slice table (URLGPU_TREE_BUDGET); the warps' stacks get the same
-    int tree_run = 6;                   // run limit t (URLGPU_TREE_RUN)
-    uint32_t tree_unit_cap = 1024;      // largest unit table r_v * prod_{i<t} r_i (URLGPU_TREE_UNIT)
+    // K1 strategy: the cube path (roots counted in shared-memory slices, the rest marginalised through HBM), or, with
+    // URLGPU_BIC_MODE=direct, direct counting of every set from the rows
+    bool bic_direct = false;
 
     // rank-space layout: binomial tables [256][K + 2] per parent limit K (tiny; kept for the life of the context so kernels in
     // flight never lose theirs), and the layout policy (URLGPU_LAYOUT=dense|rank|auto)
@@ -224,7 +216,7 @@ void fold_events(urlgpu_ctx *ctx) {
         if (cudaEventElapsedTime(&ms, ep.a, ep.b) == cudaSuccess) {
             double *dst = ep.fam == F_COUNT ? &ctx->st.ms_count : ep.fam == F_CUBE ? &ctx->st.ms_cube : ep.fam == F_CBIC ? &ctx->st.ms_cbic
                         : ep.fam == F_ACCEPT ? &ctx->st.ms_accept : ep.fam == F_PRUNE ? &ctx->st.ms_prune : ep.fam == F_GRAM ? &ctx->st.ms_gram
-                        : ep.fam == F_TREE ? &ctx->st.ms_tree : ep.fam == F_STD ? &ctx->st.ms_standardise : nullptr;
+                        : ep.fam == F_STD ? &ctx->st.ms_standardise : nullptr;
             if (dst) *dst += ms;
         }
         ctx->free_events.push_back(ep.a);
@@ -240,8 +232,7 @@ struct Region {
     Region(urlgpu_ctx *c, int f, uint64_t launches) : ctx(c), fam(f), on(c->timing) {
         c->st.launches_total += launches;
         uint64_t *cnt = f == F_COUNT ? &c->st.launches_count : f == F_CUBE ? &c->st.launches_cube : f == F_CBIC ? &c->st.launches_cbic
-                      : f == F_ACCEPT ? &c->st.launches_accept : f == F_PRUNE ? &c->st.launches_prune : f == F_TREE ? &c->st.launches_tree
-                      : &c->st.launches_other;
+                      : f == F_ACCEPT ? &c->st.launches_accept : f == F_PRUNE ? &c->st.launches_prune : &c->st.launches_other;
         *cnt += launches;
         if (on) { ep.a = get_event(c); ep.b = get_event(c); ep.fam = f; cudaEventRecord(ep.a, c->stream); }
     }
@@ -344,7 +335,6 @@ extern "C" int urlgpu_create(urlgpu_ctx **out, int device_id) {
     ctx->stream = ctx->own_stream;
     if (const char *m = getenv("URLGPU_SLICE_COUNT")) ctx->use_slice_count = atoi(m) != 0;
     if (const char *m = getenv("URLGPU_FUSE_ROOTS")) ctx->fuse_roots = atoi(m) != 0;
-    if (const char *m = getenv("URLGPU_FUSE_LEAVES")) ctx->fuse_leaves = atoi(m) != 0;
     if (const char *m = getenv("URLGPU_TABLE16")) ctx->table16 = atoi(m) != 0;
     if (const char *m = getenv("URLGPU_TABLE16_MINLAYER")) ctx->table16_min_layer = std::max(1, atoi(m));
     if (const char *m = getenv("URLGPU_ROOT_BUDGET")) ctx->root_budget = (uint32_t)std::max(1024, std::min(atoi(m), 48 * 1024)) / 4 * 4;
@@ -359,16 +349,11 @@ extern "C" int urlgpu_create(urlgpu_ctx **out, int device_id) {
 #undef URLGPU_ROOT_ATTR
     }
     if (const char *m = getenv("URLGPU_LAYOUT")) ctx->layout_policy = strcmp(m, "dense") == 0 ? 1 : strcmp(m, "rank") == 0 ? 2 : 0;
-    if (const char *m = getenv("URLGPU_BIC_MODE"))
-        ctx->bic_mode = strcmp(m, "direct") == 0 ? 1 : strcmp(m, "tree") == 0 ? 0 : 2;
-    if (const char *m = getenv("URLGPU_TREE_BUDGET")) ctx->tree_budget = (uint32_t)std::max(1024, std::min(atoi(m), 26 * 1024)) / 4 * 4;
-    if (const char *m = getenv("URLGPU_TREE_RUN")) ctx->tree_run = std::max(1, std::min(atoi(m), kTreeMaxRun));
-    if (const char *m = getenv("URLGPU_TREE_UNIT")) ctx->tree_unit_cap = (uint32_t)std::max(16, atoi(m));
-    cudaFuncSetAttribute(bic_count_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->smem_optin - 2048);
-    cudaFuncSetAttribute(bic_tree_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * ctx->tree_budget * sizeof(int)));
-    cudaFuncSetAttribute(bic_tree_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * ctx->tree_budget * sizeof(int)));
-    cudaFuncSetAttribute(bic_tree_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * ctx->tree_budget * sizeof(int)));
-    cudaFuncSetAttribute(bic_tree_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * ctx->tree_budget * sizeof(int)));
+    if (const char *m = getenv("URLGPU_BIC_MODE")) ctx->bic_direct = strcmp(m, "direct") == 0;
+    // the large dynamic shared-memory opt-ins are per device: every context sets them for its own
+    cudaFuncSetAttribute(bic_count_smem_kernel<MaskSets>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->smem_optin - 2048);
+    cudaFuncSetAttribute(bic_count_smem_kernel<RankSets>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->smem_optin - 2048);
+    cudaFuncSetAttribute(gram_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGramSmemBytes);
     if (device_id < 64) g_ctx_on_device[device_id]++;
     *out = ctx;
     return URLGPU_OK;
@@ -652,8 +637,6 @@ static int shard_finish_impl(urlgpu_ctx *ctx, const double *mean_host, const dou
         const int slices = (int)((z_stride + rps - 1) / rps);
         CK(gpart.alloc((size_t)slices * p * p * sizeof(double)));
         CK(g.alloc((size_t)p * p * sizeof(double)));
-        static bool attr = false;
-        if (!attr) { CK(cudaFuncSetAttribute(gram_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGramSmemBytes)); attr = true; }
         gram_partial_kernel<<<dim3(pairs, slices), kGramThreads, kGramSmemBytes, s>>>(zbuf, z_stride, p, rps, tiles, gpart.as<double>());
         gram_combine_kernel<<<blocks_for((uint64_t)p * p, 256), 256, 0, s>>>(gpart.as<double>(), p, slices, g.as<double>());
         ctx->st.gram_flops += 2.0 * (double)n * p * p;
@@ -783,128 +766,24 @@ static CandInfo make_candinfo(urlgpu_ctx *ctx, int variable, const std::vector<i
     return ci;
 }
 
-// Score the listed compact masks (device list for the shared-memory tiers, host list for the global tier)
-static int bic_run_global_tier(urlgpu_ctx *ctx, const BicData &bd, const CandInfo &ci, const std::vector<uint32_t> &masks,
-                               float *d_table, long long *d_llfixed, int *keep_tables_of_first /*optional host out*/, int64_t keep_cells,
-                               const RankSpace &om = RankSpace{}) {
-    if (masks.empty()) return URLGPU_OK;
-    cudaStream_t s = ctx->stream;
-    std::vector<GlobalSet> sets(masks.size());
-    size_t max_cells = 0;
-    for (size_t i = 0; i < masks.size(); i++) {
-        uint64_t cells = ci.rv;
-        for (int b = 0; b < ci.c; b++) if ((masks[i] >> b) & 1) cells *= (uint64_t)ci.card[b];
-        sets[i].mask = masks[i]; sets[i].cells = (uint32_t)cells; sets[i].table_off = 0;
-        max_cells = std::max<size_t>(max_cells, cells);
-    }
-    int rc = ensure_tables(ctx, std::max(kBatchTableElems, max_cells));
-    if (rc) return rc;
-    DevBuf dsets(ctx), dacc(ctx);
-    CK(dsets.alloc(sets.size() * sizeof(GlobalSet)));
-    CK(dacc.alloc(sets.size() * sizeof(long long)));
-    CK(cudaMemsetAsync(dacc.p, 0, sets.size() * sizeof(long long), s));
-    // batches
-    size_t i0 = 0;
-    std::vector<std::pair<size_t, size_t>> batches;
-    while (i0 < sets.size()) {
-        size_t used = 0, i1 = i0;
-        while (i1 < sets.size() && (i1 == i0 || used + sets[i1].cells <= ctx->tables_cap) && i1 - i0 < 65535) {
-            sets[i1].table_off = used;
-            used += (sets[i1].cells + 3) / 4 * 4;
-            i1++;
-        }
-        batches.push_back({i0, i1});
-        i0 = i1;
-    }
-    CK(cudaMemcpyAsync(dsets.p, sets.data(), sets.size() * sizeof(GlobalSet), cudaMemcpyHostToDevice, s));
+// A batch of B global-tier tables (zeroed, at their table_off in `tables`): count the rows of every set in row slices,
+// then score the tables into acc[set] in configuration chunks; both grids hold ~8 CTAs per SM over the batch.
+template <class Sets>
+static void launch_count_global(urlgpu_ctx *ctx, const BicData &bd, const Sets &fam, const GlobalSet *d_sets, size_t B, int *tables) {
     const int threads = 256;
-    for (auto &bt : batches) {
-        const size_t B = bt.second - bt.first;
-        size_t used = sets[bt.second - 1].table_off + sets[bt.second - 1].cells;
-        Region rg(ctx, F_COUNT, 3);
-        CK(cudaMemsetAsync(ctx->d_tables, 0, used * sizeof(int), s));
-        // row slices so that the batch fills the machine (B*R CTAs ~ 8 per SM)
-        int64_t R = std::max<int64_t>(1, (int64_t)(ctx->sm_count * 8 + B - 1) / (int64_t)B);
-        int64_t rps = (bd.n + R - 1) / R;
-        rps = std::max<int64_t>((rps + 15) / 16 * 16, 16 * threads);
-        R = (bd.n + rps - 1) / rps;
-        bic_count_global_kernel<<<dim3((unsigned)B, (unsigned)R), threads, 0, s>>>(bd, ci, dsets.as<GlobalSet>() + bt.first, ctx->d_tables, rps);
-        uint32_t maxc = 0;
-        for (size_t i = bt.first; i < bt.second; i++) maxc = std::max(maxc, sets[i].cells);
-        int64_t nconf = maxc / ci.rv;
-        int64_t chunks = std::max<int64_t>(1, std::min<int64_t>((nconf + threads * 4 - 1) / (threads * 4), (ctx->sm_count * 8 + (int64_t)B - 1) / (int64_t)B));
-        int64_t cpc = (nconf + chunks - 1) / chunks;
-        bic_score_tables_kernel<<<dim3((unsigned)B, (unsigned)chunks), threads, 0, s>>>(bd, ci, dsets.as<GlobalSet>() + bt.first, ctx->d_tables,
-                                                                                    dacc.as<long long>() + bt.first, cpc);
-        if (keep_tables_of_first && bt.first == 0) {
-            CK(cudaMemcpyAsync(keep_tables_of_first, ctx->d_tables, (size_t)keep_cells * sizeof(int), cudaMemcpyDeviceToHost, s));
-            CK(cudaStreamSynchronize(s));
-        }
-    }
-    if (d_table) {
-        Region rg(ctx, F_OTHER, 1);
-        bic_finalize_kernel<<<blocks_for(sets.size(), 256), 256, 0, s>>>(bd, ci, dsets.as<GlobalSet>(), dacc.as<long long>(), (int)sets.size(), d_table,
-                                                                         d_llfixed, om);
-    }
-    CK(cudaStreamSynchronize(s)); // dsets/dacc are freed on return
-    CK(cudaGetLastError());
-    return URLGPU_OK;
+    int64_t R = std::max<int64_t>(1, (int64_t)(ctx->sm_count * 8 + B - 1) / (int64_t)B);
+    int64_t rps = (bd.n + R - 1) / R;
+    rps = std::max<int64_t>((rps + 15) / 16 * 16, 16 * threads);
+    R = (bd.n + rps - 1) / rps;
+    bic_count_global_kernel<<<dim3((unsigned)B, (unsigned)R), threads, 0, ctx->stream>>>(bd, fam, d_sets, tables, rps);
 }
-
-static int bic_score_family_direct(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, float *d_table, long long *d_llfixed,
-                                   uint64_t *n_scored, const RankSpace &om) {
-    cudaStream_t s = ctx->stream;
-    const int c = (int)cand.size();
-    const uint64_t n_masks = (uint64_t)1 << c;
-    const uint64_t fam = family_size(c, K);
-    *n_scored = fam;
-    BicData bd{ctx->d_codes, ctx->n, ctx->n_stride, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, ctx->ds_base, ctx->ds_ess, ctx->ds_scale};
-    CandInfo ci = make_candinfo(ctx, variable, cand, K);
-    const uint32_t tier1_cells = (uint32_t)((ctx->smem_optin - 2048) / sizeof(int));
-
-    DevBuf lists(ctx), counters(ctx);
-    CK(lists.alloc(3 * fam * sizeof(uint32_t)));
-    CK(counters.alloc(4 * sizeof(unsigned long long)));
-    CK(cudaMemsetAsync(counters.p, 0, 4 * sizeof(unsigned long long), s));
-    uint32_t *l0 = lists.as<uint32_t>(), *l1 = l0 + fam, *l2 = l1 + fam;
-    {
-        Region rg(ctx, F_OTHER, 1);
-        bic_classify_kernel<<<blocks_for(n_masks, 256), 256, 0, s>>>(ci, n_masks, kTier0Cells, tier1_cells, kCellLimit, l0, l1, l2,
-                                                                    counters.as<unsigned long long>());
-    }
-    unsigned long long hc[4];
-    CK(cudaMemcpyAsync(hc, counters.p, sizeof hc, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    if (hc[3]) return ctx->fail(URLGPU_ERR_LIMIT, "a contingency table of this family has more than 2^30 cells");
-    if (hc[0]) {
-        Region rg(ctx, F_COUNT, 1);
-        const int threads = ctx->n >= 65536 ? 256 : 128;
-        bic_count_smem_kernel<<<(unsigned)hc[0], threads, kTier0Cells * sizeof(int), s>>>(bd, ci, l0, d_table, d_llfixed, nullptr, nullptr, nullptr, om);
-    }
-    if (hc[1]) {
-        Region rg(ctx, F_COUNT, 1);
-        bic_count_smem_kernel<<<(unsigned)hc[1], 1024, (size_t)tier1_cells * sizeof(int), s>>>(bd, ci, l1, d_table, d_llfixed, nullptr, nullptr, nullptr, om);
-    }
-    if (hc[2]) {
-        std::vector<uint32_t> m2(hc[2]);
-        CK(cudaMemcpyAsync(m2.data(), l2, hc[2] * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        std::sort(m2.begin(), m2.end());
-        int rc = bic_run_global_tier(ctx, bd, ci, m2, d_table, d_llfixed, nullptr, 0, om);
-        if (rc) return rc;
-    }
-    // algorithmic bytes: n*(k+1) per set (SURVEY.md §8d)
-    {
-        double bytes = 0, b = 1;
-        for (int l = 0; l <= K && l <= c; l++) { bytes += b * (double)ctx->n * (l + 1); b = b * (c - l) / (l + 1); }
-        ctx->st.algorithmic_bytes += bytes;
-        ctx->st.sets_scored += fam;
-    }
-    CK(cudaStreamSynchronize(s)); // lists/counters are freed on return
-    CK(cudaGetLastError());
-    return URLGPU_OK;
+static void launch_score_tables(urlgpu_ctx *ctx, const BicData &bd, int rv, const GlobalSet *d_sets, size_t B, uint32_t max_cells, const int *tables, long long *acc) {
+    const int threads = 256;
+    const int64_t nconf = max_cells / rv;
+    const int64_t chunks = std::max<int64_t>(1, std::min<int64_t>((nconf + threads * 4 - 1) / (threads * 4), (ctx->sm_count * 8 + (int64_t)B - 1) / (int64_t)B));
+    const int64_t cpc = (nconf + chunks - 1) / chunks;
+    bic_score_tables_kernel<<<dim3((unsigned)B, (unsigned)chunks), threads, 0, ctx->stream>>>(bd, rv, d_sets, tables, acc, cpc);
 }
-
 
 // ------------------------------------------------------------------------------------------------------------
 // Cube path: count only the root tables from the rows, derive every other table of the family by summing one
@@ -973,8 +852,7 @@ static int h2d_async(urlgpu_ctx *ctx, void *dst, const void *src, size_t bytes) 
 
 // part / parts: score only the sub-forest of the roots i with i % parts == part (and everything derived from them); the parts
 // are disjoint and cover the family (urlgpu_score_part: one variable's K1 work split over several GPUs)
-static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, float *d_table, long long *d_llfixed,
-                                 uint64_t *n_scored, bool *used, const RankSpace &om, int part = 0, int parts = 1, int *d_ovf = nullptr) {
+static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, float *d_table, uint64_t *n_scored, bool *used, const RankSpace &om, int part = 0, int parts = 1, int *d_ovf = nullptr) {
     *used = false;
     cudaStream_t s = ctx->stream;
     { int rc_ = stage_begin(ctx); if (rc_) return rc_; }
@@ -986,14 +864,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
     const auto T0 = tnow();
     const int c = (int)cand.size();
     const int Kc = std::min(K, c);
-    // Table layout arity (opt-in, URLGPU_PAD3=1).  A child of arity 3 can be laid out as if it had a fourth value that never occurs:
-    // configurations are then 16 bytes (8 in uint16 tables) and every kernel of this path moves them with one aligned vector
-    // access per lane instead of three scalar ones (ncu on the 12-byte layout: 9 of 32 bytes used per L1 sector).  The empty
-    // cells contribute nothing to any sum; the penalty uses the true arity (cube_finalize_kernel, ci_res).  Bit-exact, but
-    // measured slower at configs[3] (301 -> 332 ms per step): the kernels are bound by instruction issue, not by L1 sectors,
-    // and a third more cells are walked and a third more root slices counted.  Off by default.
-    static const bool pad3 = getenv("URLGPU_PAD3") && atoi(getenv("URLGPU_PAD3")) != 0;
-    const int rv = (ctx->card[variable] == 3 && pad3) ? 4 : ctx->card[variable];
+    const int rv = ctx->card[variable];
     const uint64_t n = (uint64_t)ctx->n;
     if (c == 0) return URLGPU_OK; // only the empty set: the direct path handles it
     // cube order: ascending arity, ties by variable index
@@ -1005,7 +876,6 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
     for (int i = 0; i < c; i++) { cube_vars[i] = cand[perm[i]]; ccard[i] = (uint64_t)ctx->card[cube_vars[i]]; }
     for (int i = 0; i < c; i++) prefix[i + 1] = std::min<uint64_t>(prefix[i] * ccard[i], (uint64_t)1 << 40);
     CandInfo ci_cube = make_candinfo(ctx, variable, cube_vars, K);
-    ci_cube.rv = rv;                               // layout arity: the counting kernels index x_v + rv * paIdx
     CandInfo ci_res = make_candinfo(ctx, variable, cand, K);
     BicData bd{ctx->d_codes, ctx->n, ctx->n_stride, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, ctx->ds_base, ctx->ds_ess, ctx->ds_scale};
     const uint32_t tier1_cells = (uint32_t)((ctx->smem_optin - 2048) / sizeof(int));
@@ -1102,7 +972,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
     if (packed_ok) {
         uint64_t maxr = (uint64_t)rv;
         for (int i = 0; i < c; i++) maxr = std::max(maxr, ccard[i]);
-        tv.c = c; tv.rv = rv; tv.max_parents = K; tv.t = 0;
+        tv.c = c; tv.rv = rv;
         tv.w = maxr <= 4 ? 2 : maxr <= 16 ? 4 : 8;
         if ((c + 1) * tv.w > 64) packed_ok = false;
         for (int i = 0; i < c; i++) tv.card[i] = (uint16_t)ccard[i];
@@ -1131,7 +1001,6 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         if (nslices > 0x3fffffffull) return false;
         r = TreeRoot{};
         r.mask = P; r.nslices = (uint32_t)nslices; r.H = (uint32_t)H; r.nseg = (uint32_t)nseg; r.z = (uint8_t)zf;
-        r.size = (uint8_t)__builtin_popcount(P);
         r.fstride[0] = 1;
         for (int b = 0; b < zf; b++) r.fstride[b + 1] = (uint16_t)((uint32_t)rv * tv.pre[b]);
         uint32_t hs = (uint32_t)U0;
@@ -1175,7 +1044,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
     // Layer Lstar lives in buffer A, Lstar-1 in B, Lstar-2 in A again, ...: each buffer is sized for its own layers only.
     // Tables that are never materialised take no room: fused roots, and below the root layer every set without cube
     // bit 0 (nothing is derived from it, its table is only scored on the fly).
-    const bool use16 = ctx->table16 && d_ovf != nullptr && !ctx->fuse_leaves;
+    const bool use16 = ctx->table16 && d_ovf != nullptr;
     size_t needA = 0, needB = 0;
     for (int l = 0; l <= Lstar; l++) {
         uint64_t off = 0;
@@ -1249,7 +1118,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         for (size_t i = 0; i < L.size(); i++) hres[i] = mine[l][i] ? L[i].res_mask : 0xffffffffu; // 0xffffffff: not this call's set
         { int rc_ = h2d_async(ctx, dres.p, hres.data(), L.size() * sizeof(uint32_t)); if (rc_) return rc_; }
         Region rg(ctx, F_OTHER, 1);
-        cube_finalize_kernel<<<blocks_for(L.size(), 256), 256, 0, s>>>(bd, ci_res, dres.as<uint32_t>(), dacc.as<long long>() + acc_off[l], (int)L.size(), d_table, d_llfixed, om);
+        cube_finalize_kernel<<<blocks_for(L.size(), 256), 256, 0, s>>>(bd, ci_res, dres.as<uint32_t>(), dacc.as<long long>() + acc_off[l], (int)L.size(), d_table, om);
         return URLGPU_OK;
     };
 
@@ -1283,15 +1152,14 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
             const bool tiny = maxc <= kTier0Cells;
             const int threads = tiny ? (ctx->n >= 65536 ? 256 : 128) : 1024;
             const size_t smem = (tiny ? (size_t)kTier0Cells : (size_t)tier1_cells) * sizeof(int);
-            bic_count_smem_kernel<<<(unsigned)small_m.size(), threads, smem, s>>>(bd, ci_cube, dwork.as<uint32_t>(), nullptr, nullptr, doffs.as<uint64_t>(), bufP,
-                                                                               score_roots ? dacc_small.as<long long>() : nullptr, RankSpace{});
+            bic_count_smem_kernel<<<(unsigned)small_m.size(), threads, smem, s>>>(bd, MaskSets{ci_cube}, dwork.as<uint32_t>(), nullptr, doffs.as<uint64_t>(), bufP,
+                                                                               score_roots ? dacc_small.as<long long>() : nullptr);
         }
         if (!big.empty()) {
             CK(dgsets.alloc(big.size() * sizeof(GlobalSet)));
             CK(dacc_big.alloc(big.size() * sizeof(long long)));
             CK(cudaMemsetAsync(dacc_big.p, 0, big.size() * sizeof(long long), s));
             { int rc_ = h2d_async(ctx, dgsets.p, big.data(), big.size() * sizeof(GlobalSet)); if (rc_) return rc_; }
-            const int threads = 256;
             // (1) roots whose table can be cut along its top digits are counted in shared-memory slices of the bucketed
             //     packed rows (bic_root_kernel, tree_kernels.cuh).  A root that is only an ancestor (layer K+1) and whose
             //     run of low digits fits one slice is FUSED: its children are marginalised, scored and written by the
@@ -1305,7 +1173,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
                 for (size_t i = 0; i < big.size(); i++) {
                     const int kind = root_kind[big_idx[i]];
                     if (!kind) continue; // RED path below
-                    const uint32_t P = big[i].mask;
+                    const uint32_t P = big[i].key;
                     const int run = std::min(c, (int)__builtin_ctz(~P));
                     CubeRoot cr{};
                     if (!slice_root(P, kind == 2 ? run : 0, cr.t)) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: root slicing is not reproducible");
@@ -1344,7 +1212,6 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
                 { int rc_ = h2d_async(ctx, dcroots.p, croots.data(), croots.size() * sizeof(CubeRoot)); if (rc_) return rc_; }
                 tv.rows = drows.as<unsigned long long>();
                 tv.prefix_off = doffp.as<uint32_t>();
-                tv.cfg_tab = nullptr;
                 Region rg(ctx, F_COUNT, 8);
                 CK(cudaMemsetAsync(dhist.p, 0, ((size_t)Pd + 1) * sizeof(uint32_t), s));
                 tree_key_kernel<<<blocks_for(n, 256), 256, 0, s>>>(bd, ci_cube, tv.dmax, dkeys.as<uint32_t>(), dhist.as<uint32_t>());
@@ -1387,20 +1254,12 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
                     Region rg(ctx, F_COUNT, (red ? 2 : 0) + (score_roots ? 1 : 0));
                     if (red) {
                         for (size_t i = i0; i < i1; i++) CK(cudaMemsetAsync(bufP + big[i].table_off, 0, big[i].cells * sizeof(int), s));
-                        int64_t Rr = std::max<int64_t>(1, (int64_t)(ctx->sm_count * 8 + B - 1) / (int64_t)B);
-                        int64_t rps = (bd.n + Rr - 1) / Rr;
-                        rps = std::max<int64_t>((rps + 15) / 16 * 16, 16 * threads);
-                        Rr = (bd.n + rps - 1) / rps;
-                        bic_count_global_kernel<<<dim3((unsigned)B, (unsigned)Rr), threads, 0, s>>>(bd, ci_cube, dgsets.as<GlobalSet>() + i0, bufP, rps);
+                        launch_count_global(ctx, bd, MaskSets{ci_cube}, dgsets.as<GlobalSet>() + i0, B, bufP);
                     }
                     if (score_roots) {
                         uint32_t maxc = 0;
                         for (size_t i = i0; i < i1; i++) maxc = std::max(maxc, big[i].cells);
-                        const int64_t nconf = maxc / rv;
-                        const int64_t chunks = std::max<int64_t>(1, std::min<int64_t>((nconf + threads * 4 - 1) / (threads * 4), (ctx->sm_count * 8 + (int64_t)B - 1) / (int64_t)B));
-                        const int64_t cpc = (nconf + chunks - 1) / chunks;
-                        bic_score_tables_kernel<<<dim3((unsigned)B, (unsigned)chunks), threads, 0, s>>>(bd, ci_cube, dgsets.as<GlobalSet>() + i0, bufP,
-                                                                                                    dacc_big.as<long long>() + i0, cpc);
+                        launch_score_tables(ctx, bd, rv, dgsets.as<GlobalSet>() + i0, B, maxc, bufP, dacc_big.as<long long>() + i0);
                     }
                 }
                 i0 = i1;
@@ -1423,14 +1282,8 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
     // ---- derived layers ----
     // Pairs are emitted grouped by PARENT: blocks are dispatched in launch order, so the children of one parent run
     // back to back and all but the first read the parent table from L2 (126 MB) instead of HBM.
-    // LEAF FUSION: a set S without cube bit 0 has no children; its table is the marginal of P = S + {0} over the least
-    // significant digit, i.e. the sum of r0 ADJACENT configurations of P.  The pair that produces P therefore scores S
-    // in the same pass (CubePair::leaf_acc) and S gets no pair of its own: half of all sets never cost a table pass.
     std::vector<CubePair> hp;
     DevBuf dcmap(ctx);
-    const int r0 = (int)ccard[0];
-    const bool fuse_leaves = ctx->fuse_leaves && r0 >= 2 && r0 <= 4 && rv >= 2 && rv <= 4;
-    std::vector<char> by_pair_prev; // layer l+1: table produced by a derive pair of the previous iteration (its leaf child was scored there)
     for (int l = Lstar - 1; l >= 0; l--) {
         auto &L = layers[l];
         auto &P = layers[l + 1];
@@ -1438,18 +1291,10 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         if (l == Lstar - 1)
             for (size_t i = 0; i < P.size(); i++) if (!fused_root[i] && mine[l + 1][i]) ctx->st.k1_bytes_written += 4.0 * (double)P[i].cells; // root tables that were written
         const bool top = l == Lstar - 1 && fused_any; // children of fused roots were produced by the root kernel
-        // the leaf child of every set of THIS layer (in layer l-1), scored by the pair that produces the set
-        std::vector<uint32_t> leaf_child(L.size(), kNoLeafAcc);
-        if (fuse_leaves && l >= 1 && l - 1 <= Kc) {
-            auto &C = layers[l - 1];
-            for (size_t i = 0; i < C.size(); i++)
-                if ((C[i].cube_mask & 1u) == 0 && mine[l - 1][i]) leaf_child[C[i].parent] = (uint32_t)i; // parent = C[i] + {0}: parent links exist (l-1 < Lstar)
-        }
         std::vector<uint32_t> first(P.size() + 1, 0), order;
         auto skip = [&](const CubeSet &cs) {
             if (!mine[l + 1][cs.parent]) return true;   // outside this call's sub-forest
-            if (top && fused_root[cs.parent]) return true;
-            return (cs.cube_mask & 1u) == 0 && !by_pair_prev.empty() && by_pair_prev[cs.parent] != 0; // scored while its parent was produced
+            return top && fused_root[cs.parent] != 0;
         };
         for (auto &cs : L) if (!skip(cs)) first[cs.parent + 1]++;
         for (size_t i = 0; i < P.size(); i++) first[i + 1] += first[i];
@@ -1458,7 +1303,6 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
             std::vector<uint32_t> pos(first.begin(), first.end() - 1);
             for (size_t i = 0; i < L.size(); i++) if (!skip(L[i])) order[pos[L[i].parent]++] = (uint32_t)i;
         }
-        std::vector<char> by_pair(L.size(), 0);
         hp.resize(order.size());
         uint64_t chunk = 0;
         for (size_t k = 0; k < order.size(); k++) {
@@ -1469,20 +1313,13 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
             pr.Bc = cs.Bc; pr.r = cs.r; pr.chunk0 = (uint32_t)chunk;
             pr.acc_index = (uint32_t)(acc_off[l] + order[k]);
             pr.leaf = (cs.cube_mask & 1u) == 0; // lowest missing bit is 0: nothing is derived from this set
-            pr.leaf_acc = kNoLeafAcc;
             pr.fmt = (P[cs.parent].t16 ? 1u : 0u) | (cs.t16 ? 2u : 0u);
             pr.magic = pr.Bc > 1 ? 0xFFFFFFFFu / pr.Bc : 0;
-            if (!pr.leaf && leaf_child[order[k]] != kNoLeafAcc) {
-                pr.leaf_acc = (uint32_t)(acc_off[l - 1] + leaf_child[order[k]]);
-                by_pair[order[k]] = 1;
-            }
             ctx->st.k1_bytes_read += (P[cs.parent].t16 ? 2.0 : 4.0) * (double)cs.cells * (double)cs.r;
             if (!pr.leaf) ctx->st.k1_bytes_written += (cs.t16 ? 2.0 : 4.0) * (double)cs.cells;
-            const uint32_t cpb = cube_configs_per_block(pr.leaf_acc != kNoLeafAcc ? (uint32_t)r0 : 1u);
-            chunk += (pr.child_configs + cpb - 1) / cpb;
+            chunk += (pr.child_configs + kCubeConfigsPerBlock - 1) / kCubeConfigsPerBlock;
             hp[k] = pr;
         }
-        by_pair_prev.swap(by_pair);
         if (chunk > 0x7fffffffull) return ctx->fail(URLGPU_ERR_LIMIT, "cube: too many blocks in one layer");
         const bool score = l <= Kc;
         { int rc_ = h2d_async(ctx, dpairs.p, hp.data(), hp.size() * sizeof(CubePair)); if (rc_) return rc_; }
@@ -1492,10 +1329,10 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
             const unsigned grid = (unsigned)chunk;
             cube_map_kernel<<<blocks_for(chunk, 256), 256, 0, s>>>(dpairs.as<CubePair>(), (int)hp.size(), grid, dcmap.as<uint32_t>());
             switch (rv) {
-            case 2: cube_derive_kernel<2><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, r0, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
-            case 3: cube_derive_kernel<3><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, r0, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
-            case 4: cube_derive_kernel<4><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, r0, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
-            default: cube_derive_kernel<0><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, r0, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
+            case 2: cube_derive_kernel<2><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
+            case 3: cube_derive_kernel<3><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
+            case 4: cube_derive_kernel<4><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
+            default: cube_derive_kernel<0><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
             }
         }
         if (score) { int rc = finalize_layer(l); if (rc) return rc; }
@@ -1514,252 +1351,6 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         ctx->st.algorithmic_bytes += bytes;
         ctx->st.sets_scored += cnt;
         if (parts > 1) *n_scored = cnt;
-    }
-    *used = true;
-    return URLGPU_OK;
-}
-
-static int bic_score_family_tree(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, float *d_table, long long *d_llfixed,
-                                 uint64_t *n_scored, bool *used, const RankSpace &om);
-
-// c <= 30 candidates: the mask-based K1 strategies; `om` says where a set's score goes (dense by mask, or rank space)
-static int bic_score_family(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, float *d_table, long long *d_llfixed,
-                            uint64_t *n_scored, const RankSpace &om, int *d_ovf = nullptr) {
-    if (ctx->ds_ess > 0.f) return bic_score_family_direct(ctx, variable, cand, K, d_table, d_llfixed, n_scored, om);   // BDeu: one table per set
-    if (ctx->bic_mode == 0) {
-        bool used = false;
-        int rc = bic_score_family_tree(ctx, variable, cand, K, d_table, d_llfixed, n_scored, &used, om);
-        if (rc || used) return rc;
-    }
-    if (ctx->bic_mode != 1) {
-        bool used = false;
-        int rc = bic_score_family_cube(ctx, variable, cand, K, d_table, d_llfixed, n_scored, &used, om, 0, 1, d_ovf);
-        if (rc || used) return rc;
-    }
-    return bic_score_family_direct(ctx, variable, cand, K, d_table, d_llfixed, n_scored, om);
-}
-
-
-// ------------------------------------------------------------------------------------------------------------
-// Tree path (tree_kernels.cuh): every contingency table is counted or marginalised in shared memory; nothing but
-// the bucketed packed rows (L2 resident) and the per-set accumulators is read from or written to device memory.
-// Returns with *used = false (nothing launched) when the family cannot be laid out this way: packed row wider
-// than 64 bits, first candidate's arity too large for a run, or a root table that cannot be cut into slices
-// that fit the shared-memory budget.  The caller then takes the cube path.
-// ------------------------------------------------------------------------------------------------------------
-template <int RV>
-static void launch_tree(const TreeVar &tv, const TreeRoot *roots, const uint32_t *map, const long long *qlog, const long long *qcfg, int cfg_min, long long *acc, uint32_t budget, unsigned grid,
-                        size_t smem, cudaStream_t s) {
-    bic_tree_kernel<RV><<<grid, kTreeThreads, smem, s>>>(tv, roots, map, qlog, qcfg, cfg_min, acc, budget, budget);
-}
-
-static int bic_score_family_tree(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, float *d_table, long long *d_llfixed,
-                                 uint64_t *n_scored, bool *used, const RankSpace &om) {
-    *used = false;
-    cudaStream_t s = ctx->stream;
-    const int c = (int)cand.size();
-    if (c == 0) return URLGPU_OK;
-    static const bool dbg = getenv("URLGPU_DEBUG_TIMING") != nullptr;
-    const auto T0 = std::chrono::steady_clock::now();
-    const int Kc = std::min(K, c);
-    const int rv = ctx->card[variable];
-    const uint64_t n = (uint64_t)ctx->n;
-    std::vector<int> perm(c);
-    for (int i = 0; i < c; i++) perm[i] = i;
-    std::stable_sort(perm.begin(), perm.end(), [&](int a, int b) { return ctx->card[cand[a]] < ctx->card[cand[b]]; });
-    std::vector<int> cube_vars(c);
-    std::vector<uint64_t> ccard(c);
-    for (int i = 0; i < c; i++) { cube_vars[i] = cand[perm[i]]; ccard[i] = (uint64_t)ctx->card[cube_vars[i]]; }
-    // ---- packed row layout: uniform field width by the largest arity ----
-    TreeVar tv{};
-    tv.c = c; tv.rv = rv; tv.max_parents = K;
-    {
-        uint64_t maxr = (uint64_t)rv;
-        for (int i = 0; i < c; i++) maxr = std::max(maxr, ccard[i]);
-        tv.w = maxr <= 4 ? 2 : maxr <= 16 ? 4 : 8;
-        if ((c + 1) * tv.w > 64) return URLGPU_OK;
-        for (int i = 0; i < c; i++) tv.card[i] = (uint16_t)ccard[i];
-    }
-    // ---- run limit t: the lowest t digits are the ones summed out on chip ----
-    const uint32_t B = ctx->tree_budget;                      // cells of the slice table; the warps' stacks get the same
-    int t = 0;
-    {
-        uint64_t R = 1;
-        while (t < c && t < ctx->tree_run && (uint64_t)rv * R * ccard[t] <= ctx->tree_unit_cap) { R *= ccard[t]; t++; }
-    }
-    if (t == 0) return URLGPU_OK;
-    tv.t = t;
-    tv.pre[0] = 1;
-    for (int b = 0; b < t; b++) tv.pre[b + 1] = tv.pre[b] * (uint32_t)ccard[b];
-    for (int b = 0; b <= t; b++) tv.magic[b] = tv.pre[b] > 1 ? 0xFFFFFFFFu / tv.pre[b] : 0;
-    const int Lstar = std::min(Kc + 1, c);
-    // ---- bucketed zone: top digits (all above the run) whose joint arity stays <= kTreeMaxBuckets ----
-    int dmax = 0;
-    uint64_t Pd = 1;
-    while (c - 1 - dmax >= t && dmax < kTreeMaxZone && Pd * ccard[c - 1 - dmax] <= kTreeMaxBuckets) { Pd *= ccard[c - 1 - dmax]; dmax++; }
-    tv.dmax = dmax; tv.P_dmax = (uint32_t)Pd;
-    // per-unit stack need (cells) for a run of z digits
-    auto stack_unit = [&](int z) {
-        uint32_t tot = 0;
-        const uint32_t U0 = (uint32_t)rv * tv.pre[z];
-        for (int d = 1; d <= z; d++) tot += (U0 / tv.pre[d] + 3u) & ~3u;
-        return tot;
-    };
-    // ---- roots ----
-    std::vector<TreeRoot> roots;
-    uint64_t covered = 0;
-    bool ok = true;
-    auto binom = [](int a, int b) { if (b < 0 || b > a) return (uint64_t)0; uint64_t r = 1; for (int i = 0; i < b; i++) r = r * (uint64_t)(a - i) / (uint64_t)(i + 1); return r; };
-    auto add_root = [&](uint32_t A, int z) {
-        const int size = __builtin_popcount(A);
-        for (int j = 0; j <= z; j++) if (size - j <= K) covered += binom(z, j);
-        const uint32_t U0 = (uint32_t)rv * tv.pre[z];
-        const uint32_t su = stack_unit(z);
-        uint64_t H = 1;
-        for (int b = z; b < c; b++) if ((A >> b) & 1) { H *= ccard[b]; if (H > ((uint64_t)1 << 40)) H = (uint64_t)1 << 40; }
-        int depth = 0;
-        uint64_t nslices = 1, nseg = 1;
-        if ((uint64_t)kTreeWarps * su > B) { ok = false; return; } // every warp needs stack space for at least one unit
-        const uint64_t max_seg = (uint64_t)1 << 22;                  // beyond (B-1)/2 - 1 segments the kernel takes its fragmented-slice loop
-        auto fits = [&](uint64_t h) { return (uint64_t)U0 * h <= B; };
-        while (!fits(H)) {
-            if (depth == dmax) { ok = false; return; }
-            const int b = c - 1 - depth;
-            depth++;
-            if ((A >> b) & 1) { H /= ccard[b]; nslices *= ccard[b]; } else nseg *= ccard[b];
-            if (nseg > max_seg) { ok = false; return; }
-        }
-        if (U0 > B || (uint64_t)U0 * H > 65535) { ok = false; return; }
-        // optional deeper cut: keep the rows of one CTA below ~32k so single CTAs do not become the tail
-        while (n / nslices > 32768 && depth < dmax) {
-            int d2 = depth;
-            uint64_t seg2 = nseg;
-            while (d2 < dmax && !((A >> (c - 1 - d2)) & 1)) { seg2 *= ccard[c - 1 - d2]; d2++; }
-            if (d2 == dmax || seg2 > 256) break;
-            const int b = c - 1 - d2;
-            H /= ccard[b]; nslices *= ccard[b]; nseg = seg2; depth = d2 + 1;
-        }
-        if (nslices > 0x3fffffffull) { ok = false; return; }
-        TreeRoot r{};
-        r.mask = A; r.nslices = (uint32_t)nslices; r.H = (uint32_t)H; r.nseg = (uint32_t)nseg;
-        r.z = (uint8_t)z; r.size = (uint8_t)size;
-        // in-slice columns: child, run digits, present digits between the run and the zone (strides < S0 <= 65535)
-        r.fstride[0] = 1;
-        for (int b = 0; b < z; b++) r.fstride[b + 1] = (uint16_t)((uint32_t)rv * tv.pre[b]);
-        uint32_t hs = U0;
-        for (int b = z; b < c - depth; b++)
-            if ((A >> b) & 1) { r.fstride[b + 1] = (uint16_t)hs; hs *= (uint32_t)ccard[b]; }
-        for (int f = 0; f <= c; f++)
-            if (r.fstride[f]) r.gmask |= (uint8_t)(1u << (f * tv.w / 8));
-        for (int g = 0; g < 8; g++) if ((r.gmask >> g) & 1) r.glist[r.ng++] = (uint8_t)g;
-        uint64_t w = 1;
-        for (int b = c - depth; b < c; b++) {
-            const uint32_t mg = ccard[b] > 1 ? (uint32_t)(0xFFFFFFFFull / ccard[b]) : 0;
-            if ((A >> b) & 1) { r.pres_card[r.npres] = (uint16_t)ccard[b]; r.pres_weight[r.npres] = (uint32_t)w; r.pres_magic[r.npres] = mg; r.npres++; }
-            else { r.abs_card[r.nabs] = (uint16_t)ccard[b]; r.abs_weight[r.nabs] = (uint32_t)w; r.abs_magic[r.nabs] = mg; r.nabs++; }
-            w *= ccard[b];
-        }
-        r.q_stride = (uint32_t)(Pd / w);
-        roots.push_back(r);
-    };
-    auto for_each_subset = [&](int bits, int pick, auto &&fn) { // all `pick`-subsets of `bits` positions, increasing
-        if (pick < 0 || pick > bits) return;
-        if (pick == 0) { fn(0u); return; }
-        uint32_t v = (1u << pick) - 1;
-        const uint64_t lim = (uint64_t)1 << bits;
-        while ((uint64_t)v < lim) {
-            fn(v);
-            if (pick == bits) break;
-            v = gosper_next(v);
-        }
-    };
-    const uint32_t low_t = (1u << t) - 1;
-    for (int i = 0; i <= c - t && t + i <= Lstar && ok; i++)      // (1) sets containing all t low bits
-        for_each_subset(c - t, i, [&](uint32_t hm) { if (ok) add_root(low_t | (hm << t), t); });
-    for (int z = 1; z < t && ok; z++)                              // (2) layer-L* sets whose lowest missing bit is z < t
-        for_each_subset(c - z - 1, Lstar - z, [&](uint32_t hm) { if (ok) add_root(((1u << z) - 1) | (hm << (z + 1)), z); });
-    if (!ok) return URLGPU_OK;
-    if (covered != family_size(c, K)) return ctx->fail(URLGPU_ERR_INTERNAL, "tree: the roots do not cover the family exactly once");
-    // heavy CTAs (few slices = many rows each) first
-    std::stable_sort(roots.begin(), roots.end(), [](const TreeRoot &a, const TreeRoot &b) { return a.nslices < b.nslices; });
-    uint64_t chunk = 0, acc_total = 0;
-    for (auto &r : roots) { r.chunk0 = (uint32_t)chunk; r.acc_off = (uint32_t)acc_total; chunk += r.nslices; acc_total += (uint64_t)1 << r.z; }
-    if (chunk > 0x7fffffffull || acc_total > 0x7fffffffull) return URLGPU_OK;
-    // ---- device side ----
-    { int rc_ = stage_begin(ctx); if (rc_) return rc_; }
-    CandInfo ci_cube = make_candinfo(ctx, variable, cube_vars, K);
-    CandInfo ci_res = make_candinfo(ctx, variable, cand, K);
-    BicData bd{ctx->d_codes, ctx->n, ctx->n_stride, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, ctx->ds_base, ctx->ds_ess, ctx->ds_scale};
-    DevBuf dkeys(ctx), dhist(ctx), doff(ctx), dcursor(ctx), drows(ctx), droots(ctx), dmap(ctx), dacc(ctx), dperm(ctx), dtmp(ctx);
-    CK(dkeys.alloc(n * sizeof(uint32_t)));
-    CK(dhist.alloc(((size_t)Pd + 1) * sizeof(uint32_t)));
-    CK(doff.alloc(((size_t)Pd + 1) * sizeof(uint32_t)));
-    CK(dcursor.alloc(((size_t)Pd + 1) * sizeof(uint32_t)));
-    CK(drows.alloc(n * sizeof(unsigned long long)));
-    CK(droots.alloc(roots.size() * sizeof(TreeRoot)));
-    CK(dmap.alloc(chunk * sizeof(uint32_t)));
-    CK(dacc.alloc(acc_total * sizeof(long long)));
-    CK(dperm.alloc(kMaxDenseCand));
-    uint8_t hperm[kMaxDenseCand] = {0};
-    for (int i = 0; i < c; i++) hperm[i] = (uint8_t)perm[i];
-    std::vector<uint16_t> cfgtab((size_t)(t + 1) << t, 0);
-    for (int z = 0; z <= t; z++)
-        for (uint32_t D = 0; D < (1u << z); D++) {
-            uint32_t v = tv.pre[z];
-            for (int i = 0; i < z; i++) if ((D >> i) & 1) v /= (uint32_t)ccard[i];
-            cfgtab[((size_t)z << t) + D] = (uint16_t)v;
-        }
-    DevBuf dcfg(ctx);
-    CK(dcfg.alloc(cfgtab.size() * sizeof(uint16_t)));
-    { int rc_ = h2d_async(ctx, dcfg.p, cfgtab.data(), cfgtab.size() * sizeof(uint16_t)); if (rc_) return rc_; }
-    tv.cfg_tab = dcfg.as<uint16_t>();
-    { int rc_ = h2d_async(ctx, droots.p, roots.data(), roots.size() * sizeof(TreeRoot)); if (rc_) return rc_; }
-    { int rc_ = h2d_async(ctx, dperm.p, hperm, kMaxDenseCand); if (rc_) return rc_; }
-    tv.rows = drows.as<unsigned long long>();
-    tv.prefix_off = doff.as<uint32_t>();
-    {
-        Region rg(ctx, F_COUNT, 5);
-        CK(cudaMemsetAsync(dhist.p, 0, ((size_t)Pd + 1) * sizeof(uint32_t), s));
-        tree_key_kernel<<<blocks_for(n, 256), 256, 0, s>>>(bd, ci_cube, dmax, dkeys.as<uint32_t>(), dhist.as<uint32_t>());
-        {
-            const uint32_t nscan = (uint32_t)(Pd + 1), ntiles = (nscan + kScanTile - 1) / kScanTile;
-            CK(dtmp.alloc(1024 * sizeof(uint32_t)));
-            bucket_scan_sums_kernel<<<ntiles, kScanThreads, 0, s>>>(dhist.as<uint32_t>(), nscan, dtmp.as<uint32_t>());
-            bucket_scan_tiles_kernel<<<1, 1024, 0, s>>>(dtmp.as<uint32_t>(), ntiles);
-            bucket_scan_final_kernel<<<ntiles, kScanThreads, 0, s>>>(dhist.as<uint32_t>(), nscan, dtmp.as<uint32_t>(), doff.as<uint32_t>());
-        }
-        CK(cudaMemcpyAsync(dcursor.p, doff.p, ((size_t)Pd + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, s));
-        tree_scatter_kernel<<<blocks_for(n, 256), 256, 0, s>>>(bd, ci_cube, tv, dkeys.as<uint32_t>(), dcursor.as<uint32_t>(), drows.as<unsigned long long>());
-        tree_map_kernel<<<blocks_for(chunk, 256), 256, 0, s>>>(droots.as<TreeRoot>(), (int)roots.size(), (uint32_t)chunk, dmap.as<uint32_t>());
-        CK(cudaMemsetAsync(dacc.p, 0, acc_total * sizeof(long long), s));
-    }
-    {
-        Region rg(ctx, F_TREE, 1);
-        const size_t smem = (size_t)2 * B * sizeof(int);
-        const unsigned grid = (unsigned)chunk;
-        switch (rv) {
-        case 2: launch_tree<2>(tv, droots.as<TreeRoot>(), dmap.as<uint32_t>(), ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), B, grid, smem, s); break;
-        case 3: launch_tree<3>(tv, droots.as<TreeRoot>(), dmap.as<uint32_t>(), ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), B, grid, smem, s); break;
-        case 4: launch_tree<4>(tv, droots.as<TreeRoot>(), dmap.as<uint32_t>(), ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), B, grid, smem, s); break;
-        default: launch_tree<0>(tv, droots.as<TreeRoot>(), dmap.as<uint32_t>(), ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), B, grid, smem, s); break;
-        }
-    }
-    {
-        Region rg(ctx, F_OTHER, 1);
-        tree_finalize_kernel<<<blocks_for(acc_total, 256), 256, 0, s>>>(bd, ci_res, droots.as<TreeRoot>(), (int)roots.size(), dperm.as<uint8_t>(), dacc.as<long long>(),
-                                                                     (uint32_t)acc_total, d_table, d_llfixed, om);
-    }
-    CK(cudaGetLastError());
-    { int rc_ = stage_end(ctx); if (rc_) return rc_; }
-    if (dbg) fprintf(stderr, "[urlgpu tree] v=%d c=%d K=%d L*=%d t=%d dmax=%d buckets=%llu roots=%zu CTAs=%llu host %.2f ms\n", variable, c, K, Lstar, t, dmax,
-                     (unsigned long long)Pd, roots.size(), (unsigned long long)chunk,
-                     std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - T0).count());
-    *n_scored = family_size(c, K);
-    {
-        double bytes = 0, b = 1;
-        for (int l = 0; l <= K && l <= c; l++) { bytes += b * (double)ctx->n * (l + 1); b = b * (c - l) / (l + 1); }
-        ctx->st.algorithmic_bytes += bytes;
-        ctx->st.sets_scored += *n_scored;
     }
     *used = true;
     return URLGPU_OK;
@@ -1959,19 +1550,6 @@ static int make_rank_space(urlgpu_ctx *ctx, int c, int K, RankSpace &rs) {
     return ensure_binom(ctx, K, &rs.binom);
 }
 
-// host-side unrank (planning of the global BIC tier)
-static void host_unrank(int c, int l, uint32_t r, int *e) {
-    int hi = c - 1;
-    for (int i = l; i >= 1; i--) {
-        int b = hi;
-        while (b >= i && binom_sat(b, i) > r) b--;
-        if (b < i) b = i - 1;
-        e[i - 1] = b;
-        r -= binom_sat(b, i);
-        hi = b - 1;
-    }
-}
-
 // ---- K3 in rank space: per-set Schur sweeps, one launch per layer, entries [first, first + count) of the index space
 static int cbic_score_rank(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, const RankSpace &rs, double lambda, uint32_t first, uint32_t count,
                            float *d_scores /*indexed by global index*/, double *d_ts64) {
@@ -2040,105 +1618,114 @@ static int cbic_score_rank(urlgpu_ctx *ctx, int variable, const std::vector<int>
     return URLGPU_OK;
 }
 
-// ---- K1 in rank space for families the mask-based strategies cannot hold (more than 30 candidates): every set of
-// [first, first + count) is counted from the rows, in three tiers by table size like bic_score_family_direct
-static int bic_score_rank_direct(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, const RankSpace &rs, uint32_t first, uint32_t count, float *d_scores) {
+// ---- K1 by direct counting: every set of [first, first + count) of the rank space is counted from the rows.  The sets
+// are named by their index (RankSets); a score goes to its index, or to its compact mask when by_mask (dense layout).
+// Sets are classified by table size: two shared-memory tiers (one CTA per set) and the global tier below.
+
+// The global tier: tables in an L2-resident scratch batch, RED atomics.  Scores (and, optionally, the fixed-point
+// log-likelihoods) go to d_scores at each set's output index; counts_out, if given, receives the table of sets[0].
+static int direct_global_tier(urlgpu_ctx *ctx, const BicData &bd, const RankSets &fam, std::vector<GlobalSet> &sets, float *d_scores,
+                              long long *d_llfixed, int32_t *counts_out, int64_t n_cells) {
     cudaStream_t s = ctx->stream;
-    const int c = rs.c;
+    size_t max_cells = 0;
+    for (auto &g : sets) max_cells = std::max<size_t>(max_cells, g.cells);
+    int rc = ensure_tables(ctx, std::max(kBatchTableElems, max_cells));
+    if (rc) return rc;
+    std::vector<std::pair<size_t, size_t>> batches;
+    for (size_t i0 = 0; i0 < sets.size();) {
+        size_t used = 0, i1 = i0;
+        while (i1 < sets.size() && (i1 == i0 || used + sets[i1].cells <= ctx->tables_cap) && i1 - i0 < 65535) {
+            sets[i1].table_off = used;
+            used += (sets[i1].cells + 3) / 4 * 4;
+            i1++;
+        }
+        batches.push_back({i0, i1});
+        i0 = i1;
+    }
+    DevBuf dsets(ctx), dacc(ctx);
+    CK(dsets.alloc(sets.size() * sizeof(GlobalSet)));
+    CK(dacc.alloc(sets.size() * sizeof(long long)));
+    CK(cudaMemsetAsync(dacc.p, 0, sets.size() * sizeof(long long), s));
+    CK(cudaMemcpyAsync(dsets.p, sets.data(), sets.size() * sizeof(GlobalSet), cudaMemcpyHostToDevice, s));
+    for (auto &bt : batches) {
+        const size_t B = bt.second - bt.first;
+        const size_t used = sets[bt.second - 1].table_off + sets[bt.second - 1].cells;
+        uint32_t maxc = 0;
+        for (size_t i = bt.first; i < bt.second; i++) maxc = std::max(maxc, sets[i].cells);
+        Region rg(ctx, F_COUNT, 3);
+        CK(cudaMemsetAsync(ctx->d_tables, 0, used * sizeof(int), s));
+        launch_count_global(ctx, bd, fam, dsets.as<GlobalSet>() + bt.first, B, ctx->d_tables);
+        launch_score_tables(ctx, bd, fam.rc.rv, dsets.as<GlobalSet>() + bt.first, B, maxc, ctx->d_tables, dacc.as<long long>() + bt.first);
+        if (counts_out && bt.first == 0) {
+            CK(cudaMemcpyAsync(counts_out, ctx->d_tables, (size_t)n_cells * sizeof(int), cudaMemcpyDeviceToHost, s));
+            CK(cudaStreamSynchronize(s));
+        }
+    }
+    if (d_scores) {
+        Region rg(ctx, F_OTHER, 1);
+        bic_finalize_kernel<<<blocks_for(sets.size(), 256), 256, 0, s>>>(bd, fam, dsets.as<GlobalSet>(), dacc.as<long long>(), (int)sets.size(), d_scores, d_llfixed);
+    }
+    CK(cudaStreamSynchronize(s)); // dsets/dacc are freed on return
+    CK(cudaGetLastError());
+    return URLGPU_OK;
+}
+
+// the candidates' variables and arities on the device (dcand, uploaded from hv, which the caller keeps until its stream has
+// been synchronised), and the key space of the direct-counting kernels over them
+static int make_rank_sets(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, const RankSpace &rs, bool by_mask, std::vector<int> &hv, DevBuf &dcand,
+                          RankSets &fam) {
+    const int c = (int)cand.size();
+    hv.assign(2 * (size_t)std::max(c, 1), 0);
+    for (int i = 0; i < c; i++) { hv[i] = cand[i]; hv[c + i] = ctx->card[cand[i]]; }
+    CK(dcand.alloc(hv.size() * sizeof(int)));
+    CK(cudaMemcpyAsync(dcand.p, hv.data(), hv.size() * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    fam = RankSets{rs, RankCand{variable, ctx->card[variable], dcand.as<int>(), dcand.as<int>() + c}, by_mask ? 1 : 0};
+    return URLGPU_OK;
+}
+
+static int bic_score_direct(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, const RankSpace &rs, uint32_t first, uint32_t count, float *d_scores,
+                            bool by_mask) {
+    cudaStream_t s = ctx->stream;
     if (rs.K + 1 > kMaxCols) return ctx->fail(URLGPU_ERR_LIMIT, "BIC: more than 31 parents in one set");
     BicData bd{ctx->d_codes, ctx->n, ctx->n_stride, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, ctx->ds_base, ctx->ds_ess, ctx->ds_scale};
     const uint32_t tier1_cells = (uint32_t)((ctx->smem_optin - 2048) / sizeof(int));
-    std::vector<int> hv(2 * (size_t)std::max(c, 1));
-    for (int i = 0; i < c; i++) { hv[i] = cand[i]; hv[c + i] = ctx->card[cand[i]]; }
+    std::vector<int> hv;
     DevBuf dcand(ctx), lists(ctx), counters(ctx);
-    CK(dcand.alloc(hv.size() * sizeof(int)));
-    CK(lists.alloc(3 * (size_t)count * sizeof(uint32_t)));
+    RankSets fam{};
+    int rc = make_rank_sets(ctx, variable, cand, rs, by_mask, hv, dcand, fam);
+    if (rc) return rc;
+    CK(lists.alloc((size_t)count * (sizeof(GlobalSet) + 2 * sizeof(uint32_t))));
     CK(counters.alloc(4 * sizeof(unsigned long long)));
-    CK(cudaMemcpyAsync(dcand.p, hv.data(), hv.size() * sizeof(int), cudaMemcpyHostToDevice, s));
     CK(cudaMemsetAsync(counters.p, 0, 4 * sizeof(unsigned long long), s));
-    RankCand rc{variable, ctx->card[variable], dcand.as<int>(), dcand.as<int>() + c};
-    uint32_t *l0 = lists.as<uint32_t>(), *l1 = l0 + count, *l2 = l1 + count;
-    const size_t bsm = rs_binom_bytes(rs);
+    GlobalSet *l2 = lists.as<GlobalSet>();
+    uint32_t *l0 = reinterpret_cast<uint32_t *>(l2 + count), *l1 = l0 + count;
     {
         Region rg(ctx, F_OTHER, 1);
-        rank_bic_classify_kernel<<<blocks_for(count, 256), 256, bsm, s>>>(rs, rc, first, count, kTier0Cells, tier1_cells, kCellLimit, l0, l1, l2,
-                                                                          counters.as<unsigned long long>());
+        bic_classify_kernel<<<blocks_for(count, 256), 256, rs_binom_bytes(rs), s>>>(fam, first, count, kTier0Cells, tier1_cells, kCellLimit, l0, l1, l2,
+                                                                                    counters.as<unsigned long long>());
     }
     unsigned long long hc[4];
     CK(cudaMemcpyAsync(hc, counters.p, sizeof hc, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     if (hc[3]) return ctx->fail(URLGPU_ERR_LIMIT, "a contingency table of this family has more than 2^30 cells");
-    static bool attr_set = false;
-    if (!attr_set) { cudaFuncSetAttribute(rank_bic_count_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->smem_optin - 2048); attr_set = true; }
     if (hc[0]) {
         Region rg(ctx, F_COUNT, 1);
         const int threads = ctx->n >= 65536 ? 256 : 128;
-        rank_bic_count_smem_kernel<<<(unsigned)hc[0], threads, kTier0Cells * sizeof(int), s>>>(bd, rs, rc, l0, d_scores);
+        bic_count_smem_kernel<<<(unsigned)hc[0], threads, kTier0Cells * sizeof(int), s>>>(bd, fam, l0, d_scores, nullptr, nullptr, nullptr);
     }
     if (hc[1]) {
         Region rg(ctx, F_COUNT, 1);
-        rank_bic_count_smem_kernel<<<(unsigned)hc[1], 1024, (size_t)tier1_cells * sizeof(int), s>>>(bd, rs, rc, l1, d_scores);
+        bic_count_smem_kernel<<<(unsigned)hc[1], 1024, (size_t)tier1_cells * sizeof(int), s>>>(bd, fam, l1, d_scores, nullptr, nullptr, nullptr);
     }
-    if (hc[2]) { // tables in an L2-resident scratch batch, RED atomics
-        std::vector<uint32_t> m2(hc[2]);
-        CK(cudaMemcpyAsync(m2.data(), l2, hc[2] * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    if (hc[2]) {
+        std::vector<GlobalSet> sets(hc[2]);
+        CK(cudaMemcpyAsync(sets.data(), l2, hc[2] * sizeof(GlobalSet), cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
-        std::sort(m2.begin(), m2.end());
-        std::vector<RankGlobalSet> sets(m2.size());
-        size_t max_cells = 0;
-        for (size_t i = 0; i < m2.size(); i++) {
-            int l = 0;
-            while (l < rs.K && m2[i] >= rs.layer_base[l + 1]) l++;
-            int e[kMaxRankLayers];
-            host_unrank(c, l, m2[i] - rs.layer_base[l], e);
-            uint64_t cells = (uint64_t)rc.rv;
-            for (int j = 0; j < l; j++) cells *= (uint64_t)ctx->card[cand[e[j]]];
-            sets[i].idx = m2[i]; sets[i].cells = (uint32_t)cells; sets[i].table_off = 0;
-            max_cells = std::max<size_t>(max_cells, cells);
-        }
-        int rcode = ensure_tables(ctx, std::max(kBatchTableElems, max_cells));
-        if (rcode) return rcode;
-        DevBuf dsets(ctx), dacc(ctx);
-        CK(dsets.alloc(sets.size() * sizeof(RankGlobalSet)));
-        CK(dacc.alloc(sets.size() * sizeof(long long)));
-        CK(cudaMemsetAsync(dacc.p, 0, sets.size() * sizeof(long long), s));
-        std::vector<std::pair<size_t, size_t>> batches;
-        for (size_t i0 = 0; i0 < sets.size();) {
-            size_t used = 0, i1 = i0;
-            while (i1 < sets.size() && (i1 == i0 || used + sets[i1].cells <= ctx->tables_cap) && i1 - i0 < 65535) {
-                sets[i1].table_off = used;
-                used += (sets[i1].cells + 3) / 4 * 4;
-                i1++;
-            }
-            batches.push_back({i0, i1});
-            i0 = i1;
-        }
-        CK(cudaMemcpyAsync(dsets.p, sets.data(), sets.size() * sizeof(RankGlobalSet), cudaMemcpyHostToDevice, s));
-        const int threads = 256;
-        for (auto &bt : batches) {
-            const size_t B = bt.second - bt.first;
-            const size_t used = sets[bt.second - 1].table_off + sets[bt.second - 1].cells;
-            Region rg(ctx, F_COUNT, 3);
-            CK(cudaMemsetAsync(ctx->d_tables, 0, used * sizeof(int), s));
-            int64_t R = std::max<int64_t>(1, (int64_t)(ctx->sm_count * 8 + B - 1) / (int64_t)B);
-            int64_t rps = (bd.n + R - 1) / R;
-            rps = std::max<int64_t>((rps + 15) / 16 * 16, 16 * threads);
-            R = (bd.n + rps - 1) / rps;
-            rank_bic_count_global_kernel<<<dim3((unsigned)B, (unsigned)R), threads, 0, s>>>(bd, rs, rc, dsets.as<RankGlobalSet>() + bt.first, ctx->d_tables, rps);
-            uint32_t maxc = 0;
-            for (size_t i = bt.first; i < bt.second; i++) maxc = std::max(maxc, sets[i].cells);
-            const int64_t nconf = maxc / rc.rv;
-            const int64_t chunks = std::max<int64_t>(1, std::min<int64_t>((nconf + threads * 4 - 1) / (threads * 4), (ctx->sm_count * 8 + (int64_t)B - 1) / (int64_t)B));
-            const int64_t cpc = (nconf + chunks - 1) / chunks;
-            rank_bic_score_tables_kernel<<<dim3((unsigned)B, (unsigned)chunks), threads, 0, s>>>(bd, rc.rv, dsets.as<RankGlobalSet>() + bt.first, ctx->d_tables,
-                                                                                             dacc.as<long long>() + bt.first, cpc);
-        }
-        {
-            Region rg(ctx, F_OTHER, 1);
-            rank_bic_finalize_kernel<<<blocks_for(sets.size(), 256), 256, 0, s>>>(bd, rs, rc, dsets.as<RankGlobalSet>(), dacc.as<long long>(), (int)sets.size(), d_scores);
-        }
+        std::sort(sets.begin(), sets.end(), [](const GlobalSet &a, const GlobalSet &b) { return a.key < b.key; });
+        rc = direct_global_tier(ctx, bd, fam, sets, d_scores, nullptr, nullptr, 0);
+        if (rc) return rc;
     }
-    {
+    {   // algorithmic bytes: n*(k+1) per set (SURVEY.md §8d)
         double bytes = 0;
         const uint64_t last = (uint64_t)first + count;
         for (int l = 0; l <= rs.K; l++) {
@@ -2148,9 +1735,24 @@ static int bic_score_rank_direct(urlgpu_ctx *ctx, int variable, const std::vecto
         ctx->st.algorithmic_bytes += bytes;
         ctx->st.sets_scored += count;
     }
-    CK(cudaStreamSynchronize(s)); // dcand / lists are freed on return
+    CK(cudaStreamSynchronize(s)); // hv / dcand / lists / counters are freed on return
     CK(cudaGetLastError());
     return URLGPU_OK;
+}
+
+// K1 for a whole family: the cube path (c <= 30, BIC / fNML), else, or when the cube path cannot lay the family out, direct
+// counting of every set.  `om` says where a set's score goes: dense by compact mask (om.binom == nullptr), or rank space.
+static int bic_score_family(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, float *d_table, uint64_t *n_scored, const RankSpace &om,
+                            int *d_ovf = nullptr) {
+    if (ctx->ds_ess == 0.f && !ctx->bic_direct && (int)cand.size() <= kMaxDenseCand) {
+        bool used = false;
+        int rc = bic_score_family_cube(ctx, variable, cand, K, d_table, n_scored, &used, om, 0, 1, d_ovf);
+        if (rc || used) return rc;
+    }
+    RankSpace rs = om;
+    if (!om.binom) { int rc = make_rank_space(ctx, (int)cand.size(), K, rs); if (rc) return rc; }
+    *n_scored = rs.layer_base[rs.K + 1];
+    return bic_score_direct(ctx, variable, cand, rs, 0, (uint32_t)*n_scored, d_table, om.binom == nullptr);
 }
 
 // K4 (MODE 0) / K5 (MODE 1) in rank space: one launch per layer, ascending
@@ -2292,7 +1894,7 @@ extern "C" int urlgpu_score_variable(urlgpu_ctx *ctx, int variable, const uint64
     cudaStream_t s = ctx->stream;
     auto cleanup = [&](int code) { pool_free(ctx, res->d_table); if (res->d_ovf) pool_free(ctx, res->d_ovf); delete res; return code; };
     res->is_bic = bic; res->score_type = score_type; res->filter_flags = filter_flags;
-    if (bic && ctx->ds_ess == 0.f && ctx->table16 && c <= kMaxDenseCand && ctx->bic_mode == 2 && !ctx->t16_overflowed.count(variable)) {
+    if (bic && ctx->ds_ess == 0.f && ctx->table16 && c <= kMaxDenseCand && !ctx->bic_direct && !ctx->t16_overflowed.count(variable)) {
         e = pool_alloc(ctx, reinterpret_cast<void **>(&res->d_ovf), sizeof(int));
         if (e != cudaSuccess) return cleanup(ctx->cuda_fail(e, "cudaMalloc(flag)", __LINE__));
         cudaMemsetAsync(res->d_ovf, 0, sizeof(int), s);
@@ -2302,14 +1904,12 @@ extern "C" int urlgpu_score_variable(urlgpu_ctx *ctx, int variable, const uint64
         const uint32_t total = (uint32_t)res->n_masks;
         res->n_scored = total;
         if (bic) {
-            if (c <= kMaxDenseCand) { // the mask-based K1 strategies, writing by rank
-                fill_u32_kernel<<<blocks_for(total, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(res->d_table), total, kSentinelBits);
-                rc = bic_score_family(ctx, variable, cand, K, res->d_table, nullptr, &res->n_scored, res->rs, res->d_ovf);
-            } else rc = bic_score_rank_direct(ctx, variable, cand, res->rs, 0, total, res->d_table);
+            fill_u32_kernel<<<blocks_for(total, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(res->d_table), total, kSentinelBits);
+            rc = bic_score_family(ctx, variable, cand, K, res->d_table, &res->n_scored, res->rs, res->d_ovf);
         } else rc = cbic_score_rank(ctx, variable, cand, res->rs, lambda, 0, total, res->d_table, nullptr);
     } else {
         fill_u32_kernel<<<blocks_for(res->n_masks, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(res->d_table), res->n_masks, kSentinelBits);
-        if (bic) rc = bic_score_family(ctx, variable, cand, K, res->d_table, nullptr, &res->n_scored, RankSpace{}, res->d_ovf);
+        if (bic) rc = bic_score_family(ctx, variable, cand, K, res->d_table, &res->n_scored, RankSpace{}, res->d_ovf);
         else rc = cbic_score_family(ctx, variable, cand, K, lambda, res->d_table, nullptr, &res->n_scored);
     }
     if (rc) return cleanup(rc);
@@ -2361,7 +1961,7 @@ extern "C" int urlgpu_score_range(urlgpu_ctx *ctx, int variable, const uint64_t 
     if (!on_device) { CK(tmp.alloc(count * sizeof(float))); d_out = tmp.as<float>(); }
     // the kernels index by global family index: shift the base so that entry `first` lands on d_out[0]
     float *d_base = d_out - first;
-    if (bic) rc = bic_score_rank_direct(ctx, variable, cand, rs, (uint32_t)first, (uint32_t)count, d_base);
+    if (bic) rc = bic_score_direct(ctx, variable, cand, rs, (uint32_t)first, (uint32_t)count, d_base, false);
     else rc = cbic_score_rank(ctx, variable, cand, rs, lambda, (uint32_t)first, (uint32_t)count, d_base, nullptr);
     if (rc) return rc;
     if (!on_device) {
@@ -2392,11 +1992,11 @@ extern "C" int urlgpu_score_part(urlgpu_ctx *ctx, int variable, const uint64_t *
     if (!on_device) { CK(tmp.alloc((size_t)total * sizeof(float))); d_out = tmp.as<float>(); }
     fill_u32_kernel<<<blocks_for(total, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(d_out), total, kSentinelBits);
     bool done = false;
-    if (bic && ctx->ds_ess == 0.f && c <= kMaxDenseCand && ctx->bic_mode == 2) { // the cube path: part = a sub-forest of the root tables
+    if (bic && ctx->ds_ess == 0.f && c <= kMaxDenseCand && !ctx->bic_direct) { // the cube path: part = a sub-forest of the root tables
         uint64_t ns = 0;
         DevBuf flag(ctx);
         if (ctx->table16) { CK(flag.alloc(sizeof(int))); CK(cudaMemsetAsync(flag.p, 0, sizeof(int), s)); }
-        rc = bic_score_family_cube(ctx, variable, cand, K, d_out, nullptr, &ns, &done, rs, part, parts, flag.as<int>());
+        rc = bic_score_family_cube(ctx, variable, cand, K, d_out, &ns, &done, rs, part, parts, flag.as<int>());
         if (rc) return rc;
         if (done && flag.p) { // 16-bit tables are speculative: check now (this entry point hands raw scores out)
             int h = 0;
@@ -2405,7 +2005,7 @@ extern "C" int urlgpu_score_part(urlgpu_ctx *ctx, int variable, const uint64_t *
             if (h) {
                 ctx->st.table16_fallbacks++;
                 fill_u32_kernel<<<blocks_for(total, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(d_out), total, kSentinelBits);
-                rc = bic_score_family_cube(ctx, variable, cand, K, d_out, nullptr, &ns, &done, rs, part, parts, nullptr);
+                rc = bic_score_family_cube(ctx, variable, cand, K, d_out, &ns, &done, rs, part, parts, nullptr);
                 if (rc) return rc;
             }
         }
@@ -2413,7 +2013,7 @@ extern "C" int urlgpu_score_part(urlgpu_ctx *ctx, int variable, const uint64_t *
     if (!done) { // a contiguous range of the canonical numbering
         const uint64_t b0 = (uint64_t)total * part / parts, b1 = (uint64_t)total * (part + 1) / parts;
         if (b1 > b0) {
-            if (bic) rc = bic_score_rank_direct(ctx, variable, cand, rs, (uint32_t)b0, (uint32_t)(b1 - b0), d_out);
+            if (bic) rc = bic_score_direct(ctx, variable, cand, rs, (uint32_t)b0, (uint32_t)(b1 - b0), d_out, false);
             else rc = cbic_score_rank(ctx, variable, cand, rs, lambda, (uint32_t)b0, (uint32_t)(b1 - b0), d_out, nullptr);
             if (rc) return rc;
         }
@@ -2632,7 +2232,7 @@ static int result_wait_counts(urlgpu_result *res) {
         uint64_t ns = 0;
         rc = select_discrete_score(ctx, res->score_type, res->variable, 1.0);   // a later call may have selected another score / arity (never BDeu: no cube path)
         if (rc) return rc;
-        rc = bic_score_family(ctx, res->variable, res->cand, res->max_parents, res->d_table, nullptr, &ns, res->rank_layout ? res->rs : RankSpace{}, nullptr);
+        rc = bic_score_family(ctx, res->variable, res->cand, res->max_parents, res->d_table, &ns, res->rank_layout ? res->rs : RankSpace{}, nullptr);
         if (rc) return rc;
         rc = apply_filters(ctx, res, true, res->filter_flags);
         if (rc) return rc;
@@ -2913,6 +2513,21 @@ static int compact_of(urlgpu_ctx *ctx, int p, int variable, const uint64_t *pare
     return URLGPU_OK;
 }
 
+// the set of all `cand` as the one entry of a global tier (key space: the family of cand with no parent limit)
+static int single_set(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, std::vector<int> &hv, DevBuf &dcand, RankSets &fam,
+                      std::vector<GlobalSet> &one) {
+    const int c = (int)cand.size();
+    uint64_t cells = (uint64_t)ctx->card[variable];
+    for (int b = 0; b < c; b++) { cells *= (uint64_t)ctx->card[cand[b]]; if (cells > kCellLimit) return ctx->fail(URLGPU_ERR_LIMIT, "contingency table exceeds 2^30 cells"); }
+    RankSpace rs{};
+    int rc = make_rank_space(ctx, c, c, rs);
+    if (rc) return rc;
+    rc = make_rank_sets(ctx, variable, cand, rs, false, hv, dcand, fam);
+    if (rc) return rc;
+    one.assign(1, GlobalSet{rs.layer_base[c], (uint32_t)cells, 0});
+    return URLGPU_OK;
+}
+
 extern "C" int urlgpu_score_one(urlgpu_ctx *ctx, int variable, const uint64_t *parents, int mask_words, int score_type, double lambda, float *score,
                                 double *value64) {
     if (!ctx || !parents || !score) return ctx ? ctx->fail(URLGPU_ERR_ARG, "score_one: null argument") : URLGPU_ERR_ARG;
@@ -2933,18 +2548,19 @@ extern "C" int urlgpu_score_one(urlgpu_ctx *ctx, int variable, const uint64_t *p
     cudaStream_t s = ctx->stream;
     if (bic) {
         if (c > kMaxDenseCand) return ctx->fail(URLGPU_ERR_LIMIT, "score_one: more than 30 parents in one set");
-        const uint32_t full = (uint32_t)(((uint64_t)1 << c) - 1);
-        DevBuf out(ctx);
+        DevBuf out(ctx), dcand(ctx);
         CK(out.alloc(sizeof(float) + sizeof(long long) + 8));
-        BicData bd{ctx->d_codes, ctx->n, ctx->n_stride, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, ctx->ds_base, ctx->ds_ess, ctx->ds_scale};
-        CandInfo ci = make_candinfo(ctx, variable, cand, c);
-        uint64_t cells = ci.rv;
-        for (int b = 0; b < c; b++) { cells *= (uint64_t)ci.card[b]; if (cells > kCellLimit) return ctx->fail(URLGPU_ERR_LIMIT, "contingency table exceeds 2^30 cells"); }
-        std::vector<uint32_t> one(1, full);
-        // the kernels index their outputs by compact mask: shift the bases so that entry `full` is element 0
+        std::vector<int> hv;
+        RankSets fam{};
+        std::vector<GlobalSet> one;
+        rc = single_set(ctx, variable, cand, hv, dcand, fam, one);
+        if (rc) return rc;
+        // the kernels index their outputs by the set's index: shift the bases so that this set's entry is element 0
+        const uint32_t idx = one[0].key;
         long long *d_ll = out.as<long long>();
         float *d_sc = reinterpret_cast<float *>(d_ll + 1);
-        rc = bic_run_global_tier(ctx, bd, ci, one, d_sc - full, d_ll - full, nullptr, 0);
+        BicData bd{ctx->d_codes, ctx->n, ctx->n_stride, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, ctx->ds_base, ctx->ds_ess, ctx->ds_scale};
+        rc = direct_global_tier(ctx, bd, fam, one, d_sc - idx, d_ll - idx, nullptr, 0);
         if (rc) return rc;
         long long fx = 0;
         CK(cudaMemcpyAsync(score, d_sc, sizeof(float), cudaMemcpyDeviceToHost, s));
@@ -2995,13 +2611,15 @@ extern "C" int urlgpu_contingency(urlgpu_ctx *ctx, int variable, const uint64_t 
     if (rc) return rc;
     const int c = (int)cand.size();
     if (c > kMaxDenseCand) return ctx->fail(URLGPU_ERR_LIMIT, "contingency: more than 30 parents in one set");
+    std::vector<int> hv;
+    DevBuf dcand(ctx);
+    RankSets fam{};
+    std::vector<GlobalSet> one;
+    rc = single_set(ctx, variable, cand, hv, dcand, fam, one);
+    if (rc) return rc;
+    if ((int64_t)one[0].cells != n_cells) return ctx->fail(URLGPU_ERR_ARG, "contingency: n_cells must be r_v * prod r_pa = " + std::to_string(one[0].cells));
     BicData bd{ctx->d_codes, ctx->n, ctx->n_stride, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, ctx->ds_base, ctx->ds_ess, ctx->ds_scale};
-    CandInfo ci = make_candinfo(ctx, variable, cand, c);
-    uint64_t cells = ci.rv;
-    for (int b = 0; b < c; b++) { cells *= (uint64_t)ci.card[b]; if (cells > kCellLimit) return ctx->fail(URLGPU_ERR_LIMIT, "contingency table exceeds 2^30 cells"); }
-    if ((int64_t)cells != n_cells) return ctx->fail(URLGPU_ERR_ARG, "contingency: n_cells must be r_v * prod r_pa = " + std::to_string(cells));
-    std::vector<uint32_t> one(1, (uint32_t)(((uint64_t)1 << c) - 1));
-    return bic_run_global_tier(ctx, bd, ci, one, nullptr, nullptr, counts, n_cells);
+    return direct_global_tier(ctx, bd, fam, one, nullptr, nullptr, counts, n_cells);
 }
 
 extern "C" int urlgpu_prune(urlgpu_ctx *ctx, const uint64_t *masks, const float *scores, uint64_t n, int mask_words, uint8_t *keep) {
