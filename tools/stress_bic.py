@@ -1,5 +1,5 @@
 """randomised parity sweep of the BIC / fNML path against the oracle (development aid): random shapes, arities (incl. arity-1
-columns), skeletons, parent limits, all K1 modes and root-kernel budgets; prints the first mismatch and exits non-zero"""
+columns), skeletons, parent limits, all K1 modes and root-kernel budgets, warps, segment caps and the slice switch; prints the first mismatch and exits non-zero"""
 import importlib, os, sys, time
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,7 +14,10 @@ cases = 0
 while time.time() < t_end:
     mode = str(rng.choice(["cube", "cube", "direct"]))
     env = {"URLGPU_BIC_MODE": mode, "URLGPU_FUSE_ROOTS": str(rng.integers(0, 2)),
-           "URLGPU_ROOT_BUDGET": str(int(rng.choice([1024, 4096, 24576, 40000])))}
+           "URLGPU_ROOT_BUDGET": str(int(rng.choice([1024, 4096, 24576, 40000]))),
+           "URLGPU_ROOT_WARPS": str(int(rng.choice([8, 12, 16]))),
+           "URLGPU_ROOT_SEGS": str(int(rng.choice([32, 256, 1024, 8192]))),
+           "URLGPU_SLICE_COUNT": str(int(rng.random() < 0.85))}
     os.environ.update(env)
     eng = pkg.Engine(0)
     p = int(rng.integers(3, 15))

@@ -340,20 +340,50 @@ extern "C" int urlgpu_create(urlgpu_ctx **out, int device_id) {
     if (const char *m = getenv("URLGPU_ROOT_BUDGET")) ctx->root_budget = (uint32_t)std::max(1024, std::min(atoi(m), 48 * 1024)) / 4 * 4;
     if (const char *m = getenv("URLGPU_ROOT_SEGS")) ctx->root_seg_cap = (uint32_t)std::max(32, std::min(atoi(m), 8192));
     if (const char *m = getenv("URLGPU_ROOT_WARPS")) ctx->root_warps = atoi(m) == 8 ? 8 : atoi(m) == 12 ? 12 : 16;
-    {
-        const int smem = (int)((ctx->root_budget + 2 * ctx->root_seg_cap + 1) * sizeof(int));
-#define URLGPU_ROOT_ATTR(RVV, NWW) cudaFuncSetAttribute(bic_root_kernel<RVV, NWW>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)
-        URLGPU_ROOT_ATTR(0, 8); URLGPU_ROOT_ATTR(2, 8); URLGPU_ROOT_ATTR(3, 8); URLGPU_ROOT_ATTR(4, 8);
-        URLGPU_ROOT_ATTR(0, 12); URLGPU_ROOT_ATTR(2, 12); URLGPU_ROOT_ATTR(3, 12); URLGPU_ROOT_ATTR(4, 12);
-        URLGPU_ROOT_ATTR(0, 16); URLGPU_ROOT_ATTR(2, 16); URLGPU_ROOT_ATTR(3, 16); URLGPU_ROOT_ATTR(4, 16);
-#undef URLGPU_ROOT_ATTR
-    }
     if (const char *m = getenv("URLGPU_LAYOUT")) ctx->layout_policy = strcmp(m, "dense") == 0 ? 1 : strcmp(m, "rank") == 0 ? 2 : 0;
     if (const char *m = getenv("URLGPU_BIC_MODE")) ctx->bic_direct = strcmp(m, "direct") == 0;
-    // the large dynamic shared-memory opt-ins are per device: every context sets them for its own
-    cudaFuncSetAttribute(bic_count_smem_kernel<MaskSets>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->smem_optin - 2048);
-    cudaFuncSetAttribute(bic_count_smem_kernel<RankSets>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ctx->smem_optin - 2048);
-    cudaFuncSetAttribute(gram_partial_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kGramSmemBytes);
+    // the large dynamic shared-memory opt-ins are per device: every context sets them for its own.  A refused opt-in fails
+    // the creation here; unchecked, it would surface as a stale error of some later, unrelated call
+    {
+        auto refuse = [&](const std::string &m) {
+            cudaGetLastError();
+            g_create_error = m + ": " + cudaGetErrorString(e);
+            cudaStreamDestroy(ctx->copy_stream);
+            cudaStreamDestroy(ctx->own_stream);
+            delete ctx;
+            return URLGPU_ERR_CUDA;
+        };
+        const void *roots[] = {(const void *)bic_root_kernel<0, 8>, (const void *)bic_root_kernel<2, 8>, (const void *)bic_root_kernel<3, 8>,
+                               (const void *)bic_root_kernel<4, 8>, (const void *)bic_root_kernel<0, 12>, (const void *)bic_root_kernel<2, 12>,
+                               (const void *)bic_root_kernel<3, 12>, (const void *)bic_root_kernel<4, 12>, (const void *)bic_root_kernel<0, 16>,
+                               (const void *)bic_root_kernel<2, 16>, (const void *)bic_root_kernel<3, 16>, (const void *)bic_root_kernel<4, 16>};
+        // bic_root_kernel holds the slice (root_budget cells), two segment tables (root_seg_cap each) and one counter in
+        // dynamic shared memory, next to its static shared memory (the byte look-up tables, the root descriptor).  Both
+        // switches at the top of their ranges ask for more than a block may opt into: the segment cap gives way first (slices
+        // with more segments take the kernel's fragmented path), then the budget
+        size_t root_static = 0;
+        for (const void *f : roots) {
+            cudaFuncAttributes fa{};
+            if ((e = cudaFuncGetAttributes(&fa, f)) != cudaSuccess) return refuse("cannot read the root kernel's attributes");
+            root_static = std::max(root_static, fa.sharedSizeBytes);
+        }
+        const int64_t cap = ((int64_t)ctx->smem_optin - (int64_t)root_static) / (int64_t)sizeof(int) - 1;   // budget + 2 * segments
+        if ((int64_t)ctx->root_budget + 2 * (int64_t)ctx->root_seg_cap > cap)
+            ctx->root_seg_cap = (uint32_t)std::max<int64_t>(32, (cap - (int64_t)ctx->root_budget) / 2);
+        if ((int64_t)ctx->root_budget + 2 * (int64_t)ctx->root_seg_cap > cap)
+            ctx->root_budget = (uint32_t)std::max<int64_t>(0, (cap - 2 * (int64_t)ctx->root_seg_cap) / 4 * 4);
+        const int smem = (int)((ctx->root_budget + 2 * ctx->root_seg_cap + 1) * sizeof(int));
+        const int big = (int)ctx->smem_optin - 2048;
+        std::vector<std::pair<const void *, int>> attrs;
+        for (const void *f : roots) attrs.push_back({f, smem});
+        attrs.push_back({(const void *)bic_count_smem_kernel<MaskSets>, big});
+        attrs.push_back({(const void *)bic_count_smem_kernel<RankSets>, big});
+        attrs.push_back({(const void *)gram_partial_kernel, (int)kGramSmemBytes});
+        for (const auto &a : attrs)
+            if ((e = cudaFuncSetAttribute(a.first, cudaFuncAttributeMaxDynamicSharedMemorySize, a.second)) != cudaSuccess)
+                return refuse("cannot opt a kernel into " + std::to_string(a.second) + " bytes of dynamic shared memory (the device allows " +
+                              std::to_string(ctx->smem_optin) + " bytes per block, static shared memory included)");
+    }
     if (device_id < 64) g_ctx_on_device[device_id]++;
     *out = ctx;
     return URLGPU_OK;
