@@ -1581,11 +1581,17 @@ static int make_rank_space(urlgpu_ctx *ctx, int c, int K, RankSpace &rs) {
 }
 
 // ---- K3 in rank space: per-set Schur sweeps, one launch per layer, entries [first, first + count) of the index space
-static int cbic_score_rank(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, const RankSpace &rs, double lambda, uint32_t first, uint32_t count,
-                           float *d_scores /*indexed by global index*/, double *d_ts64) {
+// `who` names the caller in the refusal of more than kRankGenericMaxL parents.  urlgpu_score_variable comes here only for
+// families over more than 30 candidates; the range entry points come here for every family, and for one over at most 30
+// candidates urlgpu_score_variable is the route that scores larger parent limits.
+static int cbic_score_rank(urlgpu_ctx *ctx, const char *who, int variable, const std::vector<int> &cand, const RankSpace &rs, double lambda, uint32_t first,
+                           uint32_t count, float *d_scores /*indexed by global index*/, double *d_ts64) {
     cudaStream_t s = ctx->stream;
     const int c = rs.c, p = ctx->cp;
-    if (rs.K > kRankGenericMaxL) return ctx->fail(URLGPU_ERR_LIMIT, "cBIC over more than 30 candidates handles sets of at most " + std::to_string(kRankGenericMaxL) + " parents");
+    if (rs.K > kRankGenericMaxL)
+        return ctx->fail(URLGPU_ERR_LIMIT, std::string(who) + ": cBIC scored set by set handles sets of at most " + std::to_string(kRankGenericMaxL) + " parents" +
+                                               (c > kMaxDenseCand ? " (no other cBIC route takes a family over more than 30 candidates)"
+                                                                  : " (urlgpu_score_variable scores this family, over at most 30 candidates, whole)"));
     // candidate Gram over (v, cand_0, ..): full square, row-major
     std::vector<int> order(1, variable);
     order.insert(order.end(), cand.begin(), cand.end());
@@ -1936,7 +1942,7 @@ extern "C" int urlgpu_score_variable(urlgpu_ctx *ctx, int variable, const uint64
         if (bic) {
             fill_u32_kernel<<<blocks_for(total, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(res->d_table), total, kSentinelBits);
             rc = bic_score_family(ctx, variable, cand, K, res->d_table, &res->n_scored, res->rs, res->d_ovf);
-        } else rc = cbic_score_rank(ctx, variable, cand, res->rs, lambda, 0, total, res->d_table, nullptr);
+        } else rc = cbic_score_rank(ctx, "score_variable", variable, cand, res->rs, lambda, 0, total, res->d_table, nullptr);
     } else {
         fill_u32_kernel<<<blocks_for(res->n_masks, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(res->d_table), res->n_masks, kSentinelBits);
         if (bic) rc = bic_score_family(ctx, variable, cand, K, res->d_table, &res->n_scored, RankSpace{}, res->d_ovf);
@@ -1992,7 +1998,7 @@ extern "C" int urlgpu_score_range(urlgpu_ctx *ctx, int variable, const uint64_t 
     // the kernels index by global family index: shift the base so that entry `first` lands on d_out[0]
     float *d_base = d_out - first;
     if (bic) rc = bic_score_direct(ctx, variable, cand, rs, (uint32_t)first, (uint32_t)count, d_base, false);
-    else rc = cbic_score_rank(ctx, variable, cand, rs, lambda, (uint32_t)first, (uint32_t)count, d_base, nullptr);
+    else rc = cbic_score_rank(ctx, "score_range", variable, cand, rs, lambda, (uint32_t)first, (uint32_t)count, d_base, nullptr);
     if (rc) return rc;
     if (!on_device) {
         CK(cudaMemcpyAsync(scores, d_out, count * sizeof(float), cudaMemcpyDeviceToHost, s));
@@ -2044,7 +2050,7 @@ extern "C" int urlgpu_score_part(urlgpu_ctx *ctx, int variable, const uint64_t *
         const uint64_t b0 = (uint64_t)total * part / parts, b1 = (uint64_t)total * (part + 1) / parts;
         if (b1 > b0) {
             if (bic) rc = bic_score_direct(ctx, variable, cand, rs, (uint32_t)b0, (uint32_t)(b1 - b0), d_out, false);
-            else rc = cbic_score_rank(ctx, variable, cand, rs, lambda, (uint32_t)b0, (uint32_t)(b1 - b0), d_out, nullptr);
+            else rc = cbic_score_rank(ctx, "score_part", variable, cand, rs, lambda, (uint32_t)b0, (uint32_t)(b1 - b0), d_out, nullptr);
             if (rc) return rc;
         }
     }
