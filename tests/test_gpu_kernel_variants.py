@@ -11,12 +11,8 @@ the scores with identical stored lists, cBIC within 1e-9 relative on the FP64 va
   and just above each tier boundary, a call of several global batches, and the range and part entry points;
 - one table above the global tier's batch size through ``score_one`` / ``contingency``, and the 2^30-cell refusals;
 - ``cube_derive_kernel<0>`` with 16-bit tables;
-- K3 level B: every ``cbic_dfs_kernel<0..6>`` and ``cbic_tree_kernel<7..11>``, and the process-wide switches
-  ``URLGPU_CBIC_TREE`` / ``URLGPU_CBIC_J`` in child processes.
+- K3 level B: every ``cbic_dfs_kernel<0..4>`` and ``cbic_tree_kernel<7..11>``.
 """
-import os
-import subprocess
-import sys
 from math import comb
 
 import numpy as np
@@ -25,7 +21,6 @@ import pytest
 from conftest import engine_with_env
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 T0_CELLS = 12 * 1024              # tier 0 of the direct path: tables of at most this many cells (48 KB of shared memory)
 BATCH_CELLS = 12 << 20            # the global tier's scratch: tables of one batch, int32 cells
@@ -440,8 +435,9 @@ def test_generic_arity_derive_with_16bit_tables(pkg, orc):
 
 
 # ------------------------------------------------------------------------------------------------ 6. K3 level B widths
-# Level B walks the J lowest candidate bits, J = max(min(c, 3), min(11, c - 10)): cbic_dfs_kernel<J> for J <= 6 (c <= 16),
-# cbic_tree_kernel<J> for J = 7..11 (c = 17..21 and above).  Level A sweeps the c - J high bits in 1, 2 or 3 stages.
+# Level B walks the J lowest candidate bits: J = min(c, 3) up to c = 13, 4 for c = 14..16, min(11, c - 10) above.
+# cbic_dfs_kernel<J> for J <= 4 (c <= 16), cbic_tree_kernel<J> for J = 7..11 (c = 17..21 and above).  Level A sweeps the
+# c - J high bits in 1, 2 or 3 stages.
 CBIC_P, CBIC_N, LAM = 27, 3000, 2.0
 CBIC_CS = list(range(0, 23)) + [26]
 
@@ -457,7 +453,7 @@ def cbic_data(pkg, orc):
 
 
 def test_cbic_every_level_b_width(pkg, orc, cbic_data):
-    """c = 0..22 and 26 candidates of variable 0 (K = c up to 14, then 6, then 4): every cbic_dfs_kernel<0..6>, every
+    """c = 0..22 and 26 candidates of variable 0 (K = c up to 14, then 6, then 4): every cbic_dfs_kernel<0..4>, every
     cbic_tree_kernel<7..11>, level A in 1, 2 and 3 stages, segment DPs with and without high bits.  The dense cache equals
     the rank-layout cache bit for bit (no acceptance, acceptance, prune); >= 100 sampled sets per family against the
     oracle's residual form (1e-9) and score_one (bit-equal); acceptance and prune decisions against the oracle given the
@@ -497,39 +493,3 @@ def test_cbic_every_level_b_width(pkg, orc, cbic_data):
         assert np.array_equal(mp, om[stored][keep]) and np.array_equal(sp.view(np.uint32), val[stored][keep].view(np.uint32)), c
     dense.close()
     rank.close()
-
-
-_CBIC_CHILD = r"""
-import importlib, sys
-sys.path.insert(0, sys.argv[1])
-pkg = importlib.import_module("urlearning-cpp_b200")
-x, _ = pkg.datagen.linear_gaussian_sem(p=22, n=3000, seed=22)
-eng = pkg.Engine(0)
-eng.set_continuous(x)
-with open(sys.argv[2], "wb") as f:
-    for c in range(17, 22):
-        for flags in (pkg.CBIC_NO_ACCEPT, 0, pkg.PRUNE_DOMINATED):
-            r = eng.score_variable(0, sum(1 << i for i in range(1, c + 1)), 8, pkg.CBIC, lam=2.0, flags=flags)
-            m, s = r.fetch()
-            r.free()
-            f.write(m.tobytes())
-            f.write(s.tobytes())
-eng.close()
-"""
-
-
-def test_cbic_tree_and_split_switches_in_child_processes(tmp_path):
-    """URLGPU_CBIC_TREE=0 (level B through cbic_dfs_kernel<7..11> instead of cbic_tree_kernel) and URLGPU_CBIC_J=5 (five
-    low bits in level B, the rest in two or three level-A stages) are read once per process, so each runs in a child
-    process of its own.  Every pivot sequence is the same, so for c = 17..21 both write the same cache bytes as the default"""
-    outs = {}
-    for name, extra in (("default", {}), ("no-tree", {"URLGPU_CBIC_TREE": "0"}), ("J5", {"URLGPU_CBIC_J": "5"})):
-        env = {k: v for k, v in os.environ.items() if not k.startswith("URLGPU_CBIC_")}
-        env.update({"URLGPU_LAYOUT": "dense", **extra})
-        path = str(tmp_path / f"{name}.bin")
-        out = subprocess.run([sys.executable, "-c", _CBIC_CHILD, ROOT, path], env=env, capture_output=True, text=True, timeout=600)
-        assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
-        outs[name] = open(path, "rb").read()
-    assert len(outs["default"]) > 0
-    assert outs["no-tree"] == outs["default"]
-    assert outs["J5"] == outs["default"]

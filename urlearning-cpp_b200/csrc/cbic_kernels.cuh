@@ -250,13 +250,10 @@ __global__ void __launch_bounds__(256) probe_dmma_kernel(double *out, int iters,
 // ------------------------------------------------------------------------------------------------ K3
 
 struct CbicParams {
-    int c;            // candidates
-    int J;            // low bits handled by one thread of the DFS kernel
     int max_parents;
     double n;         // row count (num_err, BIC_OLS.cpp:348)
     double lam_logn;  // lambda*log(n)  (:366, evaluated left to right)
     double log_n;     // log(n)
-    int store_mode;   // score stores of the DFS kernel: 0 default, 1 st.global.cs (streaming), 2 st.global.wt, 3 st.global.cg
     // Pivot guard (SURVEY Q13): a candidate whose Schur pivot has dropped to <= piv_tol (1e-10 * the largest diagonal entry of
     // the candidate Gram) is a linear combination of the candidates already swept.  Its sweep is skipped (inv = 0 turns every
     // FMA of the sweep into the identity), so RSS equals the least-squares RSS without that column — what arma::solve's
@@ -297,6 +294,17 @@ __device__ __forceinline__ double cbic_log(double x) {
 // packed lower-triangular index, element order (v, cand0, cand1, ...)
 __host__ __device__ __forceinline__ int tri(int a, int b) { return a * (a + 1) / 2 + b; }
 
+// One warp sweeps candidate `piv` out of the packed matrix A over (v, cand_0 .. cand_{piv-1}, ...) in shared memory:
+// the rows above the pivot are updated in place, the lanes striding over each row.
+__device__ __forceinline__ void cbic_warp_sweep(double *A, int piv, double piv_tol, int lane) {
+    const double inv = guarded_inv(A[tri(piv, piv)], piv_tol);
+    for (int a = 0; a < piv; a++) {
+        const double f = -A[tri(piv, a)] * inv;
+        for (int b = lane; b <= a; b += 32) A[tri(a, b)] = fma(f, A[tri(piv, b)], A[tri(a, b)]);
+    }
+    __syncwarp();
+}
+
 // Level A: one warp per prefix (the high candidate bits).  Starting from a matrix over (v, cand_0 .. cand_{c_in-1}), walk
 // the `bits` highest candidates from the top: an included one is swept out (Schur complement), either way it is then
 // dropped.  The prefix index p = (q << bits) | local: q selects the input matrix (in_stride = 0: one shared matrix),
@@ -316,17 +324,8 @@ __global__ void cbic_roots_kernel(const double *__restrict__ in, size_t in_strid
     const double *src = in + (size_t)(P >> bits) * in_stride;
     for (int e = lane; e < tsz; e += 32) A[e] = src[e];
     __syncwarp();
-    for (int t = bits - 1; t >= 0; t--) {
-        if ((P >> t) & 1) {
-            const int piv = c_in - bits + t + 1; // position of the candidate in (v, c0, c1, ...)
-            const double inv = guarded_inv(A[tri(piv, piv)], piv_tol);
-            for (int a = 0; a < piv; a++) {
-                const double f = -A[tri(piv, a)] * inv;
-                for (int b = lane; b <= a; b += 32) A[tri(a, b)] = fma(f, A[tri(piv, b)], A[tri(a, b)]);
-            }
-            __syncwarp();
-        }
-    }
+    for (int t = bits - 1; t >= 0; t--)
+        if ((P >> t) & 1) cbic_warp_sweep(A, c_in - bits + t + 1 /*position of the candidate in (v, c0, c1, ...)*/, piv_tol, lane);
     const int c_out = c_in - bits;
     const int outsz = (c_out + 1) * (c_out + 2) / 2;
     if (transposed) { for (int e = lane; e < outsz; e += 32) out[(size_t)e * n_out + P] = A[e]; }
@@ -349,30 +348,14 @@ __global__ void cbic_one_kernel(const double *__restrict__ sub, int k, CbicParam
     const int tsz = (k + 1) * (k + 2) / 2;
     for (int e = lane; e < tsz; e += 32) smat[e] = sub[e];
     __syncwarp();
-    for (int piv = k; piv >= 1; piv--) {
-        const double inv = guarded_inv(smat[tri(piv, piv)], prm.piv_tol);
-        for (int a = 0; a < piv; a++) {
-            const double f = -smat[tri(piv, a)] * inv;
-            for (int b = lane; b <= a; b += 32) smat[tri(a, b)] = fma(f, smat[tri(piv, b)], smat[tri(a, b)]);
-        }
-        __syncwarp();
-    }
+    for (int piv = k; piv >= 1; piv--) cbic_warp_sweep(smat, piv, prm.piv_tol, lane);
     if (lane == 0) { out[0] = cbic_the_score64(smat[0], k, prm); out[1] = smat[0]; }
 }
 
 // Level B: template-recursive DFS over the J low candidate bits.  A has (j+1)(j+2)/2 packed entries over
-// (v, cand0..cand_{j-1}).  Low masks are emitted in ascending order (exclude branch first).  Levels above
-// kInlineLevel are real calls with their matrices on the thread's stack (touched once per 2^j sets); the bottom
-// levels are fully inlined so their matrices live in registers, and the scores of the 8 sets below a level-3 node are
-// collected in registers and written as one full 32-byte sector (two 128-bit stores).
-#ifndef URLGPU_DFS_INLINE
-#define URLGPU_DFS_INLINE 4
-#endif
-constexpr int kInlineLevel = URLGPU_DFS_INLINE;
-#ifndef URLGPU_DFS_MINBLOCKS
-#define URLGPU_DFS_MINBLOCKS 5
-#endif
-
+// (v, cand0..cand_{j-1}).  Low masks are emitted in ascending order (exclude branch first).  Every level is inlined, so
+// all matrices live in registers; the scores of the 16 sets below a level-4 node are collected in registers and written
+// together.
 template <int j>
 __device__ __forceinline__ void cbic_sweep(const double *A, double *B, double piv_tol) {
     const double inv = guarded_inv(A[tri(j, j)], piv_tol);
@@ -389,17 +372,15 @@ constexpr int kBufLevel = 4;             // the scores of the 2^kBufLevel sets b
 constexpr int kBufSets = 1 << kBufLevel; // (32-byte sector writes reached DRAM as read-modify-writes: 2.7x the table size written, 0.9x read)
 
 template <int j, uint32_t LOCAL>
-__device__ __forceinline__ void cbic_dfs_buf(const double *A, uint32_t low, int k, const CbicParams &prm, float (&buf)[kBufSets], double *__restrict__ out64) {
+__device__ __forceinline__ void cbic_dfs_buf(const double *A, int k, const CbicParams &prm, float (&buf)[kBufSets]) {
     if constexpr (j == 0) {
-        const double ts = cbic_the_score64(A[0], k, prm);
-        buf[LOCAL] = (float)ts;
-        if (out64) out64[low | LOCAL] = ts;
+        buf[LOCAL] = (float)cbic_the_score64(A[0], k, prm);
     } else {
-        cbic_dfs_buf<j - 1, LOCAL>(A, low, k, prm, buf, out64);
+        cbic_dfs_buf<j - 1, LOCAL>(A, k, prm, buf);
         if (k < prm.max_parents) {
             double B[j * (j + 1) / 2];
             cbic_sweep<j>(A, B, prm.piv_tol);
-            cbic_dfs_buf<j - 1, (LOCAL | (1u << (j - 1)))>(B, low, k + 1, prm, buf, out64);
+            cbic_dfs_buf<j - 1, (LOCAL | (1u << (j - 1)))>(B, k + 1, prm, buf);
         } else {
 #pragma unroll
             for (uint32_t m = 0; m < (1u << (j - 1)); m++) buf[LOCAL | (1u << (j - 1)) | m] = sentinel();
@@ -408,60 +389,38 @@ __device__ __forceinline__ void cbic_dfs_buf(const double *A, uint32_t low, int 
 }
 
 template <int j>
-__device__ __forceinline__ void cbic_dfs_inl(const double *A, uint32_t low, int k, const CbicParams &prm, float *__restrict__ out,
-                                             double *__restrict__ out64) {
+__device__ __forceinline__ void cbic_dfs_inl(const double *A, uint32_t low, int k, const CbicParams &prm, float *__restrict__ out) {
     if constexpr (j == kBufLevel) {
         float buf[kBufSets];
-        cbic_dfs_buf<kBufLevel, 0u>(A, low, k, prm, buf, out64);
+        cbic_dfs_buf<kBufLevel, 0u>(A, k, prm, buf);
+        // streaming stores (st.global.cs) for the 2^c scores: measured 8.8 -> 8.3 ms per variable at config 3 against the
+        // default store policy
         float4 *o4 = reinterpret_cast<float4 *>(out + low); // low is a multiple of kBufSets here
 #pragma unroll
-        for (int q = 0; q < kBufSets / 4; q++) {
-            const float4 a = make_float4(buf[4 * q], buf[4 * q + 1], buf[4 * q + 2], buf[4 * q + 3]);
-            if (prm.store_mode == 1) __stcs(o4 + q, a);
-            else if (prm.store_mode == 2) __stwt(o4 + q, a);
-            else if (prm.store_mode == 3) __stcg(o4 + q, a);
-            else o4[q] = a;
-        }
+        for (int q = 0; q < kBufSets / 4; q++) __stcs(o4 + q, make_float4(buf[4 * q], buf[4 * q + 1], buf[4 * q + 2], buf[4 * q + 3]));
     } else if constexpr (j == 0) {
-        const double ts = cbic_the_score64(A[0], k, prm);
-        out[low] = (float)ts;
-        if (out64) out64[low] = ts;
+        out[low] = (float)cbic_the_score64(A[0], k, prm);
     } else {
-        cbic_dfs_inl<j - 1>(A, low, k, prm, out, out64); // candidate j-1 excluded: leading principal submatrix
+        cbic_dfs_inl<j - 1>(A, low, k, prm, out); // candidate j-1 excluded: leading principal submatrix
         if (k < prm.max_parents) {
             double B[j * (j + 1) / 2];
             cbic_sweep<j>(A, B, prm.piv_tol);
-            cbic_dfs_inl<j - 1>(B, low | (1u << (j - 1)), k + 1, prm, out, out64);
+            cbic_dfs_inl<j - 1>(B, low | (1u << (j - 1)), k + 1, prm, out);
         } else {
             for (uint32_t m = 0; m < (1u << (j - 1)); m++) out[low | (1u << (j - 1)) | m] = sentinel();
         }
     }
 }
 
-template <int j>
-__device__ __noinline__ void cbic_dfs_call(const double *A, uint32_t low, int k, const CbicParams &prm, float *__restrict__ out,
-                                           double *__restrict__ out64) {
-    if constexpr (j <= kInlineLevel) {
-        cbic_dfs_inl<j>(A, low, k, prm, out, out64);
-    } else {
-        cbic_dfs_call<j - 1>(A, low, k, prm, out, out64);
-        if (k < prm.max_parents) {
-            double B[j * (j + 1) / 2];
-            cbic_sweep<j>(A, B, prm.piv_tol);
-            cbic_dfs_call<j - 1>(B, low | (1u << (j - 1)), k + 1, prm, out, out64);
-        } else {
-            for (uint32_t m = 0; m < (1u << (j - 1)); m++) out[low | (1u << (j - 1)) | m] = sentinel();
-        }
-    }
-}
-
+// one thread per prefix, J = 0..4: kBufLevel is the widest DFS whose matrices all fit the registers the launch bound
+// leaves (J = 5 and 6 spill); wider level-B widths go to cbic_tree_kernel below
+constexpr int kDfsMinBlocks = 5;
 template <int J>
-__global__ void __launch_bounds__(128, URLGPU_DFS_MINBLOCKS) cbic_dfs_kernel(const double *__restrict__ roots, CbicParams prm, uint32_t n_prefix, float *__restrict__ ts_out,
-                                double *__restrict__ ts64_out) {
+__global__ void __launch_bounds__(128, kDfsMinBlocks) cbic_dfs_kernel(const double *__restrict__ roots, CbicParams prm, uint32_t n_prefix, float *__restrict__ ts_out) {
+    static_assert(J <= kBufLevel, "wider level-B widths use cbic_tree_kernel");
     const uint32_t P = blockIdx.x * blockDim.x + threadIdx.x;
     if (P >= n_prefix) return;
     float *out = ts_out + ((size_t)P << J);
-    double *out64 = ts64_out ? ts64_out + ((size_t)P << J) : nullptr;
     const int k0 = __popc(P);
     if (k0 > prm.max_parents) {
         for (uint32_t m = 0; m < (1u << J); m++) out[m] = sentinel();
@@ -470,12 +429,12 @@ __global__ void __launch_bounds__(128, URLGPU_DFS_MINBLOCKS) cbic_dfs_kernel(con
     double A[(J + 1) * (J + 2) / 2];
 #pragma unroll
     for (int e = 0; e < (J + 1) * (J + 2) / 2; e++) A[e] = roots[(size_t)e * n_prefix + P];
-    cbic_dfs_call<J>(A, 0u, k0, prm, out, out64);
+    cbic_dfs_inl<J>(A, 0u, k0, prm, out);
 }
 
-// Level B, CTA form (J >= 7): the DFS above keeps the matrices of its upper levels on the thread's stack — 2.9 KB per
-// thread at J = 11, 270 MB over the resident threads, which spills out of L2 and tripled the DRAM traffic of K3 (ncu,
-// round 1).  Here one CTA of 2^(J-4) threads owns one prefix: the levels J .. 5 are expanded BREADTH FIRST in shared
+// Level B, CTA form (J >= 7): a per-thread DFS this wide keeps the matrices of its upper levels on the thread's stack —
+// 2.9 KB per thread at J = 11, 270 MB over the resident threads, which spills out of L2 and tripled the DRAM traffic of
+// K3 (ncu, round 1).  Here one CTA of 2^(J-4) threads owns one prefix: the levels J .. 5 are expanded BREADTH FIRST in shared
 // memory, all threads sharing each level's element-wise sweeps, and every thread then walks its own 4-bit subtree
 // (16 sets) with all matrices in registers.  An "exclude" child is the leading principal submatrix of its parent, i.e. a
 // PREFIX of the parent's packed array: it is never copied, only "include" children get storage (2802 doubles = 22 KB at
@@ -528,9 +487,11 @@ __device__ __forceinline__ void cbic_tree_expand(double *S, double *inv /*[2][2^
     }
 }
 
+// 72 registers hold every matrix (7 CTAs of 128 threads per SM at J = 11); left to itself, ptxas picks 64 at J = 10, 11
+// and spills
 template <int J>
-__global__ void __launch_bounds__(1 << (J - kTreeJB)) cbic_tree_kernel(const double *__restrict__ roots /*[n_prefix][tri_size(J)]*/, CbicParams prm, uint32_t n_prefix,
-                                                                        float *__restrict__ ts_out, double *__restrict__ ts64_out) {
+__global__ void __maxnreg__(72) cbic_tree_kernel(const double *__restrict__ roots /*[n_prefix][tri_size(J)]*/, CbicParams prm, uint32_t n_prefix,
+                                                 float *__restrict__ ts_out) {
     constexpr int NT = 1 << (J - kTreeJB);
     __shared__ double S[cbic_tree_doubles<J>()];
     __shared__ double inv[2 * NT];
@@ -539,7 +500,6 @@ __global__ void __launch_bounds__(1 << (J - kTreeJB)) cbic_tree_kernel(const dou
     const uint32_t P = blockIdx.x;
     const int tid = threadIdx.x;
     float *out = ts_out + ((size_t)P << J);
-    double *out64 = ts64_out ? ts64_out + ((size_t)P << J) : nullptr;
     const int k0 = __popc(P);
     if (k0 > prm.max_parents) { // whole subtree unscored
         for (uint32_t m = tid; m < (1u << J); m += NT) out[m] = sentinel();
@@ -572,7 +532,7 @@ __global__ void __launch_bounds__(1 << (J - kTreeJB)) cbic_tree_kernel(const dou
     const double *src = S + cbic_tree_offset(s_base, kTreeJB, (uint32_t)tid);
 #pragma unroll
     for (int e = 0; e < tri_size(kTreeJB); e++) A[e] = src[e];
-    cbic_dfs_inl<kTreeJB>(A, low, k, prm, out, out64);
+    cbic_dfs_inl<kTreeJB>(A, low, k, prm, out);
 }
 
 // ------------------------------------------------------------------------------------------------ K4 / K5 rules
@@ -585,10 +545,10 @@ __global__ void __launch_bounds__(1 << (J - kTreeJB)) cbic_tree_kernel(const dou
 // K5 — subset-dominance prune (ScoreCalculator::prune, score_calculator.cpp:150-197) as a DP on the dense table:
 //   M(S) = max(val'(S), max_i M(S\i)),  keep S iff stored and val(S) > max_i M(S\i)  (ties: the subset, having
 //   the smaller mask, sorts first and wins — compareSecond :137-148).  The empty set is always kept.
-// URLGPU_CBIC_NO_ACCEPT: store -the_score for every scored set
-__global__ void cbic_negate_kernel(float *__restrict__ table, uint64_t n_masks) {
+// URLGPU_CBIC_NO_ACCEPT: store -the_score for every scored set (dense table or rank-space scores alike)
+__global__ void cbic_negate_kernel(float *__restrict__ table, uint64_t n) {
     const uint64_t m = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (m >= n_masks) return;
+    if (m >= n) return;
     const float ts = table[m];
     if (!is_sentinel(ts)) table[m] = -ts;
 }

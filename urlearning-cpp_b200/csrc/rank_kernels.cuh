@@ -73,20 +73,17 @@ __global__ void rank_store_rule_kernel(float *__restrict__ scores, uint32_t tota
     if (is_sentinel(s)) return;
     if (!(i == 0 ? s < 1.0f : s < 0.0f)) scores[i] = sentinel();
 }
-__global__ void rank_negate_kernel(float *__restrict__ scores, uint32_t total) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < total && !is_sentinel(scores[i])) scores[i] = -scores[i];
-}
 
 // ------------------------------------------------------------------------------------------------ K3 in rank space
 // One thread scores kRankRun consecutive sets of layer L: unrank the first, colex successor for the rest.  The set's
-// (L+1)x(L+1) sub-Gram over (v, e_1..e_L) is gathered from the candidate Gram (row-major, (c+1)^2, position 0 = v) and the
+// (L+1)x(L+1) sub-Gram over (v, e_1..e_L) is gathered from the candidate Gram (packed lower triangle over (v, cand_0, ..),
+// indexed by tri(): members ascend, so every entry read is G[tri(pos[a], pos[b])] with pos[a] >= pos[b]) and the
 // candidates are swept out highest first — the FMA sequence of cbic_roots_kernel / cbic_sweep / cbic_one_kernel.
 // Pivot guard: see CbicParams::piv_tol (cbic_kernels.cuh).
 constexpr int kRankRun = 4;
 
 template <int L>
-__device__ __forceinline__ double rank_cbic_rss(const double *__restrict__ G, int ld, const uint8_t *e, double piv_tol) {
+__device__ __forceinline__ double rank_cbic_rss(const double *__restrict__ G, const uint8_t *e, double piv_tol) {
     double A[(L + 1) * (L + 2) / 2];
     int pos[L + 1];
     pos[0] = 0;
@@ -95,7 +92,7 @@ __device__ __forceinline__ double rank_cbic_rss(const double *__restrict__ G, in
 #pragma unroll
     for (int a = 0; a <= L; a++)
 #pragma unroll
-        for (int b = 0; b <= a; b++) A[tri(a, b)] = __ldg(G + pos[a] * ld + pos[b]);
+        for (int b = 0; b <= a; b++) A[tri(a, b)] = __ldg(G + tri(pos[a], pos[b]));
 #pragma unroll
     for (int piv = L; piv >= 1; piv--) {
         const double inv = guarded_inv(A[tri(piv, piv)], piv_tol);
@@ -109,10 +106,10 @@ __device__ __forceinline__ double rank_cbic_rss(const double *__restrict__ G, in
     return A[0];
 }
 // any L (matrix in local memory): layers above 8
-__device__ __noinline__ double rank_cbic_rss_generic(const double *__restrict__ G, int ld, const uint8_t *e, int L, double piv_tol, double *A) {
+__device__ __noinline__ double rank_cbic_rss_generic(const double *__restrict__ G, const uint8_t *e, int L, double piv_tol, double *A) {
     for (int a = 0; a <= L; a++) {
         const int pa = a ? (int)e[a - 1] + 1 : 0;
-        for (int b = 0; b <= a; b++) A[tri(a, b)] = __ldg(G + pa * ld + (b ? (int)e[b - 1] + 1 : 0));
+        for (int b = 0; b <= a; b++) A[tri(a, b)] = __ldg(G + tri(pa, b ? (int)e[b - 1] + 1 : 0));
     }
     for (int piv = L; piv >= 1; piv--) {
         const double inv = guarded_inv(A[tri(piv, piv)], piv_tol);
@@ -127,8 +124,8 @@ __device__ __noinline__ double rank_cbic_rss_generic(const double *__restrict__ 
 constexpr int kRankGenericMaxL = 16;
 
 template <int L> // L = 0: generic (run-time layer `layer`)
-__global__ void __launch_bounds__(128) rank_cbic_kernel(RankSpace rs, const double *__restrict__ G, CbicParams prm, double piv_tol, int layer,
-                                                        uint32_t first /*global index*/, uint32_t count, float *__restrict__ out, double *__restrict__ out64) {
+__global__ void __launch_bounds__(128) rank_cbic_kernel(RankSpace rs, const double *__restrict__ G, CbicParams prm, int layer,
+                                                        uint32_t first /*global index*/, uint32_t count, float *__restrict__ out) {
     extern __shared__ uint32_t s_binom[];
     rs_load_binom(rs, s_binom);
     const int l = L > 0 ? L : layer;
@@ -139,17 +136,14 @@ __global__ void __launch_bounds__(128) rank_cbic_kernel(RankSpace rs, const doub
     const uint32_t nrun = (uint32_t)min((uint64_t)kRankRun, (uint64_t)count - i0);
     uint8_t e[L > 0 ? L : kRankGenericMaxL];
     rs_unrank(s_binom, rs.bstride, rs.c, l, idx0 - rs.layer_base[l], e);
-    const int ld = rs.c + 1;
     for (uint32_t u = 0; u < nrun; u++) {
         double rss;
-        if constexpr (L > 0) rss = rank_cbic_rss<L>(G, ld, e, piv_tol);
+        if constexpr (L > 0) rss = rank_cbic_rss<L>(G, e, prm.piv_tol);
         else {
             double A[(kRankGenericMaxL + 1) * (kRankGenericMaxL + 2) / 2];
-            rss = rank_cbic_rss_generic(G, ld, e, l, piv_tol, A);
+            rss = rank_cbic_rss_generic(G, e, l, prm.piv_tol, A);
         }
-        const double ts = cbic_the_score64(rss, l, prm);
-        out[idx0 + u] = (float)ts;
-        if (out64) out64[idx0 + u] = ts;
+        out[idx0 + u] = (float)cbic_the_score64(rss, l, prm);
         if (u + 1 < nrun) rs_next(l, e);
     }
 }

@@ -1386,46 +1386,48 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
     return URLGPU_OK;
 }
 
-template <int J>
-static void launch_cbic_dfs(const double *roots, const CbicParams &prm, uint32_t n_prefix, float *ts, double *ts64, cudaStream_t s) {
-    const int threads = 128;
-    cbic_dfs_kernel<J><<<blocks_for(n_prefix, threads), threads, 0, s>>>(roots, prm, n_prefix, ts, ts64);
-}
-template <int J>
-static void launch_cbic_tree(const double *roots, const CbicParams &prm, uint32_t n_prefix, float *ts, double *ts64, cudaStream_t s) {
-    cbic_tree_kernel<J><<<n_prefix, 1 << (J - kTreeJB), 0, s>>>(roots, prm, n_prefix, ts, ts64);
-}
-
-static int cbic_score_family(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, double lambda, float *d_table, double *d_ts64,
-                             uint64_t *n_scored) {
-    cudaStream_t s = ctx->stream;
-    const int c = (int)cand.size();
-    const int p = ctx->cp;
-    *n_scored = family_size(c, K);
-    // packed sub-Gram over (v, cand0, cand1, ...)
-    std::vector<int> order(1, variable);
-    order.insert(order.end(), cand.begin(), cand.end());
-    std::vector<double> sub((size_t)(c + 1) * (c + 2) / 2);
-    for (int a = 0; a <= c; a++)
-        for (int b = 0; b <= a; b++) sub[tri(a, b)] = ctx->h_gram[(size_t)order[a] * p + order[b]];
+// the K3 parameter block of a family scored with sets of at most K parents and penalty weight lambda
+static CbicParams cbic_params(const urlgpu_ctx *ctx, int K, double lambda) {
     CbicParams prm{};
-    prm.c = c;
-    prm.piv_tol = 1e-10 * ctx->gram_dmax;
-    { // low bits walked by one DFS thread: 11 by default (URLGPU_CBIC_J overrides, 3..11)
-        static const int jmax = getenv("URLGPU_CBIC_J") ? std::max(3, std::min(atoi(getenv("URLGPU_CBIC_J")), 11)) : 11;
-        prm.J = std::max(std::min(c, 3), std::min(jmax, c - 10));
-    }
     prm.max_parents = K;
     prm.n = (double)(int)ctx->cn;
     prm.lam_logn = lambda * std::log((double)(int)ctx->cn);
     prm.log_n = std::log((double)(int)ctx->cn);
-    // streaming stores (st.global.cs) for the 2^c scores: measured 8.8 -> 8.3 ms per variable at config 3 (URLGPU_CBIC_STORE=0 restores the default policy)
-    { static const int sm = getenv("URLGPU_CBIC_STORE") ? atoi(getenv("URLGPU_CBIC_STORE")) : 1; prm.store_mode = sm; }
-    const uint32_t n_prefix = 1u << (c - prm.J);
-    const int outsz = (prm.J + 1) * (prm.J + 2) / 2;
-    // level B: one CTA per prefix with the upper levels in shared memory (J >= 7), else one thread per prefix
-    static const bool tree_off = getenv("URLGPU_CBIC_TREE") && atoi(getenv("URLGPU_CBIC_TREE")) == 0;
-    const bool use_tree = prm.J >= 7 && !tree_off;
+    prm.piv_tol = 1e-10 * ctx->gram_dmax;
+    return prm;
+}
+
+// the candidate Gram: packed lower triangle over (v, cand_0, cand_1, ...), indexed by tri()
+static std::vector<double> cbic_sub_gram(const urlgpu_ctx *ctx, int variable, const std::vector<int> &cand) {
+    const int c = (int)cand.size();
+    std::vector<int> order(1, variable);
+    order.insert(order.end(), cand.begin(), cand.end());
+    std::vector<double> sub((size_t)(c + 1) * (c + 2) / 2);
+    for (int a = 0; a <= c; a++)
+        for (int b = 0; b <= a; b++) sub[tri(a, b)] = ctx->h_gram[(size_t)order[a] * ctx->cp + order[b]];
+    return sub;
+}
+
+// level B over the J low candidate bits: one thread per prefix (J <= 4), or one CTA per prefix with the upper levels in
+// shared memory (J >= 7)
+template <int J>
+static void launch_level_b(const double *roots, const CbicParams &prm, uint32_t n_prefix, float *ts, cudaStream_t s) {
+    if constexpr (J >= 7) cbic_tree_kernel<J><<<n_prefix, 1 << (J - kTreeJB), 0, s>>>(roots, prm, n_prefix, ts);
+    else cbic_dfs_kernel<J><<<blocks_for(n_prefix, 128), 128, 0, s>>>(roots, prm, n_prefix, ts);
+}
+
+static int cbic_score_family(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, int K, double lambda, float *d_table, uint64_t *n_scored) {
+    cudaStream_t s = ctx->stream;
+    const int c = (int)cand.size();
+    *n_scored = family_size(c, K);
+    const std::vector<double> sub = cbic_sub_gram(ctx, variable, cand);
+    const CbicParams prm = cbic_params(ctx, K, lambda);
+    // low bits walked in level B: the per-thread DFS keeps all its matrices in registers up to J = 4, the CTA tree takes
+    // J = 7..11; the FMA sequence of a set does not depend on where the split falls
+    const int J = c <= 13 ? std::min(c, 3) : c <= 16 ? 4 : std::min(11, c - 10);
+    const uint32_t n_prefix = 1u << (c - J);
+    const int outsz = (J + 1) * (J + 2) / 2;
+    const bool use_tree = J >= 7;
     DevBuf dsub(ctx), droots(ctx), dmid(ctx), dmid2(ctx);
     CK(dsub.alloc(sub.size() * sizeof(double)));
     CK(droots.alloc((size_t)outsz * n_prefix * sizeof(double)));
@@ -1437,7 +1439,7 @@ static int cbic_score_family(urlgpu_ctx *ctx, int variable, const std::vector<in
         Region rg(ctx, F_CBIC, 4);
         const int warps = 8;
         // level A in stages of <= 7 bits: the sweeps of the higher bits are shared by all the prefixes below them
-        const int hbits = c - prm.J;
+        const int hbits = c - J;
         const int nstages = std::max(1, (hbits + 6) / 7);
         const double *src = dsub.as<double>();
         size_t src_stride = 0;
@@ -1457,20 +1459,11 @@ static int cbic_score_family(urlgpu_ctx *ctx, int variable, const std::vector<in
             cbic_roots_kernel<<<blocks_for(n_out, warps), warps * 32, (size_t)warps * insz * sizeof(double), s>>>(src, src_stride, c_in, bits, K, n_out, dst, last && !use_tree ? 1 : 0, prm.piv_tol);
             src = dst; src_stride = osz; c_in = c_out; done += bits;
         }
-        if (use_tree) {
-            switch (prm.J) {
-            case 7: launch_cbic_tree<7>(droots.as<double>(), prm, n_prefix, d_table, d_ts64, s); break;
-            case 8: launch_cbic_tree<8>(droots.as<double>(), prm, n_prefix, d_table, d_ts64, s); break;
-            case 9: launch_cbic_tree<9>(droots.as<double>(), prm, n_prefix, d_table, d_ts64, s); break;
-            case 10: launch_cbic_tree<10>(droots.as<double>(), prm, n_prefix, d_table, d_ts64, s); break;
-            default: launch_cbic_tree<11>(droots.as<double>(), prm, n_prefix, d_table, d_ts64, s); break;
-            }
-        } else
-        switch (prm.J) {
-#define URLGPU_CASE(JJ) case JJ: launch_cbic_dfs<JJ>(droots.as<double>(), prm, n_prefix, d_table, d_ts64, s); break;
-            URLGPU_CASE(0) URLGPU_CASE(1) URLGPU_CASE(2) URLGPU_CASE(3) URLGPU_CASE(4) URLGPU_CASE(5) URLGPU_CASE(6) URLGPU_CASE(7)
-            URLGPU_CASE(8) URLGPU_CASE(9) URLGPU_CASE(10) URLGPU_CASE(11)
-#undef URLGPU_CASE
+        switch (J) {
+#define URLGPU_LEVEL_B(JJ) case JJ: launch_level_b<JJ>(droots.as<double>(), prm, n_prefix, d_table, s); break;
+            URLGPU_LEVEL_B(0) URLGPU_LEVEL_B(1) URLGPU_LEVEL_B(2) URLGPU_LEVEL_B(3) URLGPU_LEVEL_B(4)
+            URLGPU_LEVEL_B(7) URLGPU_LEVEL_B(8) URLGPU_LEVEL_B(9) URLGPU_LEVEL_B(10) URLGPU_LEVEL_B(11)
+#undef URLGPU_LEVEL_B
         default: return ctx->fail(URLGPU_ERR_INTERNAL, "bad J");
         }
     }
@@ -1585,48 +1578,33 @@ static int make_rank_space(urlgpu_ctx *ctx, int c, int K, RankSpace &rs) {
 // families over more than 30 candidates; the range entry points come here for every family, and for one over at most 30
 // candidates urlgpu_score_variable is the route that scores larger parent limits.
 static int cbic_score_rank(urlgpu_ctx *ctx, const char *who, int variable, const std::vector<int> &cand, const RankSpace &rs, double lambda, uint32_t first,
-                           uint32_t count, float *d_scores /*indexed by global index*/, double *d_ts64) {
+                           uint32_t count, float *d_scores /*indexed by global index*/) {
     cudaStream_t s = ctx->stream;
-    const int c = rs.c, p = ctx->cp;
+    const int c = rs.c;
     if (rs.K > kRankGenericMaxL)
         return ctx->fail(URLGPU_ERR_LIMIT, std::string(who) + ": cBIC scored set by set handles sets of at most " + std::to_string(kRankGenericMaxL) + " parents" +
                                                (c > kMaxDenseCand ? " (no other cBIC route takes a family over more than 30 candidates)"
                                                                   : " (urlgpu_score_variable scores this family, over at most 30 candidates, whole)"));
-    // candidate Gram over (v, cand_0, ..): full square, row-major
-    std::vector<int> order(1, variable);
-    order.insert(order.end(), cand.begin(), cand.end());
-    const int ld = c + 1;
-    std::vector<double> g((size_t)ld * ld);
-    for (int a = 0; a <= c; a++)
-        for (int b = 0; b <= c; b++) g[(size_t)a * ld + b] = ctx->h_gram[(size_t)order[a] * p + order[b]];
+    const std::vector<double> g = cbic_sub_gram(ctx, variable, cand);
     DevBuf dg(ctx);
     CK(dg.alloc(g.size() * sizeof(double)));
     { int rc_ = stage_begin(ctx); if (rc_) return rc_; }
     { int rc_ = h2d_async(ctx, dg.p, g.data(), g.size() * sizeof(double)); if (rc_) return rc_; }
-    CbicParams prm{};
-    prm.c = c; prm.J = 0; prm.max_parents = rs.K;
-    prm.n = (double)(int)ctx->cn;
-    prm.lam_logn = lambda * std::log((double)(int)ctx->cn);
-    prm.log_n = std::log((double)(int)ctx->cn);
-    const double piv_tol = 1e-10 * ctx->gram_dmax;
-    prm.piv_tol = piv_tol;
+    const CbicParams prm = cbic_params(ctx, rs.K, lambda);
     const size_t smem = rs_binom_bytes(rs);
-    const uint64_t last = (uint64_t)first + count;
-    int launches = 0;
+    // each layer's part of [first, first + count)
+    struct Span { int l; uint32_t b0, cnt; };
+    std::vector<Span> spans;
     for (int l = 0; l <= rs.K; l++) {
-        const uint64_t b0 = std::max<uint64_t>(rs.layer_base[l], first), b1 = std::min<uint64_t>(rs.layer_base[l + 1], last);
-        if (b0 >= b1) continue;
-        launches++;
+        const uint64_t b0 = std::max<uint64_t>(rs.layer_base[l], first), b1 = std::min<uint64_t>(rs.layer_base[l + 1], (uint64_t)first + count);
+        if (b0 < b1) spans.push_back({l, (uint32_t)b0, (uint32_t)(b1 - b0)});
     }
     {
-        Region rg(ctx, F_CBIC, launches);
-        for (int l = 0; l <= rs.K; l++) {
-            const uint64_t b0 = std::max<uint64_t>(rs.layer_base[l], first), b1 = std::min<uint64_t>(rs.layer_base[l + 1], last);
-            if (b0 >= b1) continue;
-            const uint32_t cnt = (uint32_t)(b1 - b0);
-            const unsigned grid = blocks_for(((uint64_t)cnt + kRankRun - 1) / kRankRun, 128);
-#define URLGPU_RANK_CBIC(LL) rank_cbic_kernel<LL><<<grid, 128, smem, s>>>(rs, dg.as<double>(), prm, piv_tol, l, (uint32_t)b0, cnt, d_scores, d_ts64)
-            switch (l) {
+        Region rg(ctx, F_CBIC, (int)spans.size());
+        for (const Span &sp : spans) {
+            const unsigned grid = blocks_for(((uint64_t)sp.cnt + kRankRun - 1) / kRankRun, 128);
+#define URLGPU_RANK_CBIC(LL) rank_cbic_kernel<LL><<<grid, 128, smem, s>>>(rs, dg.as<double>(), prm, sp.l, sp.b0, sp.cnt, d_scores)
+            switch (sp.l) {
             case 1: URLGPU_RANK_CBIC(1); break;
             case 2: URLGPU_RANK_CBIC(2); break;
             case 3: URLGPU_RANK_CBIC(3); break;
@@ -1643,10 +1621,7 @@ static int cbic_score_rank(urlgpu_ctx *ctx, const char *who, int variable, const
     { int rc_ = stage_end(ctx); if (rc_) return rc_; }
     {
         double flops = 0;
-        for (int l = 0; l <= rs.K; l++) {
-            const uint64_t b0 = std::max<uint64_t>(rs.layer_base[l], first), b1 = std::min<uint64_t>(rs.layer_base[l + 1], last);
-            if (b0 < b1) flops += (double)(b1 - b0) * ((double)l * l * l / 3.0 + 2.0 * l * l + 2.0 * l);
-        }
+        for (const Span &sp : spans) flops += (double)sp.cnt * ((double)sp.l * sp.l * sp.l / 3.0 + 2.0 * sp.l * sp.l + 2.0 * sp.l);
         ctx->st.algorithmic_flops += flops;
         ctx->st.sets_scored += count;
     }
@@ -1874,7 +1849,7 @@ static int apply_filters(urlgpu_ctx *ctx, urlgpu_result *res, bool bic, unsigned
             rank_store_rule_kernel<<<blocks_for(total, 256), 256, 0, s>>>(res->d_table, total);
         } else if (filter_flags & URLGPU_CBIC_NO_ACCEPT) {
             Region rg(ctx, F_OTHER, 1);
-            rank_negate_kernel<<<blocks_for(total, 256), 256, 0, s>>>(res->d_table, total);
+            cbic_negate_kernel<<<blocks_for(total, 256), 256, 0, s>>>(res->d_table, total);
         } else if ((rc = run_rank_dp<0>(ctx, rs, res->d_table))) return rc;
         if (filter_flags & URLGPU_PRUNE_DOMINATED) rc = run_rank_dp<1>(ctx, rs, res->d_table);
     } else {
@@ -1942,11 +1917,11 @@ extern "C" int urlgpu_score_variable(urlgpu_ctx *ctx, int variable, const uint64
         if (bic) {
             fill_u32_kernel<<<blocks_for(total, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(res->d_table), total, kSentinelBits);
             rc = bic_score_family(ctx, variable, cand, K, res->d_table, &res->n_scored, res->rs, res->d_ovf);
-        } else rc = cbic_score_rank(ctx, "score_variable", variable, cand, res->rs, lambda, 0, total, res->d_table, nullptr);
+        } else rc = cbic_score_rank(ctx, "score_variable", variable, cand, res->rs, lambda, 0, total, res->d_table);
     } else {
         fill_u32_kernel<<<blocks_for(res->n_masks, 256), 256, 0, s>>>(reinterpret_cast<uint32_t *>(res->d_table), res->n_masks, kSentinelBits);
         if (bic) rc = bic_score_family(ctx, variable, cand, K, res->d_table, &res->n_scored, RankSpace{}, res->d_ovf);
-        else rc = cbic_score_family(ctx, variable, cand, K, lambda, res->d_table, nullptr, &res->n_scored);
+        else rc = cbic_score_family(ctx, variable, cand, K, lambda, res->d_table, &res->n_scored);
     }
     if (rc) return cleanup(rc);
     const double t_score = since(T0);
@@ -1998,7 +1973,7 @@ extern "C" int urlgpu_score_range(urlgpu_ctx *ctx, int variable, const uint64_t 
     // the kernels index by global family index: shift the base so that entry `first` lands on d_out[0]
     float *d_base = d_out - first;
     if (bic) rc = bic_score_direct(ctx, variable, cand, rs, (uint32_t)first, (uint32_t)count, d_base, false);
-    else rc = cbic_score_rank(ctx, "score_range", variable, cand, rs, lambda, (uint32_t)first, (uint32_t)count, d_base, nullptr);
+    else rc = cbic_score_rank(ctx, "score_range", variable, cand, rs, lambda, (uint32_t)first, (uint32_t)count, d_base);
     if (rc) return rc;
     if (!on_device) {
         CK(cudaMemcpyAsync(scores, d_out, count * sizeof(float), cudaMemcpyDeviceToHost, s));
@@ -2050,7 +2025,7 @@ extern "C" int urlgpu_score_part(urlgpu_ctx *ctx, int variable, const uint64_t *
         const uint64_t b0 = (uint64_t)total * part / parts, b1 = (uint64_t)total * (part + 1) / parts;
         if (b1 > b0) {
             if (bic) rc = bic_score_direct(ctx, variable, cand, rs, (uint32_t)b0, (uint32_t)(b1 - b0), d_out, false);
-            else rc = cbic_score_rank(ctx, "score_part", variable, cand, rs, lambda, (uint32_t)b0, (uint32_t)(b1 - b0), d_out, nullptr);
+            else rc = cbic_score_rank(ctx, "score_part", variable, cand, rs, lambda, (uint32_t)b0, (uint32_t)(b1 - b0), d_out);
             if (rc) return rc;
         }
     }
@@ -2543,12 +2518,6 @@ extern "C" int urlgpu_spg_free(urlgpu_spg *sp) {
 
 // ============================================================================================ single set / counts / prune
 
-static int compact_of(urlgpu_ctx *ctx, int p, int variable, const uint64_t *parents, int mask_words, std::vector<int> &cand) {
-    int rc = candidates_from_mask(ctx, p, variable, parents, mask_words, cand);
-    if (rc) return rc;
-    return URLGPU_OK;
-}
-
 // the set of all `cand` as the one entry of a global tier (key space: the family of cand with no parent limit)
 static int single_set(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, std::vector<int> &hv, DevBuf &dcand, RankSets &fam,
                       std::vector<GlobalSet> &one) {
@@ -2569,14 +2538,8 @@ extern "C" int urlgpu_score_one(urlgpu_ctx *ctx, int variable, const uint64_t *p
     if (!ctx || !parents || !score) return ctx ? ctx->fail(URLGPU_ERR_ARG, "score_one: null argument") : URLGPU_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     const bool bic = is_discrete(score_type);
-    if (!bic && score_type != URLGPU_CBIC) return ctx->fail(URLGPU_ERR_ARG, "score_one: unknown score type");
-    if (bic && !ctx->have_discrete) return ctx->fail(URLGPU_ERR_ARG, "score_one: BIC / fNML need urlgpu_set_discrete first");
-    if (!bic && !ctx->have_gram) return ctx->fail(URLGPU_ERR_ARG, "score_one: cBIC needs urlgpu_set_continuous first");
-    const int p = bic ? ctx->p : ctx->cp;
-    if (variable < 0 || variable >= p) return ctx->fail(URLGPU_ERR_ARG, "score_one: variable out of range");
-    if (bic) { const int rc0 = select_discrete_score(ctx, score_type, variable, lambda); if (rc0) return rc0; }
     std::vector<int> cand;
-    int rc = compact_of(ctx, p, variable, parents, mask_words, cand);
+    int rc = check_score_args(ctx, "score_one", variable, parents, mask_words, score_type, cand, lambda);
     if (rc) return rc;
     // the set itself is the whole candidate list (compact mask all ones).  It is scored directly: one contingency table for
     // BIC, one (k+1)x(k+1) Schur sweep for cBIC — no 2^k tables
@@ -2605,18 +2568,8 @@ extern "C" int urlgpu_score_one(urlgpu_ctx *ctx, int variable, const uint64_t *p
         if (value64) *value64 = (double)fx * ctx->ds_scale;
     } else {
         if (c > 200) return ctx->fail(URLGPU_ERR_LIMIT, "score_one: more than 200 parents in one set");
-        const int p_ = ctx->cp;
-        std::vector<int> order(1, variable);
-        order.insert(order.end(), cand.begin(), cand.end());
-        std::vector<double> sub((size_t)(c + 1) * (c + 2) / 2);
-        for (int a = 0; a <= c; a++)
-            for (int b = 0; b <= a; b++) sub[tri(a, b)] = ctx->h_gram[(size_t)order[a] * p_ + order[b]];
-        CbicParams prm{};
-        prm.c = c; prm.J = 0; prm.max_parents = c;
-        prm.n = (double)(int)ctx->cn;
-        prm.lam_logn = lambda * std::log((double)(int)ctx->cn);
-        prm.log_n = std::log((double)(int)ctx->cn);
-        prm.piv_tol = 1e-10 * ctx->gram_dmax;
+        const std::vector<double> sub = cbic_sub_gram(ctx, variable, cand);
+        const CbicParams prm = cbic_params(ctx, c, lambda);
         DevBuf dsub(ctx), dout(ctx);
         CK(dsub.alloc(sub.size() * sizeof(double)));
         CK(dout.alloc(2 * sizeof(double)));
@@ -2643,7 +2596,7 @@ extern "C" int urlgpu_contingency(urlgpu_ctx *ctx, int variable, const uint64_t 
     if (!ctx->have_discrete) return ctx->fail(URLGPU_ERR_ARG, "contingency: needs urlgpu_set_discrete first");
     if (variable < 0 || variable >= ctx->p) return ctx->fail(URLGPU_ERR_ARG, "contingency: variable out of range");
     std::vector<int> cand;
-    int rc = compact_of(ctx, ctx->p, variable, parents, mask_words, cand);
+    int rc = candidates_from_mask(ctx, ctx->p, variable, parents, mask_words, cand);
     if (rc) return rc;
     const int c = (int)cand.size();
     if (c > kMaxDenseCand) return ctx->fail(URLGPU_ERR_LIMIT, "contingency: more than 30 parents in one set");
