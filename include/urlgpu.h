@@ -163,6 +163,18 @@ int urlgpu_peer_free(urlgpu_ctx *ctx, void *dev_ptr);    /* a pointer from urlgp
  * value64 (optional): BIC: exact log-likelihood before the float rounding; cBIC: the_score in FP64. */
 int urlgpu_score_one(urlgpu_ctx *ctx, int variable, const uint64_t *parents, int mask_words, int score_type,
                      double lambda, float *score, double *value64);
+/* Score n_sets arbitrary (variable, parent set) pairs in one call.  Entry i is variables[i] with the parent set
+ * parents[i*mask_words .. i*mask_words + mask_words): any variables, any order, duplicates allowed; a parent set that
+ * names the child itself has that bit ignored (as urlgpu_score_one).  scores[i] and, if values64 is not NULL,
+ * values64[i] are exactly what urlgpu_score_one returns for that entry, bit for bit (BIC / fNML / BDeu: the score and
+ * the exact fixed-point log-likelihood or BDeu sum; cBIC: -the_score and the_score in FP64).  One score type per call;
+ * `lambda` is cBIC's lambda or BDeu's equivalent sample size.  Raw scores only: no store rule, acceptance or prune
+ * (those need a subset-closed family).  Synchronous: returns when the outputs are in host memory.  The whole list is
+ * validated before anything is launched; an error about one entry names the index of the first offending entry.
+ * Limits per entry are urlgpu_score_one's: BIC / fNML / BDeu at most 30 parents and 2^30 cells, cBIC at most 200
+ * parents.  n_sets == 0 succeeds and does nothing; n_sets >= 2^32 is refused with URLGPU_ERR_LIMIT. */
+int urlgpu_score_sets(urlgpu_ctx *ctx, uint64_t n_sets, const int32_t *variables, const uint64_t *parents, int mask_words,
+                      int score_type, double lambda, float *scores, double *values64);
 /* Dense contingency counts of (variable, parents): counts[x_v + r_v*paIdx], paIdx mixed radix over the parents in
  * ascending variable index, lowest index least significant (log_likelihood_calculator.cpp:61-73). */
 int urlgpu_contingency(urlgpu_ctx *ctx, int variable, const uint64_t *parents, int mask_words, int32_t *counts,

@@ -76,10 +76,11 @@ struct SetCols {
 // How the direct-counting kernels below name a set (its 32-bit `key`).  A policy fills the set's SetCols: columns,
 // cell count, penalty and output index.  MaskSets: key = compact mask over the candidates of a CandInfo (the cube
 // path's root tables, in cube order; they never write scores).  RankSets (rank_kernels.cuh): key = colex index.
+// ListSets: key = position in a caller's list of (child, parent set) entries (urlgpu_score_sets).
 // ---------------------------------------------------------------------------------------------------------
 struct MaskSets {
     CandInfo ci;
-    __device__ __forceinline__ int rv() const { return ci.rv; }
+    __host__ __device__ __forceinline__ int rv() const { return ci.rv; }
     __device__ __forceinline__ void build_cols(const BicData &d, uint32_t mask, SetCols &sc) const {
         // child first with stride 1, then the parents in ascending variable index
         sc.col[0] = d.codes + (int64_t)ci.v * d.n_stride;
@@ -99,6 +100,34 @@ struct MaskSets {
         sc.cells = base;
         sc.tval = pen;
         sc.out = mask;
+    }
+};
+
+// The entries of one launch share the child arity `child_rv` (bic_score_tables_kernel and the fNML table take one per launch).
+// Columns, cell count and penalty are built exactly as MaskSets builds them; the score goes to the entry's position.
+struct ListSets {
+    const ListEntry *ent;
+    const int *par;     // parents of all entries, ascending per entry
+    const int *card;    // [p]
+    int child_rv;
+    __host__ __device__ __forceinline__ int rv() const { return child_rv; }
+    __device__ __forceinline__ void build_cols(const BicData &d, uint32_t key, SetCols &sc) const {
+        const ListEntry e = ent[key];
+        sc.col[0] = d.codes + (int64_t)e.v * d.n_stride;
+        sc.stride[0] = 1;
+        uint32_t base = (uint32_t)child_rv;
+        float pen = (float)(child_rv - 1);
+        for (int i = 0; i < e.k; i++) {
+            const int q = __ldg(par + e.off + i), cd = __ldg(card + q);
+            sc.col[i + 1] = d.codes + (int64_t)q * d.n_stride;
+            sc.stride[i + 1] = base;
+            base *= (uint32_t)cd;
+            pen = __fmul_rn(pen, (float)cd);
+        }
+        sc.ncols = e.k + 1;
+        sc.cells = base;
+        sc.tval = pen;
+        sc.out = key;
     }
 };
 

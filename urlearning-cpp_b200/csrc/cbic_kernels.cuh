@@ -339,17 +339,32 @@ __device__ __forceinline__ double cbic_the_score64(double rss, int k, const Cbic
     return prm.n * (cbic_log(rss) - prm.log_n) + prm.lam_logn * (double)k;
 }
 
-// One parent set (urlgpu_score_one, the per-set ScoringFunction::calculateScore plug-in): one warp sweeps every candidate
-// out of the (k+1)x(k+1) sub-Gram over (v, S), highest first — the same sequence of FMAs the family kernels apply to this
-// set — and writes RSS -> the_score.  O(k^3) work, no 2^k tables.
-__global__ void cbic_one_kernel(const double *__restrict__ sub, int k, CbicParams prm, double *__restrict__ out /*[2]: the_score, rss*/) {
+// Listed parent sets (urlgpu_score_sets; urlgpu_score_one is a list of one): one warp per set gathers the packed sub-Gram over
+// (v, parents ascending) from the p x p Gram into its slice of shared memory — the order of cbic_sub_gram — and sweeps every
+// parent out, highest first: the sequence of FMAs the family kernels apply to this set.  O(k^3) work, no 2^k tables.  One
+// launch covers the sets of one size k; `work` lists their keys (positions in the caller's list), the outputs go to the key:
+// the_score in FP64 and the float score -the_score.
+__global__ void cbic_sets_kernel(const double *__restrict__ gram, int p, const ListEntry *__restrict__ ent, const int *__restrict__ par,
+                                 const uint32_t *__restrict__ work, uint32_t count, int k, CbicParams prm, float *__restrict__ scores,
+                                 double *__restrict__ the_score) {
     extern __shared__ double smat[];
-    const int lane = threadIdx.x;
-    const int tsz = (k + 1) * (k + 2) / 2;
-    for (int e = lane; e < tsz; e += 32) smat[e] = sub[e];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t i = blockIdx.x * (blockDim.x >> 5) + warp;
+    if (i >= count) return;
+    const uint32_t key = work[i];
+    const ListEntry e = ent[key];
+    double *A = smat + (size_t)warp * ((k + 1) * (k + 2) / 2);
+    for (int a = 0; a <= k; a++) {
+        const double *row = gram + (size_t)(a == 0 ? e.v : par[e.off + a - 1]) * p;
+        for (int b = lane; b <= a; b += 32) A[tri(a, b)] = row[b == 0 ? e.v : par[e.off + b - 1]];
+    }
     __syncwarp();
-    for (int piv = k; piv >= 1; piv--) cbic_warp_sweep(smat, piv, prm.piv_tol, lane);
-    if (lane == 0) { out[0] = cbic_the_score64(smat[0], k, prm); out[1] = smat[0]; }
+    for (int piv = k; piv >= 1; piv--) cbic_warp_sweep(A, piv, prm.piv_tol, lane);
+    if (lane == 0) {
+        const double ts = cbic_the_score64(A[0], k, prm);
+        the_score[key] = ts;
+        scores[key] = -__double2float_rn(ts); // BIC_OLS.cpp:223,245,275
+    }
 }
 
 // Level B: template-recursive DFS over the J low candidate bits.  A has (j+1)(j+2)/2 packed entries over

@@ -13,6 +13,14 @@ __device__ __forceinline__ bool is_sentinel(float x) { return __float_as_uint(x)
 constexpr int kMaxDenseCand = 30;   // dense-by-compact-mask tables: 2^c floats
 constexpr int kMaxCols = 32;        // columns of one contingency table (|S|+1)
 
+// One entry of a caller's list of parent sets (urlgpu_score_sets): the child, its parent count and the first of its parents
+// in a separate array of variable indices (ascending per entry).  Shared by K1 (ListSets) and K3 (cbic_sets_kernel).
+struct ListEntry {
+    int v;
+    int k;
+    uint32_t off;
+};
+
 __device__ __forceinline__ long long warp_sum_ll(long long v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);

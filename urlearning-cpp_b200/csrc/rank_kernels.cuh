@@ -78,7 +78,7 @@ __global__ void rank_store_rule_kernel(float *__restrict__ scores, uint32_t tota
 // One thread scores kRankRun consecutive sets of layer L: unrank the first, colex successor for the rest.  The set's
 // (L+1)x(L+1) sub-Gram over (v, e_1..e_L) is gathered from the candidate Gram (packed lower triangle over (v, cand_0, ..),
 // indexed by tri(): members ascend, so every entry read is G[tri(pos[a], pos[b])] with pos[a] >= pos[b]) and the
-// candidates are swept out highest first — the FMA sequence of cbic_roots_kernel / cbic_sweep / cbic_one_kernel.
+// candidates are swept out highest first — the FMA sequence of cbic_roots_kernel / cbic_sweep / cbic_sets_kernel.
 // Pivot guard: see CbicParams::piv_tol (cbic_kernels.cuh).
 constexpr int kRankRun = 4;
 
@@ -297,7 +297,7 @@ struct RankSets {
     RankSpace rs;
     RankCand rc;
     int by_mask;
-    __device__ __forceinline__ int rv() const { return rc.rv; }
+    __host__ __device__ __forceinline__ int rv() const { return rc.rv; }
     __device__ __forceinline__ void build_cols(const BicData &d, uint32_t idx, SetCols &sc) const {
         const int l = rs_layer_of(rs, idx);
         uint8_t e[kMaxRankLayers];
