@@ -22,6 +22,7 @@
  *   urlgpu_score_one         ScoringFunction::calculateScore          scoring_function/scoring_function.h:19
  *   urlgpu_contingency       ADTree::makeContab                       ad_tree/ad_tree.cpp:95-137
  *   urlgpu_spg_build/query   SparseParentBitwise::initialize/getScore  score_cache/sparse_parent_bitwise.cpp:24-110
+ *   urlgpu_order_search      run_astar_on_one_scc (order-graph search) astar/astar_main.cpp:216-546
  *   urlgpu_prune             ScoreCalculator::prune                   scoring_function/score_calculator.cpp:150-197
  *   urlgpu_result_*          FloatMap iteration in scoringThread      score/score_main.cpp:187-200, base/typedefs.h:816
  *
@@ -194,6 +195,27 @@ int urlgpu_spg_query(urlgpu_spg *spg, const uint64_t *allowed /* nq*mask_words *
                      int64_t *best_index /* optional */);
 int urlgpu_spg_free(urlgpu_spg *spg);
 
+/* The optimal DAG of one skeleton component over the order graph, layer by layer on the device: the search of
+ * astar/astar_main.cpp:216-546 (run_astar_on_one_scc, ancestors = 0) with the cached-subset look-up of
+ * score_cache/sparse_parent_{list,bitwise}.cpp.  Entries of variable v: masks[offsets[v]..offsets[v+1]) (mask_words words
+ * each) with scores in the SEARCH side's sign (lower is better, score_cache.cpp:151).  edges: p*mask_words skeleton
+ * neighbourhoods or NULL.  Writes *cost, order[0..|C|) (first = a root) and parents[v*mask_words..] for v in C.
+ *
+ * best(v, U) is the first entry of v, in (score, |S|, mask) order, whose parent set lies inside U (FLT_MAX if none; entries
+ * with a parent outside the component never qualify).  S is reached from S\{v} if S\{v} is reached, the leaf v touches
+ * S\{v} in the skeleton (or S\{v} is empty, or there is no skeleton) and g = cost(S\{v}) + best(v, S\{v}), one float32
+ * addition, is not +inf; cost(S) is the least such g and the leaf the smallest v attaining it.  *cost is therefore the least
+ * float32 left-to-right path sum over the admissible orders: never above A*'s goal cost, and equal to it in exact
+ * arithmetic.  Among orders of equal cost the DAG may differ from A*'s.
+ * Device memory: 5*2^|C| bytes (cost + leaf per node) plus 4*2^c_v per variable (c_v = its candidate parents inside C)
+ * plus the entries, from the context's caching allocator.  Refusals, all before any launch: p < 1, mask_words outside 1..4,
+ * decreasing offsets, an empty component or one naming a variable >= p, a NaN score and an entry containing its own
+ * variable (URLGPU_ERR_ARG); |C| > 32 and a call that does not fit the device's free memory (URLGPU_ERR_LIMIT, with the
+ * bytes).  No admissible order, or a cost of +inf: URLGPU_ERR_ARG with A*'s message "No solution found.". */
+int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                        const float *scores, const uint64_t *edges, const uint64_t *component,
+                        float *cost, int32_t *order, uint64_t *parents);
+
 /* Measurement hooks: device time (CUDA events on the context's stream) and launch counts per kernel family,
  * accumulated since the last reset. */
 typedef struct urlgpu_stats {
@@ -215,6 +237,8 @@ typedef struct urlgpu_stats {
     double k1_bytes_written;   /* cube path: bytes of contingency tables the K1 kernels store */
     double ms_standardise;     /* K2: column moments + standardisation passes (HBM bound); ms_gram is the DMMA Gram kernel + combine */
     uint64_t table16_fallbacks; /* K1 cube path: variables recomputed with 32-bit tables because a cell count did not fit 16 bits */
+    double ms_order_tables;    /* urlgpu_order_search: best-parent tables (fill, scatter, subset-min transform) */
+    double ms_order_layers;    /* urlgpu_order_search: layer sweeps and the backtrack */
 } urlgpu_stats;
 int urlgpu_stats_reset(urlgpu_ctx *ctx);
 int urlgpu_stats_get(urlgpu_ctx *ctx, urlgpu_stats *out);

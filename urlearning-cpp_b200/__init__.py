@@ -37,7 +37,7 @@ ABI_SYMBOLS = [
     "urlgpu_stats_enable_timing", "urlgpu_probe_fp64", "urlgpu_family_size", "urlgpu_score_range", "urlgpu_result_from_scores", "urlgpu_score_part",
     "urlgpu_spg_build", "urlgpu_spg_query", "urlgpu_spg_free",
     "urlgpu_peer_alloc", "urlgpu_peer_open", "urlgpu_peer_close", "urlgpu_peer_free",
-    "urlgpu_result_fetch_device", "urlgpu_copy_to_host",
+    "urlgpu_result_fetch_device", "urlgpu_copy_to_host", "urlgpu_order_search",
 ]
 
 
@@ -54,7 +54,8 @@ class Stats(C.Structure):
         ("ms_prune", C.c_double), ("ms_gram", C.c_double),
         ("sets_scored", C.c_uint64), ("algorithmic_bytes", C.c_double), ("algorithmic_flops", C.c_double), ("gram_flops", C.c_double),
         ("launches_tree", C.c_uint64), ("ms_tree", C.c_double), ("k1_bytes_read", C.c_double), ("k1_bytes_written", C.c_double),
-        ("ms_standardise", C.c_double), ("table16_fallbacks", C.c_uint64),
+        ("ms_standardise", C.c_double), ("table16_fallbacks", C.c_uint64), ("ms_order_tables", C.c_double),
+        ("ms_order_layers", C.c_double),
     ]
 
     def as_dict(self):
@@ -121,6 +122,7 @@ def load_library():
     lib.urlgpu_score_range.argtypes = [vp, i32, vp, i32, i32, i32, C.c_double, u64, u64, vp, i32]
     lib.urlgpu_score_part.argtypes = [vp, i32, vp, i32, i32, i32, C.c_double, i32, i32, vp, i32]
     lib.urlgpu_result_from_scores.argtypes = [vp, i32, vp, i32, i32, i32, vp, u64, i32, C.c_uint, P(vp)]
+    lib.urlgpu_order_search.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, P(C.c_float), vp, vp]
     for name in ABI_SYMBOLS:
         if name not in ("urlgpu_last_error", "urlgpu_host_alloc", "urlgpu_host_free"):
             getattr(lib, name).restype = C.c_int
@@ -156,6 +158,27 @@ def two_hop_neighbors(edges: Sequence[int] | None, p: int, v: int) -> int:
     for j in range(p):
         if (orig >> j) & 1 and j != v:
             out |= nb(j)
+    return out
+
+
+def components(p: int, edges: Sequence[int] | None) -> list[int]:
+    """urlsearch::components (host/search_host.hpp:435-456, skeleton.cpp:187-230): the connected components of the skeleton
+    as variable masks, in the order of their smallest variable; ``edges=None`` = one component of all p variables."""
+    if edges is None:
+        return [(1 << p) - 1]
+    out, visited = [], 0
+    for v in range(p):
+        if (visited >> v) & 1:
+            continue
+        comp, stack = 0, [v]
+        while stack:
+            u = stack.pop()
+            if (visited >> u) & 1:
+                continue
+            visited |= 1 << u
+            comp |= 1 << u
+            stack.extend(i for i in range(p - 1, -1, -1) if (int(edges[u]) >> i) & 1 and not (visited >> i) & 1)
+        out.append(comp)
     return out
 
 
@@ -452,6 +475,64 @@ class Engine:
         self._check(self.lib.urlgpu_score_sets(self._h, n, var.ctypes.data, pm.ctypes.data, max(pm.shape[1], 1), score_type, float(lam),
                                                scores.ctypes.data, values.ctypes.data))
         return scores, values
+
+    def order_search(self, entries, p: int, component: int, edges: Sequence[int] | None = None):
+        """urlgpu_order_search: the optimal DAG of one skeleton component over the order graph, layer by layer on the device.
+        entries: p pairs (masks, scores) per variable in the search side's sign (lower is better), masks uint64 [n] or
+        [n, words] or ints; component: a variable mask; edges: p skeleton masks or None.
+        -> (float32 cost, order list (first = a root), parents uint64 [p] ([p, words] above 64 variables; 0 outside C))"""
+        if len(entries) != p:
+            raise ValueError(f"{len(entries)} entry lists for {p} variables")
+        words = mask_words_for(p)
+        rows, sc, offsets = [], [], np.zeros(p + 1, dtype=np.uint64)
+        for v, (m, s_) in enumerate(entries):
+            if isinstance(m, np.ndarray) and m.dtype == np.uint64:
+                m = m.reshape(-1, 1) if m.ndim == 1 else m
+                mm = np.zeros((len(m), words), dtype=np.uint64)
+                mm[:, :min(words, m.shape[1])] = m[:, :words]
+            else:
+                mm = np.array([mask_to_words(int(x), words) for x in m], dtype=np.uint64).reshape(-1, words)
+            rows.append(mm)
+            sc.append(np.asarray(s_, dtype=np.float32).reshape(-1))
+            if len(sc[-1]) != len(mm):
+                raise ValueError(f"variable {v}: {len(mm)} masks but {len(sc[-1])} scores")
+            offsets[v + 1] = offsets[v] + len(mm)
+        masks = np.ascontiguousarray(np.concatenate(rows) if rows else np.zeros((0, words), dtype=np.uint64))
+        scores = np.ascontiguousarray(np.concatenate(sc) if sc else np.zeros(0, dtype=np.float32))
+        comp = mask_to_words(int(component), words)
+        ed = None if edges is None else np.ascontiguousarray(np.stack([mask_to_words(int(e), words) for e in edges]))
+        if ed is not None and len(ed) != p:
+            raise ValueError(f"{len(ed)} skeleton rows for {p} variables")
+        cost = C.c_float()
+        order = np.zeros(max(1, bin(int(component)).count("1")), dtype=np.int32)
+        parents = np.zeros((p, words), dtype=np.uint64)
+        self._check(self.lib.urlgpu_order_search(self._h, p, words, offsets.ctypes.data, masks.ctypes.data if len(masks) else None,
+                                                 scores.ctypes.data if len(scores) else None, None if ed is None else ed.ctypes.data,
+                                                 comp.ctypes.data, C.byref(cost), order.ctypes.data, parents.ctypes.data))
+        return np.float32(cost.value), [int(x) for x in order], parents[:, 0].copy() if words == 1 else parents
+
+    def optimal_dag(self, cache, edges: Sequence[int] | None = None):
+        """urlsearch_astar (host/search_capi.cpp:64-94) with urlgpu_order_search in place of A*: the skeleton's components
+        (the rule of urlsearch::components), one search each, their costs summed in float32 in component order.
+        cache: a search.ScoreCache or a list of p (masks, scores) pairs in search sign; edges: p skeleton masks or None.
+        -> (total cost, parents uint64 [p]), the meaning and types of ScoreCache.astar's first two results"""
+        if hasattr(cache, "entries") and hasattr(cache, "p"):
+            p = cache.p
+            entries = [cache.entries(v) for v in range(p)]
+        else:
+            entries = list(cache)
+            p = len(entries)
+        total = np.float32(0)
+        parents = None
+        for comp in components(p, edges):
+            cost, _, par = self.order_search(entries, p, comp, edges)
+            total = np.float32(total + cost)
+            if parents is None:
+                parents = np.zeros_like(par)
+            for v in range(p):
+                if (comp >> v) & 1:
+                    parents[v] = par[v]
+        return float(total), parents
 
     def contingency(self, variable: int, parents: int, n_cells: int) -> np.ndarray:
         words = mask_words_for(self.p)

@@ -1,0 +1,173 @@
+// order_kernels.cuh — exact structure search over the order graph of one skeleton component, layer by layer (sm_100a).
+//
+// The search space of run_astar_on_one_scc (astar/astar_main.cpp:216-546, host/search_host.hpp:367-432): the nodes are the
+// subsets S of a component C (k = |C| <= 32 variables), S is reached from S\{v} by adding the leaf v with its best cached
+// parent set inside S\{v}, and the goal is C.  A* keeps a hash map and a heap over the nodes it generates (~70-80 bytes
+// each); here the whole graph is stored densely, 5 bytes a node (float cost + uint8 leaf, indexed by the k-bit compact mask
+// over C's positions), and swept once, one launch per layer, so every node is final when the next layer reads it.
+//
+//   best(v, U)  the first entry of v's cache, in (score, |S|, mask) order, whose parent set is inside U.  Each variable gets a
+//               dense uint32 table T_v over the lattice of its candidates cand_v (the union of its entries inside C, c_v <= 31
+//               bits): T_v[U] = the SORTED POSITION of best(v, U), kOrderNone if there is none.  Built by scattering every
+//               entry's position to its compact mask (atomicMin: duplicates keep the first) and a subset-min transform,
+//               T[U] = min(T[U], T[U\b]) for every bit b: the low kOrderSegBits bits per 2048-entry segment in shared memory
+//               (order_table_low_kernel), each higher bit in one coalesced global pass (order_table_high_kernel).  Positions
+//               order like the sparse parent list, so the list's tie rule comes for free and a look-up is one gather.
+//   layer l     order_layer_kernel: one thread takes kOrderRun consecutive colex nodes of the layer (unrank the first with the
+//               shared-memory binomial table, Gosper successor for the rest).  For every v in S, ascending: the skeleton
+//               test (astar_main.cpp:300-307: the leaf must touch S\{v} unless S\{v} is empty), cost[S\v], the compaction
+//               of S\v into cand_v's bits through four byte look-up tables in shared memory, T_v, the score, and
+//               g = cost + score rounded once (__fadd_rn).  cost[S] = min g, leaf[S] = the smallest v attaining it; a node
+//               with no admissible predecessor gets cost +inf and leaf kOrderUnreached.
+//   backtrack   order_backtrack_kernel, one thread: walks leaf[] back from C and writes the cost, the k leaves and the k
+//               sorted positions of their parent sets into one small buffer.
+//
+// Bound: a layer reads 4 + 4 bytes (cost, table) per (S, v) pair, k 2^(k-1) pairs in all, at addresses that differ from
+// node to node: HBM and L2 sector traffic, not arithmetic, sets the time.
+#pragma once
+#include "common.cuh"
+
+namespace urlgpu {
+
+constexpr int kOrderMaxVars = 32;
+constexpr int kOrderSegBits = 11;            // 2048-entry segments of the subset-min transform (8 KB of shared memory)
+constexpr int kOrderRun = 4;                 // consecutive colex nodes per thread and grid-stride step
+constexpr int kOrderBinom = kOrderMaxVars + 1;
+constexpr int kOrderBinomWords = (kOrderBinom * kOrderBinom + 3) / 4 * 4;   // padded so the OrderVar array after it stays aligned
+constexpr uint32_t kOrderNone = 0xFFFFFFFFu; // T_v: no cached subset (best = FLT_MAX)
+constexpr uint8_t kOrderUnreached = 0xFF;    // leaf[]: no admissible predecessor
+
+struct OrderVar {            // variable at position j of C
+    unsigned long long table; // offset of T_j in the table buffer (uint32 elements)
+    uint32_t score;           // offset of j's sorted scores
+    uint32_t adj;             // skeleton neighbours as a compact mask over C; all ones without a skeleton
+    uint32_t cand;            // cand_j as a compact mask over C
+    uint8_t shift[4];         // popcount of cand_j below byte b: where byte b's compacted bits go
+};
+
+__host__ __device__ __forceinline__ size_t order_smem_bytes(int k) {
+    return (size_t)kOrderBinomWords * sizeof(uint32_t) + (size_t)k * sizeof(OrderVar) + (size_t)k * 1024;
+}
+
+// ------------------------------------------------------------------------------------------------ best-parent tables
+// T[where[i]] = min(T[where[i]], pos[i])
+__global__ void __launch_bounds__(256) order_scatter_kernel(const unsigned long long *__restrict__ where, const uint32_t *__restrict__ pos, uint64_t n,
+                                                            uint32_t *__restrict__ T) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) atomicMin(T + __ldg(where + i), __ldg(pos + i));
+}
+
+// the low `bits` bits of the subset-min transform of one table, one 2^bits segment per CTA
+__global__ void __launch_bounds__(1024) order_table_low_kernel(uint32_t *__restrict__ T, int bits) {
+    __shared__ uint32_t s[1 << kOrderSegBits];
+    const uint32_t n = 1u << bits;
+    uint32_t *seg = T + ((size_t)blockIdx.x << bits);
+    for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) s[i] = seg[i];
+    __syncthreads();
+    for (int b = 0; b < bits; b++) {
+        for (uint32_t i = threadIdx.x; i < n / 2; i += blockDim.x) {
+            const uint32_t u = ((i >> b) << (b + 1)) | (i & ((1u << b) - 1));   // bit b clear
+            s[u | (1u << b)] = min(s[u | (1u << b)], s[u]);
+        }
+        __syncthreads();
+    }
+    for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) seg[i] = s[i];
+}
+
+// one bit b >= kOrderSegBits of the transform: T[U | b] = min(T[U | b], T[U]) for the 2^(c-1) masks U without b
+__global__ void __launch_bounds__(256) order_table_high_kernel(uint32_t *__restrict__ T, int b, uint64_t half) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= half) return;
+    const uint64_t u = ((i >> b) << (b + 1)) | (i & ((1ull << b) - 1));
+    const uint64_t w = u | (1ull << b);
+    T[w] = min(T[w], T[u]);
+}
+
+// ------------------------------------------------------------------------------------------------ layer sweep
+// rank r of layer l -> the k-bit mask with that colex rank (B[b * kOrderBinom + i] = C(b, i))
+__device__ __forceinline__ uint32_t order_unrank(const uint32_t *B, int k, int l, uint32_t r) {
+    uint32_t S = 0;
+    int hi = k - 1;
+    for (int i = l; i >= 1; i--) {
+        int lo = i - 1, h = hi;                   // largest b in [i-1, hi] with C(b, i) <= r
+        while (lo < h) {
+            const int mid = (lo + h + 1) >> 1;
+            if (B[mid * kOrderBinom + i] <= r) lo = mid; else h = mid - 1;
+        }
+        S |= 1u << lo;
+        r -= B[lo * kOrderBinom + i];
+        hi = lo - 1;
+    }
+    return S;
+}
+// next mask with the same popcount (Gosper); never called on the last mask of a layer, so x + low stays below 2^32
+__device__ __forceinline__ uint32_t order_next(uint32_t x) {
+    const uint32_t low = x & (~x + 1), r = x + low;
+    return r | (((x ^ r) >> 2) >> (__ffs(x) - 1));
+}
+
+__global__ void __launch_bounds__(256) order_layer_kernel(const OrderVar *__restrict__ vars, const uint8_t *__restrict__ lut, const uint32_t *__restrict__ binom,
+                                                          const uint32_t *__restrict__ T, const float *__restrict__ scores, int k, int layer,
+                                                          uint32_t count, float *__restrict__ cost, uint8_t *__restrict__ leaf) {
+    extern __shared__ __align__(16) unsigned char order_smem[];
+    uint32_t *s_binom = reinterpret_cast<uint32_t *>(order_smem);
+    OrderVar *s_var = reinterpret_cast<OrderVar *>(s_binom + kOrderBinomWords);
+    uint8_t *s_lut = reinterpret_cast<uint8_t *>(s_var + k);
+    for (int i = threadIdx.x; i < kOrderBinom * kOrderBinom; i += blockDim.x) s_binom[i] = __ldg(binom + i);
+    for (int i = threadIdx.x; i < k; i += blockDim.x) s_var[i] = vars[i];
+    for (int i = threadIdx.x; i < k * 256; i += blockDim.x) reinterpret_cast<uint32_t *>(s_lut)[i] = __ldg(reinterpret_cast<const uint32_t *>(lut) + i);
+    __syncthreads();
+    const uint32_t runs = (count + kOrderRun - 1) / kOrderRun;
+    for (uint32_t run = blockIdx.x * blockDim.x + threadIdx.x; run < runs; run += gridDim.x * blockDim.x) {
+        const uint32_t first = run * kOrderRun;
+        const uint32_t nrun = min((uint32_t)kOrderRun, count - first);
+        uint32_t S = order_unrank(s_binom, k, layer, first);
+        for (uint32_t u = 0; u < nrun; u++) {
+            float best = __int_as_float(0x7f800000);
+            uint32_t best_leaf = kOrderUnreached;
+            for (uint32_t m = S; m; m &= m - 1) {
+                const int v = __ffs(m) - 1;
+                const uint32_t prev = S ^ (1u << v);
+                const OrderVar &V = s_var[v];
+                if (prev && !(prev & V.adj)) continue;                 // the leaf must touch the sub-network
+                const float c = __ldg(cost + prev);
+                if (c == __int_as_float(0x7f800000)) continue;        // S\v unreached
+                const uint8_t *L = s_lut + v * 1024;
+                const uint32_t idx = (uint32_t)L[prev & 255] | ((uint32_t)L[256 + ((prev >> 8) & 255)] << V.shift[1]) |
+                                     ((uint32_t)L[512 + ((prev >> 16) & 255)] << V.shift[2]) | ((uint32_t)L[768 + (prev >> 24)] << V.shift[3]);
+                const uint32_t pos = __ldg(T + V.table + idx);
+                const float s = pos == kOrderNone ? 3.402823466e+38f : __ldg(scores + V.score + pos);
+                const float g = __fadd_rn(c, s);
+                if (g == __int_as_float(0x7f800000)) continue;
+                if (g < best) { best = g; best_leaf = (uint32_t)v; }   // strict: the smallest v among equal costs
+            }
+            cost[S] = best;
+            leaf[S] = (uint8_t)best_leaf;
+            if (u + 1 < nrun) S = order_next(S);
+        }
+    }
+}
+
+// out[0] = cost(C) bits, out[1] = 1 iff C was reached, out[2 + i] = leaf at step i of the order, out[2 + k + i] = its position
+__global__ void order_backtrack_kernel(const OrderVar *__restrict__ vars, const uint32_t *__restrict__ T, const float *__restrict__ cost,
+                                       const uint8_t *__restrict__ leaf, int k, uint32_t *__restrict__ out) {
+    if (blockIdx.x | threadIdx.x) return;
+    uint32_t S = k == 32 ? 0xFFFFFFFFu : (1u << k) - 1;
+    out[0] = __float_as_uint(cost[S]);
+    out[1] = 0;
+    for (int i = k - 1; i >= 0; i--) {
+        const uint32_t v = leaf[S];
+        if (v == kOrderUnreached) return;
+        const uint32_t prev = S ^ (1u << v);
+        uint32_t idx = 0;
+        int j = 0;
+        for (uint32_t m = vars[v].cand; m; m &= m - 1, j++)
+            if ((prev >> (__ffs(m) - 1)) & 1) idx |= 1u << j;
+        out[2 + i] = v;
+        out[2 + k + i] = T[vars[v].table + idx];
+        S = prev;
+    }
+    out[1] = 1;
+}
+
+} // namespace urlgpu

@@ -22,6 +22,7 @@
 #include "cbic_kernels.cuh"
 #include "rank_kernels.cuh"
 #include "spg_kernels.cuh"
+#include "order_kernels.cuh"
 #include "regret.hpp"
 
 using namespace urlgpu;
@@ -33,7 +34,7 @@ namespace {
 thread_local std::string g_create_error;
 std::atomic<int> g_ctx_on_device[64];   // live contexts per device: each budgets its share of the free memory
 
-enum Family { F_COUNT = 0, F_CUBE, F_CBIC, F_ACCEPT, F_PRUNE, F_GRAM, F_OTHER, F_STD, F_N };
+enum Family { F_COUNT = 0, F_CUBE, F_CBIC, F_ACCEPT, F_PRUNE, F_GRAM, F_OTHER, F_STD, F_ORDER_TABLES, F_ORDER_LAYERS, F_N };
 
 struct EvPair { cudaEvent_t a, b; int fam; };
 
@@ -217,7 +218,8 @@ void fold_events(urlgpu_ctx *ctx) {
         if (cudaEventElapsedTime(&ms, ep.a, ep.b) == cudaSuccess) {
             double *dst = ep.fam == F_COUNT ? &ctx->st.ms_count : ep.fam == F_CUBE ? &ctx->st.ms_cube : ep.fam == F_CBIC ? &ctx->st.ms_cbic
                         : ep.fam == F_ACCEPT ? &ctx->st.ms_accept : ep.fam == F_PRUNE ? &ctx->st.ms_prune : ep.fam == F_GRAM ? &ctx->st.ms_gram
-                        : ep.fam == F_STD ? &ctx->st.ms_standardise : nullptr;
+                        : ep.fam == F_STD ? &ctx->st.ms_standardise : ep.fam == F_ORDER_TABLES ? &ctx->st.ms_order_tables
+                        : ep.fam == F_ORDER_LAYERS ? &ctx->st.ms_order_layers : nullptr;
             if (dst) *dst += ms;
         }
         ctx->free_events.push_back(ep.a);
@@ -2525,6 +2527,200 @@ extern "C" int urlgpu_spg_free(urlgpu_spg *sp) {
     cudaStreamSynchronize(sp->ctx->stream);
     cudaFree(sp->d_masks); cudaFree(sp->d_scores); cudaFree(sp->d_not_used);
     delete sp;
+    return URLGPU_OK;
+}
+
+// ============================================================================================ order-graph search
+// urlgpu_order_search (order_kernels.cuh).  The host validates everything, translates the component's qualifying entries to
+// compact masks over C's positions once, sorts each variable's list in the (score, |S|, mask) order of SortedEntries::build,
+// and sizes the call before any allocation.  One upload of the small arrays, the table passes, k layer launches, one
+// backtrack and one copy back; the host then maps each leaf's sorted position to its parent mask.
+extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks, const float *scores,
+                                   const uint64_t *edges, const uint64_t *component, float *cost, int32_t *order, uint64_t *parents) {
+    if (!ctx) return URLGPU_ERR_ARG;
+    auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, "order_search: " + m); };
+    if (!offsets || !component || !cost || !order || !parents) return refuse(URLGPU_ERR_ARG, "null argument");
+    if (p < 1) return refuse(URLGPU_ERR_ARG, "p must be at least 1");
+    if (mask_words < 1 || mask_words > kSpgMaxWords) return refuse(URLGPU_ERR_ARG, "mask_words must be in 1.." + std::to_string(kSpgMaxWords));
+    if ((int64_t)mask_words * 64 < p) return refuse(URLGPU_ERR_ARG, "mask_words too small for the variable count");
+    for (int v = 0; v < p; v++)
+        if (offsets[v + 1] < offsets[v]) return refuse(URLGPU_ERR_ARG, "offsets decrease at variable " + std::to_string(v));
+    if (offsets[p] > offsets[0] && (!masks || !scores)) return refuse(URLGPU_ERR_ARG, "null entries");
+    auto bit = [&](const uint64_t *m, int v) { return (m[v >> 6] >> (v & 63)) & 1; };
+    std::vector<int> vars;                       // position j of C -> variable
+    std::vector<int> pos_of(p, -1);
+    for (int w = 0; w < mask_words; w++)
+        for (int b = 0; b < 64; b++) {
+            if (!((component[w] >> b) & 1)) continue;
+            if (w * 64 + b >= p) return refuse(URLGPU_ERR_ARG, "the component names variable " + std::to_string(w * 64 + b) + " >= p");
+            pos_of[w * 64 + b] = (int)vars.size();
+            vars.push_back(w * 64 + b);
+        }
+    if (vars.empty()) return refuse(URLGPU_ERR_ARG, "empty component");
+    for (int v = 0; v < p; v++)
+        for (uint64_t e = offsets[v]; e < offsets[v + 1]; e++) {
+            if (std::isnan(scores[e])) return refuse(URLGPU_ERR_ARG, "variable " + std::to_string(v) + ", entry " + std::to_string(e - offsets[v]) + ": NaN score");
+            if (bit(masks + e * mask_words, v)) return refuse(URLGPU_ERR_ARG, "variable " + std::to_string(v) + ", entry " + std::to_string(e - offsets[v]) + ": the parent set contains the variable itself");
+        }
+    const int k = (int)vars.size();
+    if (k > kOrderMaxVars) return refuse(URLGPU_ERR_LIMIT, std::to_string(k) + " variables in the component; at most " + std::to_string(kOrderMaxVars) + " are supported");
+
+    // qualifying entries (all parents inside C), compact masks, per-variable sort
+    std::vector<uint64_t> Cmask(component, component + mask_words);
+    std::vector<std::vector<uint64_t>> ent(k);   // per position: indices into masks/scores, sorted
+    std::vector<std::vector<uint32_t>> cm(k);    // compact masks in the same order
+    std::vector<OrderVar> hv(k);
+    auto compact = [&](const uint64_t *m) {
+        uint32_t c = 0;
+        for (int j = 0; j < k; j++) if (bit(m, vars[j])) c |= 1u << j;
+        return c;
+    };
+    uint64_t n_ent = 0, table_elems = 0;
+    for (int j = 0; j < k; j++) {
+        const int v = vars[j];
+        auto &E = ent[j];
+        for (uint64_t e = offsets[v]; e < offsets[v + 1]; e++) {
+            bool inside = true;
+            for (int w = 0; w < mask_words && inside; w++) inside = (masks[e * mask_words + w] & ~Cmask[w]) == 0;
+            if (inside) E.push_back(e);
+        }
+        auto card = [&](uint64_t i) { int c = 0; for (int w = 0; w < mask_words; w++) c += __builtin_popcountll(masks[i * mask_words + w]); return c; };
+        std::sort(E.begin(), E.end(), [&](uint64_t a, uint64_t b) {   // as urlgpu_spg_build (sparse_parent_list.cpp:7-9, ties by |S|, mask)
+            if (scores[a] != scores[b]) return scores[a] < scores[b];
+            const int ca = card(a), cb = card(b);
+            if (ca != cb) return ca < cb;
+            for (int w = mask_words - 1; w >= 0; w--)
+                if (masks[a * mask_words + w] != masks[b * mask_words + w]) return masks[a * mask_words + w] < masks[b * mask_words + w];
+            return a < b;
+        });
+        if (E.size() > 0xFFFFFFFEull) return refuse(URLGPU_ERR_LIMIT, "variable " + std::to_string(v) + " has 2^32 or more entries inside the component");
+        uint32_t cand = 0;
+        for (uint64_t e : E) { cm[j].push_back(compact(masks + e * mask_words)); cand |= cm[j].back(); }
+        hv[j].table = table_elems;
+        hv[j].score = (uint32_t)n_ent;
+        hv[j].cand = cand;
+        hv[j].adj = 0xFFFFFFFFu;
+        if (edges) hv[j].adj = compact(edges + (size_t)v * mask_words);
+        for (int b = 0; b < 4; b++) hv[j].shift[b] = (uint8_t)__builtin_popcount(b ? cand & (0xFFFFFFFFu >> (32 - 8 * b)) : 0u);
+        table_elems += (uint64_t)1 << __builtin_popcount(cand);
+        n_ent += E.size();
+    }
+    if (n_ent > 0xFFFFFFFFull) return refuse(URLGPU_ERR_LIMIT, "2^32 or more entries inside the component");
+
+    // the device memory of the call, before anything is allocated
+    const uint64_t nodes = (uint64_t)1 << k;
+    const size_t small_bytes = (size_t)k * sizeof(OrderVar) + (size_t)k * 1024 + (size_t)kOrderBinom * kOrderBinom * 4 + (2 + 2 * (size_t)k) * 4;
+    const size_t need = 5 * nodes + 4 * table_elems + n_ent * (8 + 4 + 4) + small_bytes;
+    CK(cudaSetDevice(ctx->device));
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    for (auto &b : ctx->pool) if (!b.used) free_b += b.bytes;      // cached blocks the allocator can hand out or release
+    auto bytes_msg = [&]() {
+        return std::to_string(need) + " bytes of device memory (" + std::to_string(5 * nodes) + " for the 2^" + std::to_string(k) + " nodes, " +
+               std::to_string(4 * table_elems) + " for the best-parent tables)";
+    };
+    if (need > free_b) return refuse(URLGPU_ERR_LIMIT, "the search needs " + bytes_msg() + ", " + std::to_string(free_b) + " are free");
+
+    // host arrays: binomials, byte look-up tables, scatter list, sorted scores
+    std::vector<uint32_t> binom(kOrderBinom * kOrderBinom, 0);
+    for (int b = 0; b < kOrderBinom; b++)
+        for (int i = 0; i <= b; i++) binom[b * kOrderBinom + i] = i == 0 || i == b ? 1u : binom[(b - 1) * kOrderBinom + i - 1] + binom[(b - 1) * kOrderBinom + i];
+    std::vector<uint8_t> lut((size_t)k * 1024);
+    for (int j = 0; j < k; j++)
+        for (int b = 0; b < 4; b++) {
+            const uint32_t cb = (hv[j].cand >> (8 * b)) & 255;
+            for (uint32_t x = 0; x < 256; x++) {
+                uint32_t c = 0; int q = 0;
+                for (int i = 0; i < 8; i++) if ((cb >> i) & 1) { if ((x >> i) & 1) c |= 1u << q; q++; }
+                lut[(size_t)j * 1024 + b * 256 + x] = (uint8_t)c;
+            }
+        }
+    std::vector<unsigned long long> where(n_ent);
+    std::vector<uint32_t> epos(n_ent);
+    std::vector<float> escore(n_ent);
+    for (int j = 0; j < k; j++) {
+        const uint32_t cand = hv[j].cand;
+        for (size_t i = 0; i < ent[j].size(); i++) {
+            uint32_t idx = 0; int q = 0;                  // compact mask over cand_j's bits
+            for (uint32_t m = cand; m; m &= m - 1, q++) if ((cm[j][i] >> __builtin_ctz(m)) & 1) idx |= 1u << q;
+            where[hv[j].score + i] = hv[j].table + idx;
+            epos[hv[j].score + i] = (uint32_t)i;
+            escore[hv[j].score + i] = scores[ent[j][i]];
+        }
+    }
+
+    cudaStream_t s = ctx->stream;
+    DevBuf d_cost(ctx), d_leaf(ctx), d_tab(ctx), d_small(ctx), d_ent(ctx);
+    auto alloc = [&](DevBuf &b, size_t bytes) {
+        const cudaError_t e = b.alloc(bytes);
+        if (e != cudaSuccess) { cudaGetLastError(); return false; }
+        return true;
+    };
+    const size_t ent_bytes = std::max<size_t>(16, n_ent * 16);
+    if (!alloc(d_cost, nodes * 4) || !alloc(d_leaf, nodes) || !alloc(d_tab, table_elems * 4) || !alloc(d_small, small_bytes + 64) || !alloc(d_ent, ent_bytes))
+        return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes_msg() + " failed");
+    // d_small: vars | lut | binom | out;  d_ent: where | pos | score
+    char *sm = d_small.as<char>();
+    OrderVar *dv = reinterpret_cast<OrderVar *>(sm);
+    uint8_t *dl = reinterpret_cast<uint8_t *>(sm + k * sizeof(OrderVar));
+    uint32_t *db = reinterpret_cast<uint32_t *>(dl + (size_t)k * 1024);
+    uint32_t *dout = db + kOrderBinom * kOrderBinom;
+    unsigned long long *dw = d_ent.as<unsigned long long>();
+    uint32_t *dp = reinterpret_cast<uint32_t *>(dw + n_ent);
+    float *ds = reinterpret_cast<float *>(dp + n_ent);
+    CK(cudaMemcpyAsync(dv, hv.data(), k * sizeof(OrderVar), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(dl, lut.data(), lut.size(), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(db, binom.data(), binom.size() * 4, cudaMemcpyHostToDevice, s));
+    if (n_ent) {
+        CK(cudaMemcpyAsync(dw, where.data(), n_ent * 8, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(dp, epos.data(), n_ent * 4, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(ds, escore.data(), n_ent * 4, cudaMemcpyHostToDevice, s));
+    }
+    uint32_t *T = d_tab.as<uint32_t>();
+    {
+        uint64_t launches = 1;
+        for (int j = 0; j < k; j++) launches += 1 + std::max(0, __builtin_popcount(hv[j].cand) - kOrderSegBits);
+        Region rg(ctx, F_ORDER_TABLES, launches);
+        CK(cudaMemsetAsync(T, 0xFF, table_elems * 4, s));
+        if (n_ent) order_scatter_kernel<<<blocks_for(n_ent, 256), 256, 0, s>>>(dw, dp, n_ent, T);
+        for (int j = 0; j < k; j++) {
+            const int c = __builtin_popcount(hv[j].cand), lb = std::min(c, kOrderSegBits);
+            uint32_t *Tj = T + hv[j].table;
+            if (lb) order_table_low_kernel<<<(unsigned)(1u << (c - lb)), std::min(1024, std::max(32, 1 << (lb - 1))), 0, s>>>(Tj, lb);
+            for (int b = lb; b < c; b++) order_table_high_kernel<<<blocks_for((uint64_t)1 << (c - 1), 256), 256, 0, s>>>(Tj, b, (uint64_t)1 << (c - 1));
+        }
+        CK(cudaGetLastError());
+    }
+    float *cst = d_cost.as<float>();
+    uint8_t *lf = d_leaf.as<uint8_t>();
+    {
+        Region rg(ctx, F_ORDER_LAYERS, (uint64_t)k + 1);
+        CK(cudaMemsetAsync(cst, 0, sizeof(float), s));            // cost(empty set) = 0
+        const size_t smem = order_smem_bytes(k);
+        int per_sm = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_layer_kernel, 256, smem));
+        const uint64_t grid_cap = (uint64_t)std::max(1, per_sm) * ctx->sm_count;
+        for (int l = 1; l <= k; l++) {
+            const uint32_t count = binom[k * kOrderBinom + l];
+            const uint64_t runs = (count + kOrderRun - 1) / kOrderRun;
+            order_layer_kernel<<<(unsigned)std::min<uint64_t>(grid_cap, (runs + 255) / 256), 256, smem, s>>>(dv, dl, db, T, ds, k, l, count, cst, lf);
+        }
+        order_backtrack_kernel<<<1, 32, 0, s>>>(dv, T, cst, lf, k, dout);
+        CK(cudaGetLastError());
+    }
+    std::vector<uint32_t> out(2 + 2 * (size_t)k);
+    CK(cudaMemcpyAsync(out.data(), dout, out.size() * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    float c;
+    memcpy(&c, &out[0], sizeof c);
+    if (!out[1] || c == INFINITY) return ctx->fail(URLGPU_ERR_ARG, "No solution found.");   // search_capi.cpp:87
+    *cost = c;
+    for (int i = 0; i < k; i++) {
+        const int j = (int)out[2 + i], v = vars[j];
+        const uint32_t q = out[2 + k + i];
+        order[i] = v;
+        for (int w = 0; w < mask_words; w++) parents[(size_t)v * mask_words + w] = q == kOrderNone ? 0 : masks[ent[j][q] * mask_words + w];
+    }
     return URLGPU_OK;
 }
 
