@@ -23,6 +23,7 @@
  *   urlgpu_contingency       ADTree::makeContab                       ad_tree/ad_tree.cpp:95-137
  *   urlgpu_spg_build/query   SparseParentBitwise::initialize/getScore  score_cache/sparse_parent_bitwise.cpp:24-110
  *   urlgpu_order_search      run_astar_on_one_scc (order-graph search) astar/astar_main.cpp:216-546
+ *   urlgpu_order_search_layered  the same, for components of up to 36 variables
  *   urlgpu_prune             ScoreCalculator::prune                   scoring_function/score_calculator.cpp:150-197
  *   urlgpu_result_*          FloatMap iteration in scoringThread      score/score_main.cpp:187-200, base/typedefs.h:816
  *
@@ -216,6 +217,17 @@ int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *
                         const float *scores, const uint64_t *edges, const uint64_t *component,
                         float *cost, int32_t *order, uint64_t *parents);
 
+/* urlgpu_order_search for components of 1..36 variables: the same arguments, contract and outputs, and the same bits
+ * wherever both run.  Costs are kept for two adjacent layers only, indexed by colex rank inside the layer, and a leaf byte
+ * for every node.  Device memory: 2^|C| + 8*C(|C|, floor(|C|/2)) bytes for the nodes, 4*2^c_v per variable for the
+ * best-parent tables, 16 per qualifying entry, and 1328*|C| + 10960 bytes of descriptors, look-up tables,
+ * binomials and output.  Refusals: every URLGPU_ERR_ARG refusal of urlgpu_order_search, with the same messages; |C| > 36
+ * and a call that does not fit the device's free memory (URLGPU_ERR_LIMIT, with the bytes split into leaves, cost layers
+ * and best-parent tables); no admissible order or a cost of +inf: URLGPU_ERR_ARG, "No solution found.". */
+int urlgpu_order_search_layered(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                                const float *scores, const uint64_t *edges, const uint64_t *component,
+                                float *cost, int32_t *order, uint64_t *parents);
+
 /* Measurement hooks: device time (CUDA events on the context's stream) and launch counts per kernel family,
  * accumulated since the last reset. */
 typedef struct urlgpu_stats {
@@ -237,8 +249,8 @@ typedef struct urlgpu_stats {
     double k1_bytes_written;   /* cube path: bytes of contingency tables the K1 kernels store */
     double ms_standardise;     /* K2: column moments + standardisation passes (HBM bound); ms_gram is the DMMA Gram kernel + combine */
     uint64_t table16_fallbacks; /* K1 cube path: variables recomputed with 32-bit tables because a cell count did not fit 16 bits */
-    double ms_order_tables;    /* urlgpu_order_search: best-parent tables (fill, scatter, subset-min transform) */
-    double ms_order_layers;    /* urlgpu_order_search: layer sweeps and the backtrack */
+    double ms_order_tables;    /* urlgpu_order_search(_layered): best-parent tables (fill, scatter, subset-min transform) */
+    double ms_order_layers;    /* urlgpu_order_search(_layered): layer sweeps and the backtrack */
 } urlgpu_stats;
 int urlgpu_stats_reset(urlgpu_ctx *ctx);
 int urlgpu_stats_get(urlgpu_ctx *ctx, urlgpu_stats *out);

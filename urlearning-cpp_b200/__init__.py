@@ -38,6 +38,7 @@ ABI_SYMBOLS = [
     "urlgpu_spg_build", "urlgpu_spg_query", "urlgpu_spg_free",
     "urlgpu_peer_alloc", "urlgpu_peer_open", "urlgpu_peer_close", "urlgpu_peer_free",
     "urlgpu_result_fetch_device", "urlgpu_copy_to_host", "urlgpu_order_search",
+    "urlgpu_order_search_layered",
 ]
 
 
@@ -123,6 +124,7 @@ def load_library():
     lib.urlgpu_score_part.argtypes = [vp, i32, vp, i32, i32, i32, C.c_double, i32, i32, vp, i32]
     lib.urlgpu_result_from_scores.argtypes = [vp, i32, vp, i32, i32, i32, vp, u64, i32, C.c_uint, P(vp)]
     lib.urlgpu_order_search.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, P(C.c_float), vp, vp]
+    lib.urlgpu_order_search_layered.argtypes = lib.urlgpu_order_search.argtypes
     for name in ABI_SYMBOLS:
         if name not in ("urlgpu_last_error", "urlgpu_host_alloc", "urlgpu_host_free"):
             getattr(lib, name).restype = C.c_int
@@ -478,9 +480,16 @@ class Engine:
 
     def order_search(self, entries, p: int, component: int, edges: Sequence[int] | None = None):
         """urlgpu_order_search: the optimal DAG of one skeleton component over the order graph, layer by layer on the device.
+        Components of more than 32 variables go to urlgpu_order_search_layered, which keeps two cost layers instead of
+        every node's cost and takes up to 36 (same contract, same bits where both run).
         entries: p pairs (masks, scores) per variable in the search side's sign (lower is better), masks uint64 [n] or
         [n, words] or ints; component: a variable mask; edges: p skeleton masks or None.
         -> (float32 cost, order list (first = a root), parents uint64 [p] ([p, words] above 64 variables; 0 outside C))"""
+        k = bin(int(component)).count("1")
+        return self._order_search("urlgpu_order_search" if k <= 32 else "urlgpu_order_search_layered", entries, p, component, edges)
+
+    def _order_search(self, symbol: str, entries, p: int, component: int, edges: Sequence[int] | None):
+        """order_search through the named entry point (measurements compare the two forms at k <= 32)"""
         if len(entries) != p:
             raise ValueError(f"{len(entries)} entry lists for {p} variables")
         words = mask_words_for(p)
@@ -506,9 +515,9 @@ class Engine:
         cost = C.c_float()
         order = np.zeros(max(1, bin(int(component)).count("1")), dtype=np.int32)
         parents = np.zeros((p, words), dtype=np.uint64)
-        self._check(self.lib.urlgpu_order_search(self._h, p, words, offsets.ctypes.data, masks.ctypes.data if len(masks) else None,
-                                                 scores.ctypes.data if len(scores) else None, None if ed is None else ed.ctypes.data,
-                                                 comp.ctypes.data, C.byref(cost), order.ctypes.data, parents.ctypes.data))
+        self._check(getattr(self.lib, symbol)(self._h, p, words, offsets.ctypes.data, masks.ctypes.data if len(masks) else None,
+                                              scores.ctypes.data if len(scores) else None, None if ed is None else ed.ctypes.data,
+                                              comp.ctypes.data, C.byref(cost), order.ctypes.data, parents.ctypes.data))
         return np.float32(cost.value), [int(x) for x in order], parents[:, 0].copy() if words == 1 else parents
 
     def optimal_dag(self, cache, edges: Sequence[int] | None = None):

@@ -24,6 +24,13 @@
 //
 // Bound: a layer reads 4 + 4 bytes (cost, table) per (S, v) pair, k 2^(k-1) pairs in all, at addresses that differ from
 // node to node: HBM and L2 sector traffic, not arithmetic, sets the time.
+//
+// Layered form (urlgpu_order_search_layered, k <= 36): a sweep of layer l reads only layer l-1, and the backtrack reads only
+// leaves, so costs are kept for two adjacent layers indexed by colex rank inside the layer, and a leaf byte for every node at
+// base_l + rank (base_l = sum_{m<l} C(k, m)): 2^k + 8 C(k, k/2) bytes instead of 5 2^k.  With S = {e_0 < ... < e_{l-1}},
+// rank(S) = sum_i C(e_i, i+1) and rank(S \ e_j) = sum_{i<j} C(e_i, i+1) + sum_{i>j} C(e_i, i): a first pass over S's bits sums
+// C(e_i, i), the leaf loop keeps both prefixes.  order_layer_rank_kernel does per (S, v) exactly the arithmetic of
+// order_layer_kernel with 64-bit masks, ranks and table indices, so both forms give the same bits wherever both run.
 #pragma once
 #include "common.cuh"
 
@@ -47,6 +54,22 @@ struct OrderVar {            // variable at position j of C
 
 __host__ __device__ __forceinline__ size_t order_smem_bytes(int k) {
     return (size_t)kOrderBinomWords * sizeof(uint32_t) + (size_t)k * sizeof(OrderVar) + (size_t)k * 1024;
+}
+
+constexpr int kOrderRankMaxVars = 36;        // 2^36 + 8 C(36, 18) = 141 GB of nodes; 37 would need 279 GB
+constexpr int kOrderRankBinom = kOrderRankMaxVars + 1;
+constexpr int kOrderRankLut = 5;             // byte look-up tables per variable: bits 0..39 of a compact mask
+
+struct OrderVarRank {        // OrderVar with 64-bit compact masks
+    unsigned long long table; // offset of T_j in the table buffer (uint32 elements)
+    unsigned long long adj;   // skeleton neighbours over C; all ones without a skeleton
+    unsigned long long cand;  // cand_j over C
+    uint32_t score;           // offset of j's sorted scores
+    uint8_t shift[kOrderRankLut];
+};
+
+__host__ __device__ __forceinline__ size_t order_rank_smem_bytes(int k) {
+    return (size_t)kOrderRankBinom * kOrderRankBinom * sizeof(unsigned long long) + (size_t)k * sizeof(OrderVarRank) + (size_t)k * kOrderRankLut * 256;
 }
 
 // ------------------------------------------------------------------------------------------------ best-parent tables
@@ -165,6 +188,119 @@ __global__ void order_backtrack_kernel(const OrderVar *__restrict__ vars, const 
             if ((prev >> (__ffs(m) - 1)) & 1) idx |= 1u << j;
         out[2 + i] = v;
         out[2 + k + i] = T[vars[v].table + idx];
+        S = prev;
+    }
+    out[1] = 1;
+}
+
+// ------------------------------------------------------------------------------------------------ layered form
+// rank r of layer l -> the k-bit mask with that colex rank (B[b * kOrderRankBinom + i] = C(b, i))
+__device__ __forceinline__ unsigned long long order_unrank64(const unsigned long long *B, int k, int l, unsigned long long r) {
+    unsigned long long S = 0;
+    int hi = k - 1;
+    for (int i = l; i >= 1; i--) {
+        int lo = i - 1, h = hi;                   // largest b in [i-1, hi] with C(b, i) <= r
+        while (lo < h) {
+            const int mid = (lo + h + 1) >> 1;
+            if (B[mid * kOrderRankBinom + i] <= r) lo = mid; else h = mid - 1;
+        }
+        S |= 1ull << lo;
+        r -= B[lo * kOrderRankBinom + i];
+        hi = lo - 1;
+    }
+    return S;
+}
+// Gosper successor; k <= 36, so x + low never overflows
+__device__ __forceinline__ unsigned long long order_next64(unsigned long long x) {
+    const unsigned long long low = x & (~x + 1), r = x + low;
+    return r | (((x ^ r) >> 2) >> (__ffsll((long long)x) - 1));
+}
+// colex rank of S inside its layer
+__device__ __forceinline__ unsigned long long order_rank64(const unsigned long long *B, unsigned long long S) {
+    unsigned long long r = 0;
+    int i = 1;
+    for (; S; S &= S - 1, i++) r += B[(__ffsll((long long)S) - 1) * kOrderRankBinom + i];
+    return r;
+}
+
+// layer `layer` from layer - 1: cost_prev / cost_cur are indexed by colex rank, leaf by `base` + rank
+__global__ void __launch_bounds__(256) order_layer_rank_kernel(const OrderVarRank *__restrict__ vars, const uint8_t *__restrict__ lut,
+                                                               const unsigned long long *__restrict__ binom, const uint32_t *__restrict__ T,
+                                                               const float *__restrict__ scores, int k, int layer, unsigned long long count,
+                                                               unsigned long long base, const float *__restrict__ cost_prev,
+                                                               float *__restrict__ cost_cur, uint8_t *__restrict__ leaf) {
+    extern __shared__ __align__(16) unsigned char order_smem[];
+    unsigned long long *s_binom = reinterpret_cast<unsigned long long *>(order_smem);
+    OrderVarRank *s_var = reinterpret_cast<OrderVarRank *>(s_binom + kOrderRankBinom * kOrderRankBinom);
+    uint8_t *s_lut = reinterpret_cast<uint8_t *>(s_var + k);
+    for (int i = threadIdx.x; i < kOrderRankBinom * kOrderRankBinom; i += blockDim.x) s_binom[i] = __ldg(binom + i);
+    for (int i = threadIdx.x; i < k; i += blockDim.x) s_var[i] = vars[i];
+    for (int i = threadIdx.x; i < k * kOrderRankLut * 64; i += blockDim.x)
+        reinterpret_cast<uint32_t *>(s_lut)[i] = __ldg(reinterpret_cast<const uint32_t *>(lut) + i);
+    __syncthreads();
+    const unsigned long long runs = (count + kOrderRun - 1) / kOrderRun;
+    for (unsigned long long run = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; run < runs; run += (unsigned long long)gridDim.x * blockDim.x) {
+        const unsigned long long first = run * kOrderRun;
+        const uint32_t nrun = (uint32_t)min((unsigned long long)kOrderRun, count - first);
+        unsigned long long S = order_unrank64(s_binom, k, layer, first);
+        for (uint32_t u = 0; u < nrun; u++) {
+            unsigned long long above = 0;                              // sum_i C(e_i, i)
+            {
+                int i = 0;
+                for (unsigned long long m = S; m; m &= m - 1, i++) above += s_binom[(__ffsll((long long)m) - 1) * kOrderRankBinom + i];
+            }
+            unsigned long long below = 0;                              // sum_{i<j} C(e_i, i+1)
+            float best = __int_as_float(0x7f800000);
+            uint32_t best_leaf = kOrderUnreached;
+            int j = 0;
+            for (unsigned long long m = S; m; m &= m - 1, j++) {
+                const int v = __ffsll((long long)m) - 1;
+                above -= s_binom[v * kOrderRankBinom + j];
+                const unsigned long long rprev = below + above;
+                below += s_binom[v * kOrderRankBinom + j + 1];
+                const unsigned long long prev = S ^ (1ull << v);
+                const OrderVarRank &V = s_var[v];
+                if (prev && !(prev & V.adj)) continue;                 // the leaf must touch the sub-network
+                const float c = __ldg(cost_prev + rprev);
+                if (c == __int_as_float(0x7f800000)) continue;        // S\v unreached
+                const uint8_t *L = s_lut + v * (kOrderRankLut * 256);
+                const unsigned long long idx = (unsigned long long)L[prev & 255] | ((unsigned long long)L[256 + ((prev >> 8) & 255)] << V.shift[1]) |
+                                               ((unsigned long long)L[512 + ((prev >> 16) & 255)] << V.shift[2]) |
+                                               ((unsigned long long)L[768 + ((prev >> 24) & 255)] << V.shift[3]) |
+                                               ((unsigned long long)L[1024 + ((prev >> 32) & 255)] << V.shift[4]);
+                const uint32_t pos = __ldg(T + V.table + idx);
+                const float s = pos == kOrderNone ? 3.402823466e+38f : __ldg(scores + V.score + pos);
+                const float g = __fadd_rn(c, s);
+                if (g == __int_as_float(0x7f800000)) continue;
+                if (g < best) { best = g; best_leaf = (uint32_t)v; }   // strict: the smallest v among equal costs
+            }
+            const unsigned long long r = first + u;
+            cost_cur[r] = best;
+            leaf[base + r] = (uint8_t)best_leaf;
+            if (u + 1 < nrun) S = order_next64(S);
+        }
+    }
+}
+
+// the output of order_backtrack_kernel; cost_full is the one cost of layer k, leaf[base_l + rank] as in the layer kernel
+__global__ void order_backtrack_rank_kernel(const OrderVarRank *__restrict__ vars, const unsigned long long *__restrict__ binom,
+                                            const uint32_t *__restrict__ T, const float *__restrict__ cost_full,
+                                            const uint8_t *__restrict__ leaf, int k, uint32_t *__restrict__ out) {
+    if (blockIdx.x | threadIdx.x) return;
+    unsigned long long S = (1ull << k) - 1, base = ((1ull << k) - 1);   // base_k = 2^k - C(k, k)
+    out[0] = __float_as_uint(cost_full[0]);
+    out[1] = 0;
+    for (int i = k - 1; i >= 0; i--) {
+        const uint32_t v = leaf[base + order_rank64(binom, S)];
+        if (v == kOrderUnreached) return;
+        const unsigned long long prev = S ^ (1ull << v);
+        unsigned long long idx = 0;
+        int j = 0;
+        for (unsigned long long m = vars[v].cand; m; m &= m - 1, j++)
+            if ((prev >> (__ffsll((long long)m) - 1)) & 1) idx |= 1ull << j;
+        out[2 + i] = v;
+        out[2 + k + i] = T[vars[v].table + idx];
+        base -= binom[k * kOrderRankBinom + i];                    // base_i = base_{i+1} - C(k, i)
         S = prev;
     }
     out[1] = 1;

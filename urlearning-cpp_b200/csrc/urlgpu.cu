@@ -384,6 +384,7 @@ extern "C" int urlgpu_create(urlgpu_ctx **out, int device_id) {
         attrs.push_back({(const void *)bic_count_smem_kernel<ListSets>, big});
         attrs.push_back({(const void *)cbic_sets_kernel, big});
         attrs.push_back({(const void *)gram_partial_kernel, (int)kGramSmemBytes});
+        attrs.push_back({(const void *)order_layer_rank_kernel, (int)order_rank_smem_bytes(kOrderRankMaxVars)});
         for (const auto &a : attrs)
             if ((e = cudaFuncSetAttribute(a.first, cudaFuncAttributeMaxDynamicSharedMemorySize, a.second)) != cudaSuccess)
                 return refuse("cannot opt a kernel into " + std::to_string(a.second) + " bytes of dynamic shared memory (the device allows " +
@@ -2531,14 +2532,16 @@ extern "C" int urlgpu_spg_free(urlgpu_spg *sp) {
 }
 
 // ============================================================================================ order-graph search
-// urlgpu_order_search (order_kernels.cuh).  The host validates everything, translates the component's qualifying entries to
-// compact masks over C's positions once, sorts each variable's list in the (score, |S|, mask) order of SortedEntries::build,
-// and sizes the call before any allocation.  One upload of the small arrays, the table passes, k layer launches, one
-// backtrack and one copy back; the host then maps each leaf's sorted position to its parent mask.
-extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks, const float *scores,
-                                   const uint64_t *edges, const uint64_t *component, float *cost, int32_t *order, uint64_t *parents) {
+// urlgpu_order_search and urlgpu_order_search_layered (order_kernels.cuh).  The host validates everything, translates the
+// component's qualifying entries to compact masks over C's positions once, sorts each variable's list in the (score, |S|,
+// mask) order of SortedEntries::build, and sizes the call before any allocation.  One upload of the small arrays, the table
+// passes, k layer launches, one backtrack and one copy back; the host then maps each leaf's sorted position to its parent
+// mask.  The two entry points differ only in the node storage, the layer launches and the backtrack.
+static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                             const float *scores, const uint64_t *edges, const uint64_t *component, float *cost, int32_t *order,
+                             uint64_t *parents) {
     if (!ctx) return URLGPU_ERR_ARG;
-    auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, "order_search: " + m); };
+    auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, (layered ? "order_search_layered: " : "order_search: ") + m); };
     if (!offsets || !component || !cost || !order || !parents) return refuse(URLGPU_ERR_ARG, "null argument");
     if (p < 1) return refuse(URLGPU_ERR_ARG, "p must be at least 1");
     if (mask_words < 1 || mask_words > kSpgMaxWords) return refuse(URLGPU_ERR_ARG, "mask_words must be in 1.." + std::to_string(kSpgMaxWords));
@@ -2563,16 +2566,17 @@ extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const
             if (bit(masks + e * mask_words, v)) return refuse(URLGPU_ERR_ARG, "variable " + std::to_string(v) + ", entry " + std::to_string(e - offsets[v]) + ": the parent set contains the variable itself");
         }
     const int k = (int)vars.size();
-    if (k > kOrderMaxVars) return refuse(URLGPU_ERR_LIMIT, std::to_string(k) + " variables in the component; at most " + std::to_string(kOrderMaxVars) + " are supported");
+    const int max_k = layered ? kOrderRankMaxVars : kOrderMaxVars;
+    if (k > max_k) return refuse(URLGPU_ERR_LIMIT, std::to_string(k) + " variables in the component; at most " + std::to_string(max_k) + " are supported");
 
     // qualifying entries (all parents inside C), compact masks, per-variable sort
     std::vector<uint64_t> Cmask(component, component + mask_words);
     std::vector<std::vector<uint64_t>> ent(k);   // per position: indices into masks/scores, sorted
-    std::vector<std::vector<uint32_t>> cm(k);    // compact masks in the same order
-    std::vector<OrderVar> hv(k);
+    std::vector<std::vector<uint64_t>> cm(k);    // compact masks in the same order
+    std::vector<OrderVarRank> hv(k);
     auto compact = [&](const uint64_t *m) {
-        uint32_t c = 0;
-        for (int j = 0; j < k; j++) if (bit(m, vars[j])) c |= 1u << j;
+        uint64_t c = 0;
+        for (int j = 0; j < k; j++) if (bit(m, vars[j])) c |= 1ull << j;
         return c;
     };
     uint64_t n_ent = 0, table_elems = 0;
@@ -2594,55 +2598,75 @@ extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const
             return a < b;
         });
         if (E.size() > 0xFFFFFFFEull) return refuse(URLGPU_ERR_LIMIT, "variable " + std::to_string(v) + " has 2^32 or more entries inside the component");
-        uint32_t cand = 0;
+        uint64_t cand = 0;
         for (uint64_t e : E) { cm[j].push_back(compact(masks + e * mask_words)); cand |= cm[j].back(); }
         hv[j].table = table_elems;
         hv[j].score = (uint32_t)n_ent;
         hv[j].cand = cand;
-        hv[j].adj = 0xFFFFFFFFu;
+        hv[j].adj = ~0ull;
         if (edges) hv[j].adj = compact(edges + (size_t)v * mask_words);
-        for (int b = 0; b < 4; b++) hv[j].shift[b] = (uint8_t)__builtin_popcount(b ? cand & (0xFFFFFFFFu >> (32 - 8 * b)) : 0u);
-        table_elems += (uint64_t)1 << __builtin_popcount(cand);
+        for (int b = 0; b < kOrderRankLut; b++) hv[j].shift[b] = (uint8_t)__builtin_popcountll(cand & ((1ull << (8 * b)) - 1));
+        table_elems += (uint64_t)1 << __builtin_popcountll(cand);
         n_ent += E.size();
     }
     if (n_ent > 0xFFFFFFFFull) return refuse(URLGPU_ERR_LIMIT, "2^32 or more entries inside the component");
 
-    // the device memory of the call, before anything is allocated
-    const uint64_t nodes = (uint64_t)1 << k;
-    const size_t small_bytes = (size_t)k * sizeof(OrderVar) + (size_t)k * 1024 + (size_t)kOrderBinom * kOrderBinom * 4 + (2 + 2 * (size_t)k) * 4;
-    const size_t need = 5 * nodes + 4 * table_elems + n_ent * (8 + 4 + 4) + small_bytes;
+    // binomials: C(b, i) for b, i <= kOrderRankMaxVars (the dense kernels take the uint32 corner b, i <= kOrderMaxVars)
+    std::vector<unsigned long long> binom(kOrderRankBinom * kOrderRankBinom, 0);
+    for (int b = 0; b < kOrderRankBinom; b++)
+        for (int i = 0; i <= b; i++) binom[b * kOrderRankBinom + i] = i == 0 || i == b ? 1ull : binom[(b - 1) * kOrderRankBinom + i - 1] + binom[(b - 1) * kOrderRankBinom + i];
+    std::vector<uint32_t> binom32(kOrderBinom * kOrderBinom);
+    for (int b = 0; b < kOrderBinom; b++)
+        for (int i = 0; i < kOrderBinom; i++) binom32[b * kOrderBinom + i] = (uint32_t)binom[b * kOrderRankBinom + i];
+
+    // the device memory of the call, before anything is allocated.  Dense: a cost and a leaf for each of the 2^k nodes.
+    // Layered: a leaf for each node and the costs of two layers, each at most C(k, k/2) nodes
+    const int n_lut = layered ? kOrderRankLut : 4;
+    const size_t var_bytes = layered ? sizeof(OrderVarRank) : sizeof(OrderVar);
+    const size_t binom_bytes = layered ? binom.size() * 8 : binom32.size() * 4;
+    const uint64_t nodes = (uint64_t)1 << k, widest = binom[k * kOrderRankBinom + k / 2];
+    const size_t small_bytes = (size_t)k * var_bytes + (size_t)k * n_lut * 256 + binom_bytes + (2 + 2 * (size_t)k) * 4;
+    const uint64_t node_bytes = layered ? nodes + 8 * widest : 5 * nodes;
+    const size_t need = node_bytes + 4 * table_elems + n_ent * (8 + 4 + 4) + small_bytes;
     CK(cudaSetDevice(ctx->device));
     size_t free_b = 0, total_b = 0;
     CK(cudaMemGetInfo(&free_b, &total_b));
     for (auto &b : ctx->pool) if (!b.used) free_b += b.bytes;      // cached blocks the allocator can hand out or release
     auto bytes_msg = [&]() {
-        return std::to_string(need) + " bytes of device memory (" + std::to_string(5 * nodes) + " for the 2^" + std::to_string(k) + " nodes, " +
-               std::to_string(4 * table_elems) + " for the best-parent tables)";
+        const std::string nodes_part = layered ? std::to_string(nodes) + " for the leaves of the 2^" + std::to_string(k) + " nodes, " +
+                                                     std::to_string(8 * widest) + " for two cost layers of C(" + std::to_string(k) + ", " + std::to_string(k / 2) + ") nodes, "
+                                               : std::to_string(5 * nodes) + " for the 2^" + std::to_string(k) + " nodes, ";
+        return std::to_string(need) + " bytes of device memory (" + nodes_part + std::to_string(4 * table_elems) + " for the best-parent tables)";
     };
     if (need > free_b) return refuse(URLGPU_ERR_LIMIT, "the search needs " + bytes_msg() + ", " + std::to_string(free_b) + " are free");
 
-    // host arrays: binomials, byte look-up tables, scatter list, sorted scores
-    std::vector<uint32_t> binom(kOrderBinom * kOrderBinom, 0);
-    for (int b = 0; b < kOrderBinom; b++)
-        for (int i = 0; i <= b; i++) binom[b * kOrderBinom + i] = i == 0 || i == b ? 1u : binom[(b - 1) * kOrderBinom + i - 1] + binom[(b - 1) * kOrderBinom + i];
-    std::vector<uint8_t> lut((size_t)k * 1024);
+    // host arrays: descriptors, byte look-up tables, scatter list, sorted scores
+    std::vector<OrderVar> hv32(layered ? 0 : k);
+    for (int j = 0; j < (int)hv32.size(); j++) {
+        hv32[j].table = hv[j].table;
+        hv32[j].score = hv[j].score;
+        hv32[j].adj = (uint32_t)hv[j].adj;
+        hv32[j].cand = (uint32_t)hv[j].cand;
+        for (int b = 0; b < 4; b++) hv32[j].shift[b] = hv[j].shift[b];
+    }
+    std::vector<uint8_t> lut((size_t)k * n_lut * 256);
     for (int j = 0; j < k; j++)
-        for (int b = 0; b < 4; b++) {
-            const uint32_t cb = (hv[j].cand >> (8 * b)) & 255;
+        for (int b = 0; b < n_lut; b++) {
+            const uint32_t cb = (uint32_t)(hv[j].cand >> (8 * b)) & 255;
             for (uint32_t x = 0; x < 256; x++) {
                 uint32_t c = 0; int q = 0;
                 for (int i = 0; i < 8; i++) if ((cb >> i) & 1) { if ((x >> i) & 1) c |= 1u << q; q++; }
-                lut[(size_t)j * 1024 + b * 256 + x] = (uint8_t)c;
+                lut[((size_t)j * n_lut + b) * 256 + x] = (uint8_t)c;
             }
         }
     std::vector<unsigned long long> where(n_ent);
     std::vector<uint32_t> epos(n_ent);
     std::vector<float> escore(n_ent);
     for (int j = 0; j < k; j++) {
-        const uint32_t cand = hv[j].cand;
+        const uint64_t cand = hv[j].cand;
         for (size_t i = 0; i < ent[j].size(); i++) {
-            uint32_t idx = 0; int q = 0;                  // compact mask over cand_j's bits
-            for (uint32_t m = cand; m; m &= m - 1, q++) if ((cm[j][i] >> __builtin_ctz(m)) & 1) idx |= 1u << q;
+            uint64_t idx = 0; int q = 0;                  // compact mask over cand_j's bits
+            for (uint64_t m = cand; m; m &= m - 1, q++) if ((cm[j][i] >> __builtin_ctzll(m)) & 1) idx |= 1ull << q;
             where[hv[j].score + i] = hv[j].table + idx;
             epos[hv[j].score + i] = (uint32_t)i;
             escore[hv[j].score + i] = scores[ent[j][i]];
@@ -2657,20 +2681,20 @@ extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const
         return true;
     };
     const size_t ent_bytes = std::max<size_t>(16, n_ent * 16);
-    if (!alloc(d_cost, nodes * 4) || !alloc(d_leaf, nodes) || !alloc(d_tab, table_elems * 4) || !alloc(d_small, small_bytes + 64) || !alloc(d_ent, ent_bytes))
+    const size_t cost_bytes = layered ? 8 * widest : 4 * nodes;
+    if (!alloc(d_cost, cost_bytes) || !alloc(d_leaf, nodes) || !alloc(d_tab, table_elems * 4) || !alloc(d_small, small_bytes + 64) || !alloc(d_ent, ent_bytes))
         return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes_msg() + " failed");
     // d_small: vars | lut | binom | out;  d_ent: where | pos | score
     char *sm = d_small.as<char>();
-    OrderVar *dv = reinterpret_cast<OrderVar *>(sm);
-    uint8_t *dl = reinterpret_cast<uint8_t *>(sm + k * sizeof(OrderVar));
-    uint32_t *db = reinterpret_cast<uint32_t *>(dl + (size_t)k * 1024);
-    uint32_t *dout = db + kOrderBinom * kOrderBinom;
+    uint8_t *dl = reinterpret_cast<uint8_t *>(sm + k * var_bytes);
+    char *db = reinterpret_cast<char *>(dl + lut.size());
+    uint32_t *dout = reinterpret_cast<uint32_t *>(db + binom_bytes);
     unsigned long long *dw = d_ent.as<unsigned long long>();
     uint32_t *dp = reinterpret_cast<uint32_t *>(dw + n_ent);
     float *ds = reinterpret_cast<float *>(dp + n_ent);
-    CK(cudaMemcpyAsync(dv, hv.data(), k * sizeof(OrderVar), cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(sm, layered ? (const void *)hv.data() : (const void *)hv32.data(), k * var_bytes, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(dl, lut.data(), lut.size(), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(db, binom.data(), binom.size() * 4, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(db, layered ? (const void *)binom.data() : (const void *)binom32.data(), binom_bytes, cudaMemcpyHostToDevice, s));
     if (n_ent) {
         CK(cudaMemcpyAsync(dw, where.data(), n_ent * 8, cudaMemcpyHostToDevice, s));
         CK(cudaMemcpyAsync(dp, epos.data(), n_ent * 4, cudaMemcpyHostToDevice, s));
@@ -2679,12 +2703,12 @@ extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const
     uint32_t *T = d_tab.as<uint32_t>();
     {
         uint64_t launches = 1;
-        for (int j = 0; j < k; j++) launches += 1 + std::max(0, __builtin_popcount(hv[j].cand) - kOrderSegBits);
+        for (int j = 0; j < k; j++) launches += 1 + std::max(0, __builtin_popcountll(hv[j].cand) - kOrderSegBits);
         Region rg(ctx, F_ORDER_TABLES, launches);
         CK(cudaMemsetAsync(T, 0xFF, table_elems * 4, s));
         if (n_ent) order_scatter_kernel<<<blocks_for(n_ent, 256), 256, 0, s>>>(dw, dp, n_ent, T);
         for (int j = 0; j < k; j++) {
-            const int c = __builtin_popcount(hv[j].cand), lb = std::min(c, kOrderSegBits);
+            const int c = __builtin_popcountll(hv[j].cand), lb = std::min(c, kOrderSegBits);
             uint32_t *Tj = T + hv[j].table;
             if (lb) order_table_low_kernel<<<(unsigned)(1u << (c - lb)), std::min(1024, std::max(32, 1 << (lb - 1))), 0, s>>>(Tj, lb);
             for (int b = lb; b < c; b++) order_table_high_kernel<<<blocks_for((uint64_t)1 << (c - 1), 256), 256, 0, s>>>(Tj, b, (uint64_t)1 << (c - 1));
@@ -2696,16 +2720,36 @@ extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const
     {
         Region rg(ctx, F_ORDER_LAYERS, (uint64_t)k + 1);
         CK(cudaMemsetAsync(cst, 0, sizeof(float), s));            // cost(empty set) = 0
-        const size_t smem = order_smem_bytes(k);
         int per_sm = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_layer_kernel, 256, smem));
-        const uint64_t grid_cap = (uint64_t)std::max(1, per_sm) * ctx->sm_count;
-        for (int l = 1; l <= k; l++) {
-            const uint32_t count = binom[k * kOrderBinom + l];
-            const uint64_t runs = (count + kOrderRun - 1) / kOrderRun;
-            order_layer_kernel<<<(unsigned)std::min<uint64_t>(grid_cap, (runs + 255) / 256), 256, smem, s>>>(dv, dl, db, T, ds, k, l, count, cst, lf);
+        if (!layered) {
+            const OrderVar *dv = reinterpret_cast<const OrderVar *>(sm);
+            const uint32_t *db32 = reinterpret_cast<const uint32_t *>(db);
+            const size_t smem = order_smem_bytes(k);
+            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_layer_kernel, 256, smem));
+            const uint64_t grid_cap = (uint64_t)std::max(1, per_sm) * ctx->sm_count;
+            for (int l = 1; l <= k; l++) {
+                const uint32_t count = binom32[k * kOrderBinom + l];
+                const uint64_t runs = (count + kOrderRun - 1) / kOrderRun;
+                order_layer_kernel<<<(unsigned)std::min<uint64_t>(grid_cap, (runs + 255) / 256), 256, smem, s>>>(dv, dl, db32, T, ds, k, l, count, cst, lf);
+            }
+            order_backtrack_kernel<<<1, 32, 0, s>>>(dv, T, cst, lf, k, dout);
+        } else {
+            const OrderVarRank *dv = reinterpret_cast<const OrderVarRank *>(sm);
+            const unsigned long long *db64 = reinterpret_cast<const unsigned long long *>(db);
+            const size_t smem = order_rank_smem_bytes(k);
+            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_layer_rank_kernel, 256, smem));
+            const uint64_t grid_cap = (uint64_t)std::max(1, per_sm) * ctx->sm_count;
+            float *layer_cost[2] = {cst, cst + widest};          // layer l is written to layer_cost[l & 1]
+            uint64_t base = 1;                                     // base_l = sum_{m<l} C(k, m)
+            for (int l = 1; l <= k; l++) {
+                const uint64_t count = binom[k * kOrderRankBinom + l];
+                const uint64_t runs = (count + kOrderRun - 1) / kOrderRun;
+                order_layer_rank_kernel<<<(unsigned)std::min<uint64_t>(grid_cap, (runs + 255) / 256), 256, smem, s>>>(
+                    dv, dl, db64, T, ds, k, l, count, base, layer_cost[(l - 1) & 1], layer_cost[l & 1], lf);
+                base += count;
+            }
+            order_backtrack_rank_kernel<<<1, 32, 0, s>>>(dv, db64, T, layer_cost[k & 1], lf, k, dout);
         }
-        order_backtrack_kernel<<<1, 32, 0, s>>>(dv, T, cst, lf, k, dout);
         CK(cudaGetLastError());
     }
     std::vector<uint32_t> out(2 + 2 * (size_t)k);
@@ -2722,6 +2766,17 @@ extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const
         for (int w = 0; w < mask_words; w++) parents[(size_t)v * mask_words + w] = q == kOrderNone ? 0 : masks[ent[j][q] * mask_words + w];
     }
     return URLGPU_OK;
+}
+
+extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks, const float *scores,
+                                   const uint64_t *edges, const uint64_t *component, float *cost, int32_t *order, uint64_t *parents) {
+    return order_search_impl(ctx, false, p, mask_words, offsets, masks, scores, edges, component, cost, order, parents);
+}
+
+extern "C" int urlgpu_order_search_layered(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                                           const float *scores, const uint64_t *edges, const uint64_t *component, float *cost,
+                                           int32_t *order, uint64_t *parents) {
+    return order_search_impl(ctx, true, p, mask_words, offsets, masks, scores, edges, component, cost, order, parents);
 }
 
 // ============================================================================================ listed sets
