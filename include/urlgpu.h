@@ -24,6 +24,7 @@
  *   urlgpu_spg_build/query   SparseParentBitwise::initialize/getScore  score_cache/sparse_parent_bitwise.cpp:24-110
  *   urlgpu_order_search      run_astar_on_one_scc (order-graph search) astar/astar_main.cpp:216-546
  *   urlgpu_order_search_layered  the same, for components of up to 36 variables
+ *   urlgpu_order_local_search    (no counterpart: insertion hill climbing over the same orders, components of up to 256)
  *   urlgpu_prune             ScoreCalculator::prune                   scoring_function/score_calculator.cpp:150-197
  *   urlgpu_result_*          FloatMap iteration in scoringThread      score/score_main.cpp:187-200, base/typedefs.h:816
  *
@@ -228,6 +229,31 @@ int urlgpu_order_search_layered(urlgpu_ctx *ctx, int p, int mask_words, const ui
                                 const float *scores, const uint64_t *edges, const uint64_t *component,
                                 float *cost, int32_t *order, uint64_t *parents);
 
+/* A DAG of one skeleton component of up to 256 variables by insertion hill climbing over its admissible orders, from
+ * `restarts` random orders.  Inputs, best(v, U), the sign of the scores and the outputs cost, order and parents mean what they
+ * mean for urlgpu_order_search.  An order pi of C is admissible when every pi_m, m >= 1, has a skeleton neighbour among
+ * pi_0..pi_{m-1} (every order without a skeleton).  Its cost is the float32 left-to-right path sum g_0 = 0,
+ * g_{m+1} = fl(g_m + best(pi_m, {pi_0..pi_{m-1}})), the objective urlgpu_order_search minimises, so *cost is never below
+ * urlgpu_order_search's cost on the same input.
+ * Restart r = 0..restarts-1 starts from a random admissible order drawn with splitmix64 from x = seed + 0xD1B54A32D192ED03 (r+1):
+ * the first variable is element draw % |C| of C in ascending index, then, until C is placed, element draw % |F| of F, the
+ * unplaced variables of C adjacent to a placed one (all unplaced ones without a skeleton), in ascending index.  It then climbs:
+ * a move (i, j), i != j, takes the variable at position i out and reinserts it at position j; among the admissible results the
+ * least cost is taken if it is strictly below the current cost (ties: smallest i, then smallest j), otherwise the restart ends.
+ * The result is the restart with the least final cost (ties: smallest r).  restart_costs[r] and restart_moves[r] (each
+ * optional, `restarts` elements) receive every restart's final cost and number of moves; a restart depends only on the input,
+ * seed and r.  Device memory: 4*2^c_v per variable for the best-parent tables, 16 per qualifying entry, 8 + 5|C| per restart
+ * and 80|C| of descriptors.  Refusals, all before any launch: every URLGPU_ERR_ARG refusal of urlgpu_order_search with the
+ * same message after "order_local_search: "; restarts outside 1..2^20 (URLGPU_ERR_ARG); a variable with more than 32 candidate
+ * parents inside C, and a call that does not fit the device's free memory (URLGPU_ERR_LIMIT, with the bytes split into
+ * best-parent tables, entries and per-restart state).  No admissible order, or a best cost of +inf: URLGPU_ERR_ARG,
+ * "No solution found.".  Times: the tables under ms_order_tables, the climb under ms_order_layers. */
+int urlgpu_order_local_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                              const float *scores, const uint64_t *edges, const uint64_t *component,
+                              uint32_t restarts, uint64_t seed,
+                              float *cost, int32_t *order, uint64_t *parents,
+                              float *restart_costs /* optional, [restarts] */, uint32_t *restart_moves /* optional, [restarts] */);
+
 /* Measurement hooks: device time (CUDA events on the context's stream) and launch counts per kernel family,
  * accumulated since the last reset. */
 typedef struct urlgpu_stats {
@@ -249,8 +275,8 @@ typedef struct urlgpu_stats {
     double k1_bytes_written;   /* cube path: bytes of contingency tables the K1 kernels store */
     double ms_standardise;     /* K2: column moments + standardisation passes (HBM bound); ms_gram is the DMMA Gram kernel + combine */
     uint64_t table16_fallbacks; /* K1 cube path: variables recomputed with 32-bit tables because a cell count did not fit 16 bits */
-    double ms_order_tables;    /* urlgpu_order_search(_layered): best-parent tables (fill, scatter, subset-min transform) */
-    double ms_order_layers;    /* urlgpu_order_search(_layered): layer sweeps and the backtrack */
+    double ms_order_tables;    /* urlgpu_order_search(_layered), urlgpu_order_local_search: best-parent tables (fill, scatter, subset-min transform) */
+    double ms_order_layers;    /* urlgpu_order_search(_layered): layer sweeps and the backtrack; urlgpu_order_local_search: the climb */
 } urlgpu_stats;
 int urlgpu_stats_reset(urlgpu_ctx *ctx);
 int urlgpu_stats_get(urlgpu_ctx *ctx, urlgpu_stats *out);

@@ -38,7 +38,7 @@ ABI_SYMBOLS = [
     "urlgpu_spg_build", "urlgpu_spg_query", "urlgpu_spg_free",
     "urlgpu_peer_alloc", "urlgpu_peer_open", "urlgpu_peer_close", "urlgpu_peer_free",
     "urlgpu_result_fetch_device", "urlgpu_copy_to_host", "urlgpu_order_search",
-    "urlgpu_order_search_layered",
+    "urlgpu_order_search_layered", "urlgpu_order_local_search",
 ]
 
 
@@ -125,6 +125,7 @@ def load_library():
     lib.urlgpu_result_from_scores.argtypes = [vp, i32, vp, i32, i32, i32, vp, u64, i32, C.c_uint, P(vp)]
     lib.urlgpu_order_search.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, P(C.c_float), vp, vp]
     lib.urlgpu_order_search_layered.argtypes = lib.urlgpu_order_search.argtypes
+    lib.urlgpu_order_local_search.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, C.c_uint32, u64, P(C.c_float), vp, vp, vp, vp]
     for name in ABI_SYMBOLS:
         if name not in ("urlgpu_last_error", "urlgpu_host_alloc", "urlgpu_host_free"):
             getattr(lib, name).restype = C.c_int
@@ -490,6 +491,18 @@ class Engine:
 
     def _order_search(self, symbol: str, entries, p: int, component: int, edges: Sequence[int] | None):
         """order_search through the named entry point (measurements compare the two forms at k <= 32)"""
+        words, offsets, masks, scores, comp, ed = self._order_args(entries, p, component, edges)
+        cost = C.c_float()
+        order = np.zeros(max(1, bin(int(component)).count("1")), dtype=np.int32)
+        parents = np.zeros((p, words), dtype=np.uint64)
+        self._check(getattr(self.lib, symbol)(self._h, p, words, offsets.ctypes.data, masks.ctypes.data if len(masks) else None,
+                                              scores.ctypes.data if len(scores) else None, None if ed is None else ed.ctypes.data,
+                                              comp.ctypes.data, C.byref(cost), order.ctypes.data, parents.ctypes.data))
+        return np.float32(cost.value), [int(x) for x in order], parents[:, 0].copy() if words == 1 else parents
+
+    @staticmethod
+    def _order_args(entries, p: int, component: int, edges: Sequence[int] | None):
+        """the C arrays of the order searches -> (words, offsets, masks, scores, component words, skeleton rows or None)"""
         if len(entries) != p:
             raise ValueError(f"{len(entries)} entry lists for {p} variables")
         words = mask_words_for(p)
@@ -512,29 +525,53 @@ class Engine:
         ed = None if edges is None else np.ascontiguousarray(np.stack([mask_to_words(int(e), words) for e in edges]))
         if ed is not None and len(ed) != p:
             raise ValueError(f"{len(ed)} skeleton rows for {p} variables")
+        return words, offsets, masks, scores, comp, ed
+
+    def order_local_search(self, entries, p: int, component: int, edges: Sequence[int] | None = None, restarts: int = 256, seed: int = 0):
+        """urlgpu_order_local_search: insertion hill climbing over the admissible orders of one skeleton component of up to 256
+        variables, from `restarts` random orders, with the objective of order_search (so its cost is never below order_search's).
+        Same input conventions as order_search.
+        -> (float32 cost, order list, parents as order_search returns them, float32 [restarts] final cost per restart,
+            uint32 [restarts] moves per restart)"""
+        words, offsets, masks, scores, comp, ed = self._order_args(entries, p, component, edges)
         cost = C.c_float()
         order = np.zeros(max(1, bin(int(component)).count("1")), dtype=np.int32)
         parents = np.zeros((p, words), dtype=np.uint64)
-        self._check(getattr(self.lib, symbol)(self._h, p, words, offsets.ctypes.data, masks.ctypes.data if len(masks) else None,
-                                              scores.ctypes.data if len(scores) else None, None if ed is None else ed.ctypes.data,
-                                              comp.ctypes.data, C.byref(cost), order.ctypes.data, parents.ctypes.data))
-        return np.float32(cost.value), [int(x) for x in order], parents[:, 0].copy() if words == 1 else parents
+        r_cost = np.zeros(max(1, int(restarts)), dtype=np.float32)
+        r_moves = np.zeros(max(1, int(restarts)), dtype=np.uint32)
+        self._check(self.lib.urlgpu_order_local_search(self._h, p, words, offsets.ctypes.data, masks.ctypes.data if len(masks) else None,
+                                                       scores.ctypes.data if len(scores) else None, None if ed is None else ed.ctypes.data,
+                                                       comp.ctypes.data, int(restarts), int(seed) & 0xFFFFFFFFFFFFFFFF, C.byref(cost),
+                                                       order.ctypes.data, parents.ctypes.data, r_cost.ctypes.data, r_moves.ctypes.data))
+        return (np.float32(cost.value), [int(x) for x in order], parents[:, 0].copy() if words == 1 else parents,
+                r_cost[:restarts], r_moves[:restarts])
+
+    @staticmethod
+    def _cache_entries(cache):
+        """a search.ScoreCache or a list of p (masks, scores) pairs -> (entries, p)"""
+        if hasattr(cache, "entries") and hasattr(cache, "p"):
+            return [cache.entries(v) for v in range(cache.p)], cache.p
+        entries = list(cache)
+        return entries, len(entries)
 
     def optimal_dag(self, cache, edges: Sequence[int] | None = None):
         """urlsearch_astar (host/search_capi.cpp:64-94) with urlgpu_order_search in place of A*: the skeleton's components
         (the rule of urlsearch::components), one search each, their costs summed in float32 in component order.
         cache: a search.ScoreCache or a list of p (masks, scores) pairs in search sign; edges: p skeleton masks or None.
         -> (total cost, parents uint64 [p]), the meaning and types of ScoreCache.astar's first two results"""
-        if hasattr(cache, "entries") and hasattr(cache, "p"):
-            p = cache.p
-            entries = [cache.entries(v) for v in range(p)]
-        else:
-            entries = list(cache)
-            p = len(entries)
+        return self._per_component(cache, edges, lambda entries, p, comp: self.order_search(entries, p, comp, edges))
+
+    def local_search_dag(self, cache, edges: Sequence[int] | None = None, restarts: int = 256, seed: int = 0):
+        """optimal_dag with order_local_search in place of order_search: one call per component, each with the same seed, the
+        costs summed in float32 in component order.  Components of any size up to 256 variables. -> (total cost, parents)"""
+        return self._per_component(cache, edges, lambda entries, p, comp: self.order_local_search(entries, p, comp, edges, restarts, seed)[:3])
+
+    def _per_component(self, cache, edges, search):
+        entries, p = self._cache_entries(cache)
         total = np.float32(0)
         parents = None
         for comp in components(p, edges):
-            cost, _, par = self.order_search(entries, p, comp, edges)
+            cost, _, par = search(entries, p, comp)
             total = np.float32(total + cost)
             if parents is None:
                 parents = np.zeros_like(par)

@@ -306,4 +306,239 @@ __global__ void order_backtrack_rank_kernel(const OrderVarRank *__restrict__ var
     out[1] = 1;
 }
 
+// ------------------------------------------------------------------------------------------------ local search
+// urlgpu_order_local_search: insertion hill climbing over the admissible orders of a component of up to 256 variables, with the
+// exact search's objective (the float32 left-to-right path sum of best(pi_m, {pi_0..pi_{m-1}})) and its best-parent tables.
+// One CTA per restart (resident CTAs stride over the restarts); the whole state of a restart lives in shared memory.
+//
+//   state       ord[m] (the variable at position m, as a position in C), at[v] (its inverse), b[m] = best(ord[m], pred_m),
+//               g[m] = the float32 sum of b[0..m) (g[0] = +0, one rounding per step), pre[m] = the set {ord[0..m)} (4 words).
+//   look-up     best(v, U) compacts U onto cand_v's <= 32 bits by testing at[] of cand_v's variables, then one gather from T_v
+//               and one from v's sorted scores, as in the exact search.
+//   iteration   one warp per source i.  For j > i the variables at i+1..j lose pi_i (X[m] = best(pi_m, pred_m \ pi_i)) and pi_i
+//               lands at j (Y[j] = best(pi_i, {pi_0..pi_j} \ pi_i)); for j < i the variables at j..i-1 gain pi_i (X[m]) and pi_i
+//               lands at j (Y[j] = best(pi_i, {pi_0..pi_{j-1}})): 2(k-1) look-ups per source, O(k^2) per iteration.  Each lane
+//               then sums its targets' paths left to right and re-adds the unchanged suffix until its running sum has the bits
+//               of the old g at the same position (from there on both sums are the same).  The argmin is a block reduction of
+//               a 64-bit key: order-preserving float bits (-0 folded to +0), then i, then j.
+//   output      per restart: the final cost, the number of moves, the order and the sorted position of each family.
+constexpr int kClimbMaxVars = 256;
+constexpr int kClimbMaxCand = 32;
+constexpr int kClimbWords = kClimbMaxVars / 64;
+constexpr int kClimbThreads = 256;
+constexpr int kClimbWarps = kClimbThreads / 32;
+
+struct OrderClimbVar {       // variable at position j of C
+    unsigned long long table;               // offset of T_j in the table buffer (uint32 elements)
+    unsigned long long adj[kClimbWords];    // skeleton neighbours over C's positions; all of C without a skeleton
+    uint32_t score;                         // offset of j's sorted scores
+    uint32_t ncand;                         // c_j
+    uint8_t cand[kClimbMaxCand];            // cand_j as positions in C, ascending
+};
+
+__host__ __device__ __forceinline__ size_t order_climb_smem_bytes(int k) {
+    return (size_t)k * sizeof(OrderClimbVar) + (size_t)(k + 1) * kClimbWords * 8 + kClimbWarps * 8 + (size_t)(2 * k + 1) * 4 +
+           (size_t)kClimbWarps * k * 2 * 4 + (size_t)k * 2 + (size_t)kClimbWarps * k * 2;
+}
+
+__device__ __forceinline__ uint64_t climb_draw(uint64_t &x) {   // splitmix64
+    uint64_t z = (x += 0x9E3779B97F4A7C15ull);
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+
+// the sorted position of best(v, U), U = {u : at[u] < lim, u != out} + {in}; kOrderNone if v has no entry inside U
+__device__ __forceinline__ uint32_t climb_best_pos(const OrderClimbVar &V, const uint8_t *at, int lim, int out, int in, const uint32_t *__restrict__ T) {
+    uint32_t idx = 0;
+    for (uint32_t t = 0; t < V.ncand; t++) {
+        const int u = V.cand[t];
+        if (((int)at[u] < lim && u != out) || u == in) idx |= 1u << t;
+    }
+    return __ldg(T + V.table + idx);
+}
+__device__ __forceinline__ float climb_best(const OrderClimbVar &V, const uint8_t *at, int lim, int out, int in, const uint32_t *__restrict__ T,
+                                            const float *__restrict__ scores) {
+    const uint32_t pos = climb_best_pos(V, at, lim, out, in, T);
+    return pos == kOrderNone ? 3.402823466e+38f : __ldg(scores + V.score + pos);
+}
+// does v have a skeleton neighbour in the set P, leaving out position `out`?
+__device__ __forceinline__ bool climb_touches(const OrderClimbVar &V, const unsigned long long *P, int out) {
+    unsigned long long any = 0;
+#pragma unroll
+    for (int w = 0; w < kClimbWords; w++) any |= V.adj[w] & P[w] & ~(w == (out >> 6) ? 1ull << (out & 63) : 0ull);
+    return any != 0;
+}
+// order-preserving key of a float32 cost, -0 folded to +0
+__device__ __forceinline__ uint32_t climb_key(float g) {
+    const uint32_t u = g == 0.0f ? 0u : __float_as_uint(g);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+__global__ void __launch_bounds__(kClimbThreads) order_climb_kernel(const OrderClimbVar *__restrict__ vars, const uint32_t *__restrict__ T,
+                                                                    const float *__restrict__ scores, int k, uint32_t restarts, unsigned long long seed,
+                                                                    float *__restrict__ r_cost, uint32_t *__restrict__ r_moves,
+                                                                    uint8_t *__restrict__ r_order, uint32_t *__restrict__ r_pos) {
+    extern __shared__ __align__(16) unsigned char climb_smem[];
+    OrderClimbVar *s_var = reinterpret_cast<OrderClimbVar *>(climb_smem);
+    unsigned long long *s_pre = reinterpret_cast<unsigned long long *>(s_var + k);         // [k + 1][kClimbWords]
+    unsigned long long *s_key = s_pre + (k + 1) * kClimbWords;                              // [kClimbWarps]
+    float *s_b = reinterpret_cast<float *>(s_key + kClimbWarps);                             // [k]
+    float *s_g = s_b + k;                                                                   // [k + 1]
+    float *s_x = s_g + k + 1;                                                               // [kClimbWarps][k]
+    float *s_y = s_x + kClimbWarps * k;                                                     // [kClimbWarps][k]
+    uint8_t *s_ord = reinterpret_cast<uint8_t *>(s_y + kClimbWarps * k);                    // [k]
+    uint8_t *s_at = s_ord + k;                                                              // [k]
+    uint8_t *s_okx = s_at + k;                                                              // [kClimbWarps][k]
+    uint8_t *s_oky = s_okx + kClimbWarps * k;                                               // [kClimbWarps][k]
+    __shared__ int s_flag;
+    __shared__ uint32_t s_moves;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int i = threadIdx.x; i < k; i += blockDim.x) s_var[i] = vars[i];
+    __syncthreads();
+
+    for (uint32_t r = blockIdx.x; r < restarts; r += gridDim.x) {
+        // start: a random admissible order (one thread; k draws)
+        if (threadIdx.x == 0) {
+            uint64_t x = seed + 0xD1B54A32D192ED03ull * ((uint64_t)r + 1);
+            unsigned long long *placed = s_pre, *front = s_pre + kClimbWords;   // scratch: pre[] is rebuilt from the order
+            for (int w = 0; w < kClimbWords; w++) placed[w] = front[w] = 0;
+            int ok = 1;
+            for (int m = 0; m < k; m++) {
+                const uint64_t z = climb_draw(x);
+                int v;
+                if (m == 0) {
+                    v = (int)(z % (uint64_t)k);
+                } else {
+                    int nf = 0;
+                    for (int w = 0; w < kClimbWords; w++) nf += __popcll(front[w]);
+                    if (nf == 0) { ok = 0; break; }
+                    int want = (int)(z % (uint64_t)nf), w = 0;
+                    while (want >= __popcll(front[w])) want -= __popcll(front[w++]);
+                    unsigned long long f = front[w];
+                    for (; want; want--) f &= f - 1;
+                    v = 64 * w + __ffsll((long long)f) - 1;
+                }
+                s_ord[m] = (uint8_t)v;
+                placed[v >> 6] |= 1ull << (v & 63);
+                for (int w = 0; w < kClimbWords; w++) front[w] = (front[w] | s_var[v].adj[w]) & ~placed[w];
+            }
+            s_flag = ok;
+            s_moves = 0;
+        }
+        __syncthreads();
+        if (!s_flag) {                                            // the component has no admissible order
+            if (threadIdx.x == 0) { r_cost[r] = __int_as_float(0x7f800000); r_moves[r] = 0; }
+            for (int m = threadIdx.x; m < k; m += blockDim.x) { r_order[(size_t)r * k + m] = 0; r_pos[(size_t)r * k + m] = kOrderNone; }
+            __syncthreads();
+            continue;
+        }
+        for (;;) {
+            // the state of the current order: at[], pre[], b[], g[]
+            for (int m = threadIdx.x; m < k; m += blockDim.x) s_at[s_ord[m]] = (uint8_t)m;
+            if (threadIdx.x < kClimbWords) {
+                unsigned long long acc = 0;
+                s_pre[threadIdx.x] = 0;
+                for (int m = 0; m < k; m++) {
+                    const int v = s_ord[m];
+                    if ((v >> 6) == (int)threadIdx.x) acc |= 1ull << (v & 63);
+                    s_pre[(m + 1) * kClimbWords + threadIdx.x] = acc;
+                }
+            }
+            __syncthreads();
+            for (int m = threadIdx.x; m < k; m += blockDim.x) s_b[m] = climb_best(s_var[s_ord[m]], s_at, m, -1, -1, T, scores);
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                float g = 0.0f;
+                s_g[0] = g;
+                for (int m = 0; m < k; m++) s_g[m + 1] = g = __fadd_rn(g, s_b[m]);
+            }
+            __syncthreads();
+
+            // every move (i, j): one warp per source i
+            float *X = s_x + warp * k, *Y = s_y + warp * k;
+            uint8_t *okX = s_okx + warp * k, *okY = s_oky + warp * k;
+            unsigned long long best = ~0ull;
+            for (int i = warp; i < k; i += kClimbWarps) {
+                const int vi = s_ord[i];
+                const OrderClimbVar &Vi = s_var[vi];
+                for (int t = lane; t < k; t += 32) {
+                    if (t == i) continue;
+                    const OrderClimbVar &Vt = s_var[s_ord[t]];
+                    if (t > i) {
+                        X[t] = climb_best(Vt, s_at, t, vi, -1, T, scores);
+                        okX[t] = t == 1 || climb_touches(Vt, s_pre + t * kClimbWords, vi);
+                        Y[t] = climb_best(Vi, s_at, t + 1, vi, -1, T, scores);
+                        okY[t] = climb_touches(Vi, s_pre + (t + 1) * kClimbWords, vi);
+                    } else {
+                        X[t] = climb_best(Vt, s_at, t, -1, vi, T, scores);
+                        okX[t] = t > 0 || ((Vt.adj[vi >> 6] >> (vi & 63)) & 1);
+                        Y[t] = climb_best(Vi, s_at, t, -1, -1, T, scores);
+                        okY[t] = t == 0 || climb_touches(Vi, s_pre + t * kClimbWords, -1);
+                    }
+                }
+                __syncwarp();
+                for (int j = lane; j < k; j += 32) {
+                    if (j == i || !okY[j]) continue;
+                    bool ok = true;
+                    float g;
+                    int m0;
+                    if (j > i) {
+                        g = s_g[i];
+                        for (int m = i + 1; m <= j && ok; m++) { ok = okX[m]; g = __fadd_rn(g, X[m]); }
+                        g = __fadd_rn(g, Y[j]);
+                        m0 = j + 1;
+                    } else {
+                        g = __fadd_rn(s_g[j], Y[j]);
+                        for (int m = j; m < i && ok; m++) { ok = okX[m]; g = __fadd_rn(g, X[m]); }
+                        m0 = i + 1;
+                    }
+                    if (!ok) continue;
+                    for (int m = m0; m < k; m++) {
+                        if (__float_as_uint(g) == __float_as_uint(s_g[m])) { g = s_g[k]; break; }
+                        g = __fadd_rn(g, s_b[m]);
+                    }
+                    const unsigned long long key = ((unsigned long long)climb_key(g) << 32) | ((unsigned long long)i << 8) | (unsigned long long)j;
+                    best = min(best, key);
+                }
+                __syncwarp();
+            }
+            for (int o = 16; o; o >>= 1) best = min(best, __shfl_xor_sync(0xFFFFFFFFu, best, o));
+            if (lane == 0) s_key[warp] = best;
+            __syncthreads();
+
+            // the move, if it strictly lowers the cost
+            if (threadIdx.x == 0) {
+                unsigned long long key = s_key[0];
+                for (int w = 1; w < kClimbWarps; w++) key = min(key, s_key[w]);
+                int take = 0;
+                if (key != ~0ull) {
+                    const uint32_t kc = (uint32_t)(key >> 32);
+                    const float c = __uint_as_float((kc & 0x80000000u) ? (kc & 0x7FFFFFFFu) : ~kc);
+                    take = c < s_g[k];
+                }
+                if (take) {
+                    const int i = (int)((key >> 8) & 255), j = (int)(key & 255);
+                    const uint8_t v = s_ord[i];
+                    if (j > i) for (int m = i; m < j; m++) s_ord[m] = s_ord[m + 1];
+                    else for (int m = i; m > j; m--) s_ord[m] = s_ord[m - 1];
+                    s_ord[j] = v;
+                    s_moves++;
+                }
+                s_flag = take;
+            }
+            __syncthreads();
+            if (!s_flag) break;
+        }
+
+        // the local optimum of restart r
+        for (int m = threadIdx.x; m < k; m += blockDim.x) {
+            r_order[(size_t)r * k + m] = s_ord[m];
+            r_pos[(size_t)r * k + m] = climb_best_pos(s_var[s_ord[m]], s_at, m, -1, -1, T);
+        }
+        if (threadIdx.x == 0) { r_cost[r] = s_g[k]; r_moves[r] = s_moves; }
+        __syncthreads();
+    }
+}
+
 } // namespace urlgpu

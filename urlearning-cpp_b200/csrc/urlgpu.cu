@@ -385,6 +385,7 @@ extern "C" int urlgpu_create(urlgpu_ctx **out, int device_id) {
         attrs.push_back({(const void *)cbic_sets_kernel, big});
         attrs.push_back({(const void *)gram_partial_kernel, (int)kGramSmemBytes});
         attrs.push_back({(const void *)order_layer_rank_kernel, (int)order_rank_smem_bytes(kOrderRankMaxVars)});
+        attrs.push_back({(const void *)order_climb_kernel, (int)order_climb_smem_bytes(kClimbMaxVars)});
         for (const auto &a : attrs)
             if ((e = cudaFuncSetAttribute(a.first, cudaFuncAttributeMaxDynamicSharedMemorySize, a.second)) != cudaSuccess)
                 return refuse("cannot opt a kernel into " + std::to_string(a.second) + " bytes of dynamic shared memory (the device allows " +
@@ -2532,17 +2533,28 @@ extern "C" int urlgpu_spg_free(urlgpu_spg *sp) {
 }
 
 // ============================================================================================ order-graph search
-// urlgpu_order_search and urlgpu_order_search_layered (order_kernels.cuh).  The host validates everything, translates the
-// component's qualifying entries to compact masks over C's positions once, sorts each variable's list in the (score, |S|,
-// mask) order of SortedEntries::build, and sizes the call before any allocation.  One upload of the small arrays, the table
-// passes, k layer launches, one backtrack and one copy back; the host then maps each leaf's sorted position to its parent
-// mask.  The two entry points differ only in the node storage, the layer launches and the backtrack.
-static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
-                             const float *scores, const uint64_t *edges, const uint64_t *component, float *cost, int32_t *order,
-                             uint64_t *parents) {
-    if (!ctx) return URLGPU_ERR_ARG;
-    auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, (layered ? "order_search_layered: " : "order_search: ") + m); };
-    if (!offsets || !component || !cost || !order || !parents) return refuse(URLGPU_ERR_ARG, "null argument");
+// urlgpu_order_search, urlgpu_order_search_layered and urlgpu_order_local_search (order_kernels.cuh).  order_prepare validates
+// everything on the host, keeps the component's qualifying entries, sorts each variable's list in the (score, |S|, mask) order
+// of SortedEntries::build and lays out the best-parent tables, compacting each entry straight from its variable-space mask onto
+// cand_v's bits.  order_tables uploads the entries and builds the tables.  Each entry point sizes its call before any
+// allocation; the host maps each chosen sorted position back to its parent mask.
+struct OrderPrep {
+    std::vector<int> vars;                       // position j of C -> variable
+    std::vector<std::vector<uint64_t>> ent;      // per position: indices into masks/scores, sorted
+    std::vector<std::vector<int>> cand;          // per position: cand_j as positions in C, ascending
+    std::vector<uint64_t> table;                 // per position: offset of T_j (uint32 elements), 2^c_j of them
+    std::vector<uint32_t> score;                 // per position: offset of j's sorted entries
+    std::vector<unsigned long long> where;       // per sorted entry: its slot in the tables
+    std::vector<uint32_t> epos;                  // per sorted entry: its position in its variable's list
+    std::vector<float> escore;                   // per sorted entry: its score
+    uint64_t n_ent = 0, table_elems = 0;
+};
+
+// every check and translation the three entry points share; `who` prefixes the messages.  Components of more than max_k
+// variables and variables with more than max_cand candidate parents inside the component are refused
+static int order_prepare(urlgpu_ctx *ctx, const std::string &who, int max_k, int max_cand, int p, int mask_words, const uint64_t *offsets,
+                         const uint64_t *masks, const float *scores, const uint64_t *component, OrderPrep &P) {
+    auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, who + m); };
     if (p < 1) return refuse(URLGPU_ERR_ARG, "p must be at least 1");
     if (mask_words < 1 || mask_words > kSpgMaxWords) return refuse(URLGPU_ERR_ARG, "mask_words must be in 1.." + std::to_string(kSpgMaxWords));
     if ((int64_t)mask_words * 64 < p) return refuse(URLGPU_ERR_ARG, "mask_words too small for the variable count");
@@ -2550,43 +2562,38 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
         if (offsets[v + 1] < offsets[v]) return refuse(URLGPU_ERR_ARG, "offsets decrease at variable " + std::to_string(v));
     if (offsets[p] > offsets[0] && (!masks || !scores)) return refuse(URLGPU_ERR_ARG, "null entries");
     auto bit = [&](const uint64_t *m, int v) { return (m[v >> 6] >> (v & 63)) & 1; };
-    std::vector<int> vars;                       // position j of C -> variable
     std::vector<int> pos_of(p, -1);
     for (int w = 0; w < mask_words; w++)
         for (int b = 0; b < 64; b++) {
             if (!((component[w] >> b) & 1)) continue;
             if (w * 64 + b >= p) return refuse(URLGPU_ERR_ARG, "the component names variable " + std::to_string(w * 64 + b) + " >= p");
-            pos_of[w * 64 + b] = (int)vars.size();
-            vars.push_back(w * 64 + b);
+            pos_of[w * 64 + b] = (int)P.vars.size();
+            P.vars.push_back(w * 64 + b);
         }
-    if (vars.empty()) return refuse(URLGPU_ERR_ARG, "empty component");
+    if (P.vars.empty()) return refuse(URLGPU_ERR_ARG, "empty component");
     for (int v = 0; v < p; v++)
         for (uint64_t e = offsets[v]; e < offsets[v + 1]; e++) {
             if (std::isnan(scores[e])) return refuse(URLGPU_ERR_ARG, "variable " + std::to_string(v) + ", entry " + std::to_string(e - offsets[v]) + ": NaN score");
             if (bit(masks + e * mask_words, v)) return refuse(URLGPU_ERR_ARG, "variable " + std::to_string(v) + ", entry " + std::to_string(e - offsets[v]) + ": the parent set contains the variable itself");
         }
-    const int k = (int)vars.size();
-    const int max_k = layered ? kOrderRankMaxVars : kOrderMaxVars;
+    const int k = (int)P.vars.size();
     if (k > max_k) return refuse(URLGPU_ERR_LIMIT, std::to_string(k) + " variables in the component; at most " + std::to_string(max_k) + " are supported");
 
-    // qualifying entries (all parents inside C), compact masks, per-variable sort
-    std::vector<uint64_t> Cmask(component, component + mask_words);
-    std::vector<std::vector<uint64_t>> ent(k);   // per position: indices into masks/scores, sorted
-    std::vector<std::vector<uint64_t>> cm(k);    // compact masks in the same order
-    std::vector<OrderVarRank> hv(k);
-    auto compact = [&](const uint64_t *m) {
-        uint64_t c = 0;
-        for (int j = 0; j < k; j++) if (bit(m, vars[j])) c |= 1ull << j;
-        return c;
-    };
-    uint64_t n_ent = 0, table_elems = 0;
+    // qualifying entries (all parents inside C), per-variable sort, cand_j, table layout
+    P.ent.assign(k, {});
+    P.cand.assign(k, {});
+    P.table.assign(k, 0);
+    P.score.assign(k, 0);
     for (int j = 0; j < k; j++) {
-        const int v = vars[j];
-        auto &E = ent[j];
+        const int v = P.vars[j];
+        auto &E = P.ent[j];
+        std::vector<uint64_t> cw(mask_words, 0);
         for (uint64_t e = offsets[v]; e < offsets[v + 1]; e++) {
             bool inside = true;
-            for (int w = 0; w < mask_words && inside; w++) inside = (masks[e * mask_words + w] & ~Cmask[w]) == 0;
-            if (inside) E.push_back(e);
+            for (int w = 0; w < mask_words && inside; w++) inside = (masks[e * mask_words + w] & ~component[w]) == 0;
+            if (!inside) continue;
+            E.push_back(e);
+            for (int w = 0; w < mask_words; w++) cw[w] |= masks[e * mask_words + w];
         }
         auto card = [&](uint64_t i) { int c = 0; for (int w = 0; w < mask_words; w++) c += __builtin_popcountll(masks[i * mask_words + w]); return c; };
         std::sort(E.begin(), E.end(), [&](uint64_t a, uint64_t b) {   // as urlgpu_spg_build (sparse_parent_list.cpp:7-9, ties by |S|, mask)
@@ -2598,18 +2605,94 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
             return a < b;
         });
         if (E.size() > 0xFFFFFFFEull) return refuse(URLGPU_ERR_LIMIT, "variable " + std::to_string(v) + " has 2^32 or more entries inside the component");
+        for (int u = 0; u < p; u++) if (bit(cw.data(), u)) P.cand[j].push_back(pos_of[u]);
+        if (P.cand[j].size() > (size_t)max_cand)
+            return refuse(URLGPU_ERR_LIMIT, "variable " + std::to_string(v) + " has " + std::to_string(P.cand[j].size()) +
+                                                " candidate parents inside the component; at most " + std::to_string(max_cand) + " are supported");
+        P.table[j] = P.table_elems;
+        P.score[j] = (uint32_t)P.n_ent;
+        P.table_elems += (uint64_t)1 << P.cand[j].size();
+        P.n_ent += E.size();
+    }
+    if (P.n_ent > 0xFFFFFFFFull) return refuse(URLGPU_ERR_LIMIT, "2^32 or more entries inside the component");
+    P.where.resize(P.n_ent);
+    P.epos.resize(P.n_ent);
+    P.escore.resize(P.n_ent);
+    for (int j = 0; j < k; j++)
+        for (size_t i = 0; i < P.ent[j].size(); i++) {
+            const uint64_t *m = masks + P.ent[j][i] * mask_words;
+            uint64_t idx = 0;                                  // the entry over cand_j's bits
+            for (size_t q = 0; q < P.cand[j].size(); q++) if (bit(m, P.vars[P.cand[j][q]])) idx |= 1ull << q;
+            P.where[P.score[j] + i] = P.table[j] + idx;
+            P.epos[P.score[j] + i] = (uint32_t)i;
+            P.escore[P.score[j] + i] = scores[P.ent[j][i]];
+        }
+    return URLGPU_OK;
+}
+
+// d_ent = where | pos | score (16 bytes an entry); T = every T_j: fill, scatter, subset-min transform, under ms_order_tables
+static int order_tables(urlgpu_ctx *ctx, const OrderPrep &P, void *d_ent, uint32_t *T) {
+    cudaStream_t s = ctx->stream;
+    const uint64_t n_ent = P.n_ent;
+    unsigned long long *dw = static_cast<unsigned long long *>(d_ent);
+    uint32_t *dp = reinterpret_cast<uint32_t *>(dw + n_ent);
+    float *ds = reinterpret_cast<float *>(dp + n_ent);
+    if (n_ent) {
+        CK(cudaMemcpyAsync(dw, P.where.data(), n_ent * 8, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(dp, P.epos.data(), n_ent * 4, cudaMemcpyHostToDevice, s));
+        CK(cudaMemcpyAsync(ds, P.escore.data(), n_ent * 4, cudaMemcpyHostToDevice, s));
+    }
+    const int k = (int)P.vars.size();
+    uint64_t launches = 1;
+    for (int j = 0; j < k; j++) launches += 1 + std::max(0, (int)P.cand[j].size() - kOrderSegBits);
+    Region rg(ctx, F_ORDER_TABLES, launches);
+    CK(cudaMemsetAsync(T, 0xFF, P.table_elems * 4, s));
+    if (n_ent) order_scatter_kernel<<<blocks_for(n_ent, 256), 256, 0, s>>>(dw, dp, n_ent, T);
+    for (int j = 0; j < k; j++) {
+        const int c = (int)P.cand[j].size(), lb = std::min(c, kOrderSegBits);
+        uint32_t *Tj = T + P.table[j];
+        if (lb) order_table_low_kernel<<<(unsigned)(1u << (c - lb)), std::min(1024, std::max(32, 1 << (lb - 1))), 0, s>>>(Tj, lb);
+        for (int b = lb; b < c; b++) order_table_high_kernel<<<blocks_for((uint64_t)1 << (c - 1), 256), 256, 0, s>>>(Tj, b, (uint64_t)1 << (c - 1));
+    }
+    CK(cudaGetLastError());
+    return URLGPU_OK;
+}
+
+// the device's free memory plus the allocator's idle blocks
+static int order_free_bytes(urlgpu_ctx *ctx, size_t *free_b) {
+    CK(cudaSetDevice(ctx->device));
+    size_t total_b = 0;
+    CK(cudaMemGetInfo(free_b, &total_b));
+    for (auto &b : ctx->pool) if (!b.used) *free_b += b.bytes;      // cached blocks the allocator can hand out or release
+    return URLGPU_OK;
+}
+
+static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                             const float *scores, const uint64_t *edges, const uint64_t *component, float *cost, int32_t *order,
+                             uint64_t *parents) {
+    if (!ctx) return URLGPU_ERR_ARG;
+    const std::string who = layered ? "order_search_layered: " : "order_search: ";
+    auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, who + m); };
+    if (!offsets || !component || !cost || !order || !parents) return refuse(URLGPU_ERR_ARG, "null argument");
+    OrderPrep P;
+    const int max_k = layered ? kOrderRankMaxVars : kOrderMaxVars;        // c_v < k, so max_k - 1 never refuses a variable
+    if (int rc = order_prepare(ctx, who, max_k, max_k - 1, p, mask_words, offsets, masks, scores, component, P)) return rc;
+    const int k = (int)P.vars.size();
+    const uint64_t n_ent = P.n_ent, table_elems = P.table_elems;
+    std::vector<OrderVarRank> hv(k);
+    for (int j = 0; j < k; j++) {
         uint64_t cand = 0;
-        for (uint64_t e : E) { cm[j].push_back(compact(masks + e * mask_words)); cand |= cm[j].back(); }
-        hv[j].table = table_elems;
-        hv[j].score = (uint32_t)n_ent;
+        for (int q : P.cand[j]) cand |= 1ull << q;
+        hv[j].table = P.table[j];
+        hv[j].score = P.score[j];
         hv[j].cand = cand;
         hv[j].adj = ~0ull;
-        if (edges) hv[j].adj = compact(edges + (size_t)v * mask_words);
+        if (edges) {
+            hv[j].adj = 0;
+            for (int i = 0; i < k; i++) if ((edges[(size_t)P.vars[j] * mask_words + (P.vars[i] >> 6)] >> (P.vars[i] & 63)) & 1) hv[j].adj |= 1ull << i;
+        }
         for (int b = 0; b < kOrderRankLut; b++) hv[j].shift[b] = (uint8_t)__builtin_popcountll(cand & ((1ull << (8 * b)) - 1));
-        table_elems += (uint64_t)1 << __builtin_popcountll(cand);
-        n_ent += E.size();
     }
-    if (n_ent > 0xFFFFFFFFull) return refuse(URLGPU_ERR_LIMIT, "2^32 or more entries inside the component");
 
     // binomials: C(b, i) for b, i <= kOrderRankMaxVars (the dense kernels take the uint32 corner b, i <= kOrderMaxVars)
     std::vector<unsigned long long> binom(kOrderRankBinom * kOrderRankBinom, 0);
@@ -2628,10 +2711,8 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
     const size_t small_bytes = (size_t)k * var_bytes + (size_t)k * n_lut * 256 + binom_bytes + (2 + 2 * (size_t)k) * 4;
     const uint64_t node_bytes = layered ? nodes + 8 * widest : 5 * nodes;
     const size_t need = node_bytes + 4 * table_elems + n_ent * (8 + 4 + 4) + small_bytes;
-    CK(cudaSetDevice(ctx->device));
-    size_t free_b = 0, total_b = 0;
-    CK(cudaMemGetInfo(&free_b, &total_b));
-    for (auto &b : ctx->pool) if (!b.used) free_b += b.bytes;      // cached blocks the allocator can hand out or release
+    size_t free_b = 0;
+    if (int rc = order_free_bytes(ctx, &free_b)) return rc;
     auto bytes_msg = [&]() {
         const std::string nodes_part = layered ? std::to_string(nodes) + " for the leaves of the 2^" + std::to_string(k) + " nodes, " +
                                                      std::to_string(8 * widest) + " for two cost layers of C(" + std::to_string(k) + ", " + std::to_string(k / 2) + ") nodes, "
@@ -2640,7 +2721,7 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
     };
     if (need > free_b) return refuse(URLGPU_ERR_LIMIT, "the search needs " + bytes_msg() + ", " + std::to_string(free_b) + " are free");
 
-    // host arrays: descriptors, byte look-up tables, scatter list, sorted scores
+    // host arrays: descriptors and byte look-up tables
     std::vector<OrderVar> hv32(layered ? 0 : k);
     for (int j = 0; j < (int)hv32.size(); j++) {
         hv32[j].table = hv[j].table;
@@ -2659,19 +2740,6 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
                 lut[((size_t)j * n_lut + b) * 256 + x] = (uint8_t)c;
             }
         }
-    std::vector<unsigned long long> where(n_ent);
-    std::vector<uint32_t> epos(n_ent);
-    std::vector<float> escore(n_ent);
-    for (int j = 0; j < k; j++) {
-        const uint64_t cand = hv[j].cand;
-        for (size_t i = 0; i < ent[j].size(); i++) {
-            uint64_t idx = 0; int q = 0;                  // compact mask over cand_j's bits
-            for (uint64_t m = cand; m; m &= m - 1, q++) if ((cm[j][i] >> __builtin_ctzll(m)) & 1) idx |= 1ull << q;
-            where[hv[j].score + i] = hv[j].table + idx;
-            epos[hv[j].score + i] = (uint32_t)i;
-            escore[hv[j].score + i] = scores[ent[j][i]];
-        }
-    }
 
     cudaStream_t s = ctx->stream;
     DevBuf d_cost(ctx), d_leaf(ctx), d_tab(ctx), d_small(ctx), d_ent(ctx);
@@ -2684,37 +2752,17 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
     const size_t cost_bytes = layered ? 8 * widest : 4 * nodes;
     if (!alloc(d_cost, cost_bytes) || !alloc(d_leaf, nodes) || !alloc(d_tab, table_elems * 4) || !alloc(d_small, small_bytes + 64) || !alloc(d_ent, ent_bytes))
         return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes_msg() + " failed");
-    // d_small: vars | lut | binom | out;  d_ent: where | pos | score
+    // d_small: vars | lut | binom | out
     char *sm = d_small.as<char>();
     uint8_t *dl = reinterpret_cast<uint8_t *>(sm + k * var_bytes);
     char *db = reinterpret_cast<char *>(dl + lut.size());
     uint32_t *dout = reinterpret_cast<uint32_t *>(db + binom_bytes);
-    unsigned long long *dw = d_ent.as<unsigned long long>();
-    uint32_t *dp = reinterpret_cast<uint32_t *>(dw + n_ent);
-    float *ds = reinterpret_cast<float *>(dp + n_ent);
     CK(cudaMemcpyAsync(sm, layered ? (const void *)hv.data() : (const void *)hv32.data(), k * var_bytes, cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(dl, lut.data(), lut.size(), cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(db, layered ? (const void *)binom.data() : (const void *)binom32.data(), binom_bytes, cudaMemcpyHostToDevice, s));
-    if (n_ent) {
-        CK(cudaMemcpyAsync(dw, where.data(), n_ent * 8, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(dp, epos.data(), n_ent * 4, cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(ds, escore.data(), n_ent * 4, cudaMemcpyHostToDevice, s));
-    }
     uint32_t *T = d_tab.as<uint32_t>();
-    {
-        uint64_t launches = 1;
-        for (int j = 0; j < k; j++) launches += 1 + std::max(0, __builtin_popcountll(hv[j].cand) - kOrderSegBits);
-        Region rg(ctx, F_ORDER_TABLES, launches);
-        CK(cudaMemsetAsync(T, 0xFF, table_elems * 4, s));
-        if (n_ent) order_scatter_kernel<<<blocks_for(n_ent, 256), 256, 0, s>>>(dw, dp, n_ent, T);
-        for (int j = 0; j < k; j++) {
-            const int c = __builtin_popcountll(hv[j].cand), lb = std::min(c, kOrderSegBits);
-            uint32_t *Tj = T + hv[j].table;
-            if (lb) order_table_low_kernel<<<(unsigned)(1u << (c - lb)), std::min(1024, std::max(32, 1 << (lb - 1))), 0, s>>>(Tj, lb);
-            for (int b = lb; b < c; b++) order_table_high_kernel<<<blocks_for((uint64_t)1 << (c - 1), 256), 256, 0, s>>>(Tj, b, (uint64_t)1 << (c - 1));
-        }
-        CK(cudaGetLastError());
-    }
+    if (int rc = order_tables(ctx, P, d_ent.p, T)) return rc;
+    const float *ds = reinterpret_cast<const float *>(reinterpret_cast<const uint32_t *>(d_ent.as<unsigned long long>() + n_ent) + n_ent);
     float *cst = d_cost.as<float>();
     uint8_t *lf = d_leaf.as<uint8_t>();
     {
@@ -2760,10 +2808,10 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
     if (!out[1] || c == INFINITY) return ctx->fail(URLGPU_ERR_ARG, "No solution found.");   // search_capi.cpp:87
     *cost = c;
     for (int i = 0; i < k; i++) {
-        const int j = (int)out[2 + i], v = vars[j];
+        const int j = (int)out[2 + i], v = P.vars[j];
         const uint32_t q = out[2 + k + i];
         order[i] = v;
-        for (int w = 0; w < mask_words; w++) parents[(size_t)v * mask_words + w] = q == kOrderNone ? 0 : masks[ent[j][q] * mask_words + w];
+        for (int w = 0; w < mask_words; w++) parents[(size_t)v * mask_words + w] = q == kOrderNone ? 0 : masks[P.ent[j][q] * mask_words + w];
     }
     return URLGPU_OK;
 }
@@ -2777,6 +2825,96 @@ extern "C" int urlgpu_order_search_layered(urlgpu_ctx *ctx, int p, int mask_word
                                            const float *scores, const uint64_t *edges, const uint64_t *component, float *cost,
                                            int32_t *order, uint64_t *parents) {
     return order_search_impl(ctx, true, p, mask_words, offsets, masks, scores, edges, component, cost, order, parents);
+}
+
+// Local search: the tables as above, then one order_climb_kernel launch over all restarts.  The host reads every restart's cost
+// and move count, takes the least cost (ties: the smallest restart), and copies back that restart's order and family positions.
+extern "C" int urlgpu_order_local_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                                         const float *scores, const uint64_t *edges, const uint64_t *component, uint32_t restarts,
+                                         uint64_t seed, float *cost, int32_t *order, uint64_t *parents, float *restart_costs,
+                                         uint32_t *restart_moves) {
+    if (!ctx) return URLGPU_ERR_ARG;
+    const std::string who = "order_local_search: ";
+    auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, who + m); };
+    if (!offsets || !component || !cost || !order || !parents) return refuse(URLGPU_ERR_ARG, "null argument");
+    if (restarts < 1 || restarts > (1u << 20)) return refuse(URLGPU_ERR_ARG, "restarts must be in 1..2^20");
+    OrderPrep P;
+    if (int rc = order_prepare(ctx, who, kClimbMaxVars, kClimbMaxCand, p, mask_words, offsets, masks, scores, component, P)) return rc;
+    const int k = (int)P.vars.size();
+    std::vector<OrderClimbVar> hv(k);
+    for (int j = 0; j < k; j++) {
+        OrderClimbVar &V = hv[j];
+        memset(&V, 0, sizeof V);
+        V.table = P.table[j];
+        V.score = P.score[j];
+        V.ncand = (uint32_t)P.cand[j].size();
+        for (size_t q = 0; q < P.cand[j].size(); q++) V.cand[q] = (uint8_t)P.cand[j][q];
+        for (int i = 0; i < k; i++)
+            if (!edges || ((edges[(size_t)P.vars[j] * mask_words + (P.vars[i] >> 6)] >> (P.vars[i] & 63)) & 1)) V.adj[i >> 6] |= 1ull << (i & 63);
+    }
+
+    // the device memory of the call: tables, entries, and per restart a cost, a move count, the order and the family positions
+    const uint64_t table_bytes = 4 * P.table_elems, ent_bytes = 16 * P.n_ent, restart_bytes = (uint64_t)restarts * (8 + 5 * (uint64_t)k);
+    const size_t var_bytes = (size_t)k * sizeof(OrderClimbVar);
+    const size_t need = table_bytes + ent_bytes + restart_bytes + var_bytes;
+    size_t free_b = 0;
+    if (int rc = order_free_bytes(ctx, &free_b)) return rc;
+    auto bytes_msg = [&]() {
+        return std::to_string(need) + " bytes of device memory (" + std::to_string(table_bytes) + " for the best-parent tables, " +
+               std::to_string(ent_bytes) + " for the entries, " + std::to_string(restart_bytes) + " for the state of " +
+               std::to_string(restarts) + " restarts)";
+    };
+    if (need > free_b) return refuse(URLGPU_ERR_LIMIT, "the search needs " + bytes_msg() + ", " + std::to_string(free_b) + " are free");
+
+    cudaStream_t s = ctx->stream;
+    DevBuf d_tab(ctx), d_ent(ctx), d_var(ctx), d_res(ctx);
+    auto alloc = [&](DevBuf &b, size_t bytes) {
+        const cudaError_t e = b.alloc(bytes);
+        if (e != cudaSuccess) { cudaGetLastError(); return false; }
+        return true;
+    };
+    if (!alloc(d_tab, table_bytes) || !alloc(d_ent, std::max<uint64_t>(16, ent_bytes)) || !alloc(d_var, var_bytes) || !alloc(d_res, restart_bytes))
+        return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes_msg() + " failed");
+    // d_res: cost | moves | positions | order
+    float *r_cost = d_res.as<float>();
+    uint32_t *r_moves = reinterpret_cast<uint32_t *>(r_cost + restarts);
+    uint32_t *r_pos = r_moves + restarts;
+    uint8_t *r_order = reinterpret_cast<uint8_t *>(r_pos + (size_t)restarts * k);
+    CK(cudaMemcpyAsync(d_var.p, hv.data(), var_bytes, cudaMemcpyHostToDevice, s));
+    uint32_t *T = d_tab.as<uint32_t>();
+    if (int rc = order_tables(ctx, P, d_ent.p, T)) return rc;
+    const float *ds = reinterpret_cast<const float *>(reinterpret_cast<const uint32_t *>(d_ent.as<unsigned long long>() + P.n_ent) + P.n_ent);
+    {
+        Region rg(ctx, F_ORDER_LAYERS, 1);
+        const size_t smem = order_climb_smem_bytes(k);
+        int per_sm = 0;
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_climb_kernel, kClimbThreads, smem));
+        const uint64_t grid = std::min<uint64_t>(restarts, (uint64_t)std::max(1, per_sm) * ctx->sm_count);
+        order_climb_kernel<<<(unsigned)grid, kClimbThreads, smem, s>>>(d_var.as<OrderClimbVar>(), T, ds, k, restarts, seed, r_cost, r_moves, r_order, r_pos);
+        CK(cudaGetLastError());
+    }
+    std::vector<float> rc_h(restarts);
+    std::vector<uint32_t> rm_h(restarts);
+    CK(cudaMemcpyAsync(rc_h.data(), r_cost, (size_t)restarts * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(rm_h.data(), r_moves, (size_t)restarts * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    uint32_t best = 0;
+    for (uint32_t r = 1; r < restarts; r++) if (rc_h[r] < rc_h[best]) best = r;
+    if (!(rc_h[best] < INFINITY)) return ctx->fail(URLGPU_ERR_ARG, "No solution found.");   // search_capi.cpp:87
+    std::vector<uint8_t> ord(k);
+    std::vector<uint32_t> pos(k);
+    CK(cudaMemcpyAsync(ord.data(), r_order + (size_t)best * k, k, cudaMemcpyDeviceToHost, s));
+    CK(cudaMemcpyAsync(pos.data(), r_pos + (size_t)best * k, (size_t)k * 4, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    *cost = rc_h[best];
+    for (int m = 0; m < k; m++) {
+        const int j = ord[m], v = P.vars[j];
+        order[m] = v;
+        for (int w = 0; w < mask_words; w++) parents[(size_t)v * mask_words + w] = pos[m] == kOrderNone ? 0 : masks[P.ent[j][pos[m]] * mask_words + w];
+    }
+    if (restart_costs) memcpy(restart_costs, rc_h.data(), (size_t)restarts * 4);
+    if (restart_moves) memcpy(restart_moves, rm_h.data(), (size_t)restarts * 4);
+    return URLGPU_OK;
 }
 
 // ============================================================================================ listed sets
