@@ -25,6 +25,8 @@
  *   urlgpu_order_search      run_astar_on_one_scc (order-graph search) astar/astar_main.cpp:216-546
  *   urlgpu_order_search_layered  the same, for components of up to 36 variables
  *   urlgpu_order_local_search    (no counterpart: insertion hill climbing over the same orders, components of up to 256)
+ *   urlgpu_order_local_search_sparse  the same climb, with SparseParentList::getScore inside the climb
+ *                                                                     score_cache/sparse_parent_list.cpp:44-55
  *   urlgpu_prune             ScoreCalculator::prune                   scoring_function/score_calculator.cpp:150-197
  *   urlgpu_result_*          FloatMap iteration in scoringThread      score/score_main.cpp:187-200, base/typedefs.h:816
  *
@@ -254,6 +256,21 @@ int urlgpu_order_local_search(urlgpu_ctx *ctx, int p, int mask_words, const uint
                               float *cost, int32_t *order, uint64_t *parents,
                               float *restart_costs /* optional, [restarts] */, uint32_t *restart_moves /* optional, [restarts] */);
 
+/* urlgpu_order_local_search with best(v, U) looked up in v's sorted list instead of a best-parent table: the first qualifying
+ * entry, in (score, |S|, mask) order, whose parent set lies inside U (SparseParentList::getScore), so a variable may have any
+ * number of candidate parents inside C.  Same arguments, contract and outputs; on every input both accept, the same cost,
+ * order, parents, restart costs and restart moves, bit for bit.  Device memory: 8 ceil(|C|/64) + 4 per qualifying entry,
+ * 8 + 5|C| per restart and 80|C| of descriptors; no tables.  Refusals, all before any launch: every URLGPU_ERR_ARG refusal of
+ * urlgpu_order_local_search with the same message after "order_local_search_sparse: "; |C| > 256, 2^32 or more qualifying
+ * entries, and a call that does not fit the device's free memory (URLGPU_ERR_LIMIT, with the bytes split into entries and
+ * per-restart state).  No admissible order, or a best cost of +inf: URLGPU_ERR_ARG, "No solution found.".  Times: the climb
+ * under ms_order_layers; ms_order_tables does not grow. */
+int urlgpu_order_local_search_sparse(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                                     const float *scores, const uint64_t *edges, const uint64_t *component,
+                                     uint32_t restarts, uint64_t seed,
+                                     float *cost, int32_t *order, uint64_t *parents,
+                                     float *restart_costs /* optional, [restarts] */, uint32_t *restart_moves /* optional, [restarts] */);
+
 /* Measurement hooks: device time (CUDA events on the context's stream) and launch counts per kernel family,
  * accumulated since the last reset. */
 typedef struct urlgpu_stats {
@@ -276,7 +293,7 @@ typedef struct urlgpu_stats {
     double ms_standardise;     /* K2: column moments + standardisation passes (HBM bound); ms_gram is the DMMA Gram kernel + combine */
     uint64_t table16_fallbacks; /* K1 cube path: variables recomputed with 32-bit tables because a cell count did not fit 16 bits */
     double ms_order_tables;    /* urlgpu_order_search(_layered), urlgpu_order_local_search: best-parent tables (fill, scatter, subset-min transform) */
-    double ms_order_layers;    /* urlgpu_order_search(_layered): layer sweeps and the backtrack; urlgpu_order_local_search: the climb */
+    double ms_order_layers;    /* urlgpu_order_search(_layered): layer sweeps and the backtrack; urlgpu_order_local_search(_sparse): the climb */
 } urlgpu_stats;
 int urlgpu_stats_reset(urlgpu_ctx *ctx);
 int urlgpu_stats_get(urlgpu_ctx *ctx, urlgpu_stats *out);

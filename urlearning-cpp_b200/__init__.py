@@ -38,7 +38,7 @@ ABI_SYMBOLS = [
     "urlgpu_spg_build", "urlgpu_spg_query", "urlgpu_spg_free",
     "urlgpu_peer_alloc", "urlgpu_peer_open", "urlgpu_peer_close", "urlgpu_peer_free",
     "urlgpu_result_fetch_device", "urlgpu_copy_to_host", "urlgpu_order_search",
-    "urlgpu_order_search_layered", "urlgpu_order_local_search",
+    "urlgpu_order_search_layered", "urlgpu_order_local_search", "urlgpu_order_local_search_sparse",
 ]
 
 
@@ -126,6 +126,7 @@ def load_library():
     lib.urlgpu_order_search.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, P(C.c_float), vp, vp]
     lib.urlgpu_order_search_layered.argtypes = lib.urlgpu_order_search.argtypes
     lib.urlgpu_order_local_search.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, C.c_uint32, u64, P(C.c_float), vp, vp, vp, vp]
+    lib.urlgpu_order_local_search_sparse.argtypes = lib.urlgpu_order_local_search.argtypes
     for name in ABI_SYMBOLS:
         if name not in ("urlgpu_last_error", "urlgpu_host_alloc", "urlgpu_host_free"):
             getattr(lib, name).restype = C.c_int
@@ -162,6 +163,25 @@ def two_hop_neighbors(edges: Sequence[int] | None, p: int, v: int) -> int:
         if (orig >> j) & 1 and j != v:
             out |= nb(j)
     return out
+
+
+def table_bytes(offsets: np.ndarray, masks: np.ndarray, comp: np.ndarray) -> int:
+    """the bytes of urlgpu_order_local_search's best-parent tables, the sum of 4 2^c_v over the component's variables, where c_v
+    is the popcount of the union of v's qualifying parent sets (those inside the component).  offsets [p + 1], masks [n, words]
+    and comp [words] as order_local_search passes them to the C ABI"""
+    inside = ~np.any(masks & ~comp, axis=1)
+    total = 0
+    for v in range(len(offsets) - 1):
+        if not (int(comp[v >> 6]) >> (v & 63)) & 1:
+            continue
+        rows = masks[int(offsets[v]):int(offsets[v + 1])][inside[int(offsets[v]):int(offsets[v + 1])]]
+        total += 4 << (int(np.bitwise_count(np.bitwise_or.reduce(rows, axis=0)).sum()) if len(rows) else 0)
+    return total
+
+
+# order_local_search takes the table form while its tables take at most this many bytes, the sparse form above (DESIGN §5).
+# A variable with c_v > 32, which the table form refuses, alone needs 32 GiB.
+TABLE_MAX_BYTES = 4 << 30
 
 
 def components(p: int, edges: Sequence[int] | None) -> list[int]:
@@ -530,19 +550,28 @@ class Engine:
     def order_local_search(self, entries, p: int, component: int, edges: Sequence[int] | None = None, restarts: int = 256, seed: int = 0):
         """urlgpu_order_local_search: insertion hill climbing over the admissible orders of one skeleton component of up to 256
         variables, from `restarts` random orders, with the objective of order_search (so its cost is never below order_search's).
-        Same input conventions as order_search.
+        Same input conventions as order_search.  When the best-parent tables, 4 2^c_v bytes per variable (c_v: the candidate
+        parents inside the component, the union of its qualifying parent sets), would take more than TABLE_MAX_BYTES, the call
+        goes to urlgpu_order_local_search_sparse, which scans sorted lists instead (same contract, same bits where both run).
         -> (float32 cost, order list, parents as order_search returns them, float32 [restarts] final cost per restart,
             uint32 [restarts] moves per restart)"""
-        words, offsets, masks, scores, comp, ed = self._order_args(entries, p, component, edges)
+        args = self._order_args(entries, p, component, edges)
+        symbol = "urlgpu_order_local_search" if table_bytes(args[1], args[2], args[4]) <= TABLE_MAX_BYTES else "urlgpu_order_local_search_sparse"
+        return self._order_local_search(symbol, entries, p, component, edges, restarts, seed, args)
+
+    def _order_local_search(self, symbol: str, entries, p: int, component: int, edges: Sequence[int] | None = None, restarts: int = 256,
+                            seed: int = 0, args=None):
+        """order_local_search through the named entry point (tests and measurements compare the table and sparse forms)"""
+        words, offsets, masks, scores, comp, ed = args if args is not None else self._order_args(entries, p, component, edges)
         cost = C.c_float()
         order = np.zeros(max(1, bin(int(component)).count("1")), dtype=np.int32)
         parents = np.zeros((p, words), dtype=np.uint64)
         r_cost = np.zeros(max(1, int(restarts)), dtype=np.float32)
         r_moves = np.zeros(max(1, int(restarts)), dtype=np.uint32)
-        self._check(self.lib.urlgpu_order_local_search(self._h, p, words, offsets.ctypes.data, masks.ctypes.data if len(masks) else None,
-                                                       scores.ctypes.data if len(scores) else None, None if ed is None else ed.ctypes.data,
-                                                       comp.ctypes.data, int(restarts), int(seed) & 0xFFFFFFFFFFFFFFFF, C.byref(cost),
-                                                       order.ctypes.data, parents.ctypes.data, r_cost.ctypes.data, r_moves.ctypes.data))
+        self._check(getattr(self.lib, symbol)(self._h, p, words, offsets.ctypes.data, masks.ctypes.data if len(masks) else None,
+                                              scores.ctypes.data if len(scores) else None, None if ed is None else ed.ctypes.data,
+                                              comp.ctypes.data, int(restarts), int(seed) & 0xFFFFFFFFFFFFFFFF, C.byref(cost),
+                                              order.ctypes.data, parents.ctypes.data, r_cost.ctypes.data, r_moves.ctypes.data))
         return (np.float32(cost.value), [int(x) for x in order], parents[:, 0].copy() if words == 1 else parents,
                 r_cost[:restarts], r_moves[:restarts])
 
@@ -563,7 +592,8 @@ class Engine:
 
     def local_search_dag(self, cache, edges: Sequence[int] | None = None, restarts: int = 256, seed: int = 0):
         """optimal_dag with order_local_search in place of order_search: one call per component, each with the same seed, the
-        costs summed in float32 in component order.  Components of any size up to 256 variables. -> (total cost, parents)"""
+        costs summed in float32 in component order.  Components of any size up to 256 variables, with any number of candidate
+        parents per variable. -> (total cost, parents)"""
         return self._per_component(cache, edges, lambda entries, p, comp: self.order_local_search(entries, p, comp, edges, restarts, seed)[:3])
 
     def _per_component(self, cache, edges, search):

@@ -313,8 +313,13 @@ __global__ void order_backtrack_rank_kernel(const OrderVarRank *__restrict__ var
 //
 //   state       ord[m] (the variable at position m, as a position in C), at[v] (its inverse), b[m] = best(ord[m], pred_m),
 //               g[m] = the float32 sum of b[0..m) (g[0] = +0, one rounding per step), pre[m] = the set {ord[0..m)} (4 words).
-//   look-up     best(v, U) compacts U onto cand_v's <= 32 bits by testing at[] of cand_v's variables, then one gather from T_v
-//               and one from v's sorted scores, as in the exact search.
+//   look-up     a policy.  ClimbTable (urlgpu_order_local_search): compact U onto cand_v's <= 32 bits by testing at[] of
+//               cand_v's variables, then one gather from T_v, as in the exact search.  ClimbList (urlgpu_order_local_search_sparse):
+//               the first entry of v's sorted list whose parent set, W = ceil(k/64) words over C's positions, lies inside U's
+//               words (pre[lim] with `out` cleared and `in` set); no limit on c_v.  Both lists and tie orders are the ones the
+//               tables are built from, so both policies return the same sorted position.  One gather from v's sorted scores.
+//               The move look-ups of ClimbList are warp-cooperative (32 consecutive entries a step, a ballot, the lowest lane),
+//               targets in descending order, so the U of pi_i's own look-ups only shrinks and each of them starts at the last hit.
 //   iteration   one warp per source i.  For j > i the variables at i+1..j lose pi_i (X[m] = best(pi_m, pred_m \ pi_i)) and pi_i
 //               lands at j (Y[j] = best(pi_i, {pi_0..pi_j} \ pi_i)); for j < i the variables at j..i-1 gain pi_i (X[m]) and pi_i
 //               lands at j (Y[j] = best(pi_i, {pi_0..pi_{j-1}})): 2(k-1) look-ups per source, O(k^2) per iteration.  Each lane
@@ -329,11 +334,14 @@ constexpr int kClimbThreads = 256;
 constexpr int kClimbWarps = kClimbThreads / 32;
 
 struct OrderClimbVar {       // variable at position j of C
-    unsigned long long table;               // offset of T_j in the table buffer (uint32 elements)
+    union {
+        unsigned long long table;           // ClimbTable: offset of T_j in the table buffer (uint32 elements)
+        unsigned long long nent;            // ClimbList: the number of j's entries
+    };
     unsigned long long adj[kClimbWords];    // skeleton neighbours over C's positions; all of C without a skeleton
-    uint32_t score;                         // offset of j's sorted scores
+    uint32_t score;                         // offset of j's sorted scores (and, for ClimbList, of its entries' words)
     uint32_t ncand;                         // c_j
-    uint8_t cand[kClimbMaxCand];            // cand_j as positions in C, ascending
+    uint8_t cand[kClimbMaxCand];            // ClimbTable: cand_j as positions in C, ascending
 };
 
 __host__ __device__ __forceinline__ size_t order_climb_smem_bytes(int k) {
@@ -348,18 +356,61 @@ __device__ __forceinline__ uint64_t climb_draw(uint64_t &x) {   // splitmix64
     return z ^ (z >> 31);
 }
 
-// the sorted position of best(v, U), U = {u : at[u] < lim, u != out} + {in}; kOrderNone if v has no entry inside U
-__device__ __forceinline__ uint32_t climb_best_pos(const OrderClimbVar &V, const uint8_t *at, int lim, int out, int in, const uint32_t *__restrict__ T) {
-    uint32_t idx = 0;
-    for (uint32_t t = 0; t < V.ncand; t++) {
-        const int u = V.cand[t];
-        if (((int)at[u] < lim && u != out) || u == in) idx |= 1u << t;
+// the sorted position of best(v, U), U = {u : at[u] < lim, u != out} + {in}, pre[lim] = {u : at[u] < lim} (kClimbWords words);
+// kOrderNone if v has no entry inside U
+struct ClimbTable {
+    static constexpr bool kWarp = false;
+    const uint32_t *__restrict__ T;         // every T_v
+    __device__ __forceinline__ uint32_t pos(const OrderClimbVar &V, const uint8_t *at, const unsigned long long *, int lim, int out, int in) const {
+        uint32_t idx = 0;
+        for (uint32_t t = 0; t < V.ncand; t++) {
+            const int u = V.cand[t];
+            if (((int)at[u] < lim && u != out) || u == in) idx |= 1u << t;
+        }
+        return __ldg(T + V.table + idx);
     }
-    return __ldg(T + V.table + idx);
-}
-__device__ __forceinline__ float climb_best(const OrderClimbVar &V, const uint8_t *at, int lim, int out, int in, const uint32_t *__restrict__ T,
-                                            const float *__restrict__ scores) {
-    const uint32_t pos = climb_best_pos(V, at, lim, out, in, T);
+};
+struct ClimbList {
+    static constexpr bool kWarp = true;         // the move look-ups by warp_pos
+    const unsigned long long *__restrict__ E;   // word w of sorted entry e at E[w * stride + e]
+    uint32_t stride;                            // the number of entries
+    int words;                                  // W = ceil(k / 64)
+    // the complement of U's words
+    __device__ __forceinline__ void outside(unsigned long long (&notU)[kClimbWords], const unsigned long long *pre, int lim, int out, int in) const {
+#pragma unroll
+        for (int w = 0; w < kClimbWords; w++)
+            notU[w] = ~((pre[lim * kClimbWords + w] & ~(w == (out >> 6) ? 1ull << (out & 63) : 0ull)) | (w == (in >> 6) ? 1ull << (in & 63) : 0ull));
+    }
+    // does sorted entry e (from the start of the entries) lie inside U?
+    __device__ __forceinline__ bool inside(const unsigned long long (&notU)[kClimbWords], uint32_t e) const {
+        unsigned long long miss = __ldg(E + e) & notU[0];
+#pragma unroll
+        for (int w = 1; w < kClimbWords; w++) if (w < words) miss |= __ldg(E + (size_t)w * stride + e) & notU[w];
+        return miss == 0;
+    }
+    __device__ __forceinline__ uint32_t pos(const OrderClimbVar &V, const uint8_t *, const unsigned long long *pre, int lim, int out, int in) const {
+        unsigned long long notU[kClimbWords];
+        outside(notU, pre, lim, out, in);
+        const uint32_t n = (uint32_t)V.nent;
+        for (uint32_t e = 0; e < n; e++) if (inside(notU, V.score + e)) return e;
+        return kOrderNone;
+    }
+    // the same look-up by the whole warp, 32 consecutive entries a step from `start` (every lane gets the answer)
+    __device__ __forceinline__ uint32_t warp_pos(const OrderClimbVar &V, const unsigned long long *pre, int lim, int out, int in, uint32_t start, int lane) const {
+        unsigned long long notU[kClimbWords];
+        outside(notU, pre, lim, out, in);
+        const uint32_t n = (uint32_t)V.nent;
+        for (uint32_t b = start; b < n; b += 32) {
+            const uint32_t hits = __ballot_sync(0xFFFFFFFFu, b + lane < n && inside(notU, V.score + b + lane));
+            if (hits) return b + __ffs(hits) - 1;
+        }
+        return kOrderNone;
+    }
+};
+template <class Look>
+__device__ __forceinline__ float climb_best(const Look &look, const OrderClimbVar &V, const uint8_t *at, const unsigned long long *pre, int lim, int out,
+                                            int in, const float *__restrict__ scores) {
+    const uint32_t pos = look.pos(V, at, pre, lim, out, in);
     return pos == kOrderNone ? 3.402823466e+38f : __ldg(scores + V.score + pos);
 }
 // does v have a skeleton neighbour in the set P, leaving out position `out`?
@@ -375,7 +426,8 @@ __device__ __forceinline__ uint32_t climb_key(float g) {
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
 }
 
-__global__ void __launch_bounds__(kClimbThreads) order_climb_kernel(const OrderClimbVar *__restrict__ vars, const uint32_t *__restrict__ T,
+template <class Look>
+__global__ void __launch_bounds__(kClimbThreads) order_climb_kernel(const OrderClimbVar *__restrict__ vars, const Look look,
                                                                     const float *__restrict__ scores, int k, uint32_t restarts, unsigned long long seed,
                                                                     float *__restrict__ r_cost, uint32_t *__restrict__ r_moves,
                                                                     uint8_t *__restrict__ r_order, uint32_t *__restrict__ r_pos) {
@@ -446,7 +498,7 @@ __global__ void __launch_bounds__(kClimbThreads) order_climb_kernel(const OrderC
                 }
             }
             __syncthreads();
-            for (int m = threadIdx.x; m < k; m += blockDim.x) s_b[m] = climb_best(s_var[s_ord[m]], s_at, m, -1, -1, T, scores);
+            for (int m = threadIdx.x; m < k; m += blockDim.x) s_b[m] = climb_best(look, s_var[s_ord[m]], s_at, s_pre, m, -1, -1, scores);
             __syncthreads();
             if (threadIdx.x == 0) {
                 float g = 0.0f;
@@ -462,18 +514,37 @@ __global__ void __launch_bounds__(kClimbThreads) order_climb_kernel(const OrderC
             for (int i = warp; i < k; i += kClimbWarps) {
                 const int vi = s_ord[i];
                 const OrderClimbVar &Vi = s_var[vi];
+                if constexpr (Look::kWarp) {
+                    // targets in descending order: U of the Y look-ups only shrinks, so each scan starts at the last hit
+                    uint32_t ystart = 0;
+                    for (int t = k - 1; t >= 0; t--) {
+                        if (t == i) continue;
+                        const OrderClimbVar &Vt = s_var[s_ord[t]];
+                        const uint32_t px = t > i ? look.warp_pos(Vt, s_pre, t, vi, -1, 0, lane) : look.warp_pos(Vt, s_pre, t, -1, vi, 0, lane);
+                        const uint32_t py = t > i ? look.warp_pos(Vi, s_pre, t + 1, vi, -1, ystart, lane) : look.warp_pos(Vi, s_pre, t, -1, -1, ystart, lane);
+                        ystart = py == kOrderNone ? (uint32_t)Vi.nent : py;
+                        if (lane == 0) {
+                            X[t] = px == kOrderNone ? 3.402823466e+38f : __ldg(scores + Vt.score + px);
+                            Y[t] = py == kOrderNone ? 3.402823466e+38f : __ldg(scores + Vi.score + py);
+                        }
+                    }
+                }
                 for (int t = lane; t < k; t += 32) {
                     if (t == i) continue;
                     const OrderClimbVar &Vt = s_var[s_ord[t]];
                     if (t > i) {
-                        X[t] = climb_best(Vt, s_at, t, vi, -1, T, scores);
+                        if constexpr (!Look::kWarp) {
+                            X[t] = climb_best(look, Vt, s_at, s_pre, t, vi, -1, scores);
+                            Y[t] = climb_best(look, Vi, s_at, s_pre, t + 1, vi, -1, scores);
+                        }
                         okX[t] = t == 1 || climb_touches(Vt, s_pre + t * kClimbWords, vi);
-                        Y[t] = climb_best(Vi, s_at, t + 1, vi, -1, T, scores);
                         okY[t] = climb_touches(Vi, s_pre + (t + 1) * kClimbWords, vi);
                     } else {
-                        X[t] = climb_best(Vt, s_at, t, -1, vi, T, scores);
+                        if constexpr (!Look::kWarp) {
+                            X[t] = climb_best(look, Vt, s_at, s_pre, t, -1, vi, scores);
+                            Y[t] = climb_best(look, Vi, s_at, s_pre, t, -1, -1, scores);
+                        }
                         okX[t] = t > 0 || ((Vt.adj[vi >> 6] >> (vi & 63)) & 1);
-                        Y[t] = climb_best(Vi, s_at, t, -1, -1, T, scores);
                         okY[t] = t == 0 || climb_touches(Vi, s_pre + t * kClimbWords, -1);
                     }
                 }
@@ -534,7 +605,7 @@ __global__ void __launch_bounds__(kClimbThreads) order_climb_kernel(const OrderC
         // the local optimum of restart r
         for (int m = threadIdx.x; m < k; m += blockDim.x) {
             r_order[(size_t)r * k + m] = s_ord[m];
-            r_pos[(size_t)r * k + m] = climb_best_pos(s_var[s_ord[m]], s_at, m, -1, -1, T);
+            r_pos[(size_t)r * k + m] = look.pos(s_var[s_ord[m]], s_at, s_pre, m, -1, -1);
         }
         if (threadIdx.x == 0) { r_cost[r] = s_g[k]; r_moves[r] = s_moves; }
         __syncthreads();

@@ -385,7 +385,8 @@ extern "C" int urlgpu_create(urlgpu_ctx **out, int device_id) {
         attrs.push_back({(const void *)cbic_sets_kernel, big});
         attrs.push_back({(const void *)gram_partial_kernel, (int)kGramSmemBytes});
         attrs.push_back({(const void *)order_layer_rank_kernel, (int)order_rank_smem_bytes(kOrderRankMaxVars)});
-        attrs.push_back({(const void *)order_climb_kernel, (int)order_climb_smem_bytes(kClimbMaxVars)});
+        attrs.push_back({(const void *)order_climb_kernel<ClimbTable>, (int)order_climb_smem_bytes(kClimbMaxVars)});
+        attrs.push_back({(const void *)order_climb_kernel<ClimbList>, (int)order_climb_smem_bytes(kClimbMaxVars)});
         for (const auto &a : attrs)
             if ((e = cudaFuncSetAttribute(a.first, cudaFuncAttributeMaxDynamicSharedMemorySize, a.second)) != cudaSuccess)
                 return refuse("cannot opt a kernel into " + std::to_string(a.second) + " bytes of dynamic shared memory (the device allows " +
@@ -2533,11 +2534,12 @@ extern "C" int urlgpu_spg_free(urlgpu_spg *sp) {
 }
 
 // ============================================================================================ order-graph search
-// urlgpu_order_search, urlgpu_order_search_layered and urlgpu_order_local_search (order_kernels.cuh).  order_prepare validates
-// everything on the host, keeps the component's qualifying entries, sorts each variable's list in the (score, |S|, mask) order
-// of SortedEntries::build and lays out the best-parent tables, compacting each entry straight from its variable-space mask onto
-// cand_v's bits.  order_tables uploads the entries and builds the tables.  Each entry point sizes its call before any
-// allocation; the host maps each chosen sorted position back to its parent mask.
+// urlgpu_order_search, urlgpu_order_search_layered, urlgpu_order_local_search and urlgpu_order_local_search_sparse
+// (order_kernels.cuh).  order_prepare validates everything on the host, keeps the component's qualifying entries, sorts each
+// variable's list in the (score, |S|, mask) order of SortedEntries::build and lays out the best-parent tables, compacting each
+// entry straight from its variable-space mask onto cand_v's bits; the sparse form has no tables and gets each entry's parent set
+// over C's positions instead.  order_tables uploads the entries and builds the tables.  Each entry point sizes its call before
+// any allocation; the host maps each chosen sorted position back to its parent mask.
 struct OrderPrep {
     std::vector<int> vars;                       // position j of C -> variable
     std::vector<std::vector<uint64_t>> ent;      // per position: indices into masks/scores, sorted
@@ -2547,12 +2549,15 @@ struct OrderPrep {
     std::vector<unsigned long long> where;       // per sorted entry: its slot in the tables
     std::vector<uint32_t> epos;                  // per sorted entry: its position in its variable's list
     std::vector<float> escore;                   // per sorted entry: its score
+    std::vector<unsigned long long> ewords;      // sparse: word w of sorted entry e's parent set over C at [w * n_ent + e]
+    int words = 0;                               // sparse: ceil(k / 64)
     uint64_t n_ent = 0, table_elems = 0;
 };
 
-// every check and translation the three entry points share; `who` prefixes the messages.  Components of more than max_k
-// variables and variables with more than max_cand candidate parents inside the component are refused
-static int order_prepare(urlgpu_ctx *ctx, const std::string &who, int max_k, int max_cand, int p, int mask_words, const uint64_t *offsets,
+// every check and translation the four entry points share; `who` prefixes the messages.  Components of more than max_k
+// variables and variables with more than max_cand candidate parents inside the component are refused.  sparse: no table
+// layout (2^c_v would overflow past 63 candidates), the entries' words over C instead
+static int order_prepare(urlgpu_ctx *ctx, const std::string &who, int max_k, int max_cand, bool sparse, int p, int mask_words, const uint64_t *offsets,
                          const uint64_t *masks, const float *scores, const uint64_t *component, OrderPrep &P) {
     auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, who + m); };
     if (p < 1) return refuse(URLGPU_ERR_ARG, "p must be at least 1");
@@ -2611,21 +2616,31 @@ static int order_prepare(urlgpu_ctx *ctx, const std::string &who, int max_k, int
                                                 " candidate parents inside the component; at most " + std::to_string(max_cand) + " are supported");
         P.table[j] = P.table_elems;
         P.score[j] = (uint32_t)P.n_ent;
-        P.table_elems += (uint64_t)1 << P.cand[j].size();
+        if (!sparse) P.table_elems += (uint64_t)1 << P.cand[j].size();
         P.n_ent += E.size();
     }
     if (P.n_ent > 0xFFFFFFFFull) return refuse(URLGPU_ERR_LIMIT, "2^32 or more entries inside the component");
-    P.where.resize(P.n_ent);
-    P.epos.resize(P.n_ent);
     P.escore.resize(P.n_ent);
+    if (sparse) {
+        P.words = (k + 63) / 64;
+        P.ewords.assign((size_t)P.words * P.n_ent, 0);
+    } else {
+        P.where.resize(P.n_ent);
+        P.epos.resize(P.n_ent);
+    }
     for (int j = 0; j < k; j++)
         for (size_t i = 0; i < P.ent[j].size(); i++) {
             const uint64_t *m = masks + P.ent[j][i] * mask_words;
+            const uint64_t e = P.score[j] + i;
+            P.escore[e] = scores[P.ent[j][i]];
+            if (sparse) {                                      // the entry over C's positions
+                for (int q : P.cand[j]) if (bit(m, P.vars[q])) P.ewords[(size_t)(q >> 6) * P.n_ent + e] |= 1ull << (q & 63);
+                continue;
+            }
             uint64_t idx = 0;                                  // the entry over cand_j's bits
             for (size_t q = 0; q < P.cand[j].size(); q++) if (bit(m, P.vars[P.cand[j][q]])) idx |= 1ull << q;
-            P.where[P.score[j] + i] = P.table[j] + idx;
-            P.epos[P.score[j] + i] = (uint32_t)i;
-            P.escore[P.score[j] + i] = scores[P.ent[j][i]];
+            P.where[e] = P.table[j] + idx;
+            P.epos[e] = (uint32_t)i;
         }
     return URLGPU_OK;
 }
@@ -2676,7 +2691,7 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
     if (!offsets || !component || !cost || !order || !parents) return refuse(URLGPU_ERR_ARG, "null argument");
     OrderPrep P;
     const int max_k = layered ? kOrderRankMaxVars : kOrderMaxVars;        // c_v < k, so max_k - 1 never refuses a variable
-    if (int rc = order_prepare(ctx, who, max_k, max_k - 1, p, mask_words, offsets, masks, scores, component, P)) return rc;
+    if (int rc = order_prepare(ctx, who, max_k, max_k - 1, false, p, mask_words, offsets, masks, scores, component, P)) return rc;
     const int k = (int)P.vars.size();
     const uint64_t n_ent = P.n_ent, table_elems = P.table_elems;
     std::vector<OrderVarRank> hv(k);
@@ -2827,40 +2842,49 @@ extern "C" int urlgpu_order_search_layered(urlgpu_ctx *ctx, int p, int mask_word
     return order_search_impl(ctx, true, p, mask_words, offsets, masks, scores, edges, component, cost, order, parents);
 }
 
-// Local search: the tables as above, then one order_climb_kernel launch over all restarts.  The host reads every restart's cost
-// and move count, takes the least cost (ties: the smallest restart), and copies back that restart's order and family positions.
-extern "C" int urlgpu_order_local_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
-                                         const float *scores, const uint64_t *edges, const uint64_t *component, uint32_t restarts,
-                                         uint64_t seed, float *cost, int32_t *order, uint64_t *parents, float *restart_costs,
-                                         uint32_t *restart_moves) {
+// Local search: the tables as above (sparse: the entries' words over C, no tables), then one order_climb_kernel launch over all
+// restarts.  The host reads every restart's cost and move count, takes the least cost (ties: the smallest restart), and copies
+// back that restart's order and family positions.
+static int order_local_search_impl(urlgpu_ctx *ctx, bool sparse, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                                   const float *scores, const uint64_t *edges, const uint64_t *component, uint32_t restarts,
+                                   uint64_t seed, float *cost, int32_t *order, uint64_t *parents, float *restart_costs,
+                                   uint32_t *restart_moves) {
     if (!ctx) return URLGPU_ERR_ARG;
-    const std::string who = "order_local_search: ";
+    const std::string who = sparse ? "order_local_search_sparse: " : "order_local_search: ";
     auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, who + m); };
     if (!offsets || !component || !cost || !order || !parents) return refuse(URLGPU_ERR_ARG, "null argument");
     if (restarts < 1 || restarts > (1u << 20)) return refuse(URLGPU_ERR_ARG, "restarts must be in 1..2^20");
     OrderPrep P;
-    if (int rc = order_prepare(ctx, who, kClimbMaxVars, kClimbMaxCand, p, mask_words, offsets, masks, scores, component, P)) return rc;
+    if (int rc = order_prepare(ctx, who, kClimbMaxVars, sparse ? kClimbMaxVars - 1 : kClimbMaxCand, sparse, p, mask_words, offsets, masks, scores,
+                               component, P))
+        return rc;
     const int k = (int)P.vars.size();
     std::vector<OrderClimbVar> hv(k);
     for (int j = 0; j < k; j++) {
         OrderClimbVar &V = hv[j];
         memset(&V, 0, sizeof V);
-        V.table = P.table[j];
         V.score = P.score[j];
         V.ncand = (uint32_t)P.cand[j].size();
-        for (size_t q = 0; q < P.cand[j].size(); q++) V.cand[q] = (uint8_t)P.cand[j][q];
+        if (sparse) {
+            V.nent = P.ent[j].size();
+        } else {
+            V.table = P.table[j];
+            for (size_t q = 0; q < P.cand[j].size(); q++) V.cand[q] = (uint8_t)P.cand[j][q];
+        }
         for (int i = 0; i < k; i++)
             if (!edges || ((edges[(size_t)P.vars[j] * mask_words + (P.vars[i] >> 6)] >> (P.vars[i] & 63)) & 1)) V.adj[i >> 6] |= 1ull << (i & 63);
     }
 
-    // the device memory of the call: tables, entries, and per restart a cost, a move count, the order and the family positions
-    const uint64_t table_bytes = 4 * P.table_elems, ent_bytes = 16 * P.n_ent, restart_bytes = (uint64_t)restarts * (8 + 5 * (uint64_t)k);
+    // the device memory of the call: tables, entries (table form: where | position | score, sparse: W words | score), and per
+    // restart a cost, a move count, the order and the family positions
+    const uint64_t table_bytes = 4 * P.table_elems, ent_bytes = (sparse ? 8 * (uint64_t)P.words + 4 : 16) * P.n_ent;
+    const uint64_t restart_bytes = (uint64_t)restarts * (8 + 5 * (uint64_t)k);
     const size_t var_bytes = (size_t)k * sizeof(OrderClimbVar);
     const size_t need = table_bytes + ent_bytes + restart_bytes + var_bytes;
     size_t free_b = 0;
     if (int rc = order_free_bytes(ctx, &free_b)) return rc;
     auto bytes_msg = [&]() {
-        return std::to_string(need) + " bytes of device memory (" + std::to_string(table_bytes) + " for the best-parent tables, " +
+        return std::to_string(need) + " bytes of device memory (" + (sparse ? "" : std::to_string(table_bytes) + " for the best-parent tables, ") +
                std::to_string(ent_bytes) + " for the entries, " + std::to_string(restart_bytes) + " for the state of " +
                std::to_string(restarts) + " restarts)";
     };
@@ -2873,7 +2897,8 @@ extern "C" int urlgpu_order_local_search(urlgpu_ctx *ctx, int p, int mask_words,
         if (e != cudaSuccess) { cudaGetLastError(); return false; }
         return true;
     };
-    if (!alloc(d_tab, table_bytes) || !alloc(d_ent, std::max<uint64_t>(16, ent_bytes)) || !alloc(d_var, var_bytes) || !alloc(d_res, restart_bytes))
+    if ((!sparse && !alloc(d_tab, table_bytes)) || !alloc(d_ent, std::max<uint64_t>(16, ent_bytes)) || !alloc(d_var, var_bytes) ||
+        !alloc(d_res, restart_bytes))
         return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes_msg() + " failed");
     // d_res: cost | moves | positions | order
     float *r_cost = d_res.as<float>();
@@ -2881,17 +2906,35 @@ extern "C" int urlgpu_order_local_search(urlgpu_ctx *ctx, int p, int mask_words,
     uint32_t *r_pos = r_moves + restarts;
     uint8_t *r_order = reinterpret_cast<uint8_t *>(r_pos + (size_t)restarts * k);
     CK(cudaMemcpyAsync(d_var.p, hv.data(), var_bytes, cudaMemcpyHostToDevice, s));
-    uint32_t *T = d_tab.as<uint32_t>();
-    if (int rc = order_tables(ctx, P, d_ent.p, T)) return rc;
-    const float *ds = reinterpret_cast<const float *>(reinterpret_cast<const uint32_t *>(d_ent.as<unsigned long long>() + P.n_ent) + P.n_ent);
+    const float *ds;
+    ClimbTable table{};
+    ClimbList list{};
+    if (sparse) {                                              // d_ent: words | score
+        list.E = d_ent.as<unsigned long long>();
+        list.stride = (uint32_t)P.n_ent;
+        list.words = P.words;
+        ds = reinterpret_cast<const float *>(list.E + P.ewords.size());
+        if (P.n_ent) {
+            CK(cudaMemcpyAsync(d_ent.p, P.ewords.data(), P.ewords.size() * 8, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(const_cast<float *>(ds), P.escore.data(), P.n_ent * 4, cudaMemcpyHostToDevice, s));
+        }
+    } else {
+        table.T = d_tab.as<uint32_t>();
+        if (int rc = order_tables(ctx, P, d_ent.p, d_tab.as<uint32_t>())) return rc;
+        ds = reinterpret_cast<const float *>(reinterpret_cast<const uint32_t *>(d_ent.as<unsigned long long>() + P.n_ent) + P.n_ent);
+    }
     {
         Region rg(ctx, F_ORDER_LAYERS, 1);
         const size_t smem = order_climb_smem_bytes(k);
-        int per_sm = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_climb_kernel, kClimbThreads, smem));
-        const uint64_t grid = std::min<uint64_t>(restarts, (uint64_t)std::max(1, per_sm) * ctx->sm_count);
-        order_climb_kernel<<<(unsigned)grid, kClimbThreads, smem, s>>>(d_var.as<OrderClimbVar>(), T, ds, k, restarts, seed, r_cost, r_moves, r_order, r_pos);
-        CK(cudaGetLastError());
+        auto launch = [&](auto kernel, const auto &look) -> int {
+            int per_sm = 0;
+            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kClimbThreads, smem));
+            const uint64_t grid = std::min<uint64_t>(restarts, (uint64_t)std::max(1, per_sm) * ctx->sm_count);
+            kernel<<<(unsigned)grid, kClimbThreads, smem, s>>>(d_var.as<OrderClimbVar>(), look, ds, k, restarts, seed, r_cost, r_moves, r_order, r_pos);
+            CK(cudaGetLastError());
+            return URLGPU_OK;
+        };
+        if (int rc = sparse ? launch(order_climb_kernel<ClimbList>, list) : launch(order_climb_kernel<ClimbTable>, table)) return rc;
     }
     std::vector<float> rc_h(restarts);
     std::vector<uint32_t> rm_h(restarts);
@@ -2915,6 +2958,22 @@ extern "C" int urlgpu_order_local_search(urlgpu_ctx *ctx, int p, int mask_words,
     if (restart_costs) memcpy(restart_costs, rc_h.data(), (size_t)restarts * 4);
     if (restart_moves) memcpy(restart_moves, rm_h.data(), (size_t)restarts * 4);
     return URLGPU_OK;
+}
+
+extern "C" int urlgpu_order_local_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                                         const float *scores, const uint64_t *edges, const uint64_t *component, uint32_t restarts,
+                                         uint64_t seed, float *cost, int32_t *order, uint64_t *parents, float *restart_costs,
+                                         uint32_t *restart_moves) {
+    return order_local_search_impl(ctx, false, p, mask_words, offsets, masks, scores, edges, component, restarts, seed, cost, order, parents,
+                                   restart_costs, restart_moves);
+}
+
+extern "C" int urlgpu_order_local_search_sparse(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
+                                                const float *scores, const uint64_t *edges, const uint64_t *component, uint32_t restarts,
+                                                uint64_t seed, float *cost, int32_t *order, uint64_t *parents, float *restart_costs,
+                                                uint32_t *restart_moves) {
+    return order_local_search_impl(ctx, true, p, mask_words, offsets, masks, scores, edges, component, restarts, seed, cost, order, parents,
+                                   restart_costs, restart_moves);
 }
 
 // ============================================================================================ listed sets
