@@ -76,7 +76,11 @@ int urlgpu_set_stream(urlgpu_ctx *ctx, void *cuda_stream);
 int urlgpu_synchronize(urlgpu_ctx *ctx);
 
 /* Data is COPIED to the device; the caller keeps ownership.  Column-major: value of variable i in record r at
- * [i*n + r].  codes are value indices < cardinality[i] (first-appearance order, base/variable.h:43-48). */
+ * [i*n + r].  codes are value indices < cardinality[i] (first-appearance order, base/variable.h:43-48).
+ * Record limits (URLGPU_ERR_LIMIT above them): a discrete data set holds at most 2e9 records (refused here); BDeu scores
+ * at most 1e8 and fNML with a child of arity >= 2 at most 238 609 293 (refused by the scoring calls: the reference's
+ * regret approximation computes 9 * N in int, and its table covers N = n + 1); BIC and fNML of a constant child take
+ * all 2e9.  Continuous data has no record limit. */
 int urlgpu_set_discrete(urlgpu_ctx *ctx, const uint8_t *codes_colmajor, int64_t n, int p, const int32_t *cardinality);
 /* same, but codes_colmajor is a DEVICE pointer on ctx's device (multi-GPU: data arrives by NCCL broadcast) */
 int urlgpu_set_discrete_device(urlgpu_ctx *ctx, const uint8_t *d_codes_colmajor, int64_t n, int p, const int32_t *cardinality);

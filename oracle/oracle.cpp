@@ -27,6 +27,19 @@
 
 static thread_local std::string g_err;
 static int fail(const std::string &m) { g_err = m; return -1; }
+
+/* fx * 2^e rounded once to float32 (the device's bic_finalize): fx to double rounded to odd (truncated, the lowest bit set when
+ * that dropped anything), then rounded to nearest float32 -- a correct single rounding also for |fx| >= 2^53, where
+ * (float)(double)fx rounds twice */
+static float fixed_to_float(int64_t fx, int e) {
+    const uint64_t mag = fx < 0 ? -(uint64_t)fx : (uint64_t)fx;
+    int drop = 0;
+    while ((mag >> drop) >= ((uint64_t)1 << 53)) drop++;
+    uint64_t kept = mag >> drop;
+    if (drop && (mag & (((uint64_t)1 << drop) - 1))) kept |= 1;           /* sticky bit: round to odd */
+    const double d = std::ldexp((double)kept, drop + e);                   /* exact: kept < 2^53 */
+    return (float)(fx < 0 ? -d : d);
+}
 extern "C" const char *orc_last_error(void) { return g_err.c_str(); }
 
 /* ------------------------------------------------------------------ helpers */
@@ -452,7 +465,7 @@ static int fnml_score_one(const BicCtx &c, const std::vector<float> &reg, int v,
                 fx -= std::llrint(std::ldexp((double)reg[nij], 23));
             }
         }
-        *score_out = (float)std::ldexp((double)fx, -23);
+        *score_out = fixed_to_float(fx, -23);
         return 0;
     }
     float ll;
@@ -550,7 +563,7 @@ static int bdeu_score_one(const BicCtx &c, float ess, int v, uint64_t parents, i
             }
             if (nij > 0) fx += std::llrint(((double)lg_ij - lgamma_r(a_ij + nij, &sg)) * 1073741824.0);
         }
-        *score_out = (float)((double)fx * (1.0 / 1073741824.0));
+        *score_out = fixed_to_float(fx, -30);
         return 0;
     }
     std::vector<int> vars;

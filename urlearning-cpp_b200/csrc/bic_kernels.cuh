@@ -190,8 +190,12 @@ __device__ __forceinline__ long long score_configs(HistPtr hist, int rv, int64_t
 }
 
 __device__ __forceinline__ float bic_finalize(long long acc, float tval, float base, double acc_scale = 1.0 / 8388608.0) {
-    // acc * 2^-23 is exact in FP64 (|acc| < 2^53); one rounding to float32, then the float32 penalty
-    const float ll = __double2float_rn(__ll2double_rn(acc) * acc_scale);
+    // one rounding of acc * acc_scale to float32, then the float32 penalty.  acc reaches FP64 rounded to odd (truncated, the
+    // lowest bit set when that dropped anything): a second rounding to 24 bits of a 53-bit round-to-odd value is the one
+    // correct rounding, also at |acc| >= 2^53 (BIC from 2^30 nats, BDeu near 1e8 records), where round-to-nearest twice is not
+    double d = __ll2double_rz(acc);
+    if (__double2ll_rz(d) != acc) d = __longlong_as_double(__double_as_longlong(d) | 1);
+    const float ll = __double2float_rn(d * acc_scale);
     return __fsub_rn(ll, __fmul_rn(tval, base)); // bic_scoring_function.cpp:73, no FMA contraction
 }
 

@@ -119,11 +119,15 @@ __global__ void tree_scatter_kernel(BicData d, CandInfo ci_cube, TreeVar tv, con
     out[atomicAdd(&cursor[keys[r]], 1u)] = w; // order inside a bucket is arbitrary: counts do not depend on it
 }
 
-// exact warp sum of int64 values with |v| < 2^50 in two 32-bit REDUX operations (24 low bits + arithmetic high part)
+// exact warp sum of any int64 values whose sum fits int64, in three 32-bit REDUX operations: bits 0-23 and 24-47 as
+// unsigned parts (32 of them sum below 2^29) and the arithmetic high part v >> 48 (|v >> 48| <= 2^15, 32 of them below 2^20).
+// Two parts (24 low bits + v >> 24 in an int) would wrap once a lane or the warp reached 2^55, i.e. 2^32 nats of a BIC
+// accumulator: one configuration of a 256-ary child holding 7.75e8 records of a slice is enough.
 __device__ __forceinline__ long long warp_sum_ll_redux(long long v) {
     const unsigned lo = __reduce_add_sync(0xffffffffu, (unsigned)(v & 0xFFFFFF));
-    const int hi = __reduce_add_sync(0xffffffffu, (int)(v >> 24));
-    return ((long long)hi << 24) + (long long)lo;
+    const unsigned mid = __reduce_add_sync(0xffffffffu, (unsigned)((v >> 24) & 0xFFFFFF));
+    const int hi = __reduce_add_sync(0xffffffffu, (int)(v >> 48));
+    return (long long)(((unsigned long long)(long long)hi << 48) + ((unsigned long long)mid << 24) + lo);   // modulo 2^64
 }
 
 // ---- count the slice's rows.  The rows are `nseg` contiguous segments of the bucketed rows; they are walked as ONE

@@ -540,6 +540,8 @@ extern "C" int urlgpu_share_discrete(urlgpu_ctx *ctx, urlgpu_ctx *owner) {
     return URLGPU_OK;
 }
 
+constexpr int64_t kFnmlMaxRecords = 238609293;   // 9 * (n + 1) <= INT_MAX: the largest fNML data set of a child of arity >= 2
+
 // Chooses what the K1 kernels compute for `variable`: BIC (log_likelihood - tVal * ln(N)/2, bic_scoring_function.cpp:73) or
 // fNML (log_likelihood - sum_j log C(N_ij, r_v), fnml_scoring_function.cpp:28-74).  The fNML per-configuration table is
 // qlog[N] + round(2^23 * (float)log C(N, r_v)): the exact-integer contract of bic_kernels.cuh extended by one more float
@@ -559,6 +561,12 @@ static int select_discrete_score(urlgpu_ctx *ctx, int score_type, int variable, 
         return URLGPU_OK;
     }
     const int r = ctx->card[variable];
+    // the table covers N = 0..n+1, and for r >= 2 every entry goes through regret::r2, whose Szpankowski branch evaluates
+    // 9 * N in int exactly as the reference writes it: that wraps from N = 238 609 295 on (NaN, then wrong values)
+    if (r >= 2 && ctx->n > kFnmlMaxRecords)
+        return ctx->fail(URLGPU_ERR_LIMIT, "fNML: more than " + std::to_string(kFnmlMaxRecords) + " records with a child of arity " + std::to_string(r) +
+                                               ": the regret C(N, 2) of the reference computes 9 * N in int, which overflows at N = " +
+                                               std::to_string(kFnmlMaxRecords + 2));
     auto it = ctx->d_qfnml.find(r);
     if (it == ctx->d_qfnml.end()) {
         const int64_t n = ctx->n;
@@ -671,7 +679,9 @@ static int shard_finish_impl(urlgpu_ctx *ctx, const double *mean_host, const dou
         const int tiles = (p + kGramTile - 1) / kGramTile;
         const int pairs = tiles * (tiles + 1) / 2;
         // row slices (multiples of the chunk): enough CTAs to fill the machine several times over, at least 1024 records each
+        // (beyond 65 535 * 8192 records the slices grow instead: gridDim.y holds at most 65 535)
         int64_t rps = std::max<int64_t>(1024, std::min<int64_t>(8192, z_stride * pairs / ((int64_t)ctx->sm_count * 8)));
+        rps = std::max<int64_t>(rps, (z_stride + 65534) / 65535);
         rps = (rps + kGramKC - 1) / kGramKC * kGramKC;
         const int slices = (int)((z_stride + rps - 1) / rps);
         CK(gpart.alloc((size_t)slices * p * p * sizeof(double)));
