@@ -338,16 +338,26 @@ __global__ void bic_store_rule_kernel(float *__restrict__ scores, uint64_t n_mas
 // ---------------------------------------------------------------------------------------------------------
 struct CubePair {
     uint64_t parent_off, child_off;   // int32 elements
-    uint32_t child_configs;           // child cells / rv
+    uint32_t groups;                  // child configurations / r0
     uint32_t Bc;                      // stride of the dropped digit, in configurations
     uint32_t r;                       // arity of the dropped digit
     uint32_t chunk0;                  // first block of this pair
     uint32_t acc_index;               // accumulator of the child
-    uint32_t leaf;                    // the child has no children of its own (cube bit 0 clear): its table is not written
+    uint32_t leaf_acc;                // accumulator of the child's leaf (the child without cube bit 0), scored from the same counts
+    uint32_t r0;                      // configurations per group: the arity of cube bit 0 when the child holds it, else 1
+    uint32_t flags;                   // kCubeStore | kCubeScoreChild | kCubeScoreLeaf
     uint32_t fmt;                     // bit 0: the parent table holds uint16 cells, bit 1: the child table does (see "16-bit tables")
-    uint32_t magic;                   // floor((2^32 - 1) / Bc): fast_div instead of a hardware division per configuration
-    uint32_t pad;
+    uint32_t magic;                   // floor((2^32 - 1) / Bc): fast_div instead of a hardware division per group
 };
+constexpr uint32_t kCubeStore = 1;      // the child has children of its own (it holds cube bit 0): its table is written
+constexpr uint32_t kCubeScoreChild = 2; // the child is a set of the family (layer <= K)
+constexpr uint32_t kCubeScoreLeaf = 4;  // the child's leaf is scored here; it gets no pair of its own
+
+// A LEAF is a set without cube bit 0: nothing is derived from it, and its parent is the set plus bit 0.  Digit 0 is the lowest
+// digit of a configuration index, so the r0 = card[bit 0] consecutive configurations g*r0 + a of a set T that holds bit 0 sum
+// to configuration g of its leaf T \ {0}.  A thread that derives T in whole groups of r0 configurations therefore has the
+// leaf's counts in registers: the leaf is scored there, without reading T again and without blocks of its own.  The dropped
+// digit z >= 1 of such a T has a stride Bc that is a multiple of r0, so a group is contiguous in the parent as well.
 
 constexpr int kCubeThreads = 256;
 #ifndef URLGPU_CUBE_UNROLL
@@ -356,22 +366,32 @@ constexpr int kCubeThreads = 256;
 constexpr int kCubeUnroll = URLGPU_CUBE_UNROLL;
 constexpr uint32_t kCubeConfigsPerBlock = 4096;
 
-template <int RV>
-__device__ __forceinline__ void load_cfg(const int *__restrict__ p, int (&v)[RV]) {
-    if constexpr (RV == 4) { const int4 t = *reinterpret_cast<const int4 *>(p); v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w; }
-    else if constexpr (RV == 2) { const int2 t = *reinterpret_cast<const int2 *>(p); v[0] = t.x; v[1] = t.y; }
-    else {
+// N consecutive cells.  p is aligned to N cells as far as the table allows (tables start 16-byte aligned and a run of N cells
+// starts at a multiple of N): the widest vector access that divides N.
+template <int N>
+__device__ __forceinline__ void load_cfg(const int *__restrict__ p, int (&v)[N]) {
+    if constexpr (N % 4 == 0) {
 #pragma unroll
-        for (int k = 0; k < RV; k++) v[k] = p[k];
+        for (int i = 0; i < N / 4; i++) { const int4 t = reinterpret_cast<const int4 *>(p)[i]; v[4 * i] = t.x; v[4 * i + 1] = t.y; v[4 * i + 2] = t.z; v[4 * i + 3] = t.w; }
+    } else if constexpr (N % 2 == 0) {
+#pragma unroll
+        for (int i = 0; i < N / 2; i++) { const int2 t = reinterpret_cast<const int2 *>(p)[i]; v[2 * i] = t.x; v[2 * i + 1] = t.y; }
+    } else {
+#pragma unroll
+        for (int k = 0; k < N; k++) v[k] = p[k];
     }
 }
-template <int RV>
-__device__ __forceinline__ void store_cfg(int *__restrict__ p, const int (&v)[RV]) {
-    if constexpr (RV == 4) *reinterpret_cast<int4 *>(p) = make_int4(v[0], v[1], v[2], v[3]);
-    else if constexpr (RV == 2) *reinterpret_cast<int2 *>(p) = make_int2(v[0], v[1]);
-    else {
+template <int N>
+__device__ __forceinline__ void store_cfg(int *__restrict__ p, const int (&v)[N]) {
+    if constexpr (N % 4 == 0) {
 #pragma unroll
-        for (int k = 0; k < RV; k++) p[k] = v[k];
+        for (int i = 0; i < N / 4; i++) reinterpret_cast<int4 *>(p)[i] = make_int4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
+    } else if constexpr (N % 2 == 0) {
+#pragma unroll
+        for (int i = 0; i < N / 2; i++) reinterpret_cast<int2 *>(p)[i] = make_int2(v[2 * i], v[2 * i + 1]);
+    } else {
+#pragma unroll
+        for (int k = 0; k < N; k++) p[k] = v[k];
     }
 }
 
@@ -380,30 +400,74 @@ __device__ __forceinline__ void store_cfg(int *__restrict__ p, const int (&v)[RV
 // uint16 cells: half the bytes through HBM for the kernel that is bound by them.  This is SPECULATIVE: a store that
 // would not fit saturates and raises a per-call flag; the caller then discards the variable's scores and recomputes them
 // with 32-bit tables (urlgpu.cu: table16 fallback), so results stay exact for any data.
-template <int RV>
-__device__ __forceinline__ void load_cfg16(const uint16_t *__restrict__ p, int (&v)[RV]) {
-    if constexpr (RV == 4) { const uint2 t = *reinterpret_cast<const uint2 *>(p); v[0] = t.x & 0xffff; v[1] = t.x >> 16; v[2] = t.y & 0xffff; v[3] = t.y >> 16; }
-    else if constexpr (RV == 2) { const uint32_t t = *reinterpret_cast<const uint32_t *>(p); v[0] = t & 0xffff; v[1] = t >> 16; }
-    else {
+__device__ __forceinline__ uint32_t pack16(int a, int b) { return (uint32_t)min(a, 65535) | ((uint32_t)min(b, 65535) << 16); }
+template <int N>
+__device__ __forceinline__ void load_cfg16(const uint16_t *__restrict__ p, int (&v)[N]) {
+    if constexpr (N % 8 == 0) {
 #pragma unroll
-        for (int k = 0; k < RV; k++) v[k] = p[k];
+        for (int i = 0; i < N / 8; i++) {
+            const uint4 t = reinterpret_cast<const uint4 *>(p)[i];
+            const uint32_t w[4] = {t.x, t.y, t.z, t.w};
+#pragma unroll
+            for (int q = 0; q < 4; q++) { v[8 * i + 2 * q] = w[q] & 0xffff; v[8 * i + 2 * q + 1] = w[q] >> 16; }
+        }
+    } else if constexpr (N % 4 == 0) {
+#pragma unroll
+        for (int i = 0; i < N / 4; i++) { const uint2 t = reinterpret_cast<const uint2 *>(p)[i]; v[4 * i] = t.x & 0xffff; v[4 * i + 1] = t.x >> 16; v[4 * i + 2] = t.y & 0xffff; v[4 * i + 3] = t.y >> 16; }
+    } else if constexpr (N % 2 == 0) {
+#pragma unroll
+        for (int i = 0; i < N / 2; i++) { const uint32_t t = reinterpret_cast<const uint32_t *>(p)[i]; v[2 * i] = t & 0xffff; v[2 * i + 1] = t >> 16; }
+    } else {
+#pragma unroll
+        for (int k = 0; k < N; k++) v[k] = p[k];
     }
 }
-template <int RV>
-__device__ __forceinline__ bool store_cfg16(uint16_t *__restrict__ p, const int (&v)[RV]) { // true: a count did not fit
+template <int N>
+__device__ __forceinline__ bool store_cfg16(uint16_t *__restrict__ p, const int (&v)[N]) { // true: a count did not fit
     int mx = v[0];
 #pragma unroll
-    for (int k = 1; k < RV; k++) mx = max(mx, v[k]);
-    if constexpr (RV == 4) *reinterpret_cast<uint2 *>(p) = make_uint2((uint32_t)min(v[0], 65535) | ((uint32_t)min(v[1], 65535) << 16), (uint32_t)min(v[2], 65535) | ((uint32_t)min(v[3], 65535) << 16));
-    else if constexpr (RV == 2) *reinterpret_cast<uint32_t *>(p) = (uint32_t)min(v[0], 65535) | ((uint32_t)min(v[1], 65535) << 16);
-    else {
+    for (int k = 1; k < N; k++) mx = max(mx, v[k]);
+    if constexpr (N % 8 == 0) {
 #pragma unroll
-        for (int k = 0; k < RV; k++) p[k] = (uint16_t)min(v[k], 65535);
+        for (int i = 0; i < N / 8; i++)
+            reinterpret_cast<uint4 *>(p)[i] = make_uint4(pack16(v[8 * i], v[8 * i + 1]), pack16(v[8 * i + 2], v[8 * i + 3]), pack16(v[8 * i + 4], v[8 * i + 5]), pack16(v[8 * i + 6], v[8 * i + 7]));
+    } else if constexpr (N % 4 == 0) {
+#pragma unroll
+        for (int i = 0; i < N / 4; i++) reinterpret_cast<uint2 *>(p)[i] = make_uint2(pack16(v[4 * i], v[4 * i + 1]), pack16(v[4 * i + 2], v[4 * i + 3]));
+    } else if constexpr (N % 2 == 0) {
+#pragma unroll
+        for (int i = 0; i < N / 2; i++) reinterpret_cast<uint32_t *>(p)[i] = pack16(v[2 * i], v[2 * i + 1]);
+    } else {
+#pragma unroll
+        for (int k = 0; k < N; k++) p[k] = (uint16_t)min(v[k], 65535);
     }
     return mx > 65535;
 }
 
-// RV > 0: compile-time child arity (2,3,4); RV == 0: generic arity rv_dyn
+// sum_k q[cnt_k] - q[n_j] of the RV counts cnt[off .. off + RV) of one configuration (q[0] = q[1] = 0)
+template <int RV, int N>
+__device__ __forceinline__ void score_cfg(long long &acc, const int (&cnt)[N], int off, const long long *__restrict__ qlog, const long long *__restrict__ qcfg, int cfg_min) {
+    int nij = 0;
+#pragma unroll
+    for (int k = 0; k < RV; k++) nij += cnt[off + k];
+    if (nij > cfg_min) {
+#pragma unroll
+        for (int k = 0; k < RV; k++)
+            if (cnt[off + k] > 1) acc += __ldg(&qlog[cnt[off + k]]);
+        acc -= __ldg(&qcfg[nij]);
+    }
+}
+// the leaf's counts of a group: its G configurations summed cell by cell
+template <int RV, int G>
+__device__ __forceinline__ void sum_group(const int (&cnt)[G * RV], int (&leaf)[RV]) {
+#pragma unroll
+    for (int k = 0; k < RV; k++) {
+        leaf[k] = cnt[k];
+#pragma unroll
+        for (int m = 1; m < G; m++) leaf[k] += cnt[m * RV + k];
+    }
+}
+
 // block -> pair map (one load per block instead of a dependent binary search by thread 0 while 255 threads wait)
 __global__ void cube_map_kernel(const CubePair *__restrict__ pairs, int npairs, uint32_t total, uint32_t *__restrict__ block_pair) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -416,113 +480,167 @@ __global__ void cube_map_kernel(const CubePair *__restrict__ pairs, int npairs, 
     block_pair[i] = (uint32_t)lo;
 }
 
+// RV > 0: compile-time child arity (2,3,4); RV == 0: generic arity rv_dyn.  A block derives kCubeConfigsPerBlock / r0 groups.
 template <int RV>
 __global__ void __launch_bounds__(kCubeThreads, RV == 4 ? 5 : 6) cube_derive_kernel(const CubePair *__restrict__ pairs, const uint32_t *__restrict__ block_pair, const int *__restrict__ parent_tab,
                                                                    int *__restrict__ child_tab, int rv_dyn, const long long *__restrict__ qlog,
-                                                                   const long long *__restrict__ qcfg, int cfg_min,
-                                                                   long long *__restrict__ acc_all, int score_child /*0: the children of this launch are ancestors only*/,
+                                                                   const long long *__restrict__ qcfg, int cfg_min, long long *__restrict__ acc_all,
                                                                    int *__restrict__ ovf_flag /*16-bit tables: a count did not fit*/,
                                                                    int qn /*entries of qlog*/) {
-    __shared__ long long red[32];
+    __shared__ long long red[2][32];
+    __shared__ uint32_t s_acc[2];   // the accumulators, parked until thread 0 needs them (registers are tight for RV = 4)
     (void)qn;
     const CubePair pr = pairs[__ldg(&block_pair[blockIdx.x])];
+    if (threadIdx.x == 0) { s_acc[0] = pr.acc_index; s_acc[1] = pr.leaf_acc; }
     const int rv = RV > 0 ? RV : rv_dyn;
-    long long *__restrict__ acc_out = score_child ? acc_all : nullptr;
-    const uint32_t j0 = (blockIdx.x - pr.chunk0) * kCubeConfigsPerBlock;
-    const uint32_t j1 = min(j0 + kCubeConfigsPerBlock, pr.child_configs);
+    const uint32_t r0 = pr.r0, gpb = kCubeConfigsPerBlock / r0;
+    const uint32_t g0 = (blockIdx.x - pr.chunk0) * gpb;
+    const uint32_t g1 = min(g0 + gpb, pr.groups);
+    const bool store = pr.flags & kCubeStore, score_child = pr.flags & kCubeScoreChild, score_leaf = pr.flags & kCubeScoreLeaf;
     const int *__restrict__ P = parent_tab + pr.parent_off;
     int *__restrict__ Cc = child_tab + pr.child_off;
-    long long acc = 0;
+    long long acc = 0, lacc = 0;   // child, leaf
     if constexpr (RV > 0) {
-        auto score_cfg = [&](const int (&cnt)[RV]) {
-            int nij = 0;
-#pragma unroll
-            for (int k = 0; k < RV; k++) nij += cnt[k];
-            if (nij > cfg_min) { // q[0] = q[1] = 0
-#pragma unroll
-                for (int k = 0; k < RV; k++)
-                    if (cnt[k] > 1) acc += __ldg(&qlog[cnt[k]]);
-                acc -= __ldg(&qcfg[nij]);
-            }
-        };
-        // kCubeUnroll configurations per thread and iteration: r * kCubeUnroll independent 128-bit loads in flight.
+        // configuration indices fit 32 bits (a table has at most 2^30 cells): one IMAD + one IMAD.WIDE per address.  Arity 4 keeps
+        // 64-bit indices: ptxas allocates 44 registers for that form and 58 (or spills) for the 32-bit one
+        using idx_t = std::conditional_t<RV == 4, uint64_t, uint32_t>;
+        // G (compile time) configurations per group, U groups per thread and iteration: r * G * U configurations' loads in flight.
         // P16 / C16 (compile time per instantiation, uniform per block): parent / child table in uint16 cells
-        auto run = [&](auto P16c, auto C16c) {
+        auto run = [&](auto GC, auto P16c, auto C16c) {
+            constexpr int G = decltype(GC)::value, N = G * RV, U = G == 1 ? kCubeUnroll : 1;
             constexpr bool P16 = decltype(P16c)::value, C16 = decltype(C16c)::value;
             const uint16_t *__restrict__ Ph = reinterpret_cast<const uint16_t *>(P);
             uint16_t *__restrict__ Ch = reinterpret_cast<uint16_t *>(Cc);
+            auto load = [&](idx_t pc, int (&v)[N]) { if constexpr (P16) load_cfg16<N>(Ph + pc * (idx_t)RV, v); else load_cfg<N>(P + pc * (idx_t)RV, v); };
             bool ovf = false;
-            for (uint32_t j = j0 + threadIdx.x; j < j1; j += kCubeUnroll * kCubeThreads) {
-                uint32_t jj[kCubeUnroll];
-                // configuration indices fit 32 bits (a table has at most 2^30 cells): one IMAD + one IMAD.WIDE per address.  Arity 4 keeps
-                // 64-bit indices: ptxas allocates 44 registers for that form and 58 (or spills) for the 32-bit one
-                using idx_t = std::conditional_t<RV == 4, uint64_t, uint32_t>;
-                idx_t pc[kCubeUnroll];
-                bool on[kCubeUnroll];
-                int cnt[kCubeUnroll][RV];
+            for (uint32_t g = g0 + threadIdx.x; g < g1; g += U * kCubeThreads) {
+                uint32_t gg[U];
+                idx_t pc[U];
+                bool on[U];
+                int cnt[U][N];
 #pragma unroll
-                for (int u = 0; u < kCubeUnroll; u++) {
-                    jj[u] = j + u * kCubeThreads;
-                    on[u] = jj[u] < j1;
-                    const uint32_t ju = on[u] ? jj[u] : j;
+                for (int u = 0; u < U; u++) {
+                    gg[u] = g + u * kCubeThreads;
+                    on[u] = gg[u] < g1;
+                    const uint32_t ju = (on[u] ? gg[u] : g) * G;
                     const uint32_t hi = fast_div(ju, pr.Bc, pr.magic), lo = ju - hi * pr.Bc;
                     pc[u] = (idx_t)lo + (idx_t)hi * pr.r * pr.Bc;
                 }
 #pragma unroll
-                for (int u = 0; u < kCubeUnroll; u++) {
-                    if constexpr (P16) load_cfg16<RV>(Ph + pc[u] * (idx_t)RV, cnt[u]); else load_cfg<RV>(P + pc[u] * (idx_t)RV, cnt[u]);
-                }
+                for (int u = 0; u < U; u++) load(pc[u], cnt[u]);
+#pragma unroll 2
                 for (uint32_t a = 1; a < pr.r; a++) {
-                    int t[kCubeUnroll][RV];
+                    int t[U][N];
 #pragma unroll
-                    for (int u = 0; u < kCubeUnroll; u++) {
-                        if constexpr (P16) load_cfg16<RV>(Ph + (pc[u] + (idx_t)a * pr.Bc) * (idx_t)RV, t[u]); else load_cfg<RV>(P + (pc[u] + (idx_t)a * pr.Bc) * (idx_t)RV, t[u]);
-                    }
+                    for (int u = 0; u < U; u++) load(pc[u] + (idx_t)a * pr.Bc, t[u]);
 #pragma unroll
-                    for (int u = 0; u < kCubeUnroll; u++)
+                    for (int u = 0; u < U; u++)
 #pragma unroll
-                        for (int k = 0; k < RV; k++) cnt[u][k] += t[u][k];
+                        for (int k = 0; k < N; k++) cnt[u][k] += t[u][k];
                 }
 #pragma unroll
-                for (int u = 0; u < kCubeUnroll; u++) {
+                for (int u = 0; u < U; u++) {
                     if (!on[u]) continue;
-                    if (!pr.leaf) {
-                        if constexpr (C16) ovf |= store_cfg16<RV>(Ch + (idx_t)jj[u] * (idx_t)RV, cnt[u]); else store_cfg<RV>(Cc + (idx_t)jj[u] * (idx_t)RV, cnt[u]);
+                    if (store) {
+                        if constexpr (C16) ovf |= store_cfg16<N>(Ch + (idx_t)gg[u] * (idx_t)N, cnt[u]); else store_cfg<N>(Cc + (idx_t)gg[u] * (idx_t)N, cnt[u]);
                     }
-                    if (acc_out) score_cfg(cnt[u]);
+                    if (score_child)
+#pragma unroll
+                        for (int m = 0; m < G; m++) score_cfg<RV>(acc, cnt[u], m * RV, qlog, qcfg, cfg_min);
+                    if (score_leaf) {
+                        int leaf[RV];
+                        sum_group<RV, G>(cnt[u], leaf);
+                        score_cfg<RV>(lacc, leaf, 0, qlog, qcfg, cfg_min);
+                    }
                 }
             }
             if (ovf) *ovf_flag = 1;
         };
+        // r0 >= 3: the group's configurations one after another, each added into the leaf's counts in registers
+        auto run_any = [&](auto P16c, auto C16c) {
+            constexpr bool P16 = decltype(P16c)::value, C16 = decltype(C16c)::value;
+            const uint16_t *__restrict__ Ph = reinterpret_cast<const uint16_t *>(P);
+            uint16_t *__restrict__ Ch = reinterpret_cast<uint16_t *>(Cc);
+            auto load = [&](idx_t pc, int (&v)[RV]) { if constexpr (P16) load_cfg16<RV>(Ph + pc * (idx_t)RV, v); else load_cfg<RV>(P + pc * (idx_t)RV, v); };
+            bool ovf = false;
+            for (uint32_t g = g0 + threadIdx.x; g < g1; g += kCubeThreads) {
+                const uint32_t jg = g * r0, hi = fast_div(jg, pr.Bc, pr.magic), lo = jg - hi * pr.Bc;
+                const idx_t pg = (idx_t)lo + (idx_t)hi * pr.r * pr.Bc;
+                int leaf[RV] = {};
+#pragma unroll 1
+                for (uint32_t m = 0; m < r0; m++) {
+                    int cnt[RV];
+                    load(pg + m, cnt);
+                    for (uint32_t a = 1; a < pr.r; a++) {
+                        int t[RV];
+                        load(pg + m + (idx_t)a * pr.Bc, t);
+#pragma unroll
+                        for (int k = 0; k < RV; k++) cnt[k] += t[k];
+                    }
+                    if (store) {
+                        if constexpr (C16) ovf |= store_cfg16<RV>(Ch + ((idx_t)jg + m) * (idx_t)RV, cnt); else store_cfg<RV>(Cc + ((idx_t)jg + m) * (idx_t)RV, cnt);
+                    }
+                    if (score_child) score_cfg<RV>(acc, cnt, 0, qlog, qcfg, cfg_min);
+#pragma unroll
+                    for (int k = 0; k < RV; k++) leaf[k] += cnt[k];
+                }
+                if (score_leaf) score_cfg<RV>(lacc, leaf, 0, qlog, qcfg, cfg_min);
+            }
+            if (ovf) *ovf_flag = 1;
+        };
+        auto by_group = [&](auto P16c, auto C16c) {
+            if (r0 == 1) run(std::integral_constant<int, 1>{}, P16c, C16c);
+            else if (r0 == 2) run(std::integral_constant<int, 2>{}, P16c, C16c);
+            else run_any(P16c, C16c);
+        };
         switch (pr.fmt & 3u) {
-        case 0: run(std::false_type{}, std::false_type{}); break;
-        case 1: run(std::true_type{}, std::false_type{}); break;
-        case 2: run(std::false_type{}, std::true_type{}); break;
-        default: run(std::true_type{}, std::true_type{}); break;
+        case 0: by_group(std::false_type{}, std::false_type{}); break;
+        case 1: by_group(std::true_type{}, std::false_type{}); break;
+        case 2: by_group(std::false_type{}, std::true_type{}); break;
+        default: by_group(std::true_type{}, std::true_type{}); break;
         }
     } else {
-        for (uint32_t j = j0 + threadIdx.x; j < j1; j += kCubeThreads) {
-            const uint32_t hi = j / pr.Bc, lo = j - hi * pr.Bc;
-            const uint64_t pc0 = (uint64_t)lo + (uint64_t)hi * pr.r * pr.Bc;
-            int nij = 0;
-            const uint16_t *Ph = reinterpret_cast<const uint16_t *>(P);
-            uint16_t *Ch = reinterpret_cast<uint16_t *>(Cc);
-            for (int k = 0; k < rv; k++) {
-                int cnt = 0;
-                for (uint32_t a = 0; a < pr.r; a++) cnt += (pr.fmt & 1u) ? (int)Ph[(pc0 + (uint64_t)a * pr.Bc) * rv + k] : P[(pc0 + (uint64_t)a * pr.Bc) * rv + k];
-                if (!pr.leaf) {
-                    if (pr.fmt & 2u) { Ch[(uint64_t)j * rv + k] = (uint16_t)min(cnt, 65535); if (cnt > 65535) *ovf_flag = 1; }
-                    else Cc[(uint64_t)j * rv + k] = cnt;
+        const uint16_t *Ph = reinterpret_cast<const uint16_t *>(P);
+        uint16_t *Ch = reinterpret_cast<uint16_t *>(Cc);
+        auto cell = [&](uint64_t i) { return (pr.fmt & 1u) ? (int)Ph[i] : P[i]; };
+        for (uint32_t g = g0 + threadIdx.x; g < g1; g += kCubeThreads) {
+            const uint32_t jg = g * r0, hi = jg / pr.Bc, lo = jg - hi * pr.Bc;
+            const uint64_t pg = (uint64_t)lo + (uint64_t)hi * pr.r * pr.Bc;
+            for (uint32_t m = 0; m < r0; m++) {
+                const uint64_t j = (uint64_t)jg + m;
+                int nij = 0;
+                for (int k = 0; k < rv; k++) {
+                    int cnt = 0;
+                    for (uint32_t a = 0; a < pr.r; a++) cnt += cell((pg + m + (uint64_t)a * pr.Bc) * rv + k);
+                    if (store) {
+                        if (pr.fmt & 2u) { Ch[j * rv + k] = (uint16_t)min(cnt, 65535); if (cnt > 65535) *ovf_flag = 1; }
+                        else Cc[j * rv + k] = cnt;
+                    }
+                    nij += cnt;
+                    if (score_child && cnt > 1) acc += __ldg(&qlog[cnt]);
                 }
-                nij += cnt;
-                if (acc_out && cnt > 1) acc += __ldg(&qlog[cnt]);
+                if (score_child && nij > cfg_min) acc -= __ldg(&qcfg[nij]);
             }
-            if (acc_out && nij > cfg_min) acc -= __ldg(&qcfg[nij]);
+            if (score_leaf) { // an arity this wide keeps no leaf counts in registers: the group's parent cells are read again (L1)
+                int nl = 0;
+                for (int k = 0; k < rv; k++) {
+                    int cnt = 0;
+                    for (uint32_t m = 0; m < r0; m++)
+                        for (uint32_t a = 0; a < pr.r; a++) cnt += cell((pg + m + (uint64_t)a * pr.Bc) * rv + k);
+                    nl += cnt;
+                    if (cnt > 1) lacc += __ldg(&qlog[cnt]);
+                }
+                if (nl > cfg_min) lacc -= __ldg(&qcfg[nl]);
+            }
         }
     }
-    if (acc_out) {
-        acc = block_sum_ll(acc, red);
-        if (threadIdx.x == 0 && acc != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_out[pr.acc_index]), (unsigned long long)acc);
+    if (score_child) {
+        acc = block_sum_ll(acc, red[0]);
+        if (threadIdx.x == 0 && acc != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_all[s_acc[0]]), (unsigned long long)acc);
+    }
+    if (score_leaf) {
+        lacc = block_sum_ll(lacc, red[1]);
+        if (threadIdx.x == 0 && lacc != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_all[s_acc[1]]), (unsigned long long)lacc);
     }
 }
 

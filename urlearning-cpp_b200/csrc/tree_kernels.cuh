@@ -207,6 +207,8 @@ __device__ __forceinline__ void tree_count_fragmented(const unsigned long long *
 //     CTA sums each run digit b < z out of the slice (a block-wide pass: the slice holds the whole run), scores
 //     child b = root \ {b} on the fly and writes the child's slice to ITS global table unless b == 0 (nothing is
 //     derived from a set that lacks bit 0).  This removes the write and the z reads of the largest layer of tables.
+//     For b >= 1 a thread sums whole groups of card[0] consecutive child configurations (pre[b] is a multiple of card[0]),
+//     so it also holds the counts of the child's leaf root \ {b, 0} and scores it (bic_kernels.cuh, "LEAF").
 // ---------------------------------------------------------------------------------------------------------
 constexpr int kRootMaxChild = 16;
 
@@ -215,8 +217,10 @@ struct CubeRoot {
     unsigned long long table_off;            // plain: the root's table in `tables` (int32 elements)
     unsigned long long child_off[kRootMaxChild];   // fused: child b's table in `child_tables`
     uint32_t child_acc[kRootMaxChild];       // and its accumulator
+    uint32_t leaf_acc[kRootMaxChild];        // accumulator of the leaf root \ {b, 0} of child b >= 1
     uint32_t nchild;                         // fused: children drop bit b, bfirst <= b < nchild (== run length)
-    uint16_t bfirst, score;                  // layers above K only hold sets with their lowest bits forced: the first droppable bit; score the children?
+    uint16_t bfirst, score;                  // layers above K only hold sets with their lowest bits forced: the first droppable bit;
+                                             // score bit 0: score the children, bit 1: score the leaves of children b >= 1
     uint32_t child16;                        // bit b: child b's table holds uint16 cells (bic_kernels.cuh, "16-bit tables")
     uint32_t pad16;
 };
@@ -233,7 +237,7 @@ __global__ void root_map_kernel(const CubeRoot *__restrict__ roots, int nroots, 
 }
 
 template <int RV, int NW>
-__global__ void __launch_bounds__(NW * 32) bic_root_kernel(TreeVar tv, const CubeRoot *__restrict__ roots, const uint32_t *__restrict__ cta_root,
+__global__ void __launch_bounds__(NW * 32, 2) bic_root_kernel(TreeVar tv, const CubeRoot *__restrict__ roots, const uint32_t *__restrict__ cta_root,
                                                                 const long long *__restrict__ qlog, const long long *__restrict__ qcfg, int cfg_min,
                                                                 int *__restrict__ tables, int *__restrict__ child_tables,
                                                                 long long *__restrict__ acc_out, uint32_t table_budget /*cells*/, uint32_t seg_cap,
@@ -241,7 +245,7 @@ __global__ void __launch_bounds__(NW * 32) bic_root_kernel(TreeVar tv, const Cub
     extern __shared__ __align__(16) int s_dyn[];              // [table_budget] slice table, then segbeg[seg_cap], segoff[seg_cap + 1]
     __shared__ CubeRoot cr;
     __shared__ uint16_t s_lut[8 * 256];
-    __shared__ unsigned long long s_cacc[kRootMaxChild]; // per-child exact sums of this CTA
+    __shared__ unsigned long long s_cacc[2][kRootMaxChild]; // per-child exact sums of this CTA: [0] the child b, [1] its leaf
     constexpr int kRootThreads = NW * 32;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int rv = RV > 0 ? RV : tv.rv;
@@ -255,7 +259,7 @@ __global__ void __launch_bounds__(NW * 32) bic_root_kernel(TreeVar tv, const Cub
     const TreeRoot &rt = cr.t;
     const int z = rt.z;
     (void)qn;
-    if (tid < kRootMaxChild) s_cacc[tid] = 0;
+    if (tid < 2 * kRootMaxChild) s_cacc[tid / kRootMaxChild][tid % kRootMaxChild] = 0;
     const uint32_t S0 = rt.H * (uint32_t)rv * tv.pre[z];
     const uint32_t si = blockIdx.x - rt.chunk0;
     {
@@ -352,7 +356,7 @@ __global__ void __launch_bounds__(NW * 32) bic_root_kernel(TreeVar tv, const Cub
     }
     // fused root: children b = bfirst .. z-1
     const uint32_t cfg_src = S0 / (uint32_t)rv;
-    const bool score = cr.score != 0;
+    const bool score = cr.score & 1u;
     for (int b = cr.bfirst; b < z; b++) {
         const uint32_t r = tv.card[b], pre = tv.pre[b], magic = tv.magic[b];
         const uint32_t cfg_dst = fast_div(cfg_src, r, tv.cmagic[b]); // r divides the run product: exact
@@ -360,83 +364,138 @@ __global__ void __launch_bounds__(NW * 32) bic_root_kernel(TreeVar tv, const Cub
         int *dst = child_tables + cr.child_off[b] + (c16 ? 0ull : (unsigned long long)si * ((unsigned long long)cfg_dst * rv));
         uint16_t *dst16 = reinterpret_cast<uint16_t *>(child_tables + cr.child_off[b]) + (unsigned long long)si * ((unsigned long long)cfg_dst * rv);
         const bool store = b > 0;
+        const bool sleaf = b > 0 && (cr.score & 2u);
+        const uint32_t r0 = b > 0 ? tv.card[0] : 1u;   // configurations per group
         bool ovf = false;
-        long long acc = 0;
+        long long acc = 0, lacc = 0;
         if constexpr (RV > 0) {
-            // R = compile-time arity of the digit summed out (2, 3, 4), 0 = run-time loop
-            auto pass = [&](auto RC) {
-                constexpr int R = decltype(RC)::value;
-                for (uint32_t j = tid; j < cfg_dst; j += kRootThreads) {
-                    const uint32_t hi = fast_div(j, pre, magic), lo = j - hi * pre;
+            // R = compile-time arity of the digit summed out (2, 3, 4), 0 = run-time loop; G = compile-time group size
+            auto pass = [&](auto RC, auto GC) {
+                constexpr int R = decltype(RC)::value, G = decltype(GC)::value, N = G * RV;
+                for (uint32_t g = tid; g < cfg_dst / G; g += kRootThreads) {
+                    const uint32_t j = g * G, hi = fast_div(j, pre, magic), lo = j - hi * pre;
                     const uint32_t p0 = lo + hi * r * pre;
-                    int cnt[RV];
-                    load_cfg<RV>(s_dyn + (size_t)p0 * RV, cnt);
+                    int cnt[N];
+                    load_cfg<N>(s_dyn + (size_t)p0 * RV, cnt);
                     if constexpr (R > 0) {
 #pragma unroll
                         for (int a = 1; a < R; a++) {
-                            int t[RV];
-                            load_cfg<RV>(s_dyn + (size_t)(p0 + a * pre) * RV, t);
+                            int t[N];
+                            load_cfg<N>(s_dyn + (size_t)(p0 + a * pre) * RV, t);
 #pragma unroll
-                            for (int k = 0; k < RV; k++) cnt[k] += t[k];
+                            for (int k = 0; k < N; k++) cnt[k] += t[k];
                         }
                     } else {
+#pragma unroll 2
                         for (uint32_t a = 1; a < r; a++) {
-                            int t[RV];
-                            load_cfg<RV>(s_dyn + (size_t)(p0 + a * pre) * RV, t);
+                            int t[N];
+                            load_cfg<N>(s_dyn + (size_t)(p0 + a * pre) * RV, t);
 #pragma unroll
-                            for (int k = 0; k < RV; k++) cnt[k] += t[k];
+                            for (int k = 0; k < N; k++) cnt[k] += t[k];
                         }
                     }
                     if (store) {
-                        if (c16) ovf |= store_cfg16<RV>(dst16 + (size_t)j * RV, cnt);
-                        else store_cfg<RV>(dst + (size_t)j * RV, cnt);
+                        if (c16) ovf |= store_cfg16<N>(dst16 + (size_t)j * RV, cnt);
+                        else store_cfg<N>(dst + (size_t)j * RV, cnt);
                     }
-                    int nij = 0;
+                    if (score)
 #pragma unroll
-                    for (int k = 0; k < RV; k++) nij += cnt[k];
-                    if (score && nij > cfg_min) {
-#pragma unroll
-                        for (int k = 0; k < RV; k++)
-                            if (cnt[k] > 1) acc += __ldg(&qlog[cnt[k]]);
-                        acc -= __ldg(&qcfg[nij]);
+                        for (int m = 0; m < G; m++) score_cfg<RV>(acc, cnt, m * RV, qlog, qcfg, cfg_min);
+                    if (sleaf) {
+                        int leaf[RV];
+                        sum_group<RV, G>(cnt, leaf);
+                        score_cfg<RV>(lacc, leaf, 0, qlog, qcfg, cfg_min);
                     }
                 }
             };
-            switch (r) {
-            case 2: pass(std::integral_constant<int, 2>{}); break;
-            case 3: pass(std::integral_constant<int, 3>{}); break;
-            case 4: pass(std::integral_constant<int, 4>{}); break;
-            default: pass(std::integral_constant<int, 0>{}); break;
-            }
-        } else {
-            for (uint32_t j = tid; j < cfg_dst; j += kRootThreads) {
-                const uint32_t hi = fast_div(j, pre, magic), lo = j - hi * pre;
-                const uint32_t p0 = lo + hi * r * pre;
-                int nij = 0;
-                for (int k = 0; k < rv; k++) {
-                    int cnt = 0;
-                    for (uint32_t a = 0; a < r; a++) cnt += s_dyn[(size_t)(p0 + a * pre) * rv + k];
-                    if (store) {
-                        if (c16) { dst16[(size_t)j * rv + k] = (uint16_t)min(cnt, 65535); ovf |= cnt > 65535; }
-                        else dst[(size_t)j * rv + k] = cnt;
+            // r0 >= 3: the group's configurations one after another, each added into the leaf's counts in registers
+            auto pass_any = [&]() {
+                for (uint32_t g = tid; g < cfg_dst / r0; g += kRootThreads) {
+                    const uint32_t jg = g * r0, hi = fast_div(jg, pre, magic), lo = jg - hi * pre;
+                    const uint32_t pg = lo + hi * r * pre;
+                    int leaf[RV] = {};
+#pragma unroll 1
+                    for (uint32_t m = 0; m < r0; m++) {
+                        int cnt[RV];
+                        load_cfg<RV>(s_dyn + (size_t)(pg + m) * RV, cnt);
+#pragma unroll 2
+                        for (uint32_t a = 1; a < r; a++) {
+                            int t[RV];
+                            load_cfg<RV>(s_dyn + (size_t)(pg + m + a * pre) * RV, t);
+#pragma unroll
+                            for (int k = 0; k < RV; k++) cnt[k] += t[k];
+                        }
+                        if (store) {
+                            if (c16) ovf |= store_cfg16<RV>(dst16 + (size_t)(jg + m) * RV, cnt);
+                            else store_cfg<RV>(dst + (size_t)(jg + m) * RV, cnt);
+                        }
+                        if (score) score_cfg<RV>(acc, cnt, 0, qlog, qcfg, cfg_min);
+#pragma unroll
+                        for (int k = 0; k < RV; k++) leaf[k] += cnt[k];
                     }
-                    nij += cnt;
-                    if (score && cnt > 1) acc += __ldg(&qlog[cnt]);
+                    if (sleaf) score_cfg<RV>(lacc, leaf, 0, qlog, qcfg, cfg_min);
                 }
-                if (score && nij > cfg_min) acc -= __ldg(&qcfg[nij]);
+            };
+            auto by_arity = [&](auto GC) {
+                switch (r) {
+                case 2: pass(std::integral_constant<int, 2>{}, GC); break;
+                case 3: pass(std::integral_constant<int, 3>{}, GC); break;
+                case 4: pass(std::integral_constant<int, 4>{}, GC); break;
+                default: pass(std::integral_constant<int, 0>{}, GC); break;
+                }
+            };
+            if (r0 == 1) by_arity(std::integral_constant<int, 1>{});
+            else if (r0 == 2) by_arity(std::integral_constant<int, 2>{});
+            else pass_any();
+        } else {
+            for (uint32_t g = tid; g < cfg_dst / r0; g += kRootThreads) {
+                const uint32_t jg = g * r0, hi = fast_div(jg, pre, magic), lo = jg - hi * pre;
+                const uint32_t pg = lo + hi * r * pre;
+                for (uint32_t m = 0; m < r0; m++) {
+                    const uint32_t j = jg + m, p0 = pg + m;
+                    int nij = 0;
+                    for (int k = 0; k < rv; k++) {
+                        int cnt = 0;
+                        for (uint32_t a = 0; a < r; a++) cnt += s_dyn[(size_t)(p0 + a * pre) * rv + k];
+                        if (store) {
+                            if (c16) { dst16[(size_t)j * rv + k] = (uint16_t)min(cnt, 65535); ovf |= cnt > 65535; }
+                            else dst[(size_t)j * rv + k] = cnt;
+                        }
+                        nij += cnt;
+                        if (score && cnt > 1) acc += __ldg(&qlog[cnt]);
+                    }
+                    if (score && nij > cfg_min) acc -= __ldg(&qcfg[nij]);
+                }
+                if (sleaf) { // the leaf's counts: the group's cells summed again from shared memory
+                    int nl = 0;
+                    for (int k = 0; k < rv; k++) {
+                        int cnt = 0;
+                        for (uint32_t m = 0; m < r0; m++)
+                            for (uint32_t a = 0; a < r; a++) cnt += s_dyn[(size_t)(pg + m + a * pre) * rv + k];
+                        nl += cnt;
+                        if (cnt > 1) lacc += __ldg(&qlog[cnt]);
+                    }
+                    if (nl > cfg_min) lacc -= __ldg(&qcfg[nl]);
+                }
             }
         }
         if (ovf) *ovf_flag = 1;
-        if (score) { // no barrier between children: every warp adds its exact partial sum to the child's shared accumulator
+        // no barrier between children: every warp adds its exact partial sums to the child's shared accumulators
+        if (score) {
             acc = warp_sum_ll_redux(acc);
-            if (lane == 0 && acc != 0) atomicAdd(&s_cacc[b], (unsigned long long)acc);
+            if (lane == 0 && acc != 0) atomicAdd(&s_cacc[0][b], (unsigned long long)acc);
+        }
+        if (sleaf) {
+            lacc = warp_sum_ll_redux(lacc);
+            if (lane == 0 && lacc != 0) atomicAdd(&s_cacc[1][b], (unsigned long long)lacc);
         }
     }
-    if (score) {
+    if (cr.score) {
         __syncthreads();
         if (tid >= (int)cr.bfirst && tid < z) {
-            const unsigned long long a = s_cacc[tid];
-            if (a != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_out[cr.child_acc[tid]]), a);
+            const unsigned long long a = s_cacc[0][tid], la = s_cacc[1][tid];
+            if (score && a != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_out[cr.child_acc[tid]]), a);
+            if (la != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_out[cr.leaf_acc[tid]]), la);
         }
     }
 }

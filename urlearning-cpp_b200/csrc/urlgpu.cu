@@ -854,6 +854,7 @@ struct CubeSet {
     uint32_t cube_mask, res_mask;
     uint64_t cells, off;
     int parent;       // index in the layer above
+    int leaf_child;   // a set that holds cube bit 0: index of its leaf child (the set without bit 0) in the layer below, or -1
     uint32_t Bc, r;
     bool t16;         // the table is stored with uint16 cells
 };
@@ -961,6 +962,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         cs.cells = (uint64_t)std::min<__uint128_t>(cells, kCellLimit + 1);
         cs.res_mask = resT[b0] | resT[256 + b1] | resT[512 + b2] | resT[768 + b3];
         cs.parent = -1;
+        cs.leaf_child = -1;
         return cs;
     };
     for (int l = 0; l <= Lmax; l++) {
@@ -1116,7 +1118,8 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         if (((Lstar - l) & 1) == 0) needA = std::max<size_t>(needA, off); else needB = std::max<size_t>(needB, off);
         if (l < Lstar) {
             auto &P = layers[l + 1];
-            for (auto &cs : layers[l]) {
+            for (size_t i = 0; i < layers[l].size(); i++) {
+                auto &cs = layers[l][i];
                 const int z = __builtin_ctz(~cs.cube_mask); // lowest missing cube bit (< c because l < Lstar <= c)
                 const uint32_t pm = cs.cube_mask | (1u << z);
                 auto it = std::lower_bound(P.begin(), P.end(), pm, [](const CubeSet &a, uint32_t m) { return a.cube_mask < m; });
@@ -1124,6 +1127,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
                 cs.parent = (int)(it - P.begin());
                 cs.Bc = (uint32_t)prefix[z];
                 cs.r = (uint32_t)ccard[z];
+                if (z == 0) it->leaf_child = (int)i;   // a leaf: its parent is the set plus bit 0
             }
         }
     }
@@ -1236,13 +1240,18 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
                     if (kind == 2) {
                         cr.nchild = (uint32_t)run;
                         cr.bfirst = (uint16_t)std::max(0, Lstar - 1 - Kc);
-                        cr.score = Lstar - 1 <= Kc ? 1 : 0;
+                        // children b >= 1 hold bit 0: the root kernel also scores their leaves root \ {b, 0} (layer Lstar - 2 <= Kc)
+                        cr.score = (Lstar - 1 <= Kc ? 1 : 0) | (run > std::max<int>(cr.bfirst, 1) ? 2 : 0);
                         for (int b = cr.bfirst; b < run; b++) {
                             const uint32_t cm = P & ~(1u << b);
                             auto it = std::lower_bound(Lc.begin(), Lc.end(), cm, [](const CubeSet &a, uint32_t m) { return a.cube_mask < m; });
                             if (it == Lc.end() || it->cube_mask != cm) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: child of a fused root missing");
                             cr.child_off[b] = it->off;
-                            cr.child_acc[b] = (uint32_t)(it - Lc.begin());
+                            cr.child_acc[b] = (uint32_t)(acc_off[Lstar - 1] + (it - Lc.begin()));
+                            if (b > 0) {
+                                if (it->leaf_child < 0) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: leaf of a fused root's child missing");
+                                cr.leaf_acc[b] = (uint32_t)(acc_off[Lstar - 2] + it->leaf_child);
+                            }
                             if (it->t16) cr.child16 |= 1u << b;
                             if (b > 0) ctx->st.k1_bytes_written += (it->t16 ? 2.0 : 4.0) * (double)it->cells; // only children that have children of their own are stored
                         }
@@ -1284,7 +1293,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
                 const size_t smem = ((size_t)RB + 2 * seg_cap + 1) * sizeof(int);
                 const unsigned grid = (unsigned)rchunk;
                 switch (rv) {
-#define URLGPU_ROOT_ARGS tv, dcroots.as<CubeRoot>(), dmap.as<uint32_t>(), ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, bufP, bufC, dacc.as<long long>() + acc_off[Lstar > 0 ? Lstar - 1 : 0], RB, seg_cap, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)
+#define URLGPU_ROOT_ARGS tv, dcroots.as<CubeRoot>(), dmap.as<uint32_t>(), ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, bufP, bufC, dacc.as<long long>(), RB, seg_cap, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)
 #define URLGPU_ROOT(RVV)                                                                             \
     do {                                                                                             \
         if (ctx->root_warps == 8) bic_root_kernel<RVV, 8><<<grid, 256, smem, s>>>(URLGPU_ROOT_ARGS); \
@@ -1350,6 +1359,9 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         std::vector<uint32_t> first(P.size() + 1, 0), order;
         auto skip = [&](const CubeSet &cs) {
             if (!mine[l + 1][cs.parent]) return true;   // outside this call's sub-forest
+            // a leaf of a derived table was scored by the pass that derived its parent (the derive or the root kernel); only
+            // leaves of root tables, which come from kernels that do not build digit-0 groups, are derived on their own
+            if ((cs.cube_mask & 1u) == 0 && l + 1 < Lstar) return true;
             return top && fused_root[cs.parent] != 0;
         };
         for (auto &cs : L) if (!skip(cs)) first[cs.parent + 1]++;
@@ -1364,16 +1376,24 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         for (size_t k = 0; k < order.size(); k++) {
             const CubeSet &cs = L[order[k]];
             CubePair pr{};
+            const bool leaf = (cs.cube_mask & 1u) == 0; // lowest missing bit is 0: nothing is derived from this set
             pr.parent_off = P[cs.parent].off; pr.child_off = cs.off;
-            pr.child_configs = (uint32_t)(cs.cells / rv);
+            pr.r0 = leaf ? 1u : (uint32_t)ccard[0];
+            pr.groups = (uint32_t)(cs.cells / rv / pr.r0);
             pr.Bc = cs.Bc; pr.r = cs.r; pr.chunk0 = (uint32_t)chunk;
             pr.acc_index = (uint32_t)(acc_off[l] + order[k]);
-            pr.leaf = (cs.cube_mask & 1u) == 0; // lowest missing bit is 0: nothing is derived from this set
+            pr.flags = (leaf ? 0u : kCubeStore) | (l <= Kc ? kCubeScoreChild : 0u);
+            if (!leaf) { // l >= 1 and l - 1 <= Kc: the leaf child exists and is scored from this pair's groups
+                if (cs.leaf_child < 0) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: leaf child missing");
+                pr.leaf_acc = (uint32_t)(acc_off[l - 1] + cs.leaf_child);
+                pr.flags |= kCubeScoreLeaf;
+            }
             pr.fmt = (P[cs.parent].t16 ? 1u : 0u) | (cs.t16 ? 2u : 0u);
             pr.magic = pr.Bc > 1 ? 0xFFFFFFFFu / pr.Bc : 0;
             ctx->st.k1_bytes_read += (P[cs.parent].t16 ? 2.0 : 4.0) * (double)cs.cells * (double)cs.r;
-            if (!pr.leaf) ctx->st.k1_bytes_written += (cs.t16 ? 2.0 : 4.0) * (double)cs.cells;
-            chunk += (pr.child_configs + kCubeConfigsPerBlock - 1) / kCubeConfigsPerBlock;
+            if (!leaf) ctx->st.k1_bytes_written += (cs.t16 ? 2.0 : 4.0) * (double)cs.cells;
+            const uint32_t gpb = kCubeConfigsPerBlock / pr.r0;
+            chunk += (pr.groups + gpb - 1) / gpb;
             hp[k] = pr;
         }
         if (chunk > 0x7fffffffull) return ctx->fail(URLGPU_ERR_LIMIT, "cube: too many blocks in one layer");
@@ -1385,10 +1405,10 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
             const unsigned grid = (unsigned)chunk;
             cube_map_kernel<<<blocks_for(chunk, 256), 256, 0, s>>>(dpairs.as<CubePair>(), (int)hp.size(), grid, dcmap.as<uint32_t>());
             switch (rv) {
-            case 2: cube_derive_kernel<2><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
-            case 3: cube_derive_kernel<3><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
-            case 4: cube_derive_kernel<4><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
-            default: cube_derive_kernel<0><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), score, d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
+            case 2: cube_derive_kernel<2><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
+            case 3: cube_derive_kernel<3><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
+            case 4: cube_derive_kernel<4><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
+            default: cube_derive_kernel<0><<<grid, kCubeThreads, 0, s>>>(dpairs.as<CubePair>(), dcmap.as<uint32_t>(), bufP, bufC, rv, ctx->d_qlog, ctx->ds_qcfg, ctx->ds_cfg_min, dacc.as<long long>(), d_ovf, (int)std::min<int64_t>(ctx->n + 2, 1 << 30)); break;
             }
         }
         if (score) { int rc = finalize_layer(l); if (rc) return rc; }
