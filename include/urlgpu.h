@@ -136,7 +136,8 @@ void urlgpu_host_free(void *p);
 /* (variable, parent-set range) shards — the multi-GPU unit of work SURVEY.md 8(e) / BASELINE.json north_star name.
  * The canonical order of a family (layer by layer, each layer in the reference's Gosper order, score_calculator.cpp:76-120)
  * numbers its sets 0 .. family_size-1; a contiguous range of that numbering is scored independently of the rest:
- *   urlgpu_family_size        number of sets: sum_{l<=max_parents} C(candidates, l)  (fails above 2^32)
+ *   urlgpu_family_size        number of sets: sum_{l<=max_parents} C(candidates, l); a family of more than 2^32 - 16 sets
+ *                             is refused (URLGPU_ERR_LIMIT): the score caches index sets with 32 bits
  *   urlgpu_score_range        RAW scores of sets [first, first+count) (BIC: the score, cBIC: the_score before negation),
  *                             into a host buffer or, on_device=1, a device buffer on ctx's device (e.g. an NCCL send buffer)
  *   urlgpu_result_from_scores the variable's owner, holding all family_size raw scores (gathered from the ranks), applies

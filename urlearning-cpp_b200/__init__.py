@@ -239,26 +239,31 @@ class Result:
         self._eng._check(self._eng.lib.urlgpu_result_scored(self._h, C.byref(n)))
         return n.value
 
-    def fetch(self, pinned: bool = False):
-        """-> (masks uint64[n, words], scores float32[n]) in canonical (|S|, mask) order.
+    def fetch(self, pinned: bool = False, first: int = 0, n: int | None = None):
+        """-> (masks uint64[n, words], scores float32[n]) in canonical (|S|, mask) order: the stored entries [first, first + n),
+        by default all of them.
         pinned=True: the arrays are views of the engine's page-locked result buffer (PCIe-speed copy, no page faults on
         fresh memory); they stay valid until the next pinned fetch on the same engine."""
-        n = self.count()
+        if n is None:
+            n = self.count() - first
         if pinned:
             masks, scores = self._eng._pinned_views(n, self.words)
         else:
             masks = np.zeros((n, self.words), dtype=np.uint64)
             scores = np.zeros(n, dtype=np.float32)
         if n:
-            self._eng._check(self._eng.lib.urlgpu_result_fetch(self._h, 0, n, masks.ctypes.data, scores.ctypes.data))
+            self._eng._check(self._eng.lib.urlgpu_result_fetch(self._h, first, n, masks.ctypes.data, scores.ctypes.data))
         return masks, scores
 
-    def fetch_device(self, masks_ptr: int, scores_ptr: int, words_out: int | None = None, shift: int = 0) -> int:
-        """write the stored entries (canonical order) to device addresses — local or peer-mapped (Engine.peer_open): masks as
-        ``words_out`` words with every variable index shifted by ``shift``, scores as float32.  -> number of entries"""
-        n = self.count()
+    def fetch_device(self, masks_ptr: int, scores_ptr: int, words_out: int | None = None, shift: int = 0, first: int = 0,
+                     n: int | None = None) -> int:
+        """write the stored entries [first, first + n) (canonical order; by default all of them) to device addresses — local or
+        peer-mapped (Engine.peer_open): masks as ``words_out`` words with every variable index shifted by ``shift``, scores as
+        float32.  A null (0) address skips that part.  -> number of entries"""
+        if n is None:
+            n = self.count() - first
         if n:
-            self._eng._check(self._eng.lib.urlgpu_result_fetch_device(self._h, 0, n, int(words_out or self.words), int(shift),
+            self._eng._check(self._eng.lib.urlgpu_result_fetch_device(self._h, first, n, int(words_out or self.words), int(shift),
                                                                       C.c_void_p(masks_ptr), C.c_void_p(scores_ptr)))
         return n
 

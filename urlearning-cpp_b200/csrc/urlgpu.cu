@@ -1741,6 +1741,8 @@ static int make_rank_sets(urlgpu_ctx *ctx, int variable, const std::vector<int> 
     return URLGPU_OK;
 }
 
+constexpr uint32_t kDirectChunk = 1u << 28;   // sets classified and counted per pass of bic_score_direct
+
 static int bic_score_direct(urlgpu_ctx *ctx, int variable, const std::vector<int> &cand, const RankSpace &rs, uint32_t first, uint32_t count, float *d_scores,
                             bool by_mask) {
     cudaStream_t s = ctx->stream;
@@ -1752,36 +1754,42 @@ static int bic_score_direct(urlgpu_ctx *ctx, int variable, const std::vector<int
     RankSets fam{};
     int rc = make_rank_sets(ctx, variable, cand, rs, by_mask, hv, dcand, fam);
     if (rc) return rc;
-    CK(lists.alloc((size_t)count * (sizeof(GlobalSet) + 2 * sizeof(uint32_t))));
+    // the range in chunks: every grid (one CTA per set in the shared-memory tiers) stays below 2^31 - 1 blocks, and the tier
+    // lists (20 bytes per set) below 5.4 GB.  Each set is scored on its own, so the chunking changes no output.
+    const uint32_t chunk = std::min(count, kDirectChunk);
+    CK(lists.alloc((size_t)chunk * (sizeof(GlobalSet) + 2 * sizeof(uint32_t))));
     CK(counters.alloc(4 * sizeof(unsigned long long)));
-    CK(cudaMemsetAsync(counters.p, 0, 4 * sizeof(unsigned long long), s));
     GlobalSet *l2 = lists.as<GlobalSet>();
-    uint32_t *l0 = reinterpret_cast<uint32_t *>(l2 + count), *l1 = l0 + count;
-    {
-        Region rg(ctx, F_OTHER, 1);
-        bic_classify_kernel<<<blocks_for(count, 256), 256, rs_binom_bytes(rs), s>>>(fam, first, count, kTier0Cells, tier1_cells, kCellLimit, l0, l1, l2,
-                                                                                    counters.as<unsigned long long>());
-    }
-    unsigned long long hc[4];
-    CK(cudaMemcpyAsync(hc, counters.p, sizeof hc, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    if (hc[3]) return ctx->fail(URLGPU_ERR_LIMIT, "a contingency table of this family has more than 2^30 cells");
-    if (hc[0]) {
-        Region rg(ctx, F_COUNT, 1);
-        const int threads = ctx->n >= 65536 ? 256 : 128;
-        bic_count_smem_kernel<<<(unsigned)hc[0], threads, kTier0Cells * sizeof(int), s>>>(bd, fam, l0, d_scores, nullptr, nullptr, nullptr);
-    }
-    if (hc[1]) {
-        Region rg(ctx, F_COUNT, 1);
-        bic_count_smem_kernel<<<(unsigned)hc[1], 1024, (size_t)tier1_cells * sizeof(int), s>>>(bd, fam, l1, d_scores, nullptr, nullptr, nullptr);
-    }
-    if (hc[2]) {
-        std::vector<GlobalSet> sets(hc[2]);
-        CK(cudaMemcpyAsync(sets.data(), l2, hc[2] * sizeof(GlobalSet), cudaMemcpyDeviceToHost, s));
+    uint32_t *l0 = reinterpret_cast<uint32_t *>(l2 + chunk), *l1 = l0 + chunk;
+    for (uint64_t c0 = 0; c0 < count; c0 += chunk) {
+        const uint32_t f = first + (uint32_t)c0, cnt = (uint32_t)std::min<uint64_t>(chunk, count - c0);
+        CK(cudaMemsetAsync(counters.p, 0, 4 * sizeof(unsigned long long), s));
+        {
+            Region rg(ctx, F_OTHER, 1);
+            bic_classify_kernel<<<blocks_for(cnt, 256), 256, rs_binom_bytes(rs), s>>>(fam, f, cnt, kTier0Cells, tier1_cells, kCellLimit, l0, l1, l2,
+                                                                                      counters.as<unsigned long long>());
+        }
+        unsigned long long hc[4];
+        CK(cudaMemcpyAsync(hc, counters.p, sizeof hc, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
-        std::sort(sets.begin(), sets.end(), [](const GlobalSet &a, const GlobalSet &b) { return a.key < b.key; });
-        rc = direct_global_tier(ctx, bd, fam, sets, d_scores, nullptr, nullptr, 0);
-        if (rc) return rc;
+        if (hc[3]) return ctx->fail(URLGPU_ERR_LIMIT, "a contingency table of this family has more than 2^30 cells");
+        if (hc[0]) {
+            Region rg(ctx, F_COUNT, 1);
+            const int threads = ctx->n >= 65536 ? 256 : 128;
+            bic_count_smem_kernel<<<(unsigned)hc[0], threads, kTier0Cells * sizeof(int), s>>>(bd, fam, l0, d_scores, nullptr, nullptr, nullptr);
+        }
+        if (hc[1]) {
+            Region rg(ctx, F_COUNT, 1);
+            bic_count_smem_kernel<<<(unsigned)hc[1], 1024, (size_t)tier1_cells * sizeof(int), s>>>(bd, fam, l1, d_scores, nullptr, nullptr, nullptr);
+        }
+        if (hc[2]) {
+            std::vector<GlobalSet> sets(hc[2]);
+            CK(cudaMemcpyAsync(sets.data(), l2, hc[2] * sizeof(GlobalSet), cudaMemcpyDeviceToHost, s));
+            CK(cudaStreamSynchronize(s));
+            std::sort(sets.begin(), sets.end(), [](const GlobalSet &a, const GlobalSet &b) { return a.key < b.key; });
+            rc = direct_global_tier(ctx, bd, fam, sets, d_scores, nullptr, nullptr, 0);
+            if (rc) return rc;
+        }
     }
     {   // algorithmic bytes: n*(k+1) per set (SURVEY.md §8d)
         double bytes = 0;
@@ -2011,7 +2019,7 @@ extern "C" int urlgpu_score_range(urlgpu_ctx *ctx, int variable, const uint64_t 
     rc = make_rank_space(ctx, (int)cand.size(), std::max(0, max_parents), rs);
     if (rc) return rc;
     const uint64_t total = rs.layer_base[rs.K + 1];
-    if (first + count > total) return ctx->fail(URLGPU_ERR_ARG, "score_range: the range exceeds the family (" + std::to_string(total) + " sets)");
+    if (first > total || count > total - first) return ctx->fail(URLGPU_ERR_ARG, "score_range: the range exceeds the family (" + std::to_string(total) + " sets)");
     if (count == 0) return URLGPU_OK;
     cudaStream_t s = ctx->stream;
     DevBuf tmp(ctx);
@@ -2330,7 +2338,7 @@ extern "C" int urlgpu_result_fetch(urlgpu_result *res, uint64_t offset, uint64_t
     CK(cudaSetDevice(ctx->device));
     int rc = result_wait_counts(res);
     if (rc) return rc;
-    if (offset + n > res->n_stored) return ctx->fail(URLGPU_ERR_ARG, "result_fetch: range exceeds the stored count");
+    if (offset > res->n_stored || n > res->n_stored - offset) return ctx->fail(URLGPU_ERR_ARG, "result_fetch: range exceeds the stored count");
     if (n == 0) return URLGPU_OK;
     cudaStream_t cs = ctx->copy_stream; // the compaction has completed (ready event): nothing here waits for later scoring work
     if (masks) {
@@ -2366,7 +2374,7 @@ extern "C" int urlgpu_result_fetch_device(urlgpu_result *res, uint64_t offset, u
     CK(cudaSetDevice(ctx->device));
     int rc = result_wait_counts(res);
     if (rc) return rc;
-    if (offset + n > res->n_stored) return ctx->fail(URLGPU_ERR_ARG, "result_fetch_device: range exceeds the stored count");
+    if (offset > res->n_stored || n > res->n_stored - offset) return ctx->fail(URLGPU_ERR_ARG, "result_fetch_device: range exceeds the stored count");
     if (variable_shift < 0 || mask_words_out < 1) return ctx->fail(URLGPU_ERR_ARG, "result_fetch_device: bad mask width or shift");
     for (int v : res->cand)
         if ((v + variable_shift) / 64 >= mask_words_out) return ctx->fail(URLGPU_ERR_ARG, "result_fetch_device: mask_words_out is too small for the shifted variables");
