@@ -216,22 +216,23 @@ int urlgpu_spg_free(urlgpu_spg *spg);
  * addition, is not +inf; cost(S) is the least such g and the leaf the smallest v attaining it.  *cost is therefore the least
  * float32 left-to-right path sum over the admissible orders: never above A*'s goal cost, and equal to it in exact
  * arithmetic.  Among orders of equal cost the DAG may differ from A*'s.
- * Device memory: 5*2^|C| bytes (cost + leaf per node) plus 4*2^c_v per variable (c_v = its candidate parents inside C)
- * plus the entries, from the context's caching allocator.  Refusals, all before any launch: p < 1, mask_words outside 1..4,
- * decreasing offsets, an empty component or one naming a variable >= p, a NaN score and an entry containing its own
+ * Costs are kept for two adjacent layers only, indexed by colex rank inside the layer, and a leaf byte for every node.
+ * Device memory, from the context's caching allocator: 2^|C| + 8*C(|C|, floor(|C|/2)) bytes for the nodes, 4*2^c_v per
+ * variable for the best-parent tables (c_v = its candidate parents inside C), 16 per qualifying entry, and
+ * 1328*|C| + 10960 bytes of descriptors, look-up tables, binomials and output.  (Before this layout the nodes took
+ * 5*2^|C| bytes, so some calls once refused for memory now run; sweeps of 24 or more variables are faster, 1.4-2.1x from
+ * 28 up, and smaller ones take about 4 us more per layer.)  Refusals, all before any launch: p < 1, mask_words outside
+ * 1..4, decreasing offsets, an empty component or one naming a variable >= p, a NaN score and an entry containing its own
  * variable (URLGPU_ERR_ARG); |C| > 32 and a call that does not fit the device's free memory (URLGPU_ERR_LIMIT, with the
- * bytes).  No admissible order, or a cost of +inf: URLGPU_ERR_ARG with A*'s message "No solution found.". */
+ * bytes split into leaves, cost layers and best-parent tables).  No admissible order, or a cost of +inf: URLGPU_ERR_ARG
+ * with A*'s message "No solution found.". */
 int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
                         const float *scores, const uint64_t *edges, const uint64_t *component,
                         float *cost, int32_t *order, uint64_t *parents);
 
-/* urlgpu_order_search for components of 1..36 variables: the same arguments, contract and outputs, and the same bits
- * wherever both run.  Costs are kept for two adjacent layers only, indexed by colex rank inside the layer, and a leaf byte
- * for every node.  Device memory: 2^|C| + 8*C(|C|, floor(|C|/2)) bytes for the nodes, 4*2^c_v per variable for the
- * best-parent tables, 16 per qualifying entry, and 1328*|C| + 10960 bytes of descriptors, look-up tables,
- * binomials and output.  Refusals: every URLGPU_ERR_ARG refusal of urlgpu_order_search, with the same messages; |C| > 36
- * and a call that does not fit the device's free memory (URLGPU_ERR_LIMIT, with the bytes split into leaves, cost layers
- * and best-parent tables); no admissible order or a cost of +inf: URLGPU_ERR_ARG, "No solution found.". */
+/* urlgpu_order_search with a limit of 36 variables (|C| > 36: URLGPU_ERR_LIMIT) and its messages prefixed
+ * "order_search_layered: " instead of "order_search: ".  Arguments, contract, device memory and outputs are
+ * urlgpu_order_search's: both run the same search and give the same bits wherever both run. */
 int urlgpu_order_search_layered(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
                                 const float *scores, const uint64_t *edges, const uint64_t *component,
                                 float *cost, int32_t *order, uint64_t *parents);

@@ -110,12 +110,12 @@ def closed_form(k):
     return np.float32(7 + 3 + 2 * (k - 2))
 
 
-# ------------------------------------------------------------------------------------------------ same bits as the dense form
+# ------------------------------------------------------------------------------------------------ same bits as urlgpu_order_search
 @pytest.mark.parametrize("k", [1, 2, 5, 9, 12, 14, 20, 24])
 @pytest.mark.parametrize("skeleton", [False, True])
 def test_bit_equal_to_dense_form(engine, k, skeleton):
-    """tie-heavy random caches with entries reaching outside the component: cost, order and parents of the layered form
-    equal the dense form's bit for bit, and the numpy restatement's where k <= 14"""
+    """tie-heavy random caches with entries reaching outside the component: cost, order and parents of
+    urlgpu_order_search_layered equal urlgpu_order_search's bit for bit, and the numpy restatement's where k <= 14"""
     rng = np.random.default_rng(7000 + 100 * k + skeleton)
     values = np.array([0.1, 0.7, 1.3, 2.0, 2.5, 3.0], dtype=np.float32)
     for _ in range(4 if k <= 14 else 2):
@@ -244,8 +244,8 @@ def test_discrete_bn_against_astar(pkg, engine, S, tmp_path, p, skeleton, seed):
 
 
 def test_components_reach_their_own_form(pkg, engine, S, tmp_path):
-    """one 34-variable component and three small ones in one skeleton: the large one through the layered form, the small
-    ones through the dense form, each once per search; the result agrees with A*"""
+    """one 34-variable component and three small ones in one skeleton: the large one through urlgpu_order_search_layered,
+    the small ones through urlgpu_order_search, each once per search; the result agrees with A*"""
     parts = [pkg.datagen.discrete_bn(p=n, n=4000, seed=s, window=3, max_indegree=2) for n, s in ((34, 1), (5, 3), (4, 4), (3, 5))]
     codes = np.concatenate([c for c, _, _, _ in parts])
     card = np.concatenate([k for _, k, _, _ in parts])

@@ -42,11 +42,8 @@ def free_memory():
 
 
 def device_bytes(form, k, cand_bits, n_ent):
-    """what the call asks for (include/urlgpu.h); the entries are the ones inside the component"""
-    tables = sum(4 << c for c in cand_bits)
-    if form == DENSE:
-        return 5 * 2 ** k + tables + 16 * n_ent + k * 24 + k * 1024 + 33 * 33 * 4 + (2 + 2 * k) * 4
-    return 2 ** k + 8 * math.comb(k, k // 2) + tables + 16 * n_ent + 1328 * k + 10960
+    """what the call asks for (include/urlgpu.h), the same for both entry points; the entries are the ones inside the component"""
+    return 2 ** k + 8 * math.comb(k, k // 2) + sum(4 << c for c in cand_bits) + 16 * n_ent + 1328 * k + 10960
 
 
 def timed(eng, form, entries, k, comp, nb):

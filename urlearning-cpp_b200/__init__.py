@@ -506,8 +506,7 @@ class Engine:
 
     def order_search(self, entries, p: int, component: int, edges: Sequence[int] | None = None):
         """urlgpu_order_search: the optimal DAG of one skeleton component over the order graph, layer by layer on the device.
-        Components of more than 32 variables go to urlgpu_order_search_layered, which keeps two cost layers instead of
-        every node's cost and takes up to 36 (same contract, same bits where both run).
+        Components of more than 32 variables go to urlgpu_order_search_layered, the same search with a limit of 36.
         entries: p pairs (masks, scores) per variable in the search side's sign (lower is better), masks uint64 [n] or
         [n, words] or ints; component: a variable mask; edges: p skeleton masks or None.
         -> (float32 cost, order list (first = a root), parents uint64 [p] ([p, words] above 64 variables; 0 outside C))"""
@@ -515,7 +514,7 @@ class Engine:
         return self._order_search("urlgpu_order_search" if k <= 32 else "urlgpu_order_search_layered", entries, p, component, edges)
 
     def _order_search(self, symbol: str, entries, p: int, component: int, edges: Sequence[int] | None):
-        """order_search through the named entry point (measurements compare the two forms at k <= 32)"""
+        """order_search through the named entry point, urlgpu_order_search or urlgpu_order_search_layered"""
         words, offsets, masks, scores, comp, ed = self._order_args(entries, p, component, edges)
         cost = C.c_float()
         order = np.zeros(max(1, bin(int(component)).count("1")), dtype=np.int32)

@@ -384,7 +384,7 @@ extern "C" int urlgpu_create(urlgpu_ctx **out, int device_id) {
         attrs.push_back({(const void *)bic_count_smem_kernel<ListSets>, big});
         attrs.push_back({(const void *)cbic_sets_kernel, big});
         attrs.push_back({(const void *)gram_partial_kernel, (int)kGramSmemBytes});
-        attrs.push_back({(const void *)order_layer_rank_kernel, (int)order_rank_smem_bytes(kOrderRankMaxVars)});
+        attrs.push_back({(const void *)order_layer_kernel, (int)order_smem_bytes(kOrderMaxVars)});
         attrs.push_back({(const void *)order_climb_kernel<ClimbTable>, (int)order_climb_smem_bytes(kClimbMaxVars)});
         attrs.push_back({(const void *)order_climb_kernel<ClimbList>, (int)order_climb_smem_bytes(kClimbMaxVars)});
         for (const auto &a : attrs)
@@ -2574,14 +2574,16 @@ extern "C" int urlgpu_spg_free(urlgpu_spg *sp) {
 // ============================================================================================ order-graph search
 // urlgpu_order_search, urlgpu_order_search_layered, urlgpu_order_local_search and urlgpu_order_local_search_sparse
 // (order_kernels.cuh).  order_prepare validates everything on the host, keeps the component's qualifying entries, sorts each
-// variable's list in the (score, |S|, mask) order of SortedEntries::build and lays out the best-parent tables, compacting each
-// entry straight from its variable-space mask onto cand_v's bits; the sparse form has no tables and gets each entry's parent set
-// over C's positions instead.  order_tables uploads the entries and builds the tables.  Each entry point sizes its call before
-// any allocation; the host maps each chosen sorted position back to its parent mask.
+// variable's list in the (score, |S|, mask) order of SortedEntries::build, translates the skeleton onto C's positions and lays
+// out the best-parent tables, compacting each entry straight from its variable-space mask onto cand_v's bits; the sparse form
+// has no tables and gets each entry's parent set over C's positions instead.  order_tables uploads the entries and builds the
+// tables.  Each entry point sizes its call before any allocation (order_fits); order_write maps each chosen sorted position
+// back to its parent mask.
 struct OrderPrep {
     std::vector<int> vars;                       // position j of C -> variable
     std::vector<std::vector<uint64_t>> ent;      // per position: indices into masks/scores, sorted
     std::vector<std::vector<int>> cand;          // per position: cand_j as positions in C, ascending
+    std::vector<unsigned long long> adj;         // per position: kClimbWords words, its skeleton neighbours over C (all of C without one)
     std::vector<uint64_t> table;                 // per position: offset of T_j (uint32 elements), 2^c_j of them
     std::vector<uint32_t> score;                 // per position: offset of j's sorted entries
     std::vector<unsigned long long> where;       // per sorted entry: its slot in the tables
@@ -2596,7 +2598,7 @@ struct OrderPrep {
 // variables and variables with more than max_cand candidate parents inside the component are refused.  sparse: no table
 // layout (2^c_v would overflow past 63 candidates), the entries' words over C instead
 static int order_prepare(urlgpu_ctx *ctx, const std::string &who, int max_k, int max_cand, bool sparse, int p, int mask_words, const uint64_t *offsets,
-                         const uint64_t *masks, const float *scores, const uint64_t *component, OrderPrep &P) {
+                         const uint64_t *masks, const float *scores, const uint64_t *edges, const uint64_t *component, OrderPrep &P) {
     auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, who + m); };
     if (p < 1) return refuse(URLGPU_ERR_ARG, "p must be at least 1");
     if (mask_words < 1 || mask_words > kSpgMaxWords) return refuse(URLGPU_ERR_ARG, "mask_words must be in 1.." + std::to_string(kSpgMaxWords));
@@ -2621,6 +2623,10 @@ static int order_prepare(urlgpu_ctx *ctx, const std::string &who, int max_k, int
         }
     const int k = (int)P.vars.size();
     if (k > max_k) return refuse(URLGPU_ERR_LIMIT, std::to_string(k) + " variables in the component; at most " + std::to_string(max_k) + " are supported");
+    P.adj.assign((size_t)k * kClimbWords, 0);
+    for (int j = 0; j < k; j++)
+        for (int i = 0; i < k; i++)
+            if (!edges || bit(edges + (size_t)P.vars[j] * mask_words, P.vars[i])) P.adj[(size_t)j * kClimbWords + (i >> 6)] |= 1ull << (i & 63);
 
     // qualifying entries (all parents inside C), per-variable sort, cand_j, table layout
     P.ent.assign(k, {});
@@ -2711,108 +2717,98 @@ static int order_tables(urlgpu_ctx *ctx, const OrderPrep &P, void *d_ent, uint32
     return URLGPU_OK;
 }
 
-// the device's free memory plus the allocator's idle blocks
-static int order_free_bytes(urlgpu_ctx *ctx, size_t *free_b) {
+// refuses a call that needs more than the device's free memory plus the allocator's idle blocks; `bytes` says what the need is
+static int order_fits(urlgpu_ctx *ctx, const std::string &who, size_t need, const std::string &bytes) {
     CK(cudaSetDevice(ctx->device));
-    size_t total_b = 0;
-    CK(cudaMemGetInfo(free_b, &total_b));
-    for (auto &b : ctx->pool) if (!b.used) *free_b += b.bytes;      // cached blocks the allocator can hand out or release
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    for (auto &b : ctx->pool) if (!b.used) free_b += b.bytes;      // cached blocks the allocator can hand out or release
+    if (need > free_b) return ctx->fail(URLGPU_ERR_LIMIT, who + "the search needs " + bytes + ", " + std::to_string(free_b) + " are free");
     return URLGPU_OK;
 }
 
-static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
-                             const float *scores, const uint64_t *edges, const uint64_t *component, float *cost, int32_t *order,
-                             uint64_t *parents) {
+// b.alloc(bytes); a failed allocation clears the error and returns false
+static bool order_alloc(DevBuf &b, size_t bytes) {
+    if (b.alloc(bytes) == cudaSuccess) return true;
+    cudaGetLastError();
+    return false;
+}
+
+// step m of the order: the variable at position ord[m] of C with its sorted entry pos[m] (kOrderNone: the empty set)
+template <class Pos>
+static void order_write(const OrderPrep &P, const uint64_t *masks, int mask_words, const Pos *ord, const uint32_t *pos, int32_t *order, uint64_t *parents) {
+    const int k = (int)P.vars.size();
+    for (int m = 0; m < k; m++) {
+        const int j = (int)ord[m], v = P.vars[j];
+        order[m] = v;
+        for (int w = 0; w < mask_words; w++) parents[(size_t)v * mask_words + w] = pos[m] == kOrderNone ? 0 : masks[P.ent[j][pos[m]] * mask_words + w];
+    }
+}
+
+static int order_search_impl(urlgpu_ctx *ctx, const std::string &who, int max_k, int p, int mask_words, const uint64_t *offsets,
+                             const uint64_t *masks, const float *scores, const uint64_t *edges, const uint64_t *component, float *cost,
+                             int32_t *order, uint64_t *parents) {
     if (!ctx) return URLGPU_ERR_ARG;
-    const std::string who = layered ? "order_search_layered: " : "order_search: ";
     auto refuse = [&](int code, const std::string &m) { return ctx->fail(code, who + m); };
     if (!offsets || !component || !cost || !order || !parents) return refuse(URLGPU_ERR_ARG, "null argument");
     OrderPrep P;
-    const int max_k = layered ? kOrderRankMaxVars : kOrderMaxVars;        // c_v < k, so max_k - 1 never refuses a variable
-    if (int rc = order_prepare(ctx, who, max_k, max_k - 1, false, p, mask_words, offsets, masks, scores, component, P)) return rc;
+    // c_v < k, so max_k - 1 never refuses a variable
+    if (int rc = order_prepare(ctx, who, max_k, max_k - 1, false, p, mask_words, offsets, masks, scores, edges, component, P)) return rc;
     const int k = (int)P.vars.size();
     const uint64_t n_ent = P.n_ent, table_elems = P.table_elems;
-    std::vector<OrderVarRank> hv(k);
+    std::vector<OrderVar> hv(k);
     for (int j = 0; j < k; j++) {
         uint64_t cand = 0;
         for (int q : P.cand[j]) cand |= 1ull << q;
         hv[j].table = P.table[j];
         hv[j].score = P.score[j];
         hv[j].cand = cand;
-        hv[j].adj = ~0ull;
-        if (edges) {
-            hv[j].adj = 0;
-            for (int i = 0; i < k; i++) if ((edges[(size_t)P.vars[j] * mask_words + (P.vars[i] >> 6)] >> (P.vars[i] & 63)) & 1) hv[j].adj |= 1ull << i;
-        }
-        for (int b = 0; b < kOrderRankLut; b++) hv[j].shift[b] = (uint8_t)__builtin_popcountll(cand & ((1ull << (8 * b)) - 1));
+        hv[j].adj = P.adj[(size_t)j * kClimbWords];                         // k <= 64: word 0 holds all of C
+        for (int b = 0; b < kOrderLut; b++) hv[j].shift[b] = (uint8_t)__builtin_popcountll(cand & ((1ull << (8 * b)) - 1));
     }
 
-    // binomials: C(b, i) for b, i <= kOrderRankMaxVars (the dense kernels take the uint32 corner b, i <= kOrderMaxVars)
-    std::vector<unsigned long long> binom(kOrderRankBinom * kOrderRankBinom, 0);
-    for (int b = 0; b < kOrderRankBinom; b++)
-        for (int i = 0; i <= b; i++) binom[b * kOrderRankBinom + i] = i == 0 || i == b ? 1ull : binom[(b - 1) * kOrderRankBinom + i - 1] + binom[(b - 1) * kOrderRankBinom + i];
-    std::vector<uint32_t> binom32(kOrderBinom * kOrderBinom);
+    // binomials: C(b, i) for b, i <= kOrderMaxVars
+    std::vector<unsigned long long> binom(kOrderBinom * kOrderBinom, 0);
     for (int b = 0; b < kOrderBinom; b++)
-        for (int i = 0; i < kOrderBinom; i++) binom32[b * kOrderBinom + i] = (uint32_t)binom[b * kOrderRankBinom + i];
+        for (int i = 0; i <= b; i++) binom[b * kOrderBinom + i] = i == 0 || i == b ? 1ull : binom[(b - 1) * kOrderBinom + i - 1] + binom[(b - 1) * kOrderBinom + i];
 
-    // the device memory of the call, before anything is allocated.  Dense: a cost and a leaf for each of the 2^k nodes.
-    // Layered: a leaf for each node and the costs of two layers, each at most C(k, k/2) nodes
-    const int n_lut = layered ? kOrderRankLut : 4;
-    const size_t var_bytes = layered ? sizeof(OrderVarRank) : sizeof(OrderVar);
-    const size_t binom_bytes = layered ? binom.size() * 8 : binom32.size() * 4;
-    const uint64_t nodes = (uint64_t)1 << k, widest = binom[k * kOrderRankBinom + k / 2];
-    const size_t small_bytes = (size_t)k * var_bytes + (size_t)k * n_lut * 256 + binom_bytes + (2 + 2 * (size_t)k) * 4;
-    const uint64_t node_bytes = layered ? nodes + 8 * widest : 5 * nodes;
-    const size_t need = node_bytes + 4 * table_elems + n_ent * (8 + 4 + 4) + small_bytes;
-    size_t free_b = 0;
-    if (int rc = order_free_bytes(ctx, &free_b)) return rc;
-    auto bytes_msg = [&]() {
-        const std::string nodes_part = layered ? std::to_string(nodes) + " for the leaves of the 2^" + std::to_string(k) + " nodes, " +
-                                                     std::to_string(8 * widest) + " for two cost layers of C(" + std::to_string(k) + ", " + std::to_string(k / 2) + ") nodes, "
-                                               : std::to_string(5 * nodes) + " for the 2^" + std::to_string(k) + " nodes, ";
-        return std::to_string(need) + " bytes of device memory (" + nodes_part + std::to_string(4 * table_elems) + " for the best-parent tables)";
-    };
-    if (need > free_b) return refuse(URLGPU_ERR_LIMIT, "the search needs " + bytes_msg() + ", " + std::to_string(free_b) + " are free");
+    // the device memory of the call, before anything is allocated: a leaf for each node and the costs of two layers, each at
+    // most C(k, k/2) nodes
+    const size_t binom_bytes = binom.size() * 8;
+    const uint64_t nodes = (uint64_t)1 << k, widest = binom[k * kOrderBinom + k / 2];
+    const size_t small_bytes = (size_t)k * sizeof(OrderVar) + (size_t)k * kOrderLut * 256 + binom_bytes + (2 + 2 * (size_t)k) * 4;
+    const size_t need = nodes + 8 * widest + 4 * table_elems + n_ent * (8 + 4 + 4) + small_bytes;
+    const std::string bytes = std::to_string(need) + " bytes of device memory (" + std::to_string(nodes) + " for the leaves of the 2^" +
+                              std::to_string(k) + " nodes, " + std::to_string(8 * widest) + " for two cost layers of C(" + std::to_string(k) +
+                              ", " + std::to_string(k / 2) + ") nodes, " + std::to_string(4 * table_elems) + " for the best-parent tables)";
+    if (int rc = order_fits(ctx, who, need, bytes)) return rc;
 
-    // host arrays: descriptors and byte look-up tables
-    std::vector<OrderVar> hv32(layered ? 0 : k);
-    for (int j = 0; j < (int)hv32.size(); j++) {
-        hv32[j].table = hv[j].table;
-        hv32[j].score = hv[j].score;
-        hv32[j].adj = (uint32_t)hv[j].adj;
-        hv32[j].cand = (uint32_t)hv[j].cand;
-        for (int b = 0; b < 4; b++) hv32[j].shift[b] = hv[j].shift[b];
-    }
-    std::vector<uint8_t> lut((size_t)k * n_lut * 256);
+    // host arrays: byte look-up tables
+    std::vector<uint8_t> lut((size_t)k * kOrderLut * 256);
     for (int j = 0; j < k; j++)
-        for (int b = 0; b < n_lut; b++) {
+        for (int b = 0; b < kOrderLut; b++) {
             const uint32_t cb = (uint32_t)(hv[j].cand >> (8 * b)) & 255;
             for (uint32_t x = 0; x < 256; x++) {
                 uint32_t c = 0; int q = 0;
                 for (int i = 0; i < 8; i++) if ((cb >> i) & 1) { if ((x >> i) & 1) c |= 1u << q; q++; }
-                lut[((size_t)j * n_lut + b) * 256 + x] = (uint8_t)c;
+                lut[((size_t)j * kOrderLut + b) * 256 + x] = (uint8_t)c;
             }
         }
 
     cudaStream_t s = ctx->stream;
     DevBuf d_cost(ctx), d_leaf(ctx), d_tab(ctx), d_small(ctx), d_ent(ctx);
-    auto alloc = [&](DevBuf &b, size_t bytes) {
-        const cudaError_t e = b.alloc(bytes);
-        if (e != cudaSuccess) { cudaGetLastError(); return false; }
-        return true;
-    };
     const size_t ent_bytes = std::max<size_t>(16, n_ent * 16);
-    const size_t cost_bytes = layered ? 8 * widest : 4 * nodes;
-    if (!alloc(d_cost, cost_bytes) || !alloc(d_leaf, nodes) || !alloc(d_tab, table_elems * 4) || !alloc(d_small, small_bytes + 64) || !alloc(d_ent, ent_bytes))
-        return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes_msg() + " failed");
+    if (!order_alloc(d_cost, 8 * widest) || !order_alloc(d_leaf, nodes) || !order_alloc(d_tab, table_elems * 4) ||
+        !order_alloc(d_small, small_bytes + 64) || !order_alloc(d_ent, ent_bytes))
+        return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes + " failed");
     // d_small: vars | lut | binom | out
-    char *sm = d_small.as<char>();
-    uint8_t *dl = reinterpret_cast<uint8_t *>(sm + k * var_bytes);
-    char *db = reinterpret_cast<char *>(dl + lut.size());
-    uint32_t *dout = reinterpret_cast<uint32_t *>(db + binom_bytes);
-    CK(cudaMemcpyAsync(sm, layered ? (const void *)hv.data() : (const void *)hv32.data(), k * var_bytes, cudaMemcpyHostToDevice, s));
+    OrderVar *dv = d_small.as<OrderVar>();
+    uint8_t *dl = reinterpret_cast<uint8_t *>(dv + k);
+    unsigned long long *db = reinterpret_cast<unsigned long long *>(dl + lut.size());
+    uint32_t *dout = reinterpret_cast<uint32_t *>(db + binom.size());
+    CK(cudaMemcpyAsync(dv, hv.data(), k * sizeof(OrderVar), cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(dl, lut.data(), lut.size(), cudaMemcpyHostToDevice, s));
-    CK(cudaMemcpyAsync(db, layered ? (const void *)binom.data() : (const void *)binom32.data(), binom_bytes, cudaMemcpyHostToDevice, s));
+    CK(cudaMemcpyAsync(db, binom.data(), binom_bytes, cudaMemcpyHostToDevice, s));
     uint32_t *T = d_tab.as<uint32_t>();
     if (int rc = order_tables(ctx, P, d_ent.p, T)) return rc;
     const float *ds = reinterpret_cast<const float *>(reinterpret_cast<const uint32_t *>(d_ent.as<unsigned long long>() + n_ent) + n_ent);
@@ -2822,35 +2818,19 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
         Region rg(ctx, F_ORDER_LAYERS, (uint64_t)k + 1);
         CK(cudaMemsetAsync(cst, 0, sizeof(float), s));            // cost(empty set) = 0
         int per_sm = 0;
-        if (!layered) {
-            const OrderVar *dv = reinterpret_cast<const OrderVar *>(sm);
-            const uint32_t *db32 = reinterpret_cast<const uint32_t *>(db);
-            const size_t smem = order_smem_bytes(k);
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_layer_kernel, 256, smem));
-            const uint64_t grid_cap = (uint64_t)std::max(1, per_sm) * ctx->sm_count;
-            for (int l = 1; l <= k; l++) {
-                const uint32_t count = binom32[k * kOrderBinom + l];
-                const uint64_t runs = (count + kOrderRun - 1) / kOrderRun;
-                order_layer_kernel<<<(unsigned)std::min<uint64_t>(grid_cap, (runs + 255) / 256), 256, smem, s>>>(dv, dl, db32, T, ds, k, l, count, cst, lf);
-            }
-            order_backtrack_kernel<<<1, 32, 0, s>>>(dv, T, cst, lf, k, dout);
-        } else {
-            const OrderVarRank *dv = reinterpret_cast<const OrderVarRank *>(sm);
-            const unsigned long long *db64 = reinterpret_cast<const unsigned long long *>(db);
-            const size_t smem = order_rank_smem_bytes(k);
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_layer_rank_kernel, 256, smem));
-            const uint64_t grid_cap = (uint64_t)std::max(1, per_sm) * ctx->sm_count;
-            float *layer_cost[2] = {cst, cst + widest};          // layer l is written to layer_cost[l & 1]
-            uint64_t base = 1;                                     // base_l = sum_{m<l} C(k, m)
-            for (int l = 1; l <= k; l++) {
-                const uint64_t count = binom[k * kOrderRankBinom + l];
-                const uint64_t runs = (count + kOrderRun - 1) / kOrderRun;
-                order_layer_rank_kernel<<<(unsigned)std::min<uint64_t>(grid_cap, (runs + 255) / 256), 256, smem, s>>>(
-                    dv, dl, db64, T, ds, k, l, count, base, layer_cost[(l - 1) & 1], layer_cost[l & 1], lf);
-                base += count;
-            }
-            order_backtrack_rank_kernel<<<1, 32, 0, s>>>(dv, db64, T, layer_cost[k & 1], lf, k, dout);
+        const size_t smem = order_smem_bytes(k);
+        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, order_layer_kernel, 256, smem));
+        const uint64_t grid_cap = (uint64_t)std::max(1, per_sm) * ctx->sm_count;
+        float *layer_cost[2] = {cst, cst + widest};              // layer l is written to layer_cost[l & 1]
+        uint64_t base = 1;                                         // base_l = sum_{m<l} C(k, m)
+        for (int l = 1; l <= k; l++) {
+            const uint64_t count = binom[k * kOrderBinom + l];
+            const uint64_t runs = (count + kOrderRun - 1) / kOrderRun;
+            order_layer_kernel<<<(unsigned)std::min<uint64_t>(grid_cap, (runs + 255) / 256), 256, smem, s>>>(
+                dv, dl, db, T, ds, k, l, count, base, layer_cost[(l - 1) & 1], layer_cost[l & 1], lf);
+            base += count;
         }
+        order_backtrack_kernel<<<1, 32, 0, s>>>(dv, db, T, layer_cost[k & 1], lf, k, dout);
         CK(cudaGetLastError());
     }
     std::vector<uint32_t> out(2 + 2 * (size_t)k);
@@ -2860,24 +2840,22 @@ static int order_search_impl(urlgpu_ctx *ctx, bool layered, int p, int mask_word
     memcpy(&c, &out[0], sizeof c);
     if (!out[1] || c == INFINITY) return ctx->fail(URLGPU_ERR_ARG, "No solution found.");   // search_capi.cpp:87
     *cost = c;
-    for (int i = 0; i < k; i++) {
-        const int j = (int)out[2 + i], v = P.vars[j];
-        const uint32_t q = out[2 + k + i];
-        order[i] = v;
-        for (int w = 0; w < mask_words; w++) parents[(size_t)v * mask_words + w] = q == kOrderNone ? 0 : masks[P.ent[j][q] * mask_words + w];
-    }
+    order_write(P, masks, mask_words, &out[2], &out[2 + k], order, parents);
     return URLGPU_OK;
 }
 
+constexpr int kOrderSearchMaxVars = 32;   // the component limit include/urlgpu.h publishes for urlgpu_order_search
+
 extern "C" int urlgpu_order_search(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks, const float *scores,
                                    const uint64_t *edges, const uint64_t *component, float *cost, int32_t *order, uint64_t *parents) {
-    return order_search_impl(ctx, false, p, mask_words, offsets, masks, scores, edges, component, cost, order, parents);
+    return order_search_impl(ctx, "order_search: ", kOrderSearchMaxVars, p, mask_words, offsets, masks, scores, edges, component, cost, order, parents);
 }
 
 extern "C" int urlgpu_order_search_layered(urlgpu_ctx *ctx, int p, int mask_words, const uint64_t *offsets, const uint64_t *masks,
                                            const float *scores, const uint64_t *edges, const uint64_t *component, float *cost,
                                            int32_t *order, uint64_t *parents) {
-    return order_search_impl(ctx, true, p, mask_words, offsets, masks, scores, edges, component, cost, order, parents);
+    return order_search_impl(ctx, "order_search_layered: ", kOrderMaxVars, p, mask_words, offsets, masks, scores, edges, component, cost, order,
+                             parents);
 }
 
 // Local search: the tables as above (sparse: the entries' words over C, no tables), then one order_climb_kernel launch over all
@@ -2894,7 +2872,7 @@ static int order_local_search_impl(urlgpu_ctx *ctx, bool sparse, int p, int mask
     if (restarts < 1 || restarts > (1u << 20)) return refuse(URLGPU_ERR_ARG, "restarts must be in 1..2^20");
     OrderPrep P;
     if (int rc = order_prepare(ctx, who, kClimbMaxVars, sparse ? kClimbMaxVars - 1 : kClimbMaxCand, sparse, p, mask_words, offsets, masks, scores,
-                               component, P))
+                               edges, component, P))
         return rc;
     const int k = (int)P.vars.size();
     std::vector<OrderClimbVar> hv(k);
@@ -2909,8 +2887,7 @@ static int order_local_search_impl(urlgpu_ctx *ctx, bool sparse, int p, int mask
             V.table = P.table[j];
             for (size_t q = 0; q < P.cand[j].size(); q++) V.cand[q] = (uint8_t)P.cand[j][q];
         }
-        for (int i = 0; i < k; i++)
-            if (!edges || ((edges[(size_t)P.vars[j] * mask_words + (P.vars[i] >> 6)] >> (P.vars[i] & 63)) & 1)) V.adj[i >> 6] |= 1ull << (i & 63);
+        for (int w = 0; w < kClimbWords; w++) V.adj[w] = P.adj[(size_t)j * kClimbWords + w];
     }
 
     // the device memory of the call: tables, entries (table form: where | position | score, sparse: W words | score), and per
@@ -2919,25 +2896,16 @@ static int order_local_search_impl(urlgpu_ctx *ctx, bool sparse, int p, int mask
     const uint64_t restart_bytes = (uint64_t)restarts * (8 + 5 * (uint64_t)k);
     const size_t var_bytes = (size_t)k * sizeof(OrderClimbVar);
     const size_t need = table_bytes + ent_bytes + restart_bytes + var_bytes;
-    size_t free_b = 0;
-    if (int rc = order_free_bytes(ctx, &free_b)) return rc;
-    auto bytes_msg = [&]() {
-        return std::to_string(need) + " bytes of device memory (" + (sparse ? "" : std::to_string(table_bytes) + " for the best-parent tables, ") +
-               std::to_string(ent_bytes) + " for the entries, " + std::to_string(restart_bytes) + " for the state of " +
-               std::to_string(restarts) + " restarts)";
-    };
-    if (need > free_b) return refuse(URLGPU_ERR_LIMIT, "the search needs " + bytes_msg() + ", " + std::to_string(free_b) + " are free");
+    const std::string bytes = std::to_string(need) + " bytes of device memory (" + (sparse ? "" : std::to_string(table_bytes) + " for the best-parent tables, ") +
+                              std::to_string(ent_bytes) + " for the entries, " + std::to_string(restart_bytes) + " for the state of " +
+                              std::to_string(restarts) + " restarts)";
+    if (int rc = order_fits(ctx, who, need, bytes)) return rc;
 
     cudaStream_t s = ctx->stream;
     DevBuf d_tab(ctx), d_ent(ctx), d_var(ctx), d_res(ctx);
-    auto alloc = [&](DevBuf &b, size_t bytes) {
-        const cudaError_t e = b.alloc(bytes);
-        if (e != cudaSuccess) { cudaGetLastError(); return false; }
-        return true;
-    };
-    if ((!sparse && !alloc(d_tab, table_bytes)) || !alloc(d_ent, std::max<uint64_t>(16, ent_bytes)) || !alloc(d_var, var_bytes) ||
-        !alloc(d_res, restart_bytes))
-        return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes_msg() + " failed");
+    if ((!sparse && !order_alloc(d_tab, table_bytes)) || !order_alloc(d_ent, std::max<uint64_t>(16, ent_bytes)) || !order_alloc(d_var, var_bytes) ||
+        !order_alloc(d_res, restart_bytes))
+        return refuse(URLGPU_ERR_LIMIT, "allocating " + bytes + " failed");
     // d_res: cost | moves | positions | order
     float *r_cost = d_res.as<float>();
     uint32_t *r_moves = reinterpret_cast<uint32_t *>(r_cost + restarts);
@@ -2988,11 +2956,7 @@ static int order_local_search_impl(urlgpu_ctx *ctx, bool sparse, int p, int mask
     CK(cudaMemcpyAsync(pos.data(), r_pos + (size_t)best * k, (size_t)k * 4, cudaMemcpyDeviceToHost, s));
     CK(cudaStreamSynchronize(s));
     *cost = rc_h[best];
-    for (int m = 0; m < k; m++) {
-        const int j = ord[m], v = P.vars[j];
-        order[m] = v;
-        for (int w = 0; w < mask_words; w++) parents[(size_t)v * mask_words + w] = pos[m] == kOrderNone ? 0 : masks[P.ent[j][pos[m]] * mask_words + w];
-    }
+    order_write(P, masks, mask_words, ord.data(), pos.data(), order, parents);
     if (restart_costs) memcpy(restart_costs, rc_h.data(), (size_t)restarts * 4);
     if (restart_moves) memcpy(restart_moves, rm_h.data(), (size_t)restarts * 4);
     return URLGPU_OK;
