@@ -338,33 +338,42 @@ __global__ void bic_store_rule_kernel(float *__restrict__ scores, uint64_t n_mas
 // ---------------------------------------------------------------------------------------------------------
 struct CubePair {
     uint64_t parent_off, child_off;   // int32 elements
-    uint32_t groups;                  // child configurations / r0
+    uint32_t groups;                  // child configurations / (g0 * g1)
     uint32_t Bc;                      // stride of the dropped digit, in configurations
     uint32_t r;                       // arity of the dropped digit
     uint32_t chunk0;                  // first block of this pair
-    uint32_t acc_index;               // accumulator of the child
-    uint32_t leaf_acc;                // accumulator of the child's leaf (the child without cube bit 0), scored from the same counts
-    uint32_t r0;                      // configurations per group: the arity of cube bit 0 when the child holds it, else 1
-    uint32_t flags;                   // kCubeStore | kCubeScoreChild | kCubeScoreLeaf
+    uint32_t acc[4];                  // accumulators of the child T, T \ {0}, T \ {1} and T \ {0,1} (see "GROUPS")
+    uint32_t g0, g1;                  // a group is g0 * g1 configurations: the arities of cube bits 0 and 1 that T holds, else 1
+    uint32_t flags;                   // kCubeStore | kCubeScore*
     uint32_t fmt;                     // bit 0: the parent table holds uint16 cells, bit 1: the child table does (see "16-bit tables")
     uint32_t magic;                   // floor((2^32 - 1) / Bc): fast_div instead of a hardware division per group
 };
-constexpr uint32_t kCubeStore = 1;      // the child has children of its own (it holds cube bit 0): its table is written
-constexpr uint32_t kCubeScoreChild = 2; // the child is a set of the family (layer <= K)
-constexpr uint32_t kCubeScoreLeaf = 4;  // the child's leaf is scored here; it gets no pair of its own
+constexpr uint32_t kCubeStore = 1;        // a later pass reads T's table: it is written
+constexpr uint32_t kCubeScoreChild = 2;   // score T (a set of the family: layer <= K); acc[s] is scored iff flags & (2 << s)
+constexpr uint32_t kCubeScoreLeaf = 4;    // score T \ {0} from the group's sums over digit 0
+constexpr uint32_t kCubeScoreDrop1 = 8;   // score T \ {1} from the sums over digit 1
+constexpr uint32_t kCubeScoreDrop01 = 16; // score T \ {0,1} from the sums over both
 
-// A LEAF is a set without cube bit 0: nothing is derived from it, and its parent is the set plus bit 0.  Digit 0 is the lowest
-// digit of a configuration index, so the r0 = card[bit 0] consecutive configurations g*r0 + a of a set T that holds bit 0 sum
-// to configuration g of its leaf T \ {0}.  A thread that derives T in whole groups of r0 configurations therefore has the
-// leaf's counts in registers: the leaf is scored there, without reading T again and without blocks of its own.  The dropped
-// digit z >= 1 of such a T has a stride Bc that is a multiple of r0, so a group is contiguous in the parent as well.
+// GROUPS.  A set T derived in a pass has children T \ {b} for the b below run(T), the number of trailing cube bits T holds.
+// Digits 0 and 1 are the two lowest digits of a configuration index, so the g0 * g1 consecutive configurations
+// a0 + g0 * (a1 + g1 * h) of T (g0, g1 = arities of bits 0 and 1) sum over a0 to configuration a1 + g1 * h of T \ {0}, over a1
+// to configuration a0 + g0 * h of T \ {1}, and over both to configuration h of T \ {0,1}.  A thread that derives T in such
+// groups holds the counts of all four sets in registers and scores them there.  So T \ {1} (run 1: its only child is
+// T \ {0,1}) needs no pass of its own, and only tables of sets with run >= 3 are written.  The dropped digit z >= 2 of such a
+// T has a stride Bc that is a multiple of g0 * g1, so a group is contiguous in the parent as well.  Where the parent's pass
+// built no two-digit groups, pairs keep the shape (card[0], 1) for a T without bit 1 (scoring T and T \ {0}) and (1, 1) for a
+// T without bit 0: the children root \ {1} and root \ {0} of a root table written by a kernel that builds no groups, and
+// the children T \ {1} of a fused root's children T (bic_root_kernel scores T and T \ {0} in groups of card[0]).
 
 constexpr int kCubeThreads = 256;
 #ifndef URLGPU_CUBE_UNROLL
 #define URLGPU_CUBE_UNROLL 2
 #endif
 constexpr int kCubeUnroll = URLGPU_CUBE_UNROLL;
-constexpr uint32_t kCubeConfigsPerBlock = 4096;
+// configurations per block: a block ends with four block-wide sums (T and its three marginals), so a block does enough
+// groups to amortise them.  On one B200 (1000 W) the derive kernel took 88.8 ms per configs[3] step at 16384, 95.1 at
+// 4096, 91.3 at 32768 (DESIGN §5)
+constexpr uint32_t kCubeConfigsPerBlock = 16384;
 
 // N consecutive cells.  p is aligned to N cells as far as the table allows (tables start 16-byte aligned and a run of N cells
 // starts at a multiple of N): the widest vector access that divides N.
@@ -457,15 +466,128 @@ __device__ __forceinline__ void score_cfg(long long &acc, const int (&cnt)[N], i
         acc -= __ldg(&qcfg[nij]);
     }
 }
-// the leaf's counts of a group: its G configurations summed cell by cell
-template <int RV, int G>
-__device__ __forceinline__ void sum_group(const int (&cnt)[G * RV], int (&leaf)[RV]) {
+// scores of a compile-time group of G0 * G1 configurations of T held in registers (see "GROUPS"): T, T \ {0}, T \ {1}, T \ {0,1}
+// add(q, v) adds v to the sum of set q (0: T, 1: T \ {0}, 2: T \ {1}, 3: T \ {0,1})
+template <int RV, int G0, int G1, typename AddFn>
+__device__ __forceinline__ void score_group(const int (&cnt)[G0 * G1 * RV], uint32_t flags, AddFn add, const long long *__restrict__ qlog,
+                                            const long long *__restrict__ qcfg, int cfg_min) {
+    // a dimension of 1 (a unary cube digit) sums one configuration: the marginal is T itself, as the flags may still ask
+    if (flags & kCubeScoreChild) {
+        long long v = 0;
 #pragma unroll
-    for (int k = 0; k < RV; k++) {
-        leaf[k] = cnt[k];
-#pragma unroll
-        for (int m = 1; m < G; m++) leaf[k] += cnt[m * RV + k];
+        for (int m = 0; m < G0 * G1; m++) score_cfg<RV>(v, cnt, m * RV, qlog, qcfg, cfg_min);
+        add(0, v);
     }
+    if (flags & kCubeScoreLeaf) {
+        long long v = 0;
+#pragma unroll
+        for (int a1 = 0; a1 < G1; a1++) {
+            int s[RV];
+#pragma unroll
+            for (int k = 0; k < RV; k++) {
+                s[k] = cnt[G0 * a1 * RV + k];
+#pragma unroll
+                for (int a0 = 1; a0 < G0; a0++) s[k] += cnt[(a0 + G0 * a1) * RV + k];
+            }
+            score_cfg<RV>(v, s, 0, qlog, qcfg, cfg_min);
+        }
+        add(1, v);
+    }
+    if (flags & kCubeScoreDrop1) {
+        long long v = 0;
+#pragma unroll
+        for (int a0 = 0; a0 < G0; a0++) {
+            int s[RV];
+#pragma unroll
+            for (int k = 0; k < RV; k++) {
+                s[k] = cnt[a0 * RV + k];
+#pragma unroll
+                for (int a1 = 1; a1 < G1; a1++) s[k] += cnt[(a0 + G0 * a1) * RV + k];
+            }
+            score_cfg<RV>(v, s, 0, qlog, qcfg, cfg_min);
+        }
+        add(2, v);
+    }
+    if (flags & kCubeScoreDrop01) {
+        int s[RV];
+#pragma unroll
+        for (int k = 0; k < RV; k++) {
+            s[k] = cnt[k];
+#pragma unroll
+            for (int m = 1; m < G0 * G1; m++) s[k] += cnt[m * RV + k];
+        }
+        long long v = 0;
+        score_cfg<RV>(v, s, 0, qlog, qcfg, cfg_min);
+        add(3, v);
+    }
+}
+
+// a group of run-time shape g0 x g1, configuration by configuration: cfg(m, cnt) gives the counts of T's configuration m of
+// the group, put(m, cnt) stores them if T is written.  T \ {0} is summed in registers on the way; T \ {1} and T \ {0,1} sum
+// across the a1 rows, so they read the group's cells again (from L1 or shared memory).
+template <int RV, typename CfgFn, typename PutFn, typename AddFn>
+__device__ __forceinline__ void score_group_any(uint32_t g0, uint32_t g1, CfgFn cfg, PutFn put, uint32_t flags, AddFn add,
+                                                const long long *__restrict__ qlog, const long long *__restrict__ qcfg, int cfg_min) {
+#pragma unroll 1
+    for (uint32_t a1 = 0; a1 < g1; a1++) {
+        int l0[RV] = {};
+#pragma unroll 1
+        for (uint32_t a0 = 0; a0 < g0; a0++) {
+            const uint32_t m = a0 + g0 * a1;
+            int cnt[RV];
+            cfg(m, cnt);
+            put(m, cnt);
+            if (flags & kCubeScoreChild) { long long v = 0; score_cfg<RV>(v, cnt, 0, qlog, qcfg, cfg_min); add(0, v); }
+#pragma unroll
+            for (int k = 0; k < RV; k++) l0[k] += cnt[k];
+        }
+        if (flags & kCubeScoreLeaf) { long long v = 0; score_cfg<RV>(v, l0, 0, qlog, qcfg, cfg_min); add(1, v); }
+    }
+    if (flags & (kCubeScoreDrop1 | kCubeScoreDrop01)) {
+        int l01[RV] = {};
+#pragma unroll 1
+        for (uint32_t a0 = 0; a0 < g0; a0++) {
+            int l1[RV] = {};
+#pragma unroll 1
+            for (uint32_t a1 = 0; a1 < g1; a1++) {
+                int t[RV];
+                cfg(a0 + g0 * a1, t);
+#pragma unroll
+                for (int k = 0; k < RV; k++) l1[k] += t[k];
+            }
+            if (flags & kCubeScoreDrop1) { long long v = 0; score_cfg<RV>(v, l1, 0, qlog, qcfg, cfg_min); add(2, v); }
+#pragma unroll
+            for (int k = 0; k < RV; k++) l01[k] += l1[k];
+        }
+        if (flags & kCubeScoreDrop01) { long long v = 0; score_cfg<RV>(v, l01, 0, qlog, qcfg, cfg_min); add(3, v); }
+    }
+}
+
+// child arity known at run time only: no counts are kept in registers.  Sum over `cell(m, k)` (cell k of T's configuration m
+// of the group) of the no configurations o of a marginal, each the sum of ni configurations o * so + i * si of T, and score them.
+template <typename CellFn>
+__device__ __forceinline__ long long score_marginal(CellFn cell, int rv, uint32_t no, uint32_t so, uint32_t ni, uint32_t si,
+                                                    const long long *__restrict__ qlog, const long long *__restrict__ qcfg, int cfg_min) {
+    long long acc = 0;
+    for (uint32_t o = 0; o < no; o++) {
+        int nij = 0;
+        for (int k = 0; k < rv; k++) {
+            int cnt = 0;
+            for (uint32_t i = 0; i < ni; i++) cnt += cell(o * so + i * si, k);
+            nij += cnt;
+            if (cnt > 1) acc += __ldg(&qlog[cnt]);
+        }
+        if (nij > cfg_min) acc -= __ldg(&qcfg[nij]);
+    }
+    return acc;
+}
+// the three marginals of a run-time group that the flags ask for
+template <typename CellFn, typename AddFn>
+__device__ __forceinline__ void score_marginals(CellFn cell, int rv, uint32_t g0, uint32_t g1, uint32_t flags, AddFn add,
+                                                const long long *__restrict__ qlog, const long long *__restrict__ qcfg, int cfg_min) {
+    if (flags & kCubeScoreLeaf) add(1, score_marginal(cell, rv, g1, g0, g0, 1, qlog, qcfg, cfg_min));
+    if (flags & kCubeScoreDrop1) add(2, score_marginal(cell, rv, g0, 1, g1, g0, qlog, qcfg, cfg_min));
+    if (flags & kCubeScoreDrop01) add(3, score_marginal(cell, rv, 1, 0, g0 * g1, 1, qlog, qcfg, cfg_min));
 }
 
 // block -> pair map (one load per block instead of a dependent binary search by thread 0 while 255 threads wait)
@@ -480,34 +602,40 @@ __global__ void cube_map_kernel(const CubePair *__restrict__ pairs, int npairs, 
     block_pair[i] = (uint32_t)lo;
 }
 
-// RV > 0: compile-time child arity (2,3,4); RV == 0: generic arity rv_dyn.  A block derives kCubeConfigsPerBlock / r0 groups.
+// RV > 0: compile-time child arity (2,3,4); RV == 0: generic arity rv_dyn.  A block derives kCubeConfigsPerBlock / (g0 * g1) groups.
 template <int RV>
 __global__ void __launch_bounds__(kCubeThreads, RV == 4 ? 5 : 6) cube_derive_kernel(const CubePair *__restrict__ pairs, const uint32_t *__restrict__ block_pair, const int *__restrict__ parent_tab,
                                                                    int *__restrict__ child_tab, int rv_dyn, const long long *__restrict__ qlog,
                                                                    const long long *__restrict__ qcfg, int cfg_min, long long *__restrict__ acc_all,
                                                                    int *__restrict__ ovf_flag /*16-bit tables: a count did not fit*/,
                                                                    int qn /*entries of qlog*/) {
-    __shared__ long long red[2][32];
-    __shared__ uint32_t s_acc[2];   // the accumulators, parked until thread 0 needs them (registers are tight for RV = 4)
+    __shared__ long long red[4][32];
+    __shared__ uint32_t s_acc[4];   // the accumulators, parked until thread 0 needs them (registers are tight for RV = 4)
+    __shared__ long long s_sum[3][kCubeThreads];   // this thread's sums of T \ {0}, T \ {1}, T \ {0,1}: registers hold T's alone
     (void)qn;
     const CubePair pr = pairs[__ldg(&block_pair[blockIdx.x])];
-    if (threadIdx.x == 0) { s_acc[0] = pr.acc_index; s_acc[1] = pr.leaf_acc; }
+    if (threadIdx.x < 4) s_acc[threadIdx.x] = pr.acc[threadIdx.x];
     const int rv = RV > 0 ? RV : rv_dyn;
-    const uint32_t r0 = pr.r0, gpb = kCubeConfigsPerBlock / r0;
+    const uint32_t G = pr.g0 * pr.g1, gpb = max(1u, kCubeConfigsPerBlock / G);
     const uint32_t g0 = (blockIdx.x - pr.chunk0) * gpb;
     const uint32_t g1 = min(g0 + gpb, pr.groups);
-    const bool store = pr.flags & kCubeStore, score_child = pr.flags & kCubeScoreChild, score_leaf = pr.flags & kCubeScoreLeaf;
+    const uint32_t flags = pr.flags;
+    const bool store = flags & kCubeStore;
     const int *__restrict__ P = parent_tab + pr.parent_off;
     int *__restrict__ Cc = child_tab + pr.child_off;
-    long long acc = 0, lacc = 0;   // child, leaf
+    long long acc = 0;   // T
+#pragma unroll
+    for (int q = 0; q < 3; q++) s_sum[q][threadIdx.x] = 0;
+    auto add = [&](int q, long long v) { if (q == 0) acc += v; else s_sum[q - 1][threadIdx.x] += v; };
     if constexpr (RV > 0) {
         // configuration indices fit 32 bits (a table has at most 2^30 cells): one IMAD + one IMAD.WIDE per address.  Arity 4 keeps
         // 64-bit indices: ptxas allocates 44 registers for that form and 58 (or spills) for the 32-bit one
         using idx_t = std::conditional_t<RV == 4, uint64_t, uint32_t>;
-        // G (compile time) configurations per group, U groups per thread and iteration: r * G * U configurations' loads in flight.
-        // P16 / C16 (compile time per instantiation, uniform per block): parent / child table in uint16 cells
-        auto run = [&](auto GC, auto P16c, auto C16c) {
-            constexpr int G = decltype(GC)::value, N = G * RV, U = G == 1 ? kCubeUnroll : 1;
+        // G0 x G1 (compile time) configurations per group, U groups per thread and iteration: r * G0 * G1 * U configurations' loads
+        // in flight.  P16 / C16 (compile time per instantiation, uniform per block): parent / child table in uint16 cells
+        auto run = [&](auto G0c, auto G1c, auto P16c, auto C16c) {
+            constexpr int G0 = decltype(G0c)::value, G1 = decltype(G1c)::value, N = G0 * G1 * RV, U = G0 * G1 == 1 ? kCubeUnroll : 1;
+            constexpr int UA = G0 * G1 == 1 ? 2 : 1;   // loads of the dropped digit in flight: one group of N cells for a group > 1
             constexpr bool P16 = decltype(P16c)::value, C16 = decltype(C16c)::value;
             const uint16_t *__restrict__ Ph = reinterpret_cast<const uint16_t *>(P);
             uint16_t *__restrict__ Ch = reinterpret_cast<uint16_t *>(Cc);
@@ -522,13 +650,13 @@ __global__ void __launch_bounds__(kCubeThreads, RV == 4 ? 5 : 6) cube_derive_ker
                 for (int u = 0; u < U; u++) {
                     gg[u] = g + u * kCubeThreads;
                     on[u] = gg[u] < g1;
-                    const uint32_t ju = (on[u] ? gg[u] : g) * G;
+                    const uint32_t ju = (on[u] ? gg[u] : g) * (G0 * G1);
                     const uint32_t hi = fast_div(ju, pr.Bc, pr.magic), lo = ju - hi * pr.Bc;
                     pc[u] = (idx_t)lo + (idx_t)hi * pr.r * pr.Bc;
                 }
 #pragma unroll
                 for (int u = 0; u < U; u++) load(pc[u], cnt[u]);
-#pragma unroll 2
+#pragma unroll UA
                 for (uint32_t a = 1; a < pr.r; a++) {
                     int t[U][N];
 #pragma unroll
@@ -544,19 +672,12 @@ __global__ void __launch_bounds__(kCubeThreads, RV == 4 ? 5 : 6) cube_derive_ker
                     if (store) {
                         if constexpr (C16) ovf |= store_cfg16<N>(Ch + (idx_t)gg[u] * (idx_t)N, cnt[u]); else store_cfg<N>(Cc + (idx_t)gg[u] * (idx_t)N, cnt[u]);
                     }
-                    if (score_child)
-#pragma unroll
-                        for (int m = 0; m < G; m++) score_cfg<RV>(acc, cnt[u], m * RV, qlog, qcfg, cfg_min);
-                    if (score_leaf) {
-                        int leaf[RV];
-                        sum_group<RV, G>(cnt[u], leaf);
-                        score_cfg<RV>(lacc, leaf, 0, qlog, qcfg, cfg_min);
-                    }
+                    score_group<RV, G0, G1>(cnt[u], flags, add, qlog, qcfg, cfg_min);
                 }
             }
             if (ovf) *ovf_flag = 1;
         };
-        // r0 >= 3: the group's configurations one after another, each added into the leaf's counts in registers
+        // any other shape: the group's configurations one after another
         auto run_any = [&](auto P16c, auto C16c) {
             constexpr bool P16 = decltype(P16c)::value, C16 = decltype(C16c)::value;
             const uint16_t *__restrict__ Ph = reinterpret_cast<const uint16_t *>(P);
@@ -564,33 +685,32 @@ __global__ void __launch_bounds__(kCubeThreads, RV == 4 ? 5 : 6) cube_derive_ker
             auto load = [&](idx_t pc, int (&v)[RV]) { if constexpr (P16) load_cfg16<RV>(Ph + pc * (idx_t)RV, v); else load_cfg<RV>(P + pc * (idx_t)RV, v); };
             bool ovf = false;
             for (uint32_t g = g0 + threadIdx.x; g < g1; g += kCubeThreads) {
-                const uint32_t jg = g * r0, hi = fast_div(jg, pr.Bc, pr.magic), lo = jg - hi * pr.Bc;
+                const uint32_t jg = g * G, hi = fast_div(jg, pr.Bc, pr.magic), lo = jg - hi * pr.Bc;
                 const idx_t pg = (idx_t)lo + (idx_t)hi * pr.r * pr.Bc;
-                int leaf[RV] = {};
-#pragma unroll 1
-                for (uint32_t m = 0; m < r0; m++) {
-                    int cnt[RV];
+                auto cfg = [&](uint32_t m, int (&cnt)[RV]) {
                     load(pg + m, cnt);
+#pragma unroll 1
                     for (uint32_t a = 1; a < pr.r; a++) {
                         int t[RV];
                         load(pg + m + (idx_t)a * pr.Bc, t);
 #pragma unroll
                         for (int k = 0; k < RV; k++) cnt[k] += t[k];
                     }
-                    if (store) {
-                        if constexpr (C16) ovf |= store_cfg16<RV>(Ch + ((idx_t)jg + m) * (idx_t)RV, cnt); else store_cfg<RV>(Cc + ((idx_t)jg + m) * (idx_t)RV, cnt);
-                    }
-                    if (score_child) score_cfg<RV>(acc, cnt, 0, qlog, qcfg, cfg_min);
-#pragma unroll
-                    for (int k = 0; k < RV; k++) leaf[k] += cnt[k];
-                }
-                if (score_leaf) score_cfg<RV>(lacc, leaf, 0, qlog, qcfg, cfg_min);
+                };
+                auto put = [&](uint32_t m, const int (&cnt)[RV]) {
+                    if (!store) return;
+                    if constexpr (C16) ovf |= store_cfg16<RV>(Ch + ((idx_t)jg + m) * (idx_t)RV, cnt); else store_cfg<RV>(Cc + ((idx_t)jg + m) * (idx_t)RV, cnt);
+                };
+                score_group_any<RV>(pr.g0, pr.g1, cfg, put, flags, add, qlog, qcfg, cfg_min);
             }
             if (ovf) *ovf_flag = 1;
         };
         auto by_group = [&](auto P16c, auto C16c) {
-            if (r0 == 1) run(std::integral_constant<int, 1>{}, P16c, C16c);
-            else if (r0 == 2) run(std::integral_constant<int, 2>{}, P16c, C16c);
+            using I1 = std::integral_constant<int, 1>;
+            using I2 = std::integral_constant<int, 2>;
+            if (pr.g0 == 2 && pr.g1 == 2) run(I2{}, I2{}, P16c, C16c);
+            else if (pr.g0 == 2 && pr.g1 == 1) run(I2{}, I1{}, P16c, C16c);
+            else if (G == 1) run(I1{}, I1{}, P16c, C16c);
             else run_any(P16c, C16c);
         };
         switch (pr.fmt & 3u) {
@@ -602,46 +722,38 @@ __global__ void __launch_bounds__(kCubeThreads, RV == 4 ? 5 : 6) cube_derive_ker
     } else {
         const uint16_t *Ph = reinterpret_cast<const uint16_t *>(P);
         uint16_t *Ch = reinterpret_cast<uint16_t *>(Cc);
-        auto cell = [&](uint64_t i) { return (pr.fmt & 1u) ? (int)Ph[i] : P[i]; };
+        auto at = [&](uint64_t i) { return (pr.fmt & 1u) ? (int)Ph[i] : P[i]; };
         for (uint32_t g = g0 + threadIdx.x; g < g1; g += kCubeThreads) {
-            const uint32_t jg = g * r0, hi = jg / pr.Bc, lo = jg - hi * pr.Bc;
+            const uint32_t jg = g * G, hi = jg / pr.Bc, lo = jg - hi * pr.Bc;
             const uint64_t pg = (uint64_t)lo + (uint64_t)hi * pr.r * pr.Bc;
-            for (uint32_t m = 0; m < r0; m++) {
+            auto cell = [&](uint32_t m, int k) {   // an arity this wide keeps no counts in registers: marginals read the cells again (L1)
+                int cnt = 0;
+                for (uint32_t a = 0; a < pr.r; a++) cnt += at((pg + m + (uint64_t)a * pr.Bc) * rv + k);
+                return cnt;
+            };
+            for (uint32_t m = 0; m < G; m++) {
                 const uint64_t j = (uint64_t)jg + m;
                 int nij = 0;
                 for (int k = 0; k < rv; k++) {
-                    int cnt = 0;
-                    for (uint32_t a = 0; a < pr.r; a++) cnt += cell((pg + m + (uint64_t)a * pr.Bc) * rv + k);
+                    const int cnt = cell(m, k);
                     if (store) {
                         if (pr.fmt & 2u) { Ch[j * rv + k] = (uint16_t)min(cnt, 65535); if (cnt > 65535) *ovf_flag = 1; }
                         else Cc[j * rv + k] = cnt;
                     }
                     nij += cnt;
-                    if (score_child && cnt > 1) acc += __ldg(&qlog[cnt]);
+                    if ((flags & kCubeScoreChild) && cnt > 1) acc += __ldg(&qlog[cnt]);
                 }
-                if (score_child && nij > cfg_min) acc -= __ldg(&qcfg[nij]);
+                if ((flags & kCubeScoreChild) && nij > cfg_min) acc -= __ldg(&qcfg[nij]);
             }
-            if (score_leaf) { // an arity this wide keeps no leaf counts in registers: the group's parent cells are read again (L1)
-                int nl = 0;
-                for (int k = 0; k < rv; k++) {
-                    int cnt = 0;
-                    for (uint32_t m = 0; m < r0; m++)
-                        for (uint32_t a = 0; a < pr.r; a++) cnt += cell((pg + m + (uint64_t)a * pr.Bc) * rv + k);
-                    nl += cnt;
-                    if (cnt > 1) lacc += __ldg(&qlog[cnt]);
-                }
-                if (nl > cfg_min) lacc -= __ldg(&qcfg[nl]);
-            }
+            score_marginals(cell, rv, pr.g0, pr.g1, flags, add, qlog, qcfg, cfg_min);
         }
     }
-    if (score_child) {
-        acc = block_sum_ll(acc, red[0]);
-        if (threadIdx.x == 0 && acc != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_all[s_acc[0]]), (unsigned long long)acc);
-    }
-    if (score_leaf) {
-        lacc = block_sum_ll(lacc, red[1]);
-        if (threadIdx.x == 0 && lacc != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_all[s_acc[1]]), (unsigned long long)lacc);
-    }
+#pragma unroll
+    for (int q = 0; q < 4; q++)
+        if (flags & (kCubeScoreChild << q)) {
+            const long long v = block_sum_ll(q == 0 ? acc : s_sum[q - 1][threadIdx.x], red[q]);
+            if (threadIdx.x == 0 && v != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_all[s_acc[q]]), (unsigned long long)v);
+        }
 }
 
 // scores[res_mask] from the exact accumulators; tVal multiplied in ascending variable order (result-order CandInfo)

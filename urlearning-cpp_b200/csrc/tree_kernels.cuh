@@ -203,26 +203,25 @@ __device__ __forceinline__ void tree_count_fragmented(const unsigned long long *
 // ---------------------------------------------------------------------------------------------------------
 // bic_root_kernel: one CTA per (root, slice) histograms the slice in shared memory from the bucketed packed rows, then
 //   * plain root (nchild == 0): the slice is written to its place in the root's dense global table;
-//   * fused root (nchild == z > 0): the root is only an ancestor (layer K+1), so its table is never written.  The
-//     CTA sums each run digit b < z out of the slice (a block-wide pass: the slice holds the whole run), scores
-//     child b = root \ {b} on the fly and writes the child's slice to ITS global table unless b == 0 (nothing is
-//     derived from a set that lacks bit 0).  This removes the write and the z reads of the largest layer of tables.
-//     For b >= 1 a thread sums whole groups of card[0] consecutive child configurations (pre[b] is a multiple of card[0]),
-//     so it also holds the counts of the child's leaf root \ {b, 0} and scores it (bic_kernels.cuh, "LEAF").
+//   * fused root (nchild == z > 0): the root is only an ancestor (layer K+1 or K+2), so its table is never written.  The
+//     CTA sums each run digit b < z out of the slice (a block-wide pass: the slice holds the whole run) and scores child
+//     T = root \ {b} on the fly.  This removes the write and the z reads of the largest layer of tables.  For b >= 1 a thread
+//     sums whole groups of card[0] consecutive child configurations (pre[b] is a multiple of card[0]), so it also holds the
+//     counts of T \ {0} and scores it (bic_kernels.cuh, "GROUPS").  T is written iff b >= 2: the derive kernel reads it for
+//     T \ {1} (and T \ {0,1}), which stay out of the root kernel, whose two CTAs per SM score less efficiently than the
+//     derive kernel's six; T = root \ {1} has no child left to derive and is not written.  The host sets which sets a pass
+//     scores (CubeRoot::flags): above layer K only sets whose lowest bits are forced belong to the family.
 // ---------------------------------------------------------------------------------------------------------
 constexpr int kRootMaxChild = 16;
 
 struct CubeRoot {
     TreeRoot t;                              // slicing description; t.z = fused run (0 for a plain root)
     unsigned long long table_off;            // plain: the root's table in `tables` (int32 elements)
-    unsigned long long child_off[kRootMaxChild];   // fused: child b's table in `child_tables`
-    uint32_t child_acc[kRootMaxChild];       // and its accumulator
-    uint32_t leaf_acc[kRootMaxChild];        // accumulator of the leaf root \ {b, 0} of child b >= 1
-    uint32_t nchild;                         // fused: children drop bit b, bfirst <= b < nchild (== run length)
-    uint16_t bfirst, score;                  // layers above K only hold sets with their lowest bits forced: the first droppable bit;
-                                             // score bit 0: score the children, bit 1: score the leaves of children b >= 1
+    unsigned long long child_off[kRootMaxChild];   // fused: table of pass b's child root \ {b} in `child_tables` (b >= 2)
+    uint32_t acc[kRootMaxChild][2];          // accumulators of pass b's sets T = root \ {b} and T \ {0}
+    uint32_t nchild;                         // fused: passes b < nchild (== run length)
     uint32_t child16;                        // bit b: child b's table holds uint16 cells (bic_kernels.cuh, "16-bit tables")
-    uint32_t pad16;
+    uint8_t flags[kRootMaxChild];            // pass b: kCubeStore | kCubeScore* (bic_kernels.cuh); 0: no pass b
 };
 
 __global__ void root_map_kernel(const CubeRoot *__restrict__ roots, int nroots, uint32_t total, uint32_t *__restrict__ cta_root) {
@@ -245,7 +244,7 @@ __global__ void __launch_bounds__(NW * 32, 2) bic_root_kernel(TreeVar tv, const 
     extern __shared__ __align__(16) int s_dyn[];              // [table_budget] slice table, then segbeg[seg_cap], segoff[seg_cap + 1]
     __shared__ CubeRoot cr;
     __shared__ uint16_t s_lut[8 * 256];
-    __shared__ unsigned long long s_cacc[2][kRootMaxChild]; // per-child exact sums of this CTA: [0] the child b, [1] its leaf
+    __shared__ unsigned long long s_cacc[kRootMaxChild][2]; // exact sums of this CTA: pass b's T and T \ {0}
     constexpr int kRootThreads = NW * 32;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int rv = RV > 0 ? RV : tv.rv;
@@ -259,7 +258,7 @@ __global__ void __launch_bounds__(NW * 32, 2) bic_root_kernel(TreeVar tv, const 
     const TreeRoot &rt = cr.t;
     const int z = rt.z;
     (void)qn;
-    if (tid < 2 * kRootMaxChild) s_cacc[tid / kRootMaxChild][tid % kRootMaxChild] = 0;
+    if (tid < 2 * kRootMaxChild) s_cacc[tid >> 1][tid & 1] = 0;
     const uint32_t S0 = rt.H * (uint32_t)rv * tv.pre[z];
     const uint32_t si = blockIdx.x - rt.chunk0;
     {
@@ -354,26 +353,27 @@ __global__ void __launch_bounds__(NW * 32, 2) bic_root_kernel(TreeVar tv, const 
         }
         return;
     }
-    // fused root: children b = bfirst .. z-1
+    // fused root: passes b < z (see the kernel's header)
     const uint32_t cfg_src = S0 / (uint32_t)rv;
-    const bool score = cr.score & 1u;
-    for (int b = cr.bfirst; b < z; b++) {
+    for (int b = 0; b < z; b++) {
+        const uint32_t flags = cr.flags[b];
+        if (!flags) continue;
         const uint32_t r = tv.card[b], pre = tv.pre[b], magic = tv.magic[b];
         const uint32_t cfg_dst = fast_div(cfg_src, r, tv.cmagic[b]); // r divides the run product: exact
+        const uint32_t G = b == 0 ? 1u : tv.card[0];   // configurations per group
         const bool c16 = (cr.child16 >> b) & 1u;
         int *dst = child_tables + cr.child_off[b] + (c16 ? 0ull : (unsigned long long)si * ((unsigned long long)cfg_dst * rv));
         uint16_t *dst16 = reinterpret_cast<uint16_t *>(child_tables + cr.child_off[b]) + (unsigned long long)si * ((unsigned long long)cfg_dst * rv);
-        const bool store = b > 0;
-        const bool sleaf = b > 0 && (cr.score & 2u);
-        const uint32_t r0 = b > 0 ? tv.card[0] : 1u;   // configurations per group
+        const bool store = flags & kCubeStore;
         bool ovf = false;
-        long long acc = 0, lacc = 0;
+        long long acc[2] = {0, 0};
+        auto add = [&](int q, long long v) { if (q < 2) acc[q] += v; };   // passes score T and T \ {0} only
         if constexpr (RV > 0) {
-            // R = compile-time arity of the digit summed out (2, 3, 4), 0 = run-time loop; G = compile-time group size
-            auto pass = [&](auto RC, auto GC) {
-                constexpr int R = decltype(RC)::value, G = decltype(GC)::value, N = G * RV;
-                for (uint32_t g = tid; g < cfg_dst / G; g += kRootThreads) {
-                    const uint32_t j = g * G, hi = fast_div(j, pre, magic), lo = j - hi * pre;
+            // R = compile-time arity of the digit summed out (2, 3, 4), 0 = run-time loop; G0 = compile-time group size
+            auto pass = [&](auto RC, auto G0c) {
+                constexpr int R = decltype(RC)::value, G0 = decltype(G0c)::value, N = G0 * RV;
+                for (uint32_t g = tid; g < cfg_dst / G0; g += kRootThreads) {
+                    const uint32_t j = g * G0, hi = fast_div(j, pre, magic), lo = j - hi * pre;
                     const uint32_t p0 = lo + hi * r * pre;
                     int cnt[N];
                     load_cfg<N>(s_dyn + (size_t)p0 * RV, cnt);
@@ -398,25 +398,15 @@ __global__ void __launch_bounds__(NW * 32, 2) bic_root_kernel(TreeVar tv, const 
                         if (c16) ovf |= store_cfg16<N>(dst16 + (size_t)j * RV, cnt);
                         else store_cfg<N>(dst + (size_t)j * RV, cnt);
                     }
-                    if (score)
-#pragma unroll
-                        for (int m = 0; m < G; m++) score_cfg<RV>(acc, cnt, m * RV, qlog, qcfg, cfg_min);
-                    if (sleaf) {
-                        int leaf[RV];
-                        sum_group<RV, G>(cnt, leaf);
-                        score_cfg<RV>(lacc, leaf, 0, qlog, qcfg, cfg_min);
-                    }
+                    score_group<RV, G0, 1>(cnt, flags, add, qlog, qcfg, cfg_min);
                 }
             };
-            // r0 >= 3: the group's configurations one after another, each added into the leaf's counts in registers
+            // any other group shape: the group's configurations one after another
             auto pass_any = [&]() {
-                for (uint32_t g = tid; g < cfg_dst / r0; g += kRootThreads) {
-                    const uint32_t jg = g * r0, hi = fast_div(jg, pre, magic), lo = jg - hi * pre;
+                for (uint32_t g = tid; g < cfg_dst / G; g += kRootThreads) {
+                    const uint32_t jg = g * G, hi = fast_div(jg, pre, magic), lo = jg - hi * pre;
                     const uint32_t pg = lo + hi * r * pre;
-                    int leaf[RV] = {};
-#pragma unroll 1
-                    for (uint32_t m = 0; m < r0; m++) {
-                        int cnt[RV];
+                    auto cfg = [&](uint32_t m, int (&cnt)[RV]) {
                         load_cfg<RV>(s_dyn + (size_t)(pg + m) * RV, cnt);
 #pragma unroll 2
                         for (uint32_t a = 1; a < r; a++) {
@@ -425,78 +415,66 @@ __global__ void __launch_bounds__(NW * 32, 2) bic_root_kernel(TreeVar tv, const 
 #pragma unroll
                             for (int k = 0; k < RV; k++) cnt[k] += t[k];
                         }
-                        if (store) {
-                            if (c16) ovf |= store_cfg16<RV>(dst16 + (size_t)(jg + m) * RV, cnt);
-                            else store_cfg<RV>(dst + (size_t)(jg + m) * RV, cnt);
-                        }
-                        if (score) score_cfg<RV>(acc, cnt, 0, qlog, qcfg, cfg_min);
-#pragma unroll
-                        for (int k = 0; k < RV; k++) leaf[k] += cnt[k];
-                    }
-                    if (sleaf) score_cfg<RV>(lacc, leaf, 0, qlog, qcfg, cfg_min);
+                    };
+                    auto put = [&](uint32_t m, const int (&cnt)[RV]) {
+                        if (!store) return;
+                        if (c16) ovf |= store_cfg16<RV>(dst16 + (size_t)(jg + m) * RV, cnt);
+                        else store_cfg<RV>(dst + (size_t)(jg + m) * RV, cnt);
+                    };
+                    score_group_any<RV>(G, 1u, cfg, put, flags, add, qlog, qcfg, cfg_min);
                 }
             };
-            auto by_arity = [&](auto GC) {
+            auto by_arity = [&](auto G0c) {
                 switch (r) {
-                case 2: pass(std::integral_constant<int, 2>{}, GC); break;
-                case 3: pass(std::integral_constant<int, 3>{}, GC); break;
-                case 4: pass(std::integral_constant<int, 4>{}, GC); break;
-                default: pass(std::integral_constant<int, 0>{}, GC); break;
+                case 2: pass(std::integral_constant<int, 2>{}, G0c); break;
+                case 3: pass(std::integral_constant<int, 3>{}, G0c); break;
+                case 4: pass(std::integral_constant<int, 4>{}, G0c); break;
+                default: pass(std::integral_constant<int, 0>{}, G0c); break;
                 }
             };
-            if (r0 == 1) by_arity(std::integral_constant<int, 1>{});
-            else if (r0 == 2) by_arity(std::integral_constant<int, 2>{});
+            if (G == 1) by_arity(std::integral_constant<int, 1>{});
+            else if (G == 2) by_arity(std::integral_constant<int, 2>{});
             else pass_any();
         } else {
-            for (uint32_t g = tid; g < cfg_dst / r0; g += kRootThreads) {
-                const uint32_t jg = g * r0, hi = fast_div(jg, pre, magic), lo = jg - hi * pre;
+            for (uint32_t g = tid; g < cfg_dst / G; g += kRootThreads) {
+                const uint32_t jg = g * G, hi = fast_div(jg, pre, magic), lo = jg - hi * pre;
                 const uint32_t pg = lo + hi * r * pre;
-                for (uint32_t m = 0; m < r0; m++) {
-                    const uint32_t j = jg + m, p0 = pg + m;
+                auto cell = [&](uint32_t m, int k) {   // marginals sum the group's cells again from shared memory
+                    int cnt = 0;
+                    for (uint32_t a = 0; a < r; a++) cnt += s_dyn[(size_t)(pg + m + a * pre) * rv + k];
+                    return cnt;
+                };
+                for (uint32_t m = 0; m < G; m++) {
+                    const uint32_t j = jg + m;
                     int nij = 0;
                     for (int k = 0; k < rv; k++) {
-                        int cnt = 0;
-                        for (uint32_t a = 0; a < r; a++) cnt += s_dyn[(size_t)(p0 + a * pre) * rv + k];
+                        const int cnt = cell(m, k);
                         if (store) {
                             if (c16) { dst16[(size_t)j * rv + k] = (uint16_t)min(cnt, 65535); ovf |= cnt > 65535; }
                             else dst[(size_t)j * rv + k] = cnt;
                         }
                         nij += cnt;
-                        if (score && cnt > 1) acc += __ldg(&qlog[cnt]);
+                        if ((flags & kCubeScoreChild) && cnt > 1) acc[0] += __ldg(&qlog[cnt]);
                     }
-                    if (score && nij > cfg_min) acc -= __ldg(&qcfg[nij]);
+                    if ((flags & kCubeScoreChild) && nij > cfg_min) acc[0] -= __ldg(&qcfg[nij]);
                 }
-                if (sleaf) { // the leaf's counts: the group's cells summed again from shared memory
-                    int nl = 0;
-                    for (int k = 0; k < rv; k++) {
-                        int cnt = 0;
-                        for (uint32_t m = 0; m < r0; m++)
-                            for (uint32_t a = 0; a < r; a++) cnt += s_dyn[(size_t)(pg + m + a * pre) * rv + k];
-                        nl += cnt;
-                        if (cnt > 1) lacc += __ldg(&qlog[cnt]);
-                    }
-                    if (nl > cfg_min) lacc -= __ldg(&qcfg[nl]);
-                }
+                score_marginals(cell, rv, G, 1u, flags, add, qlog, qcfg, cfg_min);
             }
         }
         if (ovf) *ovf_flag = 1;
-        // no barrier between children: every warp adds its exact partial sums to the child's shared accumulators
-        if (score) {
-            acc = warp_sum_ll_redux(acc);
-            if (lane == 0 && acc != 0) atomicAdd(&s_cacc[0][b], (unsigned long long)acc);
-        }
-        if (sleaf) {
-            lacc = warp_sum_ll_redux(lacc);
-            if (lane == 0 && lacc != 0) atomicAdd(&s_cacc[1][b], (unsigned long long)lacc);
-        }
+        // no barrier between passes: every warp adds its exact partial sums to the pass's shared accumulators
+#pragma unroll
+        for (int q = 0; q < 2; q++)
+            if (flags & (kCubeScoreChild << q)) {
+                const long long v = warp_sum_ll_redux(acc[q]);
+                if (lane == 0 && v != 0) atomicAdd(&s_cacc[b][q], (unsigned long long)v);
+            }
     }
-    if (cr.score) {
-        __syncthreads();
-        if (tid >= (int)cr.bfirst && tid < z) {
-            const unsigned long long a = s_cacc[0][tid], la = s_cacc[1][tid];
-            if (score && a != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_out[cr.child_acc[tid]]), a);
-            if (la != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_out[cr.leaf_acc[tid]]), la);
-        }
+    __syncthreads();
+    if (tid < 2 * z) {
+        const int b = tid >> 1, q = tid & 1;
+        const unsigned long long a = s_cacc[b][q];
+        if ((cr.flags[b] & (kCubeScoreChild << q)) && a != 0) atomicAdd(reinterpret_cast<unsigned long long *>(&acc_out[cr.acc[b][q]]), a);
     }
 }
 

@@ -854,7 +854,8 @@ struct CubeSet {
     uint32_t cube_mask, res_mask;
     uint64_t cells, off;
     int parent;       // index in the layer above
-    int leaf_child;   // a set that holds cube bit 0: index of its leaf child (the set without bit 0) in the layer below, or -1
+    int sub[3];       // indices of the set without cube bit 0, without bit 1 (both in the layer below) and without both (two
+                      // layers below), where the set holds the bits and those sets are enumerated; else -1
     uint32_t Bc, r;
     bool t16;         // the table is stored with uint16 cells
 };
@@ -962,7 +963,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         cs.cells = (uint64_t)std::min<__uint128_t>(cells, kCellLimit + 1);
         cs.res_mask = resT[b0] | resT[256 + b1] | resT[512 + b2] | resT[768 + b3];
         cs.parent = -1;
-        cs.leaf_child = -1;
+        cs.sub[0] = cs.sub[1] = cs.sub[2] = -1;
         return cs;
     };
     for (int l = 0; l <= Lmax; l++) {
@@ -1100,9 +1101,18 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
     }
     // ---- offsets and parent links ----
     // Layer Lstar lives in buffer A, Lstar-1 in B, Lstar-2 in A again, ...: each buffer is sized for its own layers only.
-    // Tables that are never materialised take no room: fused roots, and below the root layer every set without cube
-    // bit 0 (nothing is derived from it, its table is only scored on the fly).
+    // Tables that are never materialised take no room: fused roots, and below the root layer every set that no pass reads.
+    // A derived set T is read by the passes of its children T \ {b}, b >= 2 (bic_kernels.cuh, "GROUPS"), so iff it holds bits
+    // 0 to 2; a child root \ {b} of a fused root also by the pass of its own child without bit 1, so from b = 2 on
+    // (tree_kernels.cuh).
     const bool use16 = ctx->table16 && d_ovf != nullptr;
+    auto fused_parent = [&](uint32_t m) { // the set's parent (the set plus its lowest missing bit) is a fused root
+        const uint32_t pm = m | (1u << __builtin_ctz(~m));
+        auto &R = layers[Lstar];
+        auto it = std::lower_bound(R.begin(), R.end(), pm, [](const CubeSet &a, uint32_t x) { return a.cube_mask < x; });
+        return it != R.end() && it->cube_mask == pm && root_kind[it - R.begin()] == 2;
+    };
+    auto fused_child2 = [&](uint32_t m) { return (m & 7u) == 3u && fused_parent(m); };   // root \ {2} of a fused root
     size_t needA = 0, needB = 0;
     for (int l = 0; l <= Lstar; l++) {
         uint64_t off = 0;
@@ -1111,7 +1121,7 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
             cs.off = off;
             cs.t16 = false;
             if (l == Lstar && root_kind[i] == 2) continue;          // fused root
-            if (l < Lstar && (cs.cube_mask & 1u) == 0) continue;    // leaf
+            if (l < Lstar && (cs.cube_mask & 7u) != 7u && !(l == Lstar - 1 && fused_child2(cs.cube_mask))) continue;   // read by no pass
             cs.t16 = use16 && l < Lstar && l >= ctx->table16_min_layer;   // root tables stay int32 (several kernels write them)
             off += cs.t16 ? ((cs.cells + 1) / 2 + 3) / 4 * 4 : (cs.cells + 3) / 4 * 4;
         }
@@ -1127,10 +1137,17 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
                 cs.parent = (int)(it - P.begin());
                 cs.Bc = (uint32_t)prefix[z];
                 cs.r = (uint32_t)ccard[z];
-                if (z == 0) it->leaf_child = (int)i;   // a leaf: its parent is the set plus bit 0
+                if (z <= 1) it->sub[z] = (int)i;   // the set is its parent without bit 0 or without bit 1
             }
         }
     }
+    for (int l = 0; l + 2 <= Lstar; l++) // a set without bits 0 and 1 is its grandparent (the set plus both) without both
+        for (size_t i = 0; i < layers[l].size(); i++) {
+            if (layers[l][i].cube_mask & 3u) continue;
+            auto &H = layers[l + 2][layers[l + 1][layers[l][i].parent].parent];
+            if (H.cube_mask != (layers[l][i].cube_mask | 3u)) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: grandparent set missing");
+            H.sub[2] = (int)i;
+        }
     for (int l = Lstar - 1; l >= 0; l--) { // a set belongs to the sub-forest of its parent
         mine[l].resize(layers[l].size());
         for (size_t i = 0; i < layers[l].size(); i++) mine[l][i] = mine[l + 1][layers[l][i].parent];
@@ -1180,6 +1197,23 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         Region rg(ctx, F_OTHER, 1);
         cube_finalize_kernel<<<blocks_for(L.size(), 256), 256, 0, s>>>(bd, ci_res, dres.as<uint32_t>(), dacc.as<long long>() + acc_off[l], (int)L.size(), d_table, om);
         return URLGPU_OK;
+    };
+
+    // what a pass that derives T (layer l, index i) in groups scores, and into which accumulators (bic_kernels.cuh, "GROUPS"):
+    // T itself if it is a set of the family; with bit 0 in the group (g0) T \ {0}; with bits 0 and 1 (g1) T \ {1} and T \ {0,1}.
+    // Above layer Kc no set is scored
+    auto pass_scores = [&](const CubeSet &T, int l, size_t i, bool g0, bool g1, uint32_t &flags, uint32_t (&acc)[4]) -> bool {
+        flags = 0;
+        if (l <= Kc) { flags |= kCubeScoreChild; acc[0] = (uint32_t)(acc_off[l] + i); }
+        const int sl[3] = {l - 1, l - 1, l - 2};
+        const bool on[3] = {g0, g1, g1};
+        for (int q = 0; q < 3; q++) {
+            if (!on[q] || sl[q] > Kc) continue;
+            if (T.sub[q] < 0) return false;
+            flags |= kCubeScoreLeaf << q;
+            acc[q + 1] = (uint32_t)(acc_off[sl[q]] + T.sub[q]);
+        }
+        return true;
     };
 
     // ---- roots: counted from the rows ----
@@ -1238,22 +1272,23 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
                     CubeRoot cr{};
                     if (!slice_root(P, kind == 2 ? run : 0, cr.t)) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: root slicing is not reproducible");
                     if (kind == 2) {
+                        // pass b derives root \ {b} in groups of card[0] (tree_kernels.cuh); layers above Kc hold only sets with their
+                        // lowest bits forced: the droppable bits start at bfirst
                         cr.nchild = (uint32_t)run;
-                        cr.bfirst = (uint16_t)std::max(0, Lstar - 1 - Kc);
-                        // children b >= 1 hold bit 0: the root kernel also scores their leaves root \ {b, 0} (layer Lstar - 2 <= Kc)
-                        cr.score = (Lstar - 1 <= Kc ? 1 : 0) | (run > std::max<int>(cr.bfirst, 1) ? 2 : 0);
-                        for (int b = cr.bfirst; b < run; b++) {
+                        for (int b = std::max(0, Lstar - 1 - Kc); b < run; b++) {
                             const uint32_t cm = P & ~(1u << b);
                             auto it = std::lower_bound(Lc.begin(), Lc.end(), cm, [](const CubeSet &a, uint32_t m) { return a.cube_mask < m; });
                             if (it == Lc.end() || it->cube_mask != cm) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: child of a fused root missing");
-                            cr.child_off[b] = it->off;
-                            cr.child_acc[b] = (uint32_t)(acc_off[Lstar - 1] + (it - Lc.begin()));
-                            if (b > 0) {
-                                if (it->leaf_child < 0) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: leaf of a fused root's child missing");
-                                cr.leaf_acc[b] = (uint32_t)(acc_off[Lstar - 2] + it->leaf_child);
+                            uint32_t fl = 0, acc4[4] = {0, 0, 0, 0};
+                            if (!pass_scores(*it, Lstar - 1, (size_t)(it - Lc.begin()), b > 0, false, fl, acc4)) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: a set scored by a fused root's pass is missing");
+                            cr.acc[b][0] = acc4[0]; cr.acc[b][1] = acc4[1];
+                            if (b >= 2) { // read by the derive passes of its children
+                                fl |= kCubeStore;
+                                cr.child_off[b] = it->off;
+                                if (it->t16) cr.child16 |= 1u << b;
+                                ctx->st.k1_bytes_written += (it->t16 ? 2.0 : 4.0) * (double)it->cells;
                             }
-                            if (it->t16) cr.child16 |= 1u << b;
-                            if (b > 0) ctx->st.k1_bytes_written += (it->t16 ? 2.0 : 4.0) * (double)it->cells; // only children that have children of their own are stored
+                            cr.flags[b] = (uint8_t)fl;
                         }
                         fused_root[big_idx[i]] = 1;
                     } else cr.table_off = big[i].table_off;
@@ -1357,12 +1392,16 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
             for (size_t i = 0; i < P.size(); i++) if (!fused_root[i] && mine[l + 1][i]) ctx->st.k1_bytes_written += 4.0 * (double)P[i].cells; // root tables that were written
         const bool top = l == Lstar - 1 && fused_any; // children of fused roots were produced by the root kernel
         std::vector<uint32_t> first(P.size() + 1, 0), order;
+        // A set gets a pair iff it holds cube bits 0 and 1 (it is derived in groups of card[0] * card[1] configurations and scores
+        // its subsets without those bits), or its parent's pass built no such groups: a plain root's children root \ {1} (groups
+        // of card[0], scoring root \ {0, 1} too) and root \ {0} (groups of one), and the children T \ {1} of a fused root's
+        // children T (the root kernel scored T \ {0}).  Every other set is scored by the pass of the set plus bits 0 and 1
+        // (bic_kernels.cuh, "GROUPS").
         auto skip = [&](const CubeSet &cs) {
             if (!mine[l + 1][cs.parent]) return true;   // outside this call's sub-forest
-            // a leaf of a derived table was scored by the pass that derived its parent (the derive or the root kernel); only
-            // leaves of root tables, which come from kernels that do not build digit-0 groups, are derived on their own
-            if ((cs.cube_mask & 1u) == 0 && l + 1 < Lstar) return true;
-            return top && fused_root[cs.parent] != 0;
+            if (top && fused_root[cs.parent]) return true;
+            if ((cs.cube_mask & 3u) == 3u || l + 1 == Lstar) return false;
+            return !((cs.cube_mask & 1u) && l + 2 == Lstar && fused_root[P[cs.parent].parent]);
         };
         for (auto &cs : L) if (!skip(cs)) first[cs.parent + 1]++;
         for (size_t i = 0; i < P.size(); i++) first[i + 1] += first[i];
@@ -1376,23 +1415,20 @@ static int bic_score_family_cube(urlgpu_ctx *ctx, int variable, const std::vecto
         for (size_t k = 0; k < order.size(); k++) {
             const CubeSet &cs = L[order[k]];
             CubePair pr{};
-            const bool leaf = (cs.cube_mask & 1u) == 0; // lowest missing bit is 0: nothing is derived from this set
+            const bool h0 = cs.cube_mask & 1u, h01 = (cs.cube_mask & 3u) == 3u;
             pr.parent_off = P[cs.parent].off; pr.child_off = cs.off;
-            pr.r0 = leaf ? 1u : (uint32_t)ccard[0];
-            pr.groups = (uint32_t)(cs.cells / rv / pr.r0);
+            pr.g0 = h0 ? (uint32_t)ccard[0] : 1u;
+            pr.g1 = h01 ? (uint32_t)ccard[1] : 1u;
+            pr.groups = (uint32_t)(cs.cells / rv / (pr.g0 * pr.g1));
             pr.Bc = cs.Bc; pr.r = cs.r; pr.chunk0 = (uint32_t)chunk;
-            pr.acc_index = (uint32_t)(acc_off[l] + order[k]);
-            pr.flags = (leaf ? 0u : kCubeStore) | (l <= Kc ? kCubeScoreChild : 0u);
-            if (!leaf) { // l >= 1 and l - 1 <= Kc: the leaf child exists and is scored from this pair's groups
-                if (cs.leaf_child < 0) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: leaf child missing");
-                pr.leaf_acc = (uint32_t)(acc_off[l - 1] + cs.leaf_child);
-                pr.flags |= kCubeScoreLeaf;
-            }
+            if (!pass_scores(cs, l, order[k], h0, h01, pr.flags, pr.acc)) return ctx->fail(URLGPU_ERR_INTERNAL, "cube: a set scored by a derive pass is missing");
+            const bool store = (cs.cube_mask & 7u) == 7u;
+            if (store) pr.flags |= kCubeStore;
             pr.fmt = (P[cs.parent].t16 ? 1u : 0u) | (cs.t16 ? 2u : 0u);
             pr.magic = pr.Bc > 1 ? 0xFFFFFFFFu / pr.Bc : 0;
             ctx->st.k1_bytes_read += (P[cs.parent].t16 ? 2.0 : 4.0) * (double)cs.cells * (double)cs.r;
-            if (!leaf) ctx->st.k1_bytes_written += (cs.t16 ? 2.0 : 4.0) * (double)cs.cells;
-            const uint32_t gpb = kCubeConfigsPerBlock / pr.r0;
+            if (store) ctx->st.k1_bytes_written += (cs.t16 ? 2.0 : 4.0) * (double)cs.cells;
+            const uint32_t gpb = std::max(1u, kCubeConfigsPerBlock / (pr.g0 * pr.g1));
             chunk += (pr.groups + gpb - 1) / gpb;
             hp[k] = pr;
         }
